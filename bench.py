@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- the headline benchmark of the B200 KNN engine (driver contract: ONE JSON line).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Metric (BASELINE.json): SOR + normals points/sec, k = 10 / 20; ICP ms/iter at 1 M points.
@@ -36,6 +36,10 @@ Secondary blocks on the same line, at EVERY N (strong scaling: the total work is
                 bit for bit against the one-GPU call.
 --impl reference times the CPU port as the reference arm (the Rust reference cannot be built in this image: no
 cargo/rustc; see DESIGN.md); at N ranks rank 0 processes N frames per step, so both arms do the same work.
+--dump-outputs DIR writes what rank 0's last timed step of the headline returned, float32, after the timing:
+  device_points.npy / device_normals.npy (kept points and their normals, (n_kept, 3), device-resident arm) and
+  e2e_points.npy / e2e_normals.npy (the same from the host block of the end-to-end arm).  The frames are seeded, so
+  two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -51,6 +55,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: importing the package and the oracle writes nothing there
 
 K_SOR, STD_MUL, K_NORMALS = 10, 1.0, 20
 VOXEL = 0.05
@@ -196,7 +201,7 @@ def run_reference_arm(args):
     warm = max(0, min(args.warmup, 1))
     for _ in range(warm):
         cpu_reference_run(frames[:1], cores)
-    steps = max(1, min(args.steps, max(1, 8 // world)))  # bounded: a step is ~0.25 s of CPU work per frame
+    steps = args.steps  # (a step is ~0.25 s of CPU work per frame)
     times = [cpu_reference_run(frames, cores) for _ in range(steps)]
     t = float(np.mean(times))
     n_total = sum(len(f) for f in frames)
@@ -230,7 +235,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-icp", action="store_true", help="skip the ICP block")
     ap.add_argument("--no-extras", action="store_true", help="headline only: skip batch8m / icp_sharded / config3 / frames_in_flight")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the kept points and normals of rank 0's last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
 
     if args.impl == "reference":
         return run_reference_arm(args)
@@ -336,6 +347,13 @@ def main():
     barrier()
     clocks = sampler.stop()
     hints1 = ctx.hint_stats()
+
+    if args.dump_outputs and rank == 0:  # before the parity check below reruns frame 0
+        m = last["e2e_len"]
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in (("device_points", last["dev"].to_numpy()), ("device_normals", last["dev"].normals_to_numpy()),
+                        ("e2e_points", h_out[0:3, :m].numpy().T), ("e2e_normals", h_out[3:6, :m].numpy().T)):
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), np.ascontiguousarray(a, np.float32))
 
     dev_ms_max = pdist.max_over_ranks(D, dev_ms, "cuda")
     e2e_s_max = pdist.max_over_ranks(D, e2e_s, "cuda")

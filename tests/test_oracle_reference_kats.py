@@ -11,7 +11,8 @@ import os
 import numpy as np
 import pytest
 
-REF_DATA = "/root/reference/data"
+# The reference's data/ fixtures, restated as far as its tests pin them (tests/golden/reference_data/README.md)
+REF_DATA = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_data")
 
 
 def cloud(x, y=None, z=None):
@@ -155,7 +156,6 @@ def test_normals_viewpoint(oracle):  # :456-492
 
 
 # ---- data fixtures (SURVEY 8c: expected values by inspection) ------------------------------------------
-@pytest.mark.skipif(not os.path.isdir(REF_DATA), reason="reference checkout not present (GPU box)")
 def test_reference_data_fixtures(oracle):
     bunny = oracle.read_pcd_ascii(os.path.join(REF_DATA, "bunny.pcd"))
     assert bunny.tolist() == [[0.0, 0.0, 0.0]]
