@@ -242,6 +242,41 @@ int pcr_icp_point_to_plane_dev(pcr_ctx *ctx, const float *d_sx, const float *d_s
                                size_t nt, const float *d_nx, const float *d_ny, const float *d_nz,
                                size_t n_normals, const pcr_icp_params *params, pcr_icp_result *result);
 
+/* Batched ICP: many (source, target) pairs of frames in one call.  The frames sit back to back in one buffer, frame f =
+ * points [frame_offsets[f], frame_offsets[f+1]) (as in pcr_sor_normals_batch), N = frame_offsets[n_frames].  Pair p
+ * registers frame pairs[2p] (the source) onto frame pairs[2p+1] (the target); results[p] is its result.  Independent
+ * pairs and a sequence (pairs (i+1, i): frame-to-frame odometry, every frame uploaded and indexed once) are both
+ * this form, and a frame may appear in any number of pairs, on either side.
+ * Every pair is what the single-pair call on the same two clouds returns: the same parameter checks, the same empty-cloud
+ * rules (icp.rs:131-139), max_iterations == 0 computes the metrics only.  A pair's result does not depend on the other
+ * pairs of the call, and repeated calls return the same bits; against the single-pair call it agrees within f64
+ * rounding of the sums (the single-pair call orders the points inside a grid cell by atomics, the batch by index).
+ * Point-to-plane: one normal per point of the buffer (only target frames' entries are read); n_normals != N ->
+ * PCR_ERR_NORMALS_MISMATCH.  frame_offsets not starting at 0 or decreasing, a frame id >= n_frames, or a null pointer
+ * -> PCR_ERR_INVALID_ARG.  Source frames summed over the pairs reaching 2^31 points, or more than 65535 frames ->
+ * PCR_ERR_UNSUPPORTED.
+ * The batch never communicates: on a context with a communicator every rank registers the pairs it was given (frames
+ * dealt to ranks), with its whole source frames. */
+int pcr_icp_point_to_point_batch(pcr_ctx *ctx, const float *x, const float *y, const float *z,
+                                 const uint64_t *frame_offsets, size_t n_frames,
+                                 const uint32_t *pairs, size_t n_pairs,
+                                 const pcr_icp_params *params, pcr_icp_result *results /* n_pairs */);
+int pcr_icp_point_to_plane_batch(pcr_ctx *ctx, const float *x, const float *y, const float *z,
+                                 const uint64_t *frame_offsets, size_t n_frames,
+                                 const float *nx, const float *ny, const float *nz, size_t n_normals,
+                                 const uint32_t *pairs, size_t n_pairs,
+                                 const pcr_icp_params *params, pcr_icp_result *results);
+/* _dev: x .. nz are device pointers; frame_offsets, pairs, params and results stay on the host.  Synchronous. */
+int pcr_icp_point_to_point_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z,
+                                     const uint64_t *frame_offsets, size_t n_frames,
+                                     const uint32_t *pairs, size_t n_pairs,
+                                     const pcr_icp_params *params, pcr_icp_result *results);
+int pcr_icp_point_to_plane_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z,
+                                     const uint64_t *frame_offsets, size_t n_frames,
+                                     const float *d_nx, const float *d_ny, const float *d_nz, size_t n_normals,
+                                     const uint32_t *pairs, size_t n_pairs,
+                                     const pcr_icp_params *params, pcr_icp_result *results);
+
 /* ---- voxel grid filter (SURVEY 8f-2) ---------------------------------------------------------------
  * voxel_downsample (crates/filters/src/voxel_downsample.rs:12-65): one point per occupied voxel
  * (key = floor(p / voxel_size) as i32), the mean of the voxel's points summed in input order, voxels

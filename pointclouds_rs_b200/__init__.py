@@ -38,6 +38,7 @@ __all__ = [
     "PointCloud", "KdTree", "IcpResult", "Context",
     "statistical_outlier_removal", "radius_outlier_removal", "estimate_normals",
     "icp_point_to_point", "icp_point_to_plane", "apply_transform", "find_correspondences",
+    "icp_point_to_point_batch", "icp_point_to_plane_batch",
     "sor_normals_batch", "default_context", "PcrError", "euclidean_cluster", "voxel_downsample", "DeviceCloud", "ransac_plane", "PlaneResult",
 ]
 
@@ -584,6 +585,68 @@ def apply_transform(cloud: PointCloud, rotation, translation, ctx: Optional[Cont
                                          _p(r, _ffi.f32p), _p(t, _ffi.f32p), _p(ox, _ffi.f32p), _p(oy, _ffi.f32p), _p(oz, _ffi.f32p))
     _ffi.check(st, ctx._h)
     return PointCloud._from_xyz(ox, oy, oz)
+
+
+def _icp_batch_arrays(points, frame_offsets, pairs):
+    """Checks and converts the frame buffer of a batched ICP: (N,3) f32 rows, u64 offsets, (P,2) u32 pairs."""
+    pts = np.asarray(points)
+    if pts.ndim != 2 or pts.shape[1] != 3:
+        raise ValueError("points must have shape (N, 3)")
+    n = len(pts)
+    off = np.asarray(frame_offsets).reshape(-1)
+    if len(off) == 0 or off.dtype.kind not in "iu":
+        raise ValueError("frame_offsets must be n_frames + 1 integers")
+    if off[0] != 0 or off[-1] != n or np.any(np.diff(off) < 0):
+        raise ValueError(f"frame_offsets must be non-decreasing from 0 to the number of points ({n})")
+    nf = len(off) - 1
+    pr = np.asarray(pairs)
+    if pr.size == 0:
+        pr = pr.reshape(0, 2)
+    if pr.ndim != 2 or pr.shape[1] != 2 or (len(pr) and pr.dtype.kind not in "iu"):
+        raise ValueError("pairs must be an integer array of shape (P, 2): (source frame, target frame)")
+    if len(pr) and (pr.min() < 0 or pr.max() >= nf):
+        raise ValueError(f"pairs hold a frame id outside [0, {nf})")
+    return (np.ascontiguousarray(pts, np.float32), np.ascontiguousarray(off, np.uint64), np.ascontiguousarray(pr, np.uint32))
+
+
+def icp_point_to_point_batch(points: np.ndarray, frame_offsets: Sequence[int], pairs, max_iterations: int = 50,
+                             tolerance: float = 1e-5, max_correspondence_distance: float = math.inf,
+                             ctx: Optional[Context] = None) -> List[IcpResult]:
+    """Point-to-point ICP of many frame pairs in one call.  points: (N,3), every frame back to back, frame f = rows
+    [frame_offsets[f], frame_offsets[f+1]); pairs: (P,2), pair p registers frame pairs[p][0] (source) onto frame
+    pairs[p][1] (target).  -> one IcpResult per pair, each what icp_point_to_point returns for those two clouds."""
+    p = _icp_params(max_iterations, tolerance, max_correspondence_distance)
+    pts, off, pr = _icp_batch_arrays(points, frame_offsets, pairs)
+    ctx = ctx or default_context()
+    x, y, z = _soa(pts)
+    res = (_ffi.IcpResultC * max(len(pr), 1))()
+    st = _ffi.load().pcr_icp_point_to_point_batch(ctx._h, _p(x, _ffi.f32p), _p(y, _ffi.f32p), _p(z, _ffi.f32p), _p(off, _ffi.u64p),
+                                                  len(off) - 1, _p(pr, _ffi.u32p), len(pr), C.byref(p), res)
+    _ffi.check(st, ctx._h)
+    return [IcpResult(res[i]) for i in range(len(pr))]
+
+
+def icp_point_to_plane_batch(points: np.ndarray, frame_offsets: Sequence[int], pairs, normals: Optional[np.ndarray],
+                             max_iterations: int = 50, tolerance: float = 1e-5, max_correspondence_distance: float = math.inf,
+                             ctx: Optional[Context] = None) -> List[IcpResult]:
+    """Point-to-plane form of icp_point_to_point_batch.  normals: (N,3), one per row of `points` (only the rows of
+    target frames are read)."""
+    if normals is None:  # crates/python/src/registration.rs:66-71
+        raise ValueError("point-to-plane ICP needs the targets' normals. Use estimate_normals first.")
+    p = _icp_params(max_iterations, tolerance, max_correspondence_distance)
+    pts, off, pr = _icp_batch_arrays(points, frame_offsets, pairs)
+    nrm = np.asarray(normals)
+    if nrm.ndim != 2 or nrm.shape[1] != 3 or len(nrm) != len(pts):
+        raise ValueError(f"normals must have shape ({len(pts)}, 3), one per point; got {nrm.shape}")
+    ctx = ctx or default_context()
+    x, y, z = _soa(pts)
+    nx, ny, nz = _soa(np.ascontiguousarray(nrm, np.float32))
+    res = (_ffi.IcpResultC * max(len(pr), 1))()
+    st = _ffi.load().pcr_icp_point_to_plane_batch(ctx._h, _p(x, _ffi.f32p), _p(y, _ffi.f32p), _p(z, _ffi.f32p), _p(off, _ffi.u64p),
+                                                  len(off) - 1, _p(nx, _ffi.f32p), _p(ny, _ffi.f32p), _p(nz, _ffi.f32p), len(nx),
+                                                  _p(pr, _ffi.u32p), len(pr), C.byref(p), res)
+    _ffi.check(st, ctx._h)
+    return [IcpResult(res[i]) for i in range(len(pr))]
 
 
 

@@ -99,6 +99,12 @@ SIGNATURES = {
     "pcr_icp_point_to_plane": (C.c_int, [vp, f32p, f32p, f32p, C.c_size_t, f32p, f32p, f32p, C.c_size_t, f32p, f32p, f32p, C.c_size_t, C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
     "pcr_icp_point_to_point_dev": (C.c_int, [vp, vp, vp, vp, C.c_size_t, vp, vp, vp, C.c_size_t, C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
     "pcr_icp_point_to_plane_dev": (C.c_int, [vp, vp, vp, vp, C.c_size_t, vp, vp, vp, C.c_size_t, vp, vp, vp, C.c_size_t, C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
+    "pcr_icp_point_to_point_batch": (C.c_int, [vp, f32p, f32p, f32p, u64p, C.c_size_t, u32p, C.c_size_t, C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
+    "pcr_icp_point_to_plane_batch": (C.c_int, [vp, f32p, f32p, f32p, u64p, C.c_size_t, f32p, f32p, f32p, C.c_size_t, u32p, C.c_size_t,
+                                               C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
+    "pcr_icp_point_to_point_batch_dev": (C.c_int, [vp, vp, vp, vp, u64p, C.c_size_t, u32p, C.c_size_t, C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
+    "pcr_icp_point_to_plane_batch_dev": (C.c_int, [vp, vp, vp, vp, u64p, C.c_size_t, vp, vp, vp, C.c_size_t, u32p, C.c_size_t,
+                                                   C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
     "pcr_voxel_downsample": (C.c_int, [vp, f32p, f32p, f32p, C.c_size_t, C.c_float, f32p, f32p, f32p, szp]),
     "pcr_voxel_downsample_dev": (C.c_int, [vp, vp, vp, vp, C.c_size_t, C.c_float, vp, vp, vp, szp]),
     "pcr_euclidean_cluster": (C.c_int, [vp, f32p, f32p, f32p, C.c_size_t, C.c_float, C.c_size_t, C.c_size_t, u32p, u32p, szp]),

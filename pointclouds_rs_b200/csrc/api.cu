@@ -1025,6 +1025,73 @@ int pcr_icp_point_to_plane_dev(pcr_ctx *ctx, const float *sx, const float *sy, c
     return icp_entry(ctx, true, true, sx, sy, sz, ns, tx, ty, tz, nt, nx, ny, nz, n_normals, params, result);
 }
 
+// Pairs of frames of one buffer: every pair is checked and answered as the single-pair call would (icp_entry).
+static int icp_batch_entry(pcr_ctx *ctx, bool dev, bool plane, const float *x, const float *y, const float *z, const uint64_t *frame_offsets,
+                           size_t n_frames, const float *nx, const float *ny, const float *nz, size_t n_normals, const uint32_t *pairs,
+                           size_t n_pairs, const pcr_icp_params *params, pcr_icp_result *results) {
+    if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
+    Ctx *c = &ctx->c;
+    PCR_TRY(icp_check(c, params, results));
+    for (size_t p = 0; p < n_pairs; p++) icp_identity(&results[p]);
+    if (!frame_offsets || (n_pairs && !pairs)) return fail(c, PCR_ERR_INVALID_ARG, "frame_offsets/pairs is NULL");
+    if (frame_offsets[0] != 0) return fail(c, PCR_ERR_INVALID_ARG, "frame_offsets must start at 0");
+    for (size_t f = 0; f < n_frames; f++)
+        if (frame_offsets[f + 1] < frame_offsets[f]) return fail(c, PCR_ERR_INVALID_ARG, "frame_offsets must be non-decreasing");
+    const size_t n = (size_t)frame_offsets[n_frames];
+    if (plane && n_normals != n)  // icp_plane.rs:27-32, for the whole buffer
+        return fail(c, PCR_ERR_NORMALS_MISMATCH, "normals length (%zu) does not match the number of points (%zu)", n_normals, n);
+    uint64_t src_points = 0;
+    for (size_t p = 0; p < n_pairs; p++) {
+        const uint32_t s = pairs[2 * p], t = pairs[2 * p + 1];
+        if (s >= n_frames || t >= n_frames) return fail(c, PCR_ERR_INVALID_ARG, "pair %zu: frame id out of range (%zu frames)", p, n_frames);
+        src_points += frame_offsets[s + 1] - frame_offsets[s];
+    }
+    if (src_points >= (1ull << 31)) return fail(c, PCR_ERR_UNSUPPORTED, "the source frames of one batch must hold fewer than 2^31 points");
+    if (n > 0x7fffffffull) return fail(c, PCR_ERR_UNSUPPORTED, "clouds above 2^31 points are not supported");
+    if (n_frames > 65535) return fail(c, PCR_ERR_UNSUPPORTED, "at most 65535 frames per batch");
+    if (n && (!x || !y || !z || (plane && (!nx || !ny || !nz)))) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    IcpBatchArgs a;
+    a.d_x = x; a.d_y = y; a.d_z = z; a.n = n;
+    a.frame_offsets = frame_offsets; a.n_frames = n_frames;
+    a.d_nx = a.d_ny = a.d_nz = nullptr;
+    a.pairs = pairs; a.n_pairs = n_pairs;
+    a.params = *params;
+    if (dev) {
+        if (plane) { a.d_nx = nx; a.d_ny = ny; a.d_nz = nz; }
+        return icp_batch_dev(c, a, results);
+    }
+    float *dx, *dy, *dz, *dnx = nullptr, *dny = nullptr, *dnz = nullptr;
+    PCR_TRY(stage_xyz(c, c->b_in, x, y, z, n, &dx, &dy, &dz));
+    if (plane) PCR_TRY(stage_xyz(c, c->b_out, nx, ny, nz, n, &dnx, &dny, &dnz));
+    a.d_x = dx; a.d_y = dy; a.d_z = dz;
+    a.d_nx = dnx; a.d_ny = dny; a.d_nz = dnz;
+    return icp_batch_dev(c, a, results);
+    PCR_API_END(c)
+}
+
+int pcr_icp_point_to_point_batch(pcr_ctx *ctx, const float *x, const float *y, const float *z, const uint64_t *frame_offsets, size_t n_frames,
+                                 const uint32_t *pairs, size_t n_pairs, const pcr_icp_params *params, pcr_icp_result *results) {
+    return icp_batch_entry(ctx, false, false, x, y, z, frame_offsets, n_frames, nullptr, nullptr, nullptr, 0, pairs, n_pairs, params, results);
+}
+int pcr_icp_point_to_plane_batch(pcr_ctx *ctx, const float *x, const float *y, const float *z, const uint64_t *frame_offsets, size_t n_frames,
+                                 const float *nx, const float *ny, const float *nz, size_t n_normals, const uint32_t *pairs, size_t n_pairs,
+                                 const pcr_icp_params *params, pcr_icp_result *results) {
+    return icp_batch_entry(ctx, false, true, x, y, z, frame_offsets, n_frames, nx, ny, nz, n_normals, pairs, n_pairs, params, results);
+}
+int pcr_icp_point_to_point_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z, const uint64_t *frame_offsets,
+                                     size_t n_frames, const uint32_t *pairs, size_t n_pairs, const pcr_icp_params *params,
+                                     pcr_icp_result *results) {
+    return icp_batch_entry(ctx, true, false, d_x, d_y, d_z, frame_offsets, n_frames, nullptr, nullptr, nullptr, 0, pairs, n_pairs, params, results);
+}
+int pcr_icp_point_to_plane_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z, const uint64_t *frame_offsets,
+                                     size_t n_frames, const float *d_nx, const float *d_ny, const float *d_nz, size_t n_normals,
+                                     const uint32_t *pairs, size_t n_pairs, const pcr_icp_params *params, pcr_icp_result *results) {
+    return icp_batch_entry(ctx, true, true, d_x, d_y, d_z, frame_offsets, n_frames, d_nx, d_ny, d_nz, n_normals, pairs, n_pairs, params,
+                           results);
+}
+
 /* ---- multi-frame batch ---------------------------------------------------------------------------- */
 namespace pcr {
 // frames of exactly one point are returned unchanged by the reference (statistical_outlier.rs:10-12)

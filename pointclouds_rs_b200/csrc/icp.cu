@@ -109,17 +109,12 @@ __global__ void __launch_bounds__(256) src_scatter_kernel(const float *__restric
 // (A) transform + 1-NN on grid level 0, one thread per source point.  A point whose 27 cells are
 //     empty (a source that pokes out of the target, e.g. two scans that only partly overlap) is
 //     deferred to the coarser levels instead of walking shells of empty fine cells.
-__global__ void __launch_bounds__(kIcpThreads) icp_search_kernel(const GridDesc *__restrict__ grids,
-                                                                 const uint32_t *__restrict__ cell_start,
-                                                                 const float4 *__restrict__ sorted, const float4 *__restrict__ tgt4,
-                                                                 float4 *__restrict__ cur, size_t ns,
-                                                                 const IcpState *__restrict__ state, unsigned long long *__restrict__ nn,
-                                                                 uint32_t *__restrict__ defer_list,
-                                                                 uint32_t *__restrict__ defer_count, int last_level) {
-    if (state->done) return;
-    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= ns) return;
-    const GridDesc g = grids[0];
+//     (The body is shared with the batch kernel: one working-copy point i searched in target grid g.)
+__device__ __forceinline__ void icp_search_point(const GridDesc &g, const uint32_t *__restrict__ cell_start,
+                                                 const float4 *__restrict__ sorted, const float4 *__restrict__ tgt4,
+                                                 float4 *__restrict__ cur, size_t i, const IcpState *__restrict__ state,
+                                                 unsigned long long *__restrict__ nn, uint32_t *__restrict__ defer_list,
+                                                 uint32_t *__restrict__ defer_count, int last_level) {
     float4 p = cur[i];
     if (state->has_inc) {  // icp.rs:186 / icp_plane.rs:78: current = apply_transform(current, incremental)
         float a, b, c;
@@ -160,9 +155,37 @@ __global__ void __launch_bounds__(kIcpThreads) icp_search_kernel(const GridDesc 
     nn[i] = best;
 }
 
+__global__ void __launch_bounds__(kIcpThreads) icp_search_kernel(const GridDesc *__restrict__ grids,
+                                                                 const uint32_t *__restrict__ cell_start,
+                                                                 const float4 *__restrict__ sorted, const float4 *__restrict__ tgt4,
+                                                                 float4 *__restrict__ cur, size_t ns,
+                                                                 const IcpState *__restrict__ state, unsigned long long *__restrict__ nn,
+                                                                 uint32_t *__restrict__ defer_list,
+                                                                 uint32_t *__restrict__ defer_count, int last_level) {
+    if (state->done) return;
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= ns) return;
+    const GridDesc g = grids[0];
+    icp_search_point(g, cell_start, sorted, tgt4, cur, i, state, nn, defer_list, defer_count, last_level);
+}
+
 // (A') deferred source points on a coarser level, persistent over the device-side list: one warp per point
 //      (a coarse cell holds ~70 points, so the lanes are busy).  nn[i] carries the warm-start candidate the
 //      search kernel left there (or EMPTY); the warp search inserts it first and prunes with it.
+__device__ __forceinline__ void icp_deferred_point(RegTopK &tk, const GridDesc &g, const uint32_t *__restrict__ cell_start,
+                                                   const float4 *__restrict__ pts, const float4 *__restrict__ cur, uint32_t i,
+                                                   unsigned long long *__restrict__ nn, uint32_t *__restrict__ out_list,
+                                                   uint32_t *__restrict__ out_count, int last_level) {
+    const float4 p = cur[i];
+    const unsigned long long seed = nn[i];
+    if (warp_knn_search(tk, g, cell_start, pts, p.x, p.y, p.z, last_level ? kMaxRings : kLevelRings, last_level != 0, seed)) {
+        unsigned long long best = __shfl_sync(PCR_FULL, tk.K, 0);
+        if (tk.lane == 0) nn[i] = best;
+    } else if (tk.lane == 0) {
+        out_list[atomicAdd(out_count, 1u)] = i;
+    }
+}
+
 __global__ void __launch_bounds__(128) icp_deferred_kernel(const GridDesc *__restrict__ grids, const uint32_t *__restrict__ cell_start,
                                                            const float4 *__restrict__ pts, const float4 *__restrict__ cur,
                                                            const IcpState *__restrict__ state, const uint32_t *__restrict__ in_list,
@@ -177,63 +200,50 @@ __global__ void __launch_bounds__(128) icp_deferred_kernel(const GridDesc *__res
     RegTopK tk;
     tk.kk = 1;
     tk.lane = lane;
-    for (uint32_t j = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); j < n; j += warps) {
-        const uint32_t i = in_list[j];
-        const float4 p = cur[i];
-        const unsigned long long seed = nn[i];
-        if (warp_knn_search(tk, g, cell_start, pts, p.x, p.y, p.z, last_level ? kMaxRings : kLevelRings, last_level != 0, seed)) {
-            unsigned long long best = __shfl_sync(PCR_FULL, tk.K, 0);
-            if (lane == 0) nn[i] = best;
-        } else if (lane == 0) {
-            out_list[atomicAdd(out_count, 1u)] = i;
+    for (uint32_t j = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); j < n; j += warps)
+        icp_deferred_point(tk, g, cell_start, pts, cur, in_list[j], nn, out_list, out_count, last_level);
+}
+
+// (B) residuals and normal equations from the correspondences, per-block partials in a fixed order.
+//     icp_accum_point adds source point i's terms to acc; icp_block_partials folds acc over the block.
+template <bool kPlane>
+__device__ __forceinline__ void icp_accum_point(double (&acc)[NP], const float4 *__restrict__ tgt4, const float4 *__restrict__ nrm4,
+                                                const float4 *__restrict__ cur, const unsigned long long *__restrict__ nn, size_t i,
+                                                float max_distance) {
+    const unsigned long long best = nn[i];
+    if (best == PCR_EMPTY_KEY) return;
+    const float d = __fsqrt_rn(key_d2(best));
+    if (!(d <= max_distance)) return;  // correspondence.rs:28
+    const float4 p = cur[i];
+    const float4 t = __ldg(&tgt4[key_idx(best)]);
+    acc[kSumSq] += (double)__fmul_rn(d, d);  // icp.rs:279
+    acc[kCount] += 1.0;
+    if (kPlane) {  // icp_plane.rs:152-179
+        const float4 nn4 = __ldg(&nrm4[key_idx(best)]);
+        const double sx = p.x, sy = p.y, sz = p.z, n0 = nn4.x, n1 = nn4.y, n2 = nn4.z;
+        double a[6] = {sy * n2 - sz * n1, sz * n0 - sx * n2, sx * n1 - sy * n0, n0, n1, n2};
+        const double b = ((double)t.x - sx) * n0 + ((double)t.y - sy) * n1 + ((double)t.z - sz) * n2;
+        int o = 0;
+#pragma unroll
+        for (int r = 0; r < 6; r++)
+#pragma unroll
+            for (int c = r; c < 6; c++) acc[o++] += a[r] * a[c];
+#pragma unroll
+        for (int r = 0; r < 6; r++) acc[21 + r] += a[r] * b;
+    } else {  // icp.rs:221-244 (sums; centring is done in the solve)
+        const double s[3] = {p.x, p.y, p.z}, tt[3] = {t.x, t.y, t.z};
+#pragma unroll
+        for (int r = 0; r < 3; r++) {
+            acc[r] += s[r];
+            acc[3 + r] += tt[r];
+#pragma unroll
+            for (int c = 0; c < 3; c++) acc[6 + r * 3 + c] += s[r] * tt[c];
         }
     }
 }
 
-// (B) residuals and normal equations from the correspondences, per-block partials in a fixed order
-template <bool kPlane>
-__global__ void __launch_bounds__(kIcpThreads) icp_accum_kernel(const float4 *__restrict__ tgt4, const float4 *__restrict__ nrm4,
-                                                                const float4 *__restrict__ cur,
-                                                                const unsigned long long *__restrict__ nn, size_t ns,
-                                                                float max_distance, const IcpState *__restrict__ state,
-                                                                double *__restrict__ partials) {
-    if (state->done) return;
-    double acc[NP];
-#pragma unroll
-    for (int j = 0; j < NP; j++) acc[j] = 0.0;
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < ns; i += (size_t)gridDim.x * blockDim.x) {
-        const unsigned long long best = nn[i];
-        if (best == PCR_EMPTY_KEY) continue;
-        const float d = __fsqrt_rn(key_d2(best));
-        if (!(d <= max_distance)) continue;  // correspondence.rs:28
-        const float4 p = cur[i];
-        const float4 t = __ldg(&tgt4[key_idx(best)]);
-        acc[kSumSq] += (double)__fmul_rn(d, d);  // icp.rs:279
-        acc[kCount] += 1.0;
-        if (kPlane) {  // icp_plane.rs:152-179
-            const float4 nn4 = __ldg(&nrm4[key_idx(best)]);
-            const double sx = p.x, sy = p.y, sz = p.z, n0 = nn4.x, n1 = nn4.y, n2 = nn4.z;
-            double a[6] = {sy * n2 - sz * n1, sz * n0 - sx * n2, sx * n1 - sy * n0, n0, n1, n2};
-            const double b = ((double)t.x - sx) * n0 + ((double)t.y - sy) * n1 + ((double)t.z - sz) * n2;
-            int o = 0;
-#pragma unroll
-            for (int r = 0; r < 6; r++)
-#pragma unroll
-                for (int c = r; c < 6; c++) acc[o++] += a[r] * a[c];
-#pragma unroll
-            for (int r = 0; r < 6; r++) acc[21 + r] += a[r] * b;
-        } else {  // icp.rs:221-244 (sums; centring is done in the solve)
-            const double s[3] = {p.x, p.y, p.z}, tt[3] = {t.x, t.y, t.z};
-#pragma unroll
-            for (int r = 0; r < 3; r++) {
-                acc[r] += s[r];
-                acc[3 + r] += tt[r];
-#pragma unroll
-                for (int c = 0; c < 3; c++) acc[6 + r * 3 + c] += s[r] * tt[c];
-            }
-        }
-    }
-    // block reduction in a fixed order: shuffle tree inside the warp, then warps in order
+// block reduction in a fixed order: shuffle tree inside the warp, then warps in order (every thread of the block calls it)
+__device__ __forceinline__ void icp_block_partials(const double (&acc)[NP], double *__restrict__ out /* NP */) {
     __shared__ double sh[kIcpThreads / 32][NP];
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
 #pragma unroll
@@ -248,8 +258,23 @@ __global__ void __launch_bounds__(kIcpThreads) icp_accum_kernel(const float4 *__
         double v = 0.0;
 #pragma unroll
         for (int ww = 0; ww < kIcpThreads / 32; ww++) v += sh[ww][threadIdx.x];
-        partials[(size_t)blockIdx.x * NP + threadIdx.x] = v;
+        out[threadIdx.x] = v;
     }
+}
+
+template <bool kPlane>
+__global__ void __launch_bounds__(kIcpThreads) icp_accum_kernel(const float4 *__restrict__ tgt4, const float4 *__restrict__ nrm4,
+                                                                const float4 *__restrict__ cur,
+                                                                const unsigned long long *__restrict__ nn, size_t ns,
+                                                                float max_distance, const IcpState *__restrict__ state,
+                                                                double *__restrict__ partials) {
+    if (state->done) return;
+    double acc[NP];
+#pragma unroll
+    for (int j = 0; j < NP; j++) acc[j] = 0.0;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < ns; i += (size_t)gridDim.x * blockDim.x)
+        icp_accum_point<kPlane>(acc, tgt4, nrm4, cur, nn, i, max_distance);
+    icp_block_partials(acc, partials + (size_t)blockIdx.x * NP);
 }
 
 // Folds the per-block partials in a fixed order: 32 lanes per value take strided subsets, then a
@@ -276,14 +301,20 @@ __device__ __forceinline__ unsigned long long ld_acquire_sys_u64(const unsigned 
     return v;
 }
 
-__global__ void __launch_bounds__(NP * 32) icp_reduce_kernel(const double *__restrict__ partials, int n_blocks, size_t ns_local,
-                                                             IcpState *state, PeerComm pc, unsigned long long seq) {
-    if (state->done) return;
-    const int j = threadIdx.x >> 5, lane = threadIdx.x & 31;
+// sum j of n_blocks partials, in the fixed order above (one warp per value; every lane returns the sum)
+__device__ __forceinline__ double icp_fold_partials(const double *__restrict__ partials, int n_blocks, int j, int lane) {
     double v = 0.0;
     for (int b = lane; b < n_blocks; b += 32) v += partials[(size_t)b * NP + j];
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(PCR_FULL, v, o);
+    return v;
+}
+
+__global__ void __launch_bounds__(NP * 32) icp_reduce_kernel(const double *__restrict__ partials, int n_blocks, size_t ns_local,
+                                                             IcpState *state, PeerComm pc, unsigned long long seq) {
+    if (state->done) return;
+    const int j = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    double v = icp_fold_partials(partials, n_blocks, j, lane);
     v = j == kSrcN ? (double)ns_local : v;  // (every lane holds the sum)
     if (pc.world <= 1) {
         if (lane == 0) state->sums[j] = v;
@@ -585,12 +616,11 @@ __device__ void solve_p2plane(const double *sums, float *R, float *t) {
     t[2] = (float)xs[5];
 }
 
-// One thread: convergence test, solve, compose (icp.rs:154-187 / icp_plane.rs:55-79).
+// Convergence test, solve, compose (icp.rs:154-187 / icp_plane.rs:55-79) of one registration, on one thread.
+// Returns true when this step finished it (state->done was just set).
 template <bool kPlane>
-__global__ void icp_solve_kernel(IcpState *state, int metrics_only, float tolerance, int *host_done_) {
-    volatile int *host_done = host_done_;
-    if (threadIdx.x != 0 || blockIdx.x != 0) return;
-    if (state->done) return;
+__device__ __forceinline__ bool icp_step(IcpState *state, int metrics_only, float tolerance) {
+    if (state->done) return false;
     const double m = state->sums[kCount];
     const double ns = state->sums[kSrcN];
     if (metrics_only) {  // max_iterations == 0: icp.rs:190-197
@@ -599,14 +629,12 @@ __global__ void icp_solve_kernel(IcpState *state, int metrics_only, float tolera
             state->last_fitness = __fdiv_rn((float)m, (float)ns);
         }
         state->done = 1;
-        *host_done = 1;
-        return;
+        return true;
     }
     state->num_iterations += 1;
     if (!(m > 0.0)) {  // no correspondences: break
         state->done = 1;
-        *host_done = 1;
-        return;
+        return true;
     }
     const float rmse = __fsqrt_rn(__fdiv_rn((float)state->sums[kSumSq], (float)m));
     state->last_rmse = rmse;
@@ -614,8 +642,7 @@ __global__ void icp_solve_kernel(IcpState *state, int metrics_only, float tolera
     if (fabsf(__fsub_rn(state->prev_rmse, rmse)) < tolerance) {
         state->converged = 1;
         state->done = 1;
-        *host_done = 1;
-        return;
+        return true;
     }
     state->prev_rmse = rmse;
     float R[9], t[3];
@@ -640,10 +667,17 @@ __global__ void icp_solve_kernel(IcpState *state, int metrics_only, float tolera
         state->inc_t[i] = t[i];
     }
     state->has_inc = 1;
+    return false;
 }
 
-__global__ void icp_init_state_kernel(IcpState *s) {
-    if (threadIdx.x != 0) return;
+template <bool kPlane>
+__global__ void icp_solve_kernel(IcpState *state, int metrics_only, float tolerance, int *host_done_) {
+    volatile int *host_done = host_done_;
+    if (threadIdx.x != 0 || blockIdx.x != 0) return;
+    if (icp_step<kPlane>(state, metrics_only, tolerance)) *host_done = 1;
+}
+
+__device__ __forceinline__ void icp_init_state(IcpState *s) {
     for (int i = 0; i < 9; i++) {
         s->inc_R[i] = s->cum_R[i] = (i % 4 == 0) ? 1.f : 0.f;
     }
@@ -658,10 +692,148 @@ __global__ void icp_init_state_kernel(IcpState *s) {
     for (int i = 0; i < NP; i++) s->sums[i] = 0.0;
 }
 
+__global__ void icp_init_state_kernel(IcpState *s) {
+    if (threadIdx.x != 0) return;
+    icp_init_state(s);
+}
+
 __global__ void pack_normals_kernel(const float *__restrict__ nx, const float *__restrict__ ny, const float *__restrict__ nz,
                                     size_t n, float4 *__restrict__ out) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) out[i] = make_float4(nx[i], ny[i], nz[i], 0.f);
+}
+
+// ---- batch of (source, target) frame pairs ----------------------------------------------------------------
+// All pairs of one call run through the same launches.  Pair q (of the pairs with a non-empty source and target) owns
+//   - the working-copy range [cur_off[q], cur_off[q+1]): its source frame, binned by the cells of its target frame;
+//   - the accumulation blocks [blk_off[q], blk_off[q+1]): min(ceil(ns / 256), 4 SMs) of them, as in icp_dev, so its
+//     partition (and with it every bit of its result) does not depend on the other pairs of the call;
+//   - states[q], and grid tgt_frame[q] in every level of the multi-frame target index.
+// Threads resolve their pair by a binary search over cur_off (blocks: over blk_off).
+struct IcpBatchPairs {
+    const uint32_t *cur_off;    // [n_pairs + 1]
+    const uint32_t *blk_off;    // [n_pairs + 1]
+    const uint32_t *tgt_frame;  // [n_pairs]
+    const uint32_t *src_begin;  // [n_pairs]: first input point of the source frame
+    int n_pairs;
+};
+
+// Binning, deterministic: key (pair, target cell) for every working-copy point, in working-copy order, then the stable
+// radix sort; a cell's points end up in source order.  Non-finite points go to cell 0, as in src_count_kernel.
+__global__ void __launch_bounds__(256) icp_batch_bin_key_kernel(const float *__restrict__ x, const float *__restrict__ y,
+                                                                const float *__restrict__ z, IcpBatchPairs bp, uint32_t total,
+                                                                const GridDesc *__restrict__ grids, int cell_bits,
+                                                                unsigned long long *__restrict__ keys, uint32_t *__restrict__ vals) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= total) return;
+    const int q = frame_of(bp.cur_off, bp.n_pairs, i);
+    const uint32_t gi = bp.src_begin[q] + (i - bp.cur_off[q]);
+    const GridDesc g = grids[bp.tgt_frame[q]];
+    const float px = x[gi], py = y[gi], pz = z[gi];
+    uint32_t cid = 0;
+    if (finite3(px, py, pz) && g.n_cells > 0) {
+        const int c0 = cell_coord(g, 0, pick_axis(g.ax[0], px, py, pz), nullptr);
+        const int c1 = cell_coord(g, 1, pick_axis(g.ax[1], px, py, pz), nullptr);
+        const int c2 = cell_coord(g, 2, pick_axis(g.ax[2], px, py, pz), nullptr);
+        cid = cell_linear(g, c0, c1, c2) - g.cell_base;
+    }
+    keys[i] = ((unsigned long long)q << cell_bits) | cid;
+    vals[i] = gi;
+}
+
+__global__ void __launch_bounds__(256) icp_batch_bin_gather_kernel(const float *__restrict__ x, const float *__restrict__ y,
+                                                                   const float *__restrict__ z, IcpBatchPairs bp, uint32_t total,
+                                                                   int cell_bits, const unsigned long long *__restrict__ keys,
+                                                                   const uint32_t *__restrict__ vals, float4 *__restrict__ cur) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= total) return;
+    const uint32_t q = (uint32_t)(keys[i] >> cell_bits), gi = vals[i];
+    cur[i] = make_float4(x[gi], y[gi], z[gi], __uint_as_float(gi - bp.src_begin[q]));
+}
+
+__global__ void icp_batch_init_kernel(IcpState *states, int n_pairs, unsigned *active) {
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q < n_pairs) icp_init_state(states + q);
+    if (q == 0) *active = (unsigned)n_pairs;
+}
+
+__global__ void __launch_bounds__(kIcpThreads) icp_batch_search_kernel(const GridDesc *__restrict__ grids,
+                                                                       const uint32_t *__restrict__ cell_start,
+                                                                       const float4 *__restrict__ sorted,
+                                                                       const float4 *__restrict__ tgt4, float4 *__restrict__ cur,
+                                                                       uint32_t total, IcpBatchPairs bp,
+                                                                       const IcpState *__restrict__ states,
+                                                                       unsigned long long *__restrict__ nn,
+                                                                       uint32_t *__restrict__ defer_list,
+                                                                       uint32_t *__restrict__ defer_count, int last_level) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= total) return;
+    const int q = frame_of(bp.cur_off, bp.n_pairs, i);
+    const IcpState *state = states + q;
+    if (state->done) return;  // a finished pair
+    const GridDesc g = grids[bp.tgt_frame[q]];
+    icp_search_point(g, cell_start, sorted, tgt4, cur, i, state, nn, defer_list, defer_count, last_level);
+}
+
+// the deferred lists hold points of unfinished pairs only (the search kernel skips the finished ones)
+__global__ void __launch_bounds__(128) icp_batch_deferred_kernel(const GridDesc *__restrict__ grids,
+                                                                 const uint32_t *__restrict__ cell_start,
+                                                                 const float4 *__restrict__ pts, const float4 *__restrict__ cur,
+                                                                 IcpBatchPairs bp, const uint32_t *__restrict__ in_list,
+                                                                 const uint32_t *__restrict__ in_count,
+                                                                 unsigned long long *__restrict__ nn, uint32_t *__restrict__ out_list,
+                                                                 uint32_t *__restrict__ out_count, int last_level) {
+    const uint32_t n = *in_count;
+    const uint32_t warps = gridDim.x * (blockDim.x >> 5);
+    RegTopK tk;
+    tk.kk = 1;
+    tk.lane = threadIdx.x & 31;
+    for (uint32_t j = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); j < n; j += warps) {
+        const uint32_t i = in_list[j];
+        const GridDesc g = grids[bp.tgt_frame[frame_of(bp.cur_off, bp.n_pairs, i)]];
+        icp_deferred_point(tk, g, cell_start, pts, cur, i, nn, out_list, out_count, last_level);
+    }
+}
+
+template <bool kPlane>
+__global__ void __launch_bounds__(kIcpThreads) icp_batch_accum_kernel(const float4 *__restrict__ tgt4, const float4 *__restrict__ nrm4,
+                                                                      const float4 *__restrict__ cur,
+                                                                      const unsigned long long *__restrict__ nn, IcpBatchPairs bp,
+                                                                      float max_distance, const IcpState *__restrict__ states,
+                                                                      double *__restrict__ partials) {
+    const int q = frame_of(bp.blk_off, bp.n_pairs, blockIdx.x);
+    if (states[q].done) return;
+    const uint32_t b0 = bp.cur_off[q], ns = bp.cur_off[q + 1] - b0;
+    const uint32_t nb = bp.blk_off[q + 1] - bp.blk_off[q], lb = blockIdx.x - bp.blk_off[q];
+    double acc[NP];
+#pragma unroll
+    for (int j = 0; j < NP; j++) acc[j] = 0.0;
+    for (size_t i = (size_t)lb * blockDim.x + threadIdx.x; i < ns; i += (size_t)nb * blockDim.x)
+        icp_accum_point<kPlane>(acc, tgt4, nrm4, cur + b0, nn + b0, i, max_distance);
+    icp_block_partials(acc, partials + (size_t)blockIdx.x * NP);
+}
+
+// one block per pair: its partials folded exactly as icp_reduce_kernel folds them for one GPU
+__global__ void __launch_bounds__(NP * 32) icp_batch_reduce_kernel(const double *__restrict__ partials, IcpBatchPairs bp,
+                                                                   IcpState *states) {
+    const int q = blockIdx.x;
+    IcpState *state = states + q;
+    if (state->done) return;
+    const int j = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint32_t b0 = bp.blk_off[q];
+    double v = icp_fold_partials(partials + (size_t)b0 * NP, (int)(bp.blk_off[q + 1] - b0), j, lane);
+    v = j == kSrcN ? (double)(bp.cur_off[q + 1] - bp.cur_off[q]) : v;
+    if (lane == 0) state->sums[j] = v;
+}
+
+// one thread per pair; the pair that finishes last raises the host flag
+template <bool kPlane>
+__global__ void icp_batch_solve_kernel(IcpState *states, int n_pairs, int metrics_only, float tolerance, unsigned *active,
+                                       int *host_done_) {
+    volatile int *host_done = host_done_;
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= n_pairs) return;
+    if (icp_step<kPlane>(states + q, metrics_only, tolerance) && atomicSub(active, 1u) == 1u) *host_done = 1;
 }
 
 }  // namespace
@@ -843,6 +1015,182 @@ int icp_dev(Ctx *ctx, const IcpArgs &a, pcr_icp_result *result) {
     result->rmse = h_state->last_rmse;
     result->converged = h_state->converged;
     result->num_iterations = h_state->num_iterations;
+    return PCR_OK;
+}
+
+// Many (source frame, target frame) pairs in one device-resident loop: one multi-frame index (and its coarser levels)
+// over every frame, one working copy per pair, and per pass the same seven launches as icp_dev for all pairs together.
+// The host waits only for the index build and the results.  No communication: each rank registers its own pairs.
+int icp_batch_dev(Ctx *ctx, const IcpBatchArgs &a, pcr_icp_result *results) {
+    cudaStream_t st = ctx->stream;
+    const bool plane = a.d_nx != nullptr;
+    const uint64_t *off = a.frame_offsets;
+    // pairs with an empty side are answered here (icp.rs:131-139: the identity the caller stored, 0 iterations); the
+    // others are numbered q = 0 .. Q - 1
+    std::vector<uint32_t> act, cur_off(1, 0), blk_off(1, 0), tgt_frame, src_begin;
+    const uint64_t blk_cap = (uint64_t)ctx->sm_count * 4;
+    for (size_t p = 0; p < a.n_pairs; p++) {
+        const uint32_t s = a.pairs[2 * p], t = a.pairs[2 * p + 1];
+        const uint64_t ns = off[s + 1] - off[s], nt = off[t + 1] - off[t];
+        if (ns == 0 || nt == 0) {
+            results[p].converged = (ns == 0 && nt == 0) ? 1 : 0;
+            continue;
+        }
+        act.push_back((uint32_t)p);
+        cur_off.push_back(cur_off.back() + (uint32_t)ns);  // (the caller checked that the sum stays below 2^31)
+        blk_off.push_back(blk_off.back() + (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>((ns + kIcpThreads - 1) / kIcpThreads, blk_cap)));
+        tgt_frame.push_back(t);
+        src_begin.push_back((uint32_t)off[s]);
+    }
+    const int Q = (int)act.size();
+    if (Q == 0) return PCR_OK;
+    const uint32_t total = cur_off.back(), n_blocks = blk_off.back();
+
+    Index *tgt = nullptr;
+    BuildOpts bo;
+    bo.k_hint = 1;
+    bo.transient = true;
+    bo.n_frames = (int)a.n_frames;
+    bo.frame_offsets = a.frame_offsets;
+    PCR_TRY(index_build_dev(ctx, a.d_x, a.d_y, a.d_z, a.n, bo, &tgt));
+    struct Guard {
+        Index *ix;
+        ~Guard() { index_free(ix); }
+    } guard{tgt};
+    Index *levels[kMaxLevels] = {tgt, nullptr, nullptr, nullptr};
+    for (int l = 1; l < kMaxLevels; l++) PCR_TRY(index_coarser_level(levels[l - 1], &levels[l]));
+
+    // one allocation: working copy | nn | deferred lists (counters, active-pair counter, 2 lists) | partials | states |
+    // pair table | packed normals
+    auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    const size_t o_nn = up(sizeof(float4) * total);
+    const size_t o_dl = o_nn + up(sizeof(unsigned long long) * total);
+    const size_t o_part = o_dl + up(sizeof(uint32_t) * (64 + 2 * (size_t)total));
+    const size_t o_state = o_part + up(sizeof(double) * NP * (size_t)n_blocks);
+    const size_t o_tab = o_state + up(sizeof(IcpState) * Q);
+    const size_t tab_words = 4 * (size_t)Q + 2;
+    const size_t o_nrm = o_tab + up(sizeof(uint32_t) * tab_words);
+    const size_t bytes = o_nrm + (plane ? sizeof(float4) * a.n : 0);
+    char *mem = nullptr;
+    PCR_CUDA(ctx, cudaMallocAsync((void **)&mem, bytes, st));
+    struct FreeLater {
+        void *p;
+        cudaStream_t s;
+        ~FreeLater() {
+            if (p) cudaFreeAsync(p, s);
+        }
+    } f1{mem, st};
+    float4 *cur = (float4 *)mem;
+    unsigned long long *nn = (unsigned long long *)(mem + o_nn);
+    uint32_t *dcount = (uint32_t *)(mem + o_dl);  // [kMaxLevels]
+    unsigned *active = dcount + 32;
+    uint32_t *dl[2] = {dcount + 64, dcount + 64 + total};
+    double *partials = (double *)(mem + o_part);
+    IcpState *d_states = (IcpState *)(mem + o_state);
+    uint32_t *d_tab = (uint32_t *)(mem + o_tab);
+    float4 *nrm4 = plane ? (float4 *)(mem + o_nrm) : nullptr;
+
+    // the pair table goes up through the pinned mailbox (word 0 is the host flag, the table starts at byte 256)
+    const size_t state_bytes = sizeof(IcpState) * Q;
+    PCR_TRY(ensure_pinned(ctx, 256 + std::max(sizeof(uint32_t) * tab_words, state_bytes)));
+    volatile int *h_done = (volatile int *)ctx->pinned;
+    *h_done = 0;
+    uint32_t *h_tab = (uint32_t *)((char *)ctx->pinned + 256);
+    memcpy(h_tab, cur_off.data(), sizeof(uint32_t) * (Q + 1));
+    memcpy(h_tab + Q + 1, blk_off.data(), sizeof(uint32_t) * (Q + 1));
+    memcpy(h_tab + 2 * Q + 2, tgt_frame.data(), sizeof(uint32_t) * Q);
+    memcpy(h_tab + 3 * Q + 2, src_begin.data(), sizeof(uint32_t) * Q);
+    PCR_CUDA(ctx, cudaMemcpyAsync(d_tab, h_tab, sizeof(uint32_t) * tab_words, cudaMemcpyHostToDevice, st));
+    IcpBatchPairs bp;
+    bp.cur_off = d_tab;
+    bp.blk_off = d_tab + Q + 1;
+    bp.tgt_frame = d_tab + 2 * Q + 2;
+    bp.src_begin = d_tab + 3 * Q + 2;
+    bp.n_pairs = Q;
+
+    if (plane) {
+        pack_normals_kernel<<<(unsigned)((a.n + 255) / 256), 256, 0, st>>>(a.d_nx, a.d_ny, a.d_nz, a.n, nrm4);
+        PCR_LAUNCH_CHECK(ctx);
+    }
+    {  // working copies, binned by target cell in a deterministic order
+        TimeScope ts(ctx, kTagOther);
+        uint32_t max_cells = 1;
+        for (int q = 0; q < Q; q++) max_cells = std::max(max_cells, tgt->grids_h[tgt_frame[q]].n_cells);
+        const int cell_bits = bits_for(max_cells);
+        const int key_bits = cell_bits + bits_for((uint64_t)Q);
+        const size_t hist_words = radix_sort_hist_words(total);
+        char *sm = nullptr;
+        PCR_CUDA(ctx, cudaMallocAsync((void **)&sm, up(2 * sizeof(unsigned long long) * total) + up(2 * sizeof(uint32_t) * total) +
+                                                        sizeof(uint32_t) * hist_words, st));
+        FreeLater f2{sm, st};
+        unsigned long long *kA = (unsigned long long *)sm, *kB = kA + total;
+        uint32_t *vA = (uint32_t *)(sm + up(2 * sizeof(unsigned long long) * total)), *vB = vA + total;
+        uint32_t *hist = (uint32_t *)((char *)vA + up(2 * sizeof(uint32_t) * total));
+        const unsigned nb = (total + 255) / 256;
+        icp_batch_bin_key_kernel<<<nb, 256, 0, st>>>(a.d_x, a.d_y, a.d_z, bp, total, tgt->grids, cell_bits, kA, vA);
+        PCR_LAUNCH_CHECK(ctx);
+        PCR_TRY(radix_sort_pairs_dev(ctx, &kA, &vA, &kB, &vB, total, key_bits, hist));
+        icp_batch_bin_gather_kernel<<<nb, 256, 0, st>>>(a.d_x, a.d_y, a.d_z, bp, total, cell_bits, kA, vA, cur);
+        PCR_LAUNCH_CHECK(ctx);
+    }
+    icp_batch_init_kernel<<<(Q + 127) / 128, 128, 0, st>>>(d_states, Q, active);
+    PCR_LAUNCH_CHECK(ctx);
+
+    auto one_pass = [&](int metrics_only) -> int {
+        {
+            TimeScope ts(ctx, kTagIcpStep);
+            PCR_CUDA(ctx, cudaMemsetAsync(dcount, 0, sizeof(uint32_t) * kMaxLevels, st));
+            icp_batch_search_kernel<<<(total + kIcpThreads - 1) / kIcpThreads, kIcpThreads, 0, st>>>(
+                tgt->grids, tgt->cell_start, tgt->sorted, tgt->orig4, cur, total, bp, d_states, nn, dl[0], dcount + 0, 0);
+            PCR_LAUNCH_CHECK(ctx);
+            for (int l = 1; l < kMaxLevels; l++) {  // (launch sizes as in icp_dev)
+                const bool last = l == kMaxLevels - 1;
+                icp_batch_deferred_kernel<<<ctx->sm_count * (l == 1 ? 8 : 2), 128, 0, st>>>(
+                    levels[l]->grids, levels[l]->cell_start, levels[l]->sorted, cur, bp, dl[(l - 1) & 1], dcount + (l - 1), nn, dl[l & 1],
+                    dcount + l, last ? 1 : 0);
+                PCR_LAUNCH_CHECK(ctx);
+            }
+            if (plane)
+                icp_batch_accum_kernel<true><<<n_blocks, kIcpThreads, 0, st>>>(tgt->orig4, nrm4, cur, nn, bp,
+                                                                               a.params.max_correspondence_distance, d_states, partials);
+            else
+                icp_batch_accum_kernel<false><<<n_blocks, kIcpThreads, 0, st>>>(tgt->orig4, nullptr, cur, nn, bp,
+                                                                                a.params.max_correspondence_distance, d_states, partials);
+            PCR_LAUNCH_CHECK(ctx);
+        }
+        TimeScope ts2(ctx, kTagIcpSolve);
+        icp_batch_reduce_kernel<<<Q, NP * 32, 0, st>>>(partials, bp, d_states);
+        PCR_LAUNCH_CHECK(ctx);
+        if (plane)
+            icp_batch_solve_kernel<true><<<(Q + 31) / 32, 32, 0, st>>>(d_states, Q, metrics_only, a.params.tolerance, active, (int *)h_done);
+        else
+            icp_batch_solve_kernel<false><<<(Q + 31) / 32, 32, 0, st>>>(d_states, Q, metrics_only, a.params.tolerance, active, (int *)h_done);
+        PCR_LAUNCH_CHECK(ctx);
+        return PCR_OK;
+    };
+
+    if (a.params.max_iterations == 0) {
+        PCR_TRY(one_pass(1));
+    } else {
+        for (uint64_t it = 0; it < a.params.max_iterations; it++) {
+            if (*h_done) break;  // every pair has finished; later passes would be no-ops
+            PCR_TRY(one_pass(0));
+            if ((it & 3) == 3) cudaStreamQuery(st);  // flush, so the flag is seen soon after the last pair finishes
+        }
+    }
+    IcpState *h_states = (IcpState *)((char *)ctx->pinned + 256);
+    PCR_CUDA(ctx, cudaMemcpyAsync(h_states, d_states, state_bytes, cudaMemcpyDeviceToHost, st));
+    PCR_CUDA(ctx, cudaStreamSynchronize(st));
+    for (int q = 0; q < Q; q++) {
+        const IcpState &s = h_states[q];
+        pcr_icp_result &r = results[act[q]];
+        memcpy(r.rotation, s.cum_R, sizeof(float) * 9);
+        memcpy(r.translation, s.cum_t, sizeof(float) * 3);
+        r.fitness = s.last_fitness;
+        r.rmse = s.last_rmse;
+        r.converged = s.converged;
+        r.num_iterations = s.num_iterations;
+    }
     return PCR_OK;
 }
 

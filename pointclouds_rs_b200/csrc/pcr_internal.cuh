@@ -314,6 +314,18 @@ struct IcpArgs {
     pcr_icp_params params;
 };
 int icp_dev(Ctx *ctx, const IcpArgs &a, pcr_icp_result *result);
+// Pairs of frames of one buffer (pcr_icp_point_to_*_batch, arguments checked by the caller, results preset to the identity).
+struct IcpBatchArgs {
+    const float *d_x, *d_y, *d_z;  // every frame, back to back
+    size_t n;
+    const uint64_t *frame_offsets;  // host, n_frames + 1
+    size_t n_frames;
+    const float *d_nx, *d_ny, *d_nz;  // one normal per point; nullptr for point-to-point
+    const uint32_t *pairs;            // host: pair p = (source frame, target frame)
+    size_t n_pairs;
+    pcr_icp_params params;
+};
+int icp_batch_dev(Ctx *ctx, const IcpBatchArgs &a, pcr_icp_result *results);
 int find_correspondences_dev(Index *target, const float *dsx, const float *dsy, const float *dsz,
                              size_t ns, float max_distance, uint32_t *d_tgt, float *d_dist);
 int apply_transform_dev(Ctx *ctx, const float *dx, const float *dy, const float *dz, size_t n,
@@ -330,6 +342,8 @@ int voxel_downsample_dev(Ctx *ctx, const float *dx, const float *dy, const float
                          bool allow_guess = true /* frame streams: size the table from the previous frame's key box */);
 int radix_sort_pairs_dev(Ctx *ctx, unsigned long long **keys, uint32_t **vals, unsigned long long **keys_alt, uint32_t **vals_alt,
                          size_t n, int bits, uint32_t *d_hist);
+size_t radix_sort_hist_words(size_t n);  // u32 words of radix_sort_pairs_dev's d_hist for n pairs
+int bits_for(uint64_t range);            // smallest b with 2^b >= range
 
 // ransac_plane_seeded for given samples (ransac.cu); h_samples: HOST array of m index triples
 int ransac_plane_samples_dev(Ctx *ctx, const float *dx, const float *dy, const float *dz, size_t n, float threshold,

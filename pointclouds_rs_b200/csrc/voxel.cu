@@ -494,13 +494,15 @@ __global__ void __launch_bounds__(256) vox_out_stats_kernel(const float *__restr
     }
 }
 
+}  // namespace
+
 int bits_for(uint64_t range) {  // smallest b with 2^b >= range
     int b = 0;
     while (b < 64 && (1ull << b) < range) b++;
     return b;
 }
 
-}  // namespace
+size_t radix_sort_hist_words(size_t n) { return (size_t)256 * ((n + kSortTile - 1) / kSortTile) + 1; }
 
 // Sorts the n (key, val) pairs by the low `bits` bits of the key, stably.  The result is in
 // (*keys, *vals): the pointers are swapped with the alternate buffers after every pass.

@@ -51,6 +51,29 @@ def kitti_scene(seed: int = 42, counts=KITTI_COUNTS["frame122k"]) -> np.ndarray:
     return np.ascontiguousarray(np.vstack(parts), dtype=np.float32)
 
 
+def kitti_points(counts) -> int:
+    """Points of kitti_scene(seed, counts) (two cars)."""
+    n_ground, n_car, n_ped, n_noise = counts
+    return int(n_ground + 2 * n_car + n_ped + n_noise)
+
+
+def kitti_sequence(n_frames: int, seed: int = 42, counts=KITTI_COUNTS["frame122k"], step=(0.4, 0.05, 0.0), yaw: float = 0.01,
+                   jitter: float = 0.01) -> list:
+    """A LiDAR drive through one KITTI-shaped scene: frame i sees a different random subset of kitti_points(counts) points
+    of a 25 % denser scene, in the sensor frame of pose i (pose i+1 = pose i moved by `step` metres and turned by `yaw`
+    radians about z), with Gaussian jitter.  Consecutive frames are a small rigid motion apart (odometry input)."""
+    world = kitti_scene(seed, tuple(int(c * 1.25) for c in counts))
+    n = kitti_points(counts)
+    rng = np.random.default_rng(seed + 1)
+    out = []
+    for i in range(n_frames):
+        idx = np.sort(rng.permutation(len(world))[:n])
+        r = rot_z(-yaw * i).astype(np.float64)
+        p = (world[idx].astype(np.float64) - np.asarray(step, np.float64) * i) @ r.T
+        out.append(np.ascontiguousarray(p + rng.normal(0.0, jitter, (n, 3)), dtype=np.float32))
+    return out
+
+
 def aerial_scene(seed: int = 42, scale: float = 0.1) -> np.ndarray:
     """scale=0.1 -> 241 000 points (config 3); scale=0.415 -> 1 000 150 points (config 4)."""
     rng = np.random.default_rng(seed)
