@@ -18,6 +18,8 @@
  *   pcr_icp_point_to_plane      icp_point_to_plane              crates/registration/src/icp_plane.rs:20-97,131-236
  *   pcr_sor_normals_batch       the SOR -> normals chain of the demo pipelines, per frame
  *                               (examples/python/kitti_obstacle_detection.py:99-101)
+ *   pcr_voxel_downsample_batch / pcr_estimate_normals_batch / pcr_icp_point_to_*_batch
+ *                               voxel_downsample, estimate_normals and ICP of many frames per call
  *
  * The reference calls its kd-tree once per point inside serial loops; a per-query C call would be
  * useless on a GPU, so the boundary is BATCHED and sits one level up: it replaces the bodies of the
@@ -335,6 +337,36 @@ int pcr_sor_normals_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, 
                               size_t k_sor, float std_mul, size_t k_normals,
                               const float viewpoint[3], uint8_t *d_keep, float *d_nx, float *d_ny,
                               float *d_nz);
+
+/* Batched voxel_downsample and estimate_normals: the steps in front of pcr_sor_normals_batch and of the ICP batch, for
+ * many frames in one call.  The frames sit back to back as above, N = frame_offsets[n_frames]; every frame is processed
+ * as if it were alone.
+ * Voxel: frame f's voxels are written to [out_offsets[f], out_offsets[f+1]) of ox/oy/oz (sized N); out_offsets is HOST
+ * memory of n_frames + 1 entries, out_offsets[0] = 0, so it can be passed as the frame_offsets of the other batch calls.
+ * Those entries are bit for bit what pcr_voxel_downsample returns for frame f alone: the same key order and input-order
+ * f32 sums, non-finite points skipped, a frame that is empty or holds no finite point gives 0 voxels, saturated i32 keys
+ * merge.  voxel_size not finite or <= 0 -> PCR_ERR_INVALID_ARG.  The batch neither reads nor updates the frame-stream
+ * voxel key box of the context (pcr_ctx_set_frame_stream), and leaves pcr_ctx_get_hint_stats unchanged.
+ * Normals: one normal per input point, each frame searched only within itself; frame f's entries are bit for bit what
+ * pcr_estimate_normals returns for frame f alone.  k == 0 or N == 0 -> PCR_OK and nothing is written; k > PCR_MAX_K ->
+ * PCR_ERR_UNSUPPORTED; a null viewpoint -> PCR_ERR_INVALID_ARG.
+ * Both: frame_offsets not starting at 0 or decreasing, or a null pointer -> PCR_ERR_INVALID_ARG; N >= 2^31 or more than
+ * 65535 frames -> PCR_ERR_UNSUPPORTED.  Neither batch communicates or shards its queries: on a context with a communicator
+ * every rank processes the frames it was given. */
+int pcr_voxel_downsample_batch(pcr_ctx *ctx, const float *x, const float *y, const float *z,
+                               const uint64_t *frame_offsets, size_t n_frames, float voxel_size,
+                               float *ox, float *oy, float *oz, uint64_t *out_offsets);
+/* _dev: x .. oz are device pointers; frame_offsets and out_offsets stay on the host.  Synchronous. */
+int pcr_voxel_downsample_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z,
+                                   const uint64_t *frame_offsets /* HOST */, size_t n_frames, float voxel_size,
+                                   float *d_ox, float *d_oy, float *d_oz, uint64_t *out_offsets /* HOST */);
+int pcr_estimate_normals_batch(pcr_ctx *ctx, const float *x, const float *y, const float *z,
+                               const uint64_t *frame_offsets, size_t n_frames, size_t k,
+                               const float viewpoint[3], float *nx, float *ny, float *nz);
+/* _dev: device pointers, frame_offsets on the host; enqueued on the context's stream like pcr_sor_normals_batch_dev. */
+int pcr_estimate_normals_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z,
+                                   const uint64_t *frame_offsets /* HOST */, size_t n_frames, size_t k,
+                                   const float viewpoint[3], float *d_nx, float *d_ny, float *d_nz);
 
 /* ---- device-resident clouds (SURVEY 8f-3) ---------------------------------------------------------
  * PointCloud (crates/core/src/cloud.rs:4-18) kept in HBM between the steps of a pipeline: one upload,

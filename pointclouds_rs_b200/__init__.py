@@ -38,7 +38,7 @@ __all__ = [
     "PointCloud", "KdTree", "IcpResult", "Context",
     "statistical_outlier_removal", "radius_outlier_removal", "estimate_normals",
     "icp_point_to_point", "icp_point_to_plane", "apply_transform", "find_correspondences",
-    "icp_point_to_point_batch", "icp_point_to_plane_batch",
+    "icp_point_to_point_batch", "icp_point_to_plane_batch", "voxel_downsample_batch", "estimate_normals_batch",
     "sor_normals_batch", "default_context", "PcrError", "euclidean_cluster", "voxel_downsample", "DeviceCloud", "ransac_plane", "PlaneResult",
 ]
 
@@ -587,8 +587,8 @@ def apply_transform(cloud: PointCloud, rotation, translation, ctx: Optional[Cont
     return PointCloud._from_xyz(ox, oy, oz)
 
 
-def _icp_batch_arrays(points, frame_offsets, pairs):
-    """Checks and converts the frame buffer of a batched ICP: (N,3) f32 rows, u64 offsets, (P,2) u32 pairs."""
+def _batch_frames(points, frame_offsets):
+    """Checks and converts the frame buffer of a batch call: (N,3) f32 rows, frames back to back, u64 offsets."""
     pts = np.asarray(points)
     if pts.ndim != 2 or pts.shape[1] != 3:
         raise ValueError("points must have shape (N, 3)")
@@ -598,6 +598,12 @@ def _icp_batch_arrays(points, frame_offsets, pairs):
         raise ValueError("frame_offsets must be n_frames + 1 integers")
     if off[0] != 0 or off[-1] != n or np.any(np.diff(off) < 0):
         raise ValueError(f"frame_offsets must be non-decreasing from 0 to the number of points ({n})")
+    return np.ascontiguousarray(pts, np.float32), np.ascontiguousarray(off, np.uint64)
+
+
+def _icp_batch_arrays(points, frame_offsets, pairs):
+    """Checks and converts the frame buffer of a batched ICP: (N,3) f32 rows, u64 offsets, (P,2) u32 pairs."""
+    pts, off = _batch_frames(points, frame_offsets)
     nf = len(off) - 1
     pr = np.asarray(pairs)
     if pr.size == 0:
@@ -606,7 +612,7 @@ def _icp_batch_arrays(points, frame_offsets, pairs):
         raise ValueError("pairs must be an integer array of shape (P, 2): (source frame, target frame)")
     if len(pr) and (pr.min() < 0 or pr.max() >= nf):
         raise ValueError(f"pairs hold a frame id outside [0, {nf})")
-    return (np.ascontiguousarray(pts, np.float32), np.ascontiguousarray(off, np.uint64), np.ascontiguousarray(pr, np.uint32))
+    return pts, off, np.ascontiguousarray(pr, np.uint32)
 
 
 def icp_point_to_point_batch(points: np.ndarray, frame_offsets: Sequence[int], pairs, max_iterations: int = 50,
@@ -858,6 +864,43 @@ def sor_normals_batch(points: np.ndarray, frame_offsets: Sequence[int], k_sor: i
                                                 _p(vp, _ffi.f32p), _p(keep, _ffi.u8p), _p(nrm, _ffi.f32p), _p(kept, _ffi.u64p))
     _ffi.check(st, ctx._h)
     return keep[:n], nrm[:n], kept[:nf]
+
+
+def voxel_downsample_batch(points: np.ndarray, frame_offsets: Sequence[int], voxel_size: float, ctx: Optional[Context] = None):
+    """voxel_downsample of every frame of a batch in one call.  points: (N,3), frame f = rows [frame_offsets[f],
+    frame_offsets[f+1]).  -> (voxels (M,3) f32, offsets (F+1,) u64): frame f's voxels are rows [offsets[f], offsets[f+1]),
+    bit for bit what voxel_downsample returns for the frame alone; the offsets can be passed to the other batch calls."""
+    pts, off = _batch_frames(points, frame_offsets)
+    if not math.isfinite(voxel_size) or voxel_size <= 0.0:
+        raise ValueError("voxel_size must be > 0 and finite")
+    ctx = ctx or default_context()
+    x, y, z = _soa(pts)
+    n = len(pts)
+    ox, oy, oz = (np.zeros(max(n, 1), np.float32) for _ in range(3))
+    out_off = np.zeros(len(off), np.uint64)
+    st = _ffi.load().pcr_voxel_downsample_batch(ctx._h, _p(x, _ffi.f32p), _p(y, _ffi.f32p), _p(z, _ffi.f32p), _p(off, _ffi.u64p), len(off) - 1,
+                                                float(voxel_size), _p(ox, _ffi.f32p), _p(oy, _ffi.f32p), _p(oz, _ffi.f32p), _p(out_off, _ffi.u64p))
+    _ffi.check(st, ctx._h)
+    m = int(out_off[-1])
+    return np.stack([ox[:m], oy[:m], oz[:m]], axis=1), out_off
+
+
+def estimate_normals_batch(points: np.ndarray, frame_offsets: Sequence[int], k: int, viewpoint=(0.0, 0.0, 0.0),
+                           ctx: Optional[Context] = None) -> np.ndarray:
+    """estimate_normals_with_viewpoint of every frame of a batch in one call, each frame searched only within itself.
+    -> (N,3) f32, frame f's rows bit for bit what normals_array returns for the frame alone ((0,3) if k == 0)."""
+    pts, off = _batch_frames(points, frame_offsets)
+    ctx = ctx or default_context()
+    n = len(pts)
+    if n == 0 or k == 0:
+        return np.zeros((0, 3), np.float32)
+    vp = np.asarray(viewpoint, np.float32).reshape(3)
+    x, y, z = _soa(pts)
+    nx, ny, nz = (np.empty(n, np.float32) for _ in range(3))
+    st = _ffi.load().pcr_estimate_normals_batch(ctx._h, _p(x, _ffi.f32p), _p(y, _ffi.f32p), _p(z, _ffi.f32p), _p(off, _ffi.u64p), len(off) - 1,
+                                                k, _p(vp, _ffi.f32p), _p(nx, _ffi.f32p), _p(ny, _ffi.f32p), _p(nz, _ffi.f32p))
+    _ffi.check(st, ctx._h)
+    return np.stack([nx, ny, nz], axis=1)
 
 
 def sor_normals_batch_raw(ctx: Context, x, y, z, n: int, frame_offsets: np.ndarray, k_sor: int, std_mul: float,

@@ -107,6 +107,10 @@ SIGNATURES = {
                                                    C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
     "pcr_voxel_downsample": (C.c_int, [vp, f32p, f32p, f32p, C.c_size_t, C.c_float, f32p, f32p, f32p, szp]),
     "pcr_voxel_downsample_dev": (C.c_int, [vp, vp, vp, vp, C.c_size_t, C.c_float, vp, vp, vp, szp]),
+    "pcr_voxel_downsample_batch": (C.c_int, [vp, f32p, f32p, f32p, u64p, C.c_size_t, C.c_float, f32p, f32p, f32p, u64p]),
+    "pcr_voxel_downsample_batch_dev": (C.c_int, [vp, vp, vp, vp, u64p, C.c_size_t, C.c_float, vp, vp, vp, u64p]),
+    "pcr_estimate_normals_batch": (C.c_int, [vp, f32p, f32p, f32p, u64p, C.c_size_t, C.c_size_t, f32p, f32p, f32p, f32p]),
+    "pcr_estimate_normals_batch_dev": (C.c_int, [vp, vp, vp, vp, u64p, C.c_size_t, C.c_size_t, f32p, vp, vp, vp]),
     "pcr_euclidean_cluster": (C.c_int, [vp, f32p, f32p, f32p, C.c_size_t, C.c_float, C.c_size_t, C.c_size_t, u32p, u32p, szp]),
     "pcr_cluster_labels_dev": (C.c_int, [vp, vp, vp, vp, C.c_size_t, C.c_float, vp]),
     "pcr_radius_outlier_dev": (C.c_int, [vp, vp, vp, vp, C.c_size_t, C.c_float, C.c_size_t, vp]),

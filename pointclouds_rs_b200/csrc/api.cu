@@ -1025,6 +1025,22 @@ int pcr_icp_point_to_plane_dev(pcr_ctx *ctx, const float *sx, const float *sy, c
     return icp_entry(ctx, true, true, sx, sy, sz, ns, tx, ty, tz, nt, nx, ny, nz, n_normals, params, result);
 }
 
+// Frame offsets of a batch call (ICP, voxel_downsample and estimate_normals batches): frame f = points
+// [frame_offsets[f], frame_offsets[f+1]), starting at 0, never decreasing.
+static int batch_offsets_check(Ctx *c, const uint64_t *frame_offsets, size_t n_frames) {
+    if (!frame_offsets) return fail(c, PCR_ERR_INVALID_ARG, "frame_offsets is NULL");
+    if (frame_offsets[0] != 0) return fail(c, PCR_ERR_INVALID_ARG, "frame_offsets must start at 0");
+    for (size_t f = 0; f < n_frames; f++)
+        if (frame_offsets[f + 1] < frame_offsets[f]) return fail(c, PCR_ERR_INVALID_ARG, "frame_offsets must be non-decreasing");
+    return PCR_OK;
+}
+// ... and the sizes their kernels are built for: u32 point indices, one grid row per frame
+static int batch_size_check(Ctx *c, size_t n, size_t n_frames) {
+    if (n > 0x7fffffffull) return fail(c, PCR_ERR_UNSUPPORTED, "clouds above 2^31 points are not supported");
+    if (n_frames > 65535) return fail(c, PCR_ERR_UNSUPPORTED, "at most 65535 frames per batch");
+    return PCR_OK;
+}
+
 // Pairs of frames of one buffer: every pair is checked and answered as the single-pair call would (icp_entry).
 static int icp_batch_entry(pcr_ctx *ctx, bool dev, bool plane, const float *x, const float *y, const float *z, const uint64_t *frame_offsets,
                            size_t n_frames, const float *nx, const float *ny, const float *nz, size_t n_normals, const uint32_t *pairs,
@@ -1033,10 +1049,8 @@ static int icp_batch_entry(pcr_ctx *ctx, bool dev, bool plane, const float *x, c
     Ctx *c = &ctx->c;
     PCR_TRY(icp_check(c, params, results));
     for (size_t p = 0; p < n_pairs; p++) icp_identity(&results[p]);
-    if (!frame_offsets || (n_pairs && !pairs)) return fail(c, PCR_ERR_INVALID_ARG, "frame_offsets/pairs is NULL");
-    if (frame_offsets[0] != 0) return fail(c, PCR_ERR_INVALID_ARG, "frame_offsets must start at 0");
-    for (size_t f = 0; f < n_frames; f++)
-        if (frame_offsets[f + 1] < frame_offsets[f]) return fail(c, PCR_ERR_INVALID_ARG, "frame_offsets must be non-decreasing");
+    if (n_pairs && !pairs) return fail(c, PCR_ERR_INVALID_ARG, "pairs is NULL");
+    PCR_TRY(batch_offsets_check(c, frame_offsets, n_frames));
     const size_t n = (size_t)frame_offsets[n_frames];
     if (plane && n_normals != n)  // icp_plane.rs:27-32, for the whole buffer
         return fail(c, PCR_ERR_NORMALS_MISMATCH, "normals length (%zu) does not match the number of points (%zu)", n_normals, n);
@@ -1047,8 +1061,7 @@ static int icp_batch_entry(pcr_ctx *ctx, bool dev, bool plane, const float *x, c
         src_points += frame_offsets[s + 1] - frame_offsets[s];
     }
     if (src_points >= (1ull << 31)) return fail(c, PCR_ERR_UNSUPPORTED, "the source frames of one batch must hold fewer than 2^31 points");
-    if (n > 0x7fffffffull) return fail(c, PCR_ERR_UNSUPPORTED, "clouds above 2^31 points are not supported");
-    if (n_frames > 65535) return fail(c, PCR_ERR_UNSUPPORTED, "at most 65535 frames per batch");
+    PCR_TRY(batch_size_check(c, n, n_frames));
     if (n && (!x || !y || !z || (plane && (!nx || !ny || !nz)))) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     PCR_API_BEGIN
     DevSetter ds(c);
@@ -1090,6 +1103,104 @@ int pcr_icp_point_to_plane_batch_dev(pcr_ctx *ctx, const float *d_x, const float
                                      const uint32_t *pairs, size_t n_pairs, const pcr_icp_params *params, pcr_icp_result *results) {
     return icp_batch_entry(ctx, true, true, d_x, d_y, d_z, frame_offsets, n_frames, d_nx, d_ny, d_nz, n_normals, pairs, n_pairs, params,
                            results);
+}
+
+/* ---- batched voxel_downsample and estimate_normals --------------------------------------------------- */
+// Frames back to back; every frame gets what the single call returns for it alone.  Neither batch communicates or
+// shards its queries: on a context with a communicator each rank processes the frames it was given.
+static int voxel_batch_entry(pcr_ctx *ctx, bool dev, const float *x, const float *y, const float *z, const uint64_t *frame_offsets,
+                             size_t n_frames, float voxel_size, float *ox, float *oy, float *oz, uint64_t *out_offsets) {
+    if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
+    Ctx *c = &ctx->c;
+    if (!out_offsets) return fail(c, PCR_ERR_INVALID_ARG, "out_offsets is NULL");
+    out_offsets[0] = 0;
+    PCR_TRY(batch_offsets_check(c, frame_offsets, n_frames));
+    for (size_t f = 1; f <= n_frames; f++) out_offsets[f] = 0;
+    const size_t n = (size_t)frame_offsets[n_frames];
+    PCR_TRY(batch_size_check(c, n, n_frames));
+    if (!std::isfinite(voxel_size) || !(voxel_size > 0.f)) return fail(c, PCR_ERR_INVALID_ARG, "voxel_size must be > 0 and finite");
+    if (n && (!x || !y || !z || !ox || !oy || !oz)) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    if (n == 0) return PCR_OK;
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    if (dev) return voxel_downsample_batch_dev(c, x, y, z, frame_offsets, n_frames, voxel_size, ox, oy, oz, out_offsets);
+    float *dx, *dy, *dz;
+    PCR_TRY(stage_xyz(c, c->b_in, x, y, z, n, &dx, &dy, &dz));
+    const size_t stride = (n + 63) & ~(size_t)63;
+    PCR_TRY(ensure(c, c->b_out, sizeof(float) * 3 * stride));
+    float *o0 = (float *)c->b_out.p, *o1 = o0 + stride, *o2 = o1 + stride;
+    PCR_TRY(voxel_downsample_batch_dev(c, dx, dy, dz, frame_offsets, n_frames, voxel_size, o0, o1, o2, out_offsets));
+    const size_t m = (size_t)out_offsets[n_frames];
+    if (m) {
+        PCR_CUDA(c, cudaMemcpyAsync(ox, o0, m * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+        PCR_CUDA(c, cudaMemcpyAsync(oy, o1, m * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+        PCR_CUDA(c, cudaMemcpyAsync(oz, o2, m * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+        PCR_CUDA(c, cudaStreamSynchronize(c->stream));
+    }
+    return PCR_OK;
+    PCR_API_END(c)
+}
+
+int pcr_voxel_downsample_batch(pcr_ctx *ctx, const float *x, const float *y, const float *z, const uint64_t *frame_offsets, size_t n_frames,
+                               float voxel_size, float *ox, float *oy, float *oz, uint64_t *out_offsets) {
+    return voxel_batch_entry(ctx, false, x, y, z, frame_offsets, n_frames, voxel_size, ox, oy, oz, out_offsets);
+}
+int pcr_voxel_downsample_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z, const uint64_t *frame_offsets,
+                                   size_t n_frames, float voxel_size, float *d_ox, float *d_oy, float *d_oz, uint64_t *out_offsets) {
+    return voxel_batch_entry(ctx, true, d_x, d_y, d_z, frame_offsets, n_frames, voxel_size, d_ox, d_oy, d_oz, out_offsets);
+}
+
+// One transient index over all frames (each frame searched only within itself), then the normals of every point: the
+// non-SOR half of batch_core.
+static int normals_batch_core(Ctx *c, const float *dx, const float *dy, const float *dz, const uint64_t *frame_offsets, size_t n_frames,
+                              size_t n, size_t k, const float vp[3], float *d_nx, float *d_ny, float *d_nz) {
+    BuildOpts bo;
+    bo.k_hint = k;
+    bo.self_knn = true;
+    bo.n_frames = (int)n_frames;
+    bo.frame_offsets = frame_offsets;
+    bo.transient = true;
+    Index *ix = nullptr;
+    PCR_TRY(index_build_dev(c, dx, dy, dz, n, bo, &ix));
+    const int s = normals_dev(ix, k, vp, d_nx, d_ny, d_nz, nullptr, /*allow_shard=*/false);
+    index_free(ix);
+    return s;
+}
+
+static int normals_batch_entry(pcr_ctx *ctx, bool dev, const float *x, const float *y, const float *z, const uint64_t *frame_offsets,
+                               size_t n_frames, size_t k, const float viewpoint[3], float *nx, float *ny, float *nz) {
+    if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
+    Ctx *c = &ctx->c;
+    PCR_TRY(batch_offsets_check(c, frame_offsets, n_frames));
+    const size_t n = (size_t)frame_offsets[n_frames];
+    PCR_TRY(batch_size_check(c, n, n_frames));
+    if (n == 0 || k == 0) return PCR_OK;  // estimate.rs:25-31, as the single call
+    if (!x || !y || !z || !nx || !ny || !nz || !viewpoint) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    if (k > PCR_MAX_K) return fail(c, PCR_ERR_UNSUPPORTED, "k = %zu exceeds PCR_MAX_K = %d", k, PCR_MAX_K);
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    if (dev) return normals_batch_core(c, x, y, z, frame_offsets, n_frames, n, k, viewpoint, nx, ny, nz);
+    float *dx, *dy, *dz;
+    PCR_TRY(stage_xyz(c, c->b_in, x, y, z, n, &dx, &dy, &dz));
+    const size_t stride = (n + 63) & ~(size_t)63;
+    PCR_TRY(ensure(c, c->b_out, stride * 3 * sizeof(float)));
+    float *dnx = (float *)c->b_out.p, *dny = dnx + stride, *dnz = dny + stride;
+    PCR_TRY(normals_batch_core(c, dx, dy, dz, frame_offsets, n_frames, n, k, viewpoint, dnx, dny, dnz));
+    PCR_CUDA(c, cudaMemcpyAsync(nx, dnx, n * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    PCR_CUDA(c, cudaMemcpyAsync(ny, dny, n * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    PCR_CUDA(c, cudaMemcpyAsync(nz, dnz, n * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    PCR_CUDA(c, cudaStreamSynchronize(c->stream));
+    return PCR_OK;
+    PCR_API_END(c)
+}
+
+int pcr_estimate_normals_batch(pcr_ctx *ctx, const float *x, const float *y, const float *z, const uint64_t *frame_offsets, size_t n_frames,
+                               size_t k, const float viewpoint[3], float *nx, float *ny, float *nz) {
+    return normals_batch_entry(ctx, false, x, y, z, frame_offsets, n_frames, k, viewpoint, nx, ny, nz);
+}
+int pcr_estimate_normals_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z, const uint64_t *frame_offsets,
+                                   size_t n_frames, size_t k, const float viewpoint[3], float *d_nx, float *d_ny, float *d_nz) {
+    return normals_batch_entry(ctx, true, d_x, d_y, d_z, frame_offsets, n_frames, k, viewpoint, d_nx, d_ny, d_nz);
 }
 
 /* ---- multi-frame batch ---------------------------------------------------------------------------- */

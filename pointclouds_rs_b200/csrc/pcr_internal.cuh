@@ -340,6 +340,10 @@ size_t clusters_from_labels(const uint32_t *labels, size_t n, size_t min_size, s
 int voxel_downsample_dev(Ctx *ctx, const float *dx, const float *dy, const float *dz, size_t n, float voxel, float *d_ox, float *d_oy,
                          float *d_oz, size_t *n_out, CloudStats *stats_out = nullptr /* host; filled (valid = 1) when it comes for free */,
                          bool allow_guess = true /* frame streams: size the table from the previous frame's key box */);
+// every frame of a batch in one call (pcr_voxel_downsample_batch, arguments checked by the caller); out_offsets: host,
+// n_frames + 1, frame f's voxels are [out_offsets[f], out_offsets[f+1]) of the outputs (sized frame_offsets[n_frames])
+int voxel_downsample_batch_dev(Ctx *ctx, const float *dx, const float *dy, const float *dz, const uint64_t *frame_offsets,
+                               size_t n_frames, float voxel, float *d_ox, float *d_oy, float *d_oz, uint64_t *out_offsets);
 int radix_sort_pairs_dev(Ctx *ctx, unsigned long long **keys, uint32_t **vals, unsigned long long **keys_alt, uint32_t **vals_alt,
                          size_t n, int bits, uint32_t *d_hist);
 size_t radix_sort_hist_words(size_t n);  // u32 words of radix_sort_pairs_dev's d_hist for n pairs

@@ -56,19 +56,30 @@ struct VoxRange {
 // voxel_downsample.rs:32-36: (p / voxel).floor() as i32 -- IEEE division, round down, saturate, NaN -> 0
 __device__ __forceinline__ int vox_cell(float v, float voxel) { return __float2int_rd(__fdiv_rn(v, voxel)); }
 
-__global__ void vox_init_kernel(VoxRange *r) {
-    for (int a = 0; a < 3; a++) {
-        r->mn[a] = 2147483647;
-        r->mx[a] = -2147483647 - 1;
+__global__ void vox_init_kernel(VoxRange *r, int n_ranges) {
+    for (int f = blockIdx.x * blockDim.x + threadIdx.x; f < n_ranges; f += gridDim.x * blockDim.x) {
+        for (int a = 0; a < 3; a++) {
+            r[f].mn[a] = 2147483647;
+            r[f].mx[a] = -2147483647 - 1;
+        }
+        r[f].finite = 0;
     }
-    r->finite = 0;
 }
 
+// frame_off == nullptr: the range of the n points.  Otherwise (batch) frame blockIdx.y = points [frame_off[y],
+// frame_off[y + 1]) and its range goes to r[y]: a block never crosses a frame, so the reductions below stay per frame.
 __global__ void __launch_bounds__(256) vox_range_kernel(const float *__restrict__ x, const float *__restrict__ y,
-                                                        const float *__restrict__ z, size_t n, float voxel, VoxRange *r) {
+                                                        const float *__restrict__ z, const uint32_t *__restrict__ frame_off,
+                                                        size_t n, float voxel, VoxRange *r) {
     int mn[3] = {2147483647, 2147483647, 2147483647}, mx[3] = {-2147483647 - 1, -2147483647 - 1, -2147483647 - 1};
     unsigned cnt = 0;
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+    size_t b = 0, e = n;
+    if (frame_off) {
+        b = frame_off[blockIdx.y];
+        e = frame_off[blockIdx.y + 1];
+        r += blockIdx.y;
+    }
+    for (size_t i = b + (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < e; i += (size_t)gridDim.x * blockDim.x) {
         const float px = x[i], py = y[i], pz = z[i];
         if (!finite3(px, py, pz)) continue;  // :28-30
         const int k[3] = {vox_cell(px, voxel), vox_cell(py, voxel), vox_cell(pz, voxel)};
@@ -114,11 +125,14 @@ __global__ void __launch_bounds__(256) vox_range_kernel(const float *__restrict_
 
 // axis < 0: packed key ((kx - mn0) << s0) | ((ky - mn1) << s1) | (kz - mn2); axis 0..2: that axis alone
 // (biased to unsigned).  Non-finite points get `last`, above every real key.
+// Batch (fr != nullptr): the point's frame f (frame_of over frame_off) takes the biases from its own range fr[f] and
+// leads the packed key, (f << fshift) | ...; axis 3 is the frame id alone.
 __global__ void __launch_bounds__(256) vox_pack_kernel(const float *__restrict__ x, const float *__restrict__ y,
                                                        const float *__restrict__ z, const uint32_t *order, size_t n,
                                                        float voxel, int axis, int mn0, int mn1, int mn2, int s0, int s1,
                                                        unsigned long long last, unsigned long long *__restrict__ keys,
-                                                       uint32_t *vals /* may alias order */) {
+                                                       uint32_t *vals /* may alias order */, const uint32_t *__restrict__ frame_off,
+                                                       int n_frames, const VoxRange *__restrict__ fr, int fshift) {
     const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= n) return;
     const uint32_t i = order ? order[t] : (uint32_t)t;
@@ -126,11 +140,22 @@ __global__ void __launch_bounds__(256) vox_pack_kernel(const float *__restrict__
     unsigned long long key = last;
     if (finite3(px, py, pz)) {
         const int kx = vox_cell(px, voxel), ky = vox_cell(py, voxel), kz = vox_cell(pz, voxel);
-        if (axis < 0)
-            key = ((unsigned long long)(uint32_t)(kx - mn0) << s0) | ((unsigned long long)(uint32_t)(ky - mn1) << s1) |
+        if (axis < 0) {
+            unsigned long long head = 0;
+            if (fr) {
+                const int f = frame_of(frame_off, n_frames, i);
+                mn0 = fr[f].mn[0];
+                mn1 = fr[f].mn[1];
+                mn2 = fr[f].mn[2];
+                head = (unsigned long long)f << fshift;
+            }
+            key = head | ((unsigned long long)(uint32_t)(kx - mn0) << s0) | ((unsigned long long)(uint32_t)(ky - mn1) << s1) |
                   (unsigned long long)(uint32_t)(kz - mn2);
-        else
+        } else if (axis == 3) {
+            key = (unsigned long long)frame_of(frame_off, n_frames, i);
+        } else {
             key = (unsigned long long)((uint32_t)(axis == 0 ? kx : (axis == 1 ? ky : kz)) ^ 0x80000000u);
+        }
     }
     keys[t] = key;
     vals[t] = i;
@@ -205,10 +230,12 @@ __global__ void __launch_bounds__(256) vox_heads_kernel(const unsigned long long
     flag[i] = (i < m && (i == 0 || keys[i] != keys[i - 1])) ? 1u : 0u;  // flag[m] = 0: slot of the total
 }
 
-// the three-pass (z, y, x) fallback has no packed key: heads are compared on the recomputed triple
+// the three-pass (z, y, x) fallback has no packed key: heads are compared on the recomputed triple (and, in a batch,
+// on the frame: the same voxel of two frames is two voxels)
 __global__ void __launch_bounds__(256) vox_heads_triple_kernel(const float *__restrict__ x, const float *__restrict__ y,
                                                                const float *__restrict__ z, const uint32_t *__restrict__ vals, uint32_t m,
-                                                               float voxel, uint32_t *__restrict__ flag) {
+                                                               float voxel, const uint32_t *__restrict__ frame_off, int n_frames,
+                                                               uint32_t *__restrict__ flag) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i > m) return;
     uint32_t f = 0;
@@ -217,7 +244,7 @@ __global__ void __launch_bounds__(256) vox_heads_triple_kernel(const float *__re
         if (i > 0) {
             const uint32_t a = vals[i], b = vals[i - 1];
             f = (vox_cell(x[a], voxel) != vox_cell(x[b], voxel) || vox_cell(y[a], voxel) != vox_cell(y[b], voxel) ||
-                 vox_cell(z[a], voxel) != vox_cell(z[b], voxel))
+                 vox_cell(z[a], voxel) != vox_cell(z[b], voxel) || frame_of(frame_off, n_frames, a) != frame_of(frame_off, n_frames, b))
                     ? 1u
                     : 0u;
         }
@@ -494,6 +521,21 @@ __global__ void __launch_bounds__(256) vox_out_stats_kernel(const float *__restr
     }
 }
 
+// Batch: out_off[f] = first voxel of frame f, out_off[n_frames] = number of voxels.  The m finite points are sorted by
+// frame first, so thread i in [0, m] writes the entries of the frames that start between sorted positions i - 1 and i
+// (empty frames and frames without a finite point included): all of them start at voxel vid[i].
+__global__ void __launch_bounds__(256) vox_frame_starts_kernel(const unsigned long long *__restrict__ keys, const uint32_t *__restrict__ vals,
+                                                               uint32_t m, int fshift /* < 0: no frame in the key */,
+                                                               const uint32_t *__restrict__ frame_off, int n_frames,
+                                                               const uint32_t *__restrict__ vid, uint32_t *__restrict__ out_off) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i > m) return;
+    auto frame = [&](uint32_t j) { return fshift >= 0 ? (int)(keys[j] >> fshift) : frame_of(frame_off, n_frames, vals[j]); };
+    const int hi = i < m ? frame(i) : n_frames;
+    const int lo = i > 0 ? frame(i - 1) : -1;
+    for (int f = lo + 1; f <= hi; f++) out_off[f] = vid[i];
+}
+
 }  // namespace
 
 int bits_for(uint64_t range) {  // smallest b with 2^b >= range
@@ -552,10 +594,10 @@ int voxel_downsample_dev(Ctx *ctx, const float *dx, const float *dy, const float
         }
         m = (uint32_t)n;  // (an upper bound is all the sizing below needs)
     } else {
-        vox_init_kernel<<<1, 1, 0, st>>>(d_range);
+        vox_init_kernel<<<1, 1, 0, st>>>(d_range, 1);
         PCR_LAUNCH_CHECK(ctx);
         const unsigned bx = (unsigned)std::min<size_t>((n + 255) / 256, (size_t)ctx->sm_count * 2);
-        vox_range_kernel<<<bx, 256, 0, st>>>(dx, dy, dz, n, voxel, d_range);
+        vox_range_kernel<<<bx, 256, 0, st>>>(dx, dy, dz, nullptr, n, voxel, d_range);
         PCR_LAUNCH_CHECK(ctx);
         PCR_CUDA(ctx, cudaMemcpyAsync(h_range, d_range, sizeof(VoxRange), cudaMemcpyDeviceToHost, st));
         PCR_MARK("voxel: wait for range");
@@ -692,7 +734,7 @@ int voxel_downsample_dev(Ctx *ctx, const float *dx, const float *dy, const float
     if (packed) {
         const unsigned long long last = 1ull << total_bits;  // non-finite points: above every real key
         vox_pack_kernel<<<nb, 256, 0, st>>>(dx, dy, dz, nullptr, n, voxel, -1, h_range->mn[0], h_range->mn[1], h_range->mn[2],
-                                            bits[1] + bits[2], bits[2], last, kA, vA);
+                                            bits[1] + bits[2], bits[2], last, kA, vA, nullptr, 1, nullptr, 0);
         PCR_LAUNCH_CHECK(ctx);
         PCR_TRY(radix_sort_pairs_dev(ctx, &kA, &vA, &kB, &vB, n, total_bits + 1, hist));
         vox_heads_kernel<<<(m + 1 + 255) / 256, 256, 0, st>>>(kA, m, vid);
@@ -701,11 +743,12 @@ int voxel_downsample_dev(Ctx *ctx, const float *dx, const float *dy, const float
         const unsigned long long last = 1ull << 32;
         for (int axis = 2; axis >= 0; axis--) {  // LSD over the axes: z, y, x
             // after the first pass vA holds the order so far; the pack kernel reads and rewrites it in place
-            vox_pack_kernel<<<nb, 256, 0, st>>>(dx, dy, dz, axis == 2 ? nullptr : vA, n, voxel, axis, 0, 0, 0, 0, 0, last, kA, vA);
+            vox_pack_kernel<<<nb, 256, 0, st>>>(dx, dy, dz, axis == 2 ? nullptr : vA, n, voxel, axis, 0, 0, 0, 0, 0, last, kA, vA, nullptr, 1,
+                                                nullptr, 0);
             PCR_LAUNCH_CHECK(ctx);
             PCR_TRY(radix_sort_pairs_dev(ctx, &kA, &vA, &kB, &vB, n, 33, hist));
         }
-        vox_heads_triple_kernel<<<(m + 1 + 255) / 256, 256, 0, st>>>(dx, dy, dz, vA, m, voxel, vid);
+        vox_heads_triple_kernel<<<(m + 1 + 255) / 256, 256, 0, st>>>(dx, dy, dz, vA, m, voxel, nullptr, 1, vid);
         PCR_LAUNCH_CHECK(ctx);
     }
     PCR_TRY(exclusive_scan_u32_dev(ctx, vid, (size_t)m + 1));  // vid[m] = number of voxels
@@ -718,6 +761,117 @@ int voxel_downsample_dev(Ctx *ctx, const float *dx, const float *dy, const float
     PCR_CUDA(ctx, cudaMemcpyAsync(mail, d_nvox, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     PCR_CUDA(ctx, cudaStreamSynchronize(st));
     *n_out = *mail;
+    return PCR_OK;
+}
+
+// voxel_downsample of every frame of a batch (frame f = points [frame_offsets[f], frame_offsets[f+1]), offsets on the
+// host, checked by the caller) in one set of launches: the radix path above with the frame as the most significant
+// part of the key.  Frame f's voxels go to [out_offsets[f], out_offsets[f+1]) of the outputs (sized n), bit for bit
+// what voxel_downsample_dev returns for the frame alone: the same key order and the same input-order sums, since the
+// sort is stable and a frame's points keep their order.  Two host round trips: the per-frame key ranges, and the
+// per-frame voxel counts.  The frame-stream key box (ctx->vox_cache) is neither read nor written.
+int voxel_downsample_batch_dev(Ctx *ctx, const float *dx, const float *dy, const float *dz, const uint64_t *frame_offsets,
+                               size_t n_frames, float voxel, float *d_ox, float *d_oy, float *d_oz, uint64_t *out_offsets) {
+    const int F = (int)n_frames;
+    for (int f = 0; f <= F; f++) out_offsets[f] = 0;
+    const size_t n = F ? (size_t)frame_offsets[F] : 0;
+    if (n == 0) return PCR_OK;
+    cudaStream_t st = ctx->stream;
+    TimeScope ts(ctx, kTagOther);
+    // scratch (b_table): keys A/B u64[n] | vals A/B u32[n] | hist u32[256 * tiles + 1] | flag/vid u32[n + 1] | start u32[n + 1]
+    //                    | frame offsets u32[F + 1] | out offsets u32[F + 1] | ranges VoxRange[F]
+    const size_t n_tiles = (n + kSortTile - 1) / kSortTile;
+    const size_t need = 2 * sizeof(unsigned long long) * n + sizeof(uint32_t) * (2 * n + 256 * n_tiles + 1 + 2 * (n + 1)) +
+                        sizeof(uint32_t) * 2 * (F + 1) + sizeof(VoxRange) * F + 1024;
+    PCR_TRY(ensure(ctx, ctx->b_table, need));
+    PCR_TRY(ensure_pinned(ctx, std::max<size_t>(4096, std::max(sizeof(VoxRange) * F, sizeof(uint32_t) * (F + 1)))));
+    char *p = (char *)ctx->b_table.p;
+    unsigned long long *kA = (unsigned long long *)p;
+    p += sizeof(unsigned long long) * n;
+    unsigned long long *kB = (unsigned long long *)p;
+    p += sizeof(unsigned long long) * n;
+    uint32_t *vA = (uint32_t *)p;
+    p += sizeof(uint32_t) * n;
+    uint32_t *vB = (uint32_t *)p;
+    p += sizeof(uint32_t) * n;
+    uint32_t *hist = (uint32_t *)p;
+    p += sizeof(uint32_t) * (256 * n_tiles + 1);
+    uint32_t *vid = (uint32_t *)p;
+    p += sizeof(uint32_t) * (n + 1);
+    uint32_t *start = (uint32_t *)p;
+    p += sizeof(uint32_t) * (n + 1);
+    uint32_t *d_off = (uint32_t *)p;
+    p += sizeof(uint32_t) * (F + 1);
+    uint32_t *d_out_off = (uint32_t *)p;
+    p += sizeof(uint32_t) * (F + 1);
+    VoxRange *d_range = (VoxRange *)p;
+
+    // per-frame key ranges, ONE round trip for all of them
+    std::vector<uint32_t> h_off(F + 1);
+    size_t longest = 0;
+    for (int f = 0; f <= F; f++) h_off[f] = (uint32_t)frame_offsets[f];
+    for (int f = 0; f < F; f++) longest = std::max<size_t>(longest, h_off[f + 1] - h_off[f]);
+    // (pageable source: the copy has taken the bytes when it returns)
+    PCR_CUDA(ctx, cudaMemcpyAsync(d_off, h_off.data(), sizeof(uint32_t) * (F + 1), cudaMemcpyHostToDevice, st));
+    vox_init_kernel<<<(F + 255) / 256, 256, 0, st>>>(d_range, F);
+    PCR_LAUNCH_CHECK(ctx);
+    const unsigned bx = (unsigned)std::max<size_t>(1, std::min<size_t>((longest + 255) / 256, (size_t)ctx->sm_count * 8 / F));
+    vox_range_kernel<<<dim3(bx, F), 256, 0, st>>>(dx, dy, dz, d_off, n, voxel, d_range);
+    PCR_LAUNCH_CHECK(ctx);
+    VoxRange *h_range = (VoxRange *)ctx->pinned;
+    PCR_CUDA(ctx, cudaMemcpyAsync(h_range, d_range, sizeof(VoxRange) * F, cudaMemcpyDeviceToHost, st));
+    PCR_MARK("voxel batch: wait for ranges");
+    PCR_CUDA(ctx, cudaStreamSynchronize(st));
+    uint64_t m64 = 0;
+    int bits[3] = {0, 0, 0};  // per axis, the widest frame's
+    for (int f = 0; f < F; f++) {
+        if (!h_range[f].finite) continue;
+        m64 += h_range[f].finite;
+        for (int a = 0; a < 3; a++)
+            bits[a] = std::max(bits[a], bits_for((uint64_t)((int64_t)h_range[f].mx[a] - (int64_t)h_range[f].mn[a]) + 1));
+    }
+    if (m64 == 0) return PCR_OK;  // :45-47, in every frame
+    const uint32_t m = (uint32_t)m64;
+    const int fbits = bits_for((uint64_t)F), key_bits = bits[0] + bits[1] + bits[2];
+    const bool packed = fbits + key_bits <= 63;
+
+    // one stable sort of all frames: (frame, key, index) order
+    const unsigned nb = (unsigned)((n + 255) / 256);
+    if (packed) {
+        const unsigned long long last = 1ull << (fbits + key_bits);  // non-finite points: above every real key of every frame
+        vox_pack_kernel<<<nb, 256, 0, st>>>(dx, dy, dz, nullptr, n, voxel, -1, 0, 0, 0, bits[1] + bits[2], bits[2], last, kA, vA, d_off, F,
+                                            d_range, key_bits);
+        PCR_LAUNCH_CHECK(ctx);
+        PCR_TRY(radix_sort_pairs_dev(ctx, &kA, &vA, &kB, &vB, n, fbits + key_bits + 1, hist));
+        vox_heads_kernel<<<(m + 1 + 255) / 256, 256, 0, st>>>(kA, m, vid);
+        PCR_LAUNCH_CHECK(ctx);
+    } else {  // LSD over z, y, x as in the single call, then one more stable pass on the frame id
+        for (int axis = 2; axis >= 0; axis--) {
+            vox_pack_kernel<<<nb, 256, 0, st>>>(dx, dy, dz, axis == 2 ? nullptr : vA, n, voxel, axis, 0, 0, 0, 0, 0, 1ull << 32, kA, vA, nullptr, 1,
+                                                nullptr, 0);
+            PCR_LAUNCH_CHECK(ctx);
+            PCR_TRY(radix_sort_pairs_dev(ctx, &kA, &vA, &kB, &vB, n, 33, hist));
+        }
+        if (F > 1) {
+            vox_pack_kernel<<<nb, 256, 0, st>>>(dx, dy, dz, vA, n, voxel, 3, 0, 0, 0, 0, 0, (unsigned long long)F, kA, vA, d_off, F, nullptr, 0);
+            PCR_LAUNCH_CHECK(ctx);
+            PCR_TRY(radix_sort_pairs_dev(ctx, &kA, &vA, &kB, &vB, n, bits_for((uint64_t)F + 1), hist));
+        }
+        vox_heads_triple_kernel<<<(m + 1 + 255) / 256, 256, 0, st>>>(dx, dy, dz, vA, m, voxel, d_off, F, vid);
+        PCR_LAUNCH_CHECK(ctx);
+    }
+    PCR_TRY(exclusive_scan_u32_dev(ctx, vid, (size_t)m + 1));  // vid[m] = number of voxels
+    vox_starts_kernel<<<(m + 1 + 255) / 256, 256, 0, st>>>(vid, m, start);
+    PCR_LAUNCH_CHECK(ctx);
+    vox_mean_kernel<<<(m + 127) / 128, 128, 0, st>>>(dx, dy, dz, vA, start, vid + m, d_ox, d_oy, d_oz);
+    PCR_LAUNCH_CHECK(ctx);
+    vox_frame_starts_kernel<<<(m + 1 + 255) / 256, 256, 0, st>>>(kA, vA, m, packed ? key_bits : -1, d_off, F, vid, d_out_off);
+    PCR_LAUNCH_CHECK(ctx);
+    uint32_t *h_out = (uint32_t *)ctx->pinned;
+    PCR_CUDA(ctx, cudaMemcpyAsync(h_out, d_out_off, sizeof(uint32_t) * (F + 1), cudaMemcpyDeviceToHost, st));
+    PCR_MARK("voxel batch: wait for counts");
+    PCR_CUDA(ctx, cudaStreamSynchronize(st));
+    for (int f = 0; f <= F; f++) out_offsets[f] = h_out[f];
     return PCR_OK;
 }
 
