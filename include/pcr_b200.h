@@ -20,6 +20,9 @@
  *                               (examples/python/kitti_obstacle_detection.py:99-101)
  *   pcr_voxel_downsample_batch / pcr_estimate_normals_batch / pcr_icp_point_to_*_batch
  *                               voxel_downsample, estimate_normals and ICP of many frames per call
+ *   pcr_ransac_plane_samples_batch / pcr_euclidean_cluster_batch
+ *                               the plane fit and clustering of the obstacle pipeline, many frames per call
+ *                               (examples/python/kitti_obstacle_detection.py:87-122)
  *
  * The reference calls its kd-tree once per point inside serial loops; a per-query C call would be
  * useless on a GPU, so the boundary is BATCHED and sits one level up: it replaces the bodies of the
@@ -317,6 +320,51 @@ int pcr_ransac_plane_samples(pcr_ctx *ctx, const float *x, const float *y, const
                              uint32_t *inliers, size_t *n_inliers);
 int pcr_cloud_ransac_plane_samples(const pcr_cloud *cloud, float distance_threshold, const uint32_t *samples,
                                    size_t m, float model[4], uint32_t *inliers, size_t *n_inliers);
+
+/* Batched plane fit and clustering: the back end of the obstacle pipeline (voxel -> SOR -> ransac_plane -> select_inverse
+ * -> euclidean_cluster) for many frames per call.  The frames sit back to back, frame f = points
+ * [frame_offsets[f], frame_offsets[f+1]), N = frame_offsets[n_frames]; every frame gets bit for bit what the single call
+ * returns for that frame alone.  Indices in and out are FRAME-LOCAL.
+ * RANSAC: frame f's triples are samples[3 * sample_offsets[f] .. 3 * sample_offsets[f+1]) (HOST, sample_offsets
+ * n_frames + 1 entries; both may be NULL when no frame has triples).  models[4f .. 4f+4) (HOST) and the ascending inlier
+ * list inliers[inlier_offsets[f] .. inlier_offsets[f+1]) (inlier_offsets HOST, n_frames + 1; inliers sized N) are what
+ * pcr_ransac_plane_samples returns for frame f and its triples: the default model and no inliers below 3 points, the
+ * default model when no triple is valid (its inliers are still those of the plane z = 0), and the choice rule applied
+ * with the frame's own point and triple counts.  A triple index >= the frame's point count (in a frame of 3 points or
+ * more), or sample_offsets not starting at 0 or decreasing -> PCR_ERR_INVALID_ARG.
+ * Clustering: frame f's clusters are c in [cluster_offsets[f], cluster_offsets[f+1]) (HOST, n_frames + 1), cluster c is
+ * indices[offsets[c] .. offsets[c+1]) (offsets sized N + 1, indices N).  Minus offsets[cluster_offsets[f]], frame f's
+ * CSR is pcr_euclidean_cluster's for the frame alone (size descending, then first index ascending, indices ascending).
+ * threshold <= 0 or min_size == 0 -> no cluster in any frame and offsets[0] = 0; N >= 2^30 -> PCR_ERR_UNSUPPORTED.
+ * Both: frame_offsets not starting at 0 or decreasing, or a null pointer -> PCR_ERR_INVALID_ARG; more than 65535 frames
+ * -> PCR_ERR_UNSUPPORTED.  Neither batch communicates: on a context with a communicator every rank processes the frames
+ * it was given.  Synchronous, two host round trips each whatever the number of frames.  Measured on an NVIDIA B200 at a
+ * 1000 W power limit, 100 frames of 65 K points after voxel 0.15 and SOR: RANSAC with 500 triples per frame 1.88 ms
+ * against 23.9 ms for 100 single calls on resident clouds, clustering of their 487 K non-ground points 0.99 ms against
+ * 36.4 ms (DESIGN section 6). */
+int pcr_ransac_plane_samples_batch(pcr_ctx *ctx, const float *x, const float *y, const float *z,
+                                   const uint64_t *frame_offsets, size_t n_frames, float distance_threshold,
+                                   const uint32_t *samples, const uint64_t *sample_offsets, float *models,
+                                   uint32_t *inliers, uint64_t *inlier_offsets);
+/* _dev: x, y, z and inliers are device pointers; everything else stays on the host. */
+int pcr_ransac_plane_samples_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z,
+                                       const uint64_t *frame_offsets /* HOST */, size_t n_frames, float distance_threshold,
+                                       const uint32_t *samples /* HOST */, const uint64_t *sample_offsets /* HOST */,
+                                       float *models /* HOST */, uint32_t *d_inliers, uint64_t *inlier_offsets /* HOST */);
+int pcr_euclidean_cluster_batch(pcr_ctx *ctx, const float *x, const float *y, const float *z,
+                                const uint64_t *frame_offsets, size_t n_frames, float distance_threshold,
+                                size_t min_size, size_t max_size, uint32_t *offsets, uint32_t *indices,
+                                uint64_t *cluster_offsets);
+/* _dev: x, y, z, offsets and indices are device pointers; frame_offsets and cluster_offsets stay on the host. */
+int pcr_euclidean_cluster_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z,
+                                    const uint64_t *frame_offsets /* HOST */, size_t n_frames, float distance_threshold,
+                                    size_t min_size, size_t max_size, uint32_t *d_offsets, uint32_t *d_indices,
+                                    uint64_t *cluster_offsets /* HOST */);
+/* d_labels[i] = smallest FRAME-LOCAL index of the component of point i inside its frame (pcr_cluster_labels_dev of each
+ * frame alone).  threshold <= 0 -> PCR_ERR_INVALID_ARG.  Enqueued on the context's stream like pcr_cluster_labels_dev. */
+int pcr_cluster_labels_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z,
+                                 const uint64_t *frame_offsets /* HOST */, size_t n_frames, float distance_threshold,
+                                 uint32_t *d_labels);
 
 /* ---- multi-frame batch (BASELINE config 5) ------------------------------------------------------
  * Frames are independent clouds stored back to back: frame f = points [frame_offsets[f],

@@ -40,6 +40,7 @@ __all__ = [
     "icp_point_to_point", "icp_point_to_plane", "apply_transform", "find_correspondences",
     "icp_point_to_point_batch", "icp_point_to_plane_batch", "voxel_downsample_batch", "estimate_normals_batch",
     "sor_normals_batch", "default_context", "PcrError", "euclidean_cluster", "voxel_downsample", "DeviceCloud", "ransac_plane", "PlaneResult",
+    "ransac_plane_samples_batch", "ransac_plane_batch", "cluster_arrays_batch", "euclidean_cluster_batch",
 ]
 
 
@@ -901,6 +902,86 @@ def estimate_normals_batch(points: np.ndarray, frame_offsets: Sequence[int], k: 
                                                 k, _p(vp, _ffi.f32p), _p(nx, _ffi.f32p), _p(ny, _ffi.f32p), _p(nz, _ffi.f32p))
     _ffi.check(st, ctx._h)
     return np.stack([nx, ny, nz], axis=1)
+
+
+def _frame_samples(samples, off):
+    """Checks and stacks the per-frame triples of a batched RANSAC: one (m_f, 3) integer array of frame-LOCAL indices per
+    frame -> (triples (M, 3) u32, sample offsets (F+1,) u64)."""
+    nf = len(off) - 1
+    if isinstance(samples, (str, bytes)) or not hasattr(samples, "__len__") or len(samples) != nf:
+        raise ValueError(f"samples must hold one (m, 3) array of triples per frame ({nf} frames)")
+    parts, s_off = [], np.zeros(nf + 1, np.uint64)
+    for f, smp in enumerate(samples):
+        a = np.asarray(smp)
+        if a.size == 0:
+            a = a.reshape(0, 3)
+        if a.ndim != 2 or a.shape[1] != 3 or (len(a) and a.dtype.kind not in "iu"):
+            raise ValueError(f"samples[{f}] must be an integer array of shape (m, 3)")
+        n_f = int(off[f + 1] - off[f])
+        if len(a) and (int(a.min()) < 0 or int(a.max()) >= n_f):
+            bad = int(a.min()) if int(a.min()) < 0 else int(a.max())
+            raise IndexError(f"frame {f}: sample index {bad} out of bounds for a frame with {n_f} points")
+        parts.append(a.astype(np.uint32))
+        s_off[f + 1] = s_off[f] + len(a)
+    smp = np.ascontiguousarray(np.vstack(parts) if parts else np.zeros((0, 3), np.uint32), np.uint32)
+    return smp, s_off
+
+
+def ransac_plane_samples_batch(points: np.ndarray, frame_offsets: Sequence[int], distance_threshold: float, samples,
+                               ctx: Optional[Context] = None):
+    """ransac_plane_samples of every frame of a batch in one call.  points: (N,3), frame f = rows [frame_offsets[f],
+    frame_offsets[f+1]); samples: one (m_f, 3) array of frame-local index triples per frame.  -> (models (F,4) f32
+    [nx, ny, nz, d], inliers u32, inlier_offsets (F+1,) u64): frame f's model and its ascending frame-local inliers
+    inliers[inlier_offsets[f]:inlier_offsets[f+1]] are bit for bit what ransac_plane_samples returns for the frame alone."""
+    pts, off = _batch_frames(points, frame_offsets)
+    smp, s_off = _frame_samples(samples, off)
+    ctx = ctx or default_context()
+    x, y, z = _soa(pts)
+    n, nf = len(pts), len(off) - 1
+    models = np.zeros((max(nf, 1), 4), np.float32)
+    inl = np.zeros(max(n, 1), np.uint32)
+    inl_off = np.zeros(nf + 1, np.uint64)
+    st = _ffi.load().pcr_ransac_plane_samples_batch(ctx._h, _p(x, _ffi.f32p), _p(y, _ffi.f32p), _p(z, _ffi.f32p), _p(off, _ffi.u64p), nf,
+                                                    float(distance_threshold), _p(smp, _ffi.u32p), _p(s_off, _ffi.u64p),
+                                                    _p(models, _ffi.f32p), _p(inl, _ffi.u32p), _p(inl_off, _ffi.u64p))
+    _ffi.check(st, ctx._h)
+    return models[:nf], inl[:int(inl_off[-1])].copy(), inl_off
+
+
+def ransac_plane_batch(points: np.ndarray, frame_offsets: Sequence[int], distance_threshold: float, iterations: int, seed=None,
+                       ctx: Optional[Context] = None):
+    """ransac_plane of every frame of a batch: frame f's triples are draw_plane_samples(n_f, iterations, [seed, f]) (a
+    fresh random draw per frame when seed is None).  -> as ransac_plane_samples_batch."""
+    _, off = _batch_frames(points, frame_offsets)
+    samples = [draw_plane_samples(int(off[f + 1] - off[f]), iterations, None if seed is None else [seed, f]) for f in range(len(off) - 1)]
+    return ransac_plane_samples_batch(points, off, distance_threshold, samples, ctx)
+
+
+def cluster_arrays_batch(points: np.ndarray, frame_offsets: Sequence[int], distance_threshold: float, min_size: int, max_size: int,
+                         ctx: Optional[Context] = None):
+    """euclidean_cluster of every frame of a batch in one call, CSR form.  -> (cluster_offsets (F+1,) u64, offsets u32,
+    indices u32): frame f's clusters are c in [cluster_offsets[f], cluster_offsets[f+1]), cluster c is the frame-local
+    indices[offsets[c]:offsets[c+1]], in the order cluster_arrays returns for the frame alone."""
+    pts, off = _batch_frames(points, frame_offsets)
+    ctx = ctx or default_context()
+    x, y, z = _soa(pts)
+    n, nf = len(pts), len(off) - 1
+    offsets = np.zeros(n + 1, np.uint32)
+    idx = np.zeros(max(n, 1), np.uint32)
+    c_off = np.zeros(nf + 1, np.uint64)
+    st = _ffi.load().pcr_euclidean_cluster_batch(ctx._h, _p(x, _ffi.f32p), _p(y, _ffi.f32p), _p(z, _ffi.f32p), _p(off, _ffi.u64p), nf,
+                                                 float(distance_threshold), int(min_size), int(max_size), _p(offsets, _ffi.u32p),
+                                                 _p(idx, _ffi.u32p), _p(c_off, _ffi.u64p))
+    _ffi.check(st, ctx._h)
+    k = int(c_off[-1])
+    return c_off, offsets[:k + 1].copy(), idx[:int(offsets[k])].copy()
+
+
+def euclidean_cluster_batch(points: np.ndarray, frame_offsets: Sequence[int], distance_threshold: float, min_size: int, max_size: int,
+                            ctx: Optional[Context] = None) -> List[List[List[int]]]:
+    """-> one list of index lists per frame, each what euclidean_cluster returns for the frame alone."""
+    c_off, offsets, idx = cluster_arrays_batch(points, frame_offsets, distance_threshold, min_size, max_size, ctx)
+    return [[idx[offsets[c]:offsets[c + 1]].tolist() for c in range(int(c_off[f]), int(c_off[f + 1]))] for f in range(len(c_off) - 1)]
 
 
 def sor_normals_batch_raw(ctx: Context, x, y, z, n: int, frame_offsets: np.ndarray, k_sor: int, std_mul: float,

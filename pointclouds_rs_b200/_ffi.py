@@ -138,6 +138,11 @@ SIGNATURES = {
     "pcr_cloud_icp_point_to_plane": (C.c_int, [vp, vp, C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
     "pcr_ransac_plane_samples": (C.c_int, [vp, f32p, f32p, f32p, C.c_size_t, C.c_float, u32p, C.c_size_t, f32p, u32p, szp]),
     "pcr_cloud_ransac_plane_samples": (C.c_int, [vp, C.c_float, u32p, C.c_size_t, f32p, u32p, szp]),
+    "pcr_ransac_plane_samples_batch": (C.c_int, [vp, f32p, f32p, f32p, u64p, C.c_size_t, C.c_float, u32p, u64p, f32p, u32p, u64p]),
+    "pcr_ransac_plane_samples_batch_dev": (C.c_int, [vp, vp, vp, vp, u64p, C.c_size_t, C.c_float, u32p, u64p, f32p, vp, u64p]),
+    "pcr_euclidean_cluster_batch": (C.c_int, [vp, f32p, f32p, f32p, u64p, C.c_size_t, C.c_float, C.c_size_t, C.c_size_t, u32p, u32p, u64p]),
+    "pcr_euclidean_cluster_batch_dev": (C.c_int, [vp, vp, vp, vp, u64p, C.c_size_t, C.c_float, C.c_size_t, C.c_size_t, vp, vp, u64p]),
+    "pcr_cluster_labels_batch_dev": (C.c_int, [vp, vp, vp, vp, u64p, C.c_size_t, C.c_float, vp]),
     "pcr_sor_normals_batch": (C.c_int, [vp, f32p, f32p, f32p, u64p, C.c_size_t, C.c_size_t, C.c_float, C.c_size_t, f32p, u8p, f32p, f32p, f32p, u64p]),
     "pcr_sor_normals_batch_rows": (C.c_int, [vp, f32p, u64p, C.c_size_t, C.c_size_t, C.c_float, C.c_size_t, f32p, u8p, f32p, u64p]),
     "pcr_sor_normals_batch_dev": (C.c_int, [vp, vp, vp, vp, u64p, C.c_size_t, C.c_size_t, C.c_float, C.c_size_t, f32p, vp, vp, vp, vp]),

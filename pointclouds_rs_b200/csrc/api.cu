@@ -1025,7 +1025,7 @@ int pcr_icp_point_to_plane_dev(pcr_ctx *ctx, const float *sx, const float *sy, c
     return icp_entry(ctx, true, true, sx, sy, sz, ns, tx, ty, tz, nt, nx, ny, nz, n_normals, params, result);
 }
 
-// Frame offsets of a batch call (ICP, voxel_downsample and estimate_normals batches): frame f = points
+// Frame offsets of a batch call (ICP, voxel_downsample, estimate_normals, RANSAC and clustering batches): frame f = points
 // [frame_offsets[f], frame_offsets[f+1]), starting at 0, never decreasing.
 static int batch_offsets_check(Ctx *c, const uint64_t *frame_offsets, size_t n_frames) {
     if (!frame_offsets) return fail(c, PCR_ERR_INVALID_ARG, "frame_offsets is NULL");
@@ -1201,6 +1201,134 @@ int pcr_estimate_normals_batch(pcr_ctx *ctx, const float *x, const float *y, con
 int pcr_estimate_normals_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z, const uint64_t *frame_offsets,
                                    size_t n_frames, size_t k, const float viewpoint[3], float *d_nx, float *d_ny, float *d_nz) {
     return normals_batch_entry(ctx, true, d_x, d_y, d_z, frame_offsets, n_frames, k, viewpoint, d_nx, d_ny, d_nz);
+}
+
+/* ---- batched RANSAC plane fit and euclidean_cluster ------------------------------------------------- */
+// The back end of the obstacle pipeline over many frames; every frame gets what the single call returns for it alone.
+// Neither batch communicates: on a context with a communicator each rank processes the frames it was given.
+static int ransac_batch_entry(pcr_ctx *ctx, bool dev, const float *x, const float *y, const float *z, const uint64_t *frame_offsets,
+                              size_t n_frames, float distance_threshold, const uint32_t *samples, const uint64_t *sample_offsets,
+                              float *models, uint32_t *inliers, uint64_t *inlier_offsets) {
+    if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
+    Ctx *c = &ctx->c;
+    if (!models || !inlier_offsets) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    inlier_offsets[0] = 0;
+    PCR_TRY(batch_offsets_check(c, frame_offsets, n_frames));
+    for (size_t f = 1; f <= n_frames; f++) inlier_offsets[f] = 0;
+    const size_t n = (size_t)frame_offsets[n_frames];
+    PCR_TRY(batch_size_check(c, n, n_frames));
+    if (sample_offsets) {
+        if (sample_offsets[0] != 0) return fail(c, PCR_ERR_INVALID_ARG, "sample_offsets must start at 0");
+        for (size_t f = 0; f < n_frames; f++)
+            if (sample_offsets[f + 1] < sample_offsets[f]) return fail(c, PCR_ERR_INVALID_ARG, "sample_offsets must be non-decreasing");
+        if (sample_offsets[n_frames] && !samples) return fail(c, PCR_ERR_INVALID_ARG, "samples is NULL");
+        if (sample_offsets[n_frames] > 0x7fffffffull) return fail(c, PCR_ERR_UNSUPPORTED, "at most 2^31 - 1 sample triples per batch");
+    } else if (samples) {
+        return fail(c, PCR_ERR_INVALID_ARG, "sample_offsets is NULL");
+    }
+    if (n && (!x || !y || !z || !inliers)) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    if (dev || n == 0)
+        return ransac_plane_samples_batch_dev(c, x, y, z, frame_offsets, n_frames, distance_threshold, samples, sample_offsets, models, inliers,
+                                              inlier_offsets);
+    float *dx, *dy, *dz;
+    PCR_TRY(stage_xyz(c, c->b_in, x, y, z, n, &dx, &dy, &dz));
+    PCR_TRY(ensure(c, c->b_out, sizeof(uint32_t) * n));
+    uint32_t *d_inl = (uint32_t *)c->b_out.p;
+    PCR_TRY(ransac_plane_samples_batch_dev(c, dx, dy, dz, frame_offsets, n_frames, distance_threshold, samples, sample_offsets, models, d_inl,
+                                           inlier_offsets));
+    const size_t k = (size_t)inlier_offsets[n_frames];
+    if (k) {
+        PCR_CUDA(c, cudaMemcpyAsync(inliers, d_inl, sizeof(uint32_t) * k, cudaMemcpyDeviceToHost, c->stream));
+        PCR_CUDA(c, cudaStreamSynchronize(c->stream));
+    }
+    return PCR_OK;
+    PCR_API_END(c)
+}
+
+int pcr_ransac_plane_samples_batch(pcr_ctx *ctx, const float *x, const float *y, const float *z, const uint64_t *frame_offsets, size_t n_frames,
+                                   float distance_threshold, const uint32_t *samples, const uint64_t *sample_offsets, float *models,
+                                   uint32_t *inliers, uint64_t *inlier_offsets) {
+    return ransac_batch_entry(ctx, false, x, y, z, frame_offsets, n_frames, distance_threshold, samples, sample_offsets, models, inliers,
+                              inlier_offsets);
+}
+int pcr_ransac_plane_samples_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z, const uint64_t *frame_offsets,
+                                       size_t n_frames, float distance_threshold, const uint32_t *samples, const uint64_t *sample_offsets,
+                                       float *models, uint32_t *d_inliers, uint64_t *inlier_offsets) {
+    return ransac_batch_entry(ctx, true, d_x, d_y, d_z, frame_offsets, n_frames, distance_threshold, samples, sample_offsets, models, d_inliers,
+                              inlier_offsets);
+}
+
+static int cluster_batch_entry(pcr_ctx *ctx, bool dev, const float *x, const float *y, const float *z, const uint64_t *frame_offsets,
+                               size_t n_frames, float distance_threshold, size_t min_size, size_t max_size, uint32_t *offsets,
+                               uint32_t *indices, uint64_t *cluster_offsets) {
+    if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
+    Ctx *c = &ctx->c;
+    if (!offsets || !cluster_offsets) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    cluster_offsets[0] = 0;
+    if (!dev) offsets[0] = 0;
+    PCR_TRY(batch_offsets_check(c, frame_offsets, n_frames));
+    for (size_t f = 1; f <= n_frames; f++) cluster_offsets[f] = 0;
+    const size_t n = (size_t)frame_offsets[n_frames];
+    PCR_TRY(batch_size_check(c, n, n_frames));
+    if (n && (!x || !y || !z || !indices)) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    if (n == 0 || distance_threshold <= 0.0f || min_size == 0) {  // euclidean_cluster.rs:102-104, in every frame
+        if (dev) {
+            PCR_CUDA(c, cudaMemsetAsync(offsets, 0, sizeof(uint32_t), c->stream));
+            PCR_CUDA(c, cudaStreamSynchronize(c->stream));
+        }
+        return PCR_OK;
+    }
+    size_t total = 0;
+    if (dev)
+        return euclidean_cluster_batch_dev(c, x, y, z, frame_offsets, n_frames, distance_threshold, min_size, max_size, offsets, indices,
+                                           cluster_offsets, &total);
+    float *dx, *dy, *dz;
+    PCR_TRY(stage_xyz(c, c->b_in, x, y, z, n, &dx, &dy, &dz));
+    PCR_TRY(ensure(c, c->b_out, sizeof(uint32_t) * (2 * n + 1)));
+    uint32_t *d_off = (uint32_t *)c->b_out.p, *d_idx = d_off + n + 1;
+    PCR_TRY(euclidean_cluster_batch_dev(c, dx, dy, dz, frame_offsets, n_frames, distance_threshold, min_size, max_size, d_off, d_idx,
+                                        cluster_offsets, &total));
+    const size_t k = (size_t)cluster_offsets[n_frames];
+    if (k) {
+        PCR_CUDA(c, cudaMemcpyAsync(offsets, d_off, sizeof(uint32_t) * (k + 1), cudaMemcpyDeviceToHost, c->stream));
+        PCR_CUDA(c, cudaMemcpyAsync(indices, d_idx, sizeof(uint32_t) * total, cudaMemcpyDeviceToHost, c->stream));
+        PCR_CUDA(c, cudaStreamSynchronize(c->stream));
+    }
+    return PCR_OK;
+    PCR_API_END(c)
+}
+
+int pcr_euclidean_cluster_batch(pcr_ctx *ctx, const float *x, const float *y, const float *z, const uint64_t *frame_offsets, size_t n_frames,
+                                float distance_threshold, size_t min_size, size_t max_size, uint32_t *offsets, uint32_t *indices,
+                                uint64_t *cluster_offsets) {
+    return cluster_batch_entry(ctx, false, x, y, z, frame_offsets, n_frames, distance_threshold, min_size, max_size, offsets, indices,
+                               cluster_offsets);
+}
+int pcr_euclidean_cluster_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z, const uint64_t *frame_offsets,
+                                    size_t n_frames, float distance_threshold, size_t min_size, size_t max_size, uint32_t *d_offsets,
+                                    uint32_t *d_indices, uint64_t *cluster_offsets) {
+    return cluster_batch_entry(ctx, true, d_x, d_y, d_z, frame_offsets, n_frames, distance_threshold, min_size, max_size, d_offsets, d_indices,
+                               cluster_offsets);
+}
+
+int pcr_cluster_labels_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z, const uint64_t *frame_offsets,
+                                 size_t n_frames, float distance_threshold, uint32_t *d_labels) {
+    if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
+    Ctx *c = &ctx->c;
+    PCR_TRY(batch_offsets_check(c, frame_offsets, n_frames));
+    const size_t n = (size_t)frame_offsets[n_frames];
+    PCR_TRY(batch_size_check(c, n, n_frames));
+    if (n && (!d_x || !d_y || !d_z || !d_labels)) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    if (distance_threshold <= 0.0f) return fail(c, PCR_ERR_INVALID_ARG, "distance_threshold must be > 0");
+    if (n == 0) return PCR_OK;
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    return cluster_labels_batch_dev(c, d_x, d_y, d_z, frame_offsets, n_frames, distance_threshold, d_labels);
+    PCR_API_END(c)
 }
 
 /* ---- multi-frame batch ---------------------------------------------------------------------------- */

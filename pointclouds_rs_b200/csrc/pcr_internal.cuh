@@ -332,9 +332,19 @@ int apply_transform_dev(Ctx *ctx, const float *dx, const float *dy, const float 
                         const float R[9], const float t[3], float *ox, float *oy, float *oz);
 
 // euclidean_cluster (cluster.cu): labels[i] = smallest index of the component of point i
-int cluster_labels_dev(Ctx *ctx, const float *dx, const float *dy, const float *dz, size_t n, float threshold, uint32_t *d_labels);
+// (d_frame_off: device frame offsets of a batch, no component crosses a frame; labels stay global indices)
+int cluster_labels_dev(Ctx *ctx, const float *dx, const float *dy, const float *dz, size_t n, float threshold, uint32_t *d_labels,
+                       const uint32_t *d_frame_off = nullptr, int n_frames = 1);
 size_t clusters_from_labels(const uint32_t *labels, size_t n, size_t min_size, size_t max_size, uint32_t *offsets, uint32_t *indices,
                             std::vector<uint32_t> &scratch);
+// every frame of a batch (pcr_cluster_labels_batch_dev / pcr_euclidean_cluster_batch, arguments checked by the caller):
+// frame-local labels, and the CSR of every frame in the single call's order (frame f's clusters are
+// [cluster_offsets[f], cluster_offsets[f+1]), host; *total = clustered points)
+int cluster_labels_batch_dev(Ctx *ctx, const float *dx, const float *dy, const float *dz, const uint64_t *frame_offsets, size_t n_frames,
+                             float threshold, uint32_t *d_labels);
+int euclidean_cluster_batch_dev(Ctx *ctx, const float *dx, const float *dy, const float *dz, const uint64_t *frame_offsets, size_t n_frames,
+                                float threshold, size_t min_size, size_t max_size, uint32_t *d_offsets, uint32_t *d_indices,
+                                uint64_t *cluster_offsets, size_t *total);
 
 // voxel_downsample + the stable radix sort it uses (voxel.cu)
 int voxel_downsample_dev(Ctx *ctx, const float *dx, const float *dy, const float *dz, size_t n, float voxel, float *d_ox, float *d_oy,
@@ -352,6 +362,12 @@ int bits_for(uint64_t range);            // smallest b with 2^b >= range
 // ransac_plane_seeded for given samples (ransac.cu); h_samples: HOST array of m index triples
 int ransac_plane_samples_dev(Ctx *ctx, const float *dx, const float *dy, const float *dz, size_t n, float threshold,
                              const uint32_t *h_samples, size_t m, float model_out[4], uint32_t *d_inliers, size_t *n_inliers);
+// every frame of a batch (pcr_ransac_plane_samples_batch, frame and sample offsets checked by the caller): h_samples holds
+// frame-LOCAL triples, frame f's are [sample_offsets[f], sample_offsets[f+1]); models_out 4 per frame (host), frame f's
+// ascending frame-local inliers at [inlier_offsets[f], inlier_offsets[f+1]) of d_inliers (inlier_offsets: host)
+int ransac_plane_samples_batch_dev(Ctx *ctx, const float *dx, const float *dy, const float *dz, const uint64_t *frame_offsets,
+                                   size_t n_frames, float threshold, const uint32_t *h_samples, const uint64_t *sample_offsets,
+                                   float *models_out, uint32_t *d_inliers, uint64_t *inlier_offsets);
 
 // NCCL plumbing (comm.cu)
 int comm_unique_id(void *out);

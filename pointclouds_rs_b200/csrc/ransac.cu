@@ -13,6 +13,8 @@
 //                         early exit (:95-121), or first-maximum for the parallel path (:82-93)
 //   ransac_inlier_kernel  inlier flags of the winner -> exclusive scan -> ascending index list (:123-126)
 // f32 arithmetic is the reference's, operation by operation (no FMA: the library is built -fmad=false).
+// A batch (frames back to back) fits all frames' triples in one launch, counts with blocks that never cross a frame
+// against that frame's models only, and writes every frame's inliers with one scan (ransac_plane_samples_batch_dev).
 #include "pcr_internal.cuh"
 
 #include <algorithm>
@@ -58,14 +60,13 @@ __global__ void __launch_bounds__(256) ransac_fit_kernel(const float *__restrict
     models[t] = mdl;
 }
 
-__global__ void __launch_bounds__(kRansacThreads) ransac_count_kernel(const float *__restrict__ x, const float *__restrict__ y,
-                                                                      const float *__restrict__ z, size_t n, float threshold,
-                                                                      const float4 *__restrict__ models, size_t m,
-                                                                      uint32_t *__restrict__ counts) {
+// one block's share of the counts: points base + j * kRansacThreads (j < kRansacItems) below n, against the m models
+__device__ __forceinline__ void ransac_count_block(const float *__restrict__ x, const float *__restrict__ y, const float *__restrict__ z,
+                                                   size_t base, size_t n, float threshold, const float4 *__restrict__ models, size_t m,
+                                                   uint32_t *__restrict__ counts) {
     __shared__ float4 smodel[kModelChunk];
     __shared__ uint32_t scount[kModelChunk];
     float px[kRansacItems], py[kRansacItems], pz[kRansacItems];
-    const size_t base = (size_t)blockIdx.x * (kRansacThreads * kRansacItems) + threadIdx.x;
 #pragma unroll
     for (int j = 0; j < kRansacItems; j++) {
         const size_t i = base + (size_t)j * kRansacThreads;
@@ -97,6 +98,25 @@ __global__ void __launch_bounds__(kRansacThreads) ransac_count_kernel(const floa
     }
 }
 
+__global__ void __launch_bounds__(kRansacThreads) ransac_count_kernel(const float *__restrict__ x, const float *__restrict__ y,
+                                                                      const float *__restrict__ z, size_t n, float threshold,
+                                                                      const float4 *__restrict__ models, size_t m,
+                                                                      uint32_t *__restrict__ counts) {
+    ransac_count_block(x, y, z, (size_t)blockIdx.x * (kRansacThreads * kRansacItems) + threadIdx.x, n, threshold, models, m, counts);
+}
+
+// Batch: every block holds kRansacThreads * kRansacItems points of ONE frame (blocks[b] = {frame, first point}) and
+// streams only that frame's models, [model_off[f], model_off[f+1]).
+__global__ void __launch_bounds__(kRansacThreads) ransac_count_batch_kernel(const float *__restrict__ x, const float *__restrict__ y,
+                                                                            const float *__restrict__ z, const uint2 *__restrict__ blocks,
+                                                                            const uint32_t *__restrict__ frame_off,
+                                                                            const uint32_t *__restrict__ model_off, float threshold,
+                                                                            const float4 *__restrict__ models, uint32_t *__restrict__ counts) {
+    const uint2 b = blocks[blockIdx.x];
+    const uint32_t m0 = model_off[b.x];
+    ransac_count_block(x, y, z, (size_t)b.y + threadIdx.x, frame_off[b.x + 1], threshold, models + m0, model_off[b.x + 1] - m0, counts + m0);
+}
+
 __global__ void __launch_bounds__(256) ransac_inlier_kernel(const float *__restrict__ x, const float *__restrict__ y,
                                                             const float *__restrict__ z, size_t n, float4 model, float threshold,
                                                             uint32_t *__restrict__ flag) {
@@ -109,6 +129,64 @@ __global__ void __launch_bounds__(256) ransac_emit_kernel(const uint32_t *__rest
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     if (pos[i + 1] != pos[i]) out[pos[i]] = (uint32_t)i;
+}
+
+// Batch: the inlier flags of every point against its frame's winner (a frame of fewer than 3 points has none, :64-66) ...
+__global__ void __launch_bounds__(256) ransac_inlier_batch_kernel(const float *__restrict__ x, const float *__restrict__ y,
+                                                                  const float *__restrict__ z, size_t n, const uint32_t *__restrict__ frame_off,
+                                                                  int n_frames, const float4 *__restrict__ best, float threshold,
+                                                                  uint32_t *__restrict__ flag) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i > n) return;
+    uint32_t v = 0;
+    if (i < n) {
+        const int f = frame_of(frame_off, n_frames, (uint32_t)i);
+        v = (frame_off[f + 1] - frame_off[f] >= 3 && plane_dist(best[f], x[i], y[i], z[i]) <= threshold) ? 1u : 0u;
+    }
+    flag[i] = v;
+}
+
+// ... the frame-local index of every inlier at its scanned position ...
+__global__ void __launch_bounds__(256) ransac_emit_batch_kernel(const uint32_t *__restrict__ pos, size_t n, const uint32_t *__restrict__ frame_off,
+                                                                int n_frames, uint32_t *__restrict__ out) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n || pos[i + 1] == pos[i]) return;
+    out[pos[i]] = (uint32_t)i - frame_off[frame_of(frame_off, n_frames, (uint32_t)i)];
+}
+
+// ... and the first inlier of every frame (entry n_frames: the total)
+__global__ void ransac_frame_starts_kernel(const uint32_t *__restrict__ pos, const uint32_t *__restrict__ frame_off, int n_frames,
+                                           uint32_t *__restrict__ out) {
+    const int f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f <= n_frames) out[f] = pos[frame_off[f]];
+}
+
+// the reference's choice rule (:80-121), replayed on the counts of one cloud's m hypotheses (0xffffffff: collinear sample)
+float4 ransac_choose(const uint32_t *counts, const float4 *models, size_t m, size_t n) {
+    float4 best = make_float4(0.f, 0.f, 1.f, 0.f);
+    const bool parallel = n >= 10000 && m >= 16;  // :80
+    size_t best_count = 0;
+    bool have = false;
+    for (size_t it = 0; it < m; it++) {
+        if (counts[it] == 0xffffffffu) continue;  // collinear sample (:86 / :98-101)
+        const size_t cnt = counts[it];
+        if (parallel) {  // :84-93: first hypothesis with the largest count
+            if (!have || cnt > best_count) {
+                have = true;
+                best_count = cnt;
+                best = models[it];
+            }
+        } else if (cnt > best_count) {  // :106
+            best_count = cnt;
+            best = models[it];
+            const double w = (double)best_count / (double)n;  // :110-117
+            if (w > 0.5) {
+                const double needed = std::log(1.0 - 0.999) / std::log(1.0 - w * w * w);
+                if ((double)it > needed) break;
+            }
+        }
+    }
+    return best;
 }
 
 }  // namespace
@@ -148,29 +226,7 @@ int ransac_plane_samples_dev(Ctx *ctx, const float *dx, const float *dy, const f
         PCR_CUDA(ctx, cudaMemcpyAsync(counts.data(), d_counts, sizeof(uint32_t) * m, cudaMemcpyDeviceToHost, st));
         PCR_CUDA(ctx, cudaMemcpyAsync(models.data(), d_models, sizeof(float4) * m, cudaMemcpyDeviceToHost, st));
         PCR_CUDA(ctx, cudaStreamSynchronize(st));
-        // the reference's choice rule, replayed on the counts
-        const bool parallel = n >= 10000 && m >= 16;  // :80
-        size_t best_count = 0;
-        bool have = false;
-        for (size_t it = 0; it < m; it++) {
-            if (counts[it] == 0xffffffffu) continue;  // collinear sample (:86 / :98-101)
-            const size_t cnt = counts[it];
-            if (parallel) {  // :84-93: first hypothesis with the largest count
-                if (!have || cnt > best_count) {
-                    have = true;
-                    best_count = cnt;
-                    best = models[it];
-                }
-            } else if (cnt > best_count) {  // :106
-                best_count = cnt;
-                best = models[it];
-                const double w = (double)best_count / (double)n;  // :110-117
-                if (w > 0.5) {
-                    const double needed = std::log(1.0 - 0.999) / std::log(1.0 - w * w * w);
-                    if ((double)it > needed) break;
-                }
-            }
-        }
+        best = ransac_choose(counts.data(), models.data(), m, n);
     }
     model_out[0] = best.x; model_out[1] = best.y; model_out[2] = best.z; model_out[3] = best.w;
     ransac_inlier_kernel<<<(unsigned)((n + 1 + 255) / 256), 256, 0, st>>>(dx, dy, dz, n, best, threshold, d_pos);
@@ -182,6 +238,119 @@ int ransac_plane_samples_dev(Ctx *ctx, const float *dx, const float *dy, const f
     PCR_CUDA(ctx, cudaMemcpyAsync(mail, d_pos + n, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     PCR_CUDA(ctx, cudaStreamSynchronize(st));
     *n_inliers = *mail;
+    return PCR_OK;
+}
+
+// Every frame of a batch in one set of launches; frame f gets what ransac_plane_samples_dev returns for it alone with its
+// own triples (its own n and m in the choice rule).  The triples are turned into global indices while they are staged,
+// so the fit is the single call's kernel over all M triples.  Two host round trips: all counts and models, then the
+// per-frame inlier offsets.
+int ransac_plane_samples_batch_dev(Ctx *ctx, const float *dx, const float *dy, const float *dz, const uint64_t *frame_offsets,
+                                   size_t n_frames, float threshold, const uint32_t *h_samples, const uint64_t *sample_offsets,
+                                   float *models_out, uint32_t *d_inliers, uint64_t *inlier_offsets) {
+    const int F = (int)n_frames;
+    for (int f = 0; f < F; f++) {
+        float *mo = models_out + 4 * f;
+        mo[0] = 0.f; mo[1] = 0.f; mo[2] = 1.f; mo[3] = 0.f;  // PlaneModel::default(), :23-30
+    }
+    for (int f = 0; f <= F; f++) inlier_offsets[f] = 0;
+    const size_t n = F ? (size_t)frame_offsets[F] : 0;
+    if (n == 0) return PCR_OK;
+    // host staging, ONE copy: triples u32[3M] (global indices) | frame offsets u32[F + 1] | model offsets u32[F + 1] |
+    // count blocks uint2[B].  A frame below 3 points keeps none of its triples (the single call returns before it
+    // reads them, :64-66).
+    const size_t per_block = (size_t)kRansacThreads * kRansacItems;
+    std::vector<uint32_t> moff(F + 1, 0);
+    size_t n_blocks = 0;
+    for (int f = 0; f < F; f++) {
+        const uint64_t b = frame_offsets[f], nf = frame_offsets[f + 1] - b;
+        const uint64_t mf = sample_offsets ? sample_offsets[f + 1] - sample_offsets[f] : 0;
+        moff[f + 1] = moff[f];
+        if (nf < 3 || mf == 0) continue;
+        const uint32_t *t = h_samples + 3 * sample_offsets[f];
+        for (uint64_t j = 0; j < 3 * mf; j++)
+            if (t[j] >= nf)
+                return fail(ctx, PCR_ERR_INVALID_ARG, "frame %d: sample index %u out of bounds for a frame with %llu points", f, t[j],
+                            (unsigned long long)nf);
+        moff[f + 1] += (uint32_t)mf;
+        n_blocks += (nf + per_block - 1) / per_block;
+    }
+    const size_t M = moff[F];
+    const size_t o_foff = (3 * M + 3) & ~(size_t)3, o_moff = (o_foff + F + 1 + 3) & ~(size_t)3, o_blk = (o_moff + F + 1 + 3) & ~(size_t)3;
+    std::vector<uint32_t> stage(o_blk + 2 * n_blocks);
+    for (int f = 0; f < F; f++) {
+        const uint32_t b = (uint32_t)frame_offsets[f], nf = (uint32_t)(frame_offsets[f + 1] - b);
+        stage[o_foff + f] = b;
+        stage[o_moff + f] = moff[f];
+        const uint32_t mf = moff[f + 1] - moff[f];
+        if (!mf) continue;
+        const uint32_t *t = h_samples + 3 * sample_offsets[f];
+        for (uint32_t j = 0; j < 3 * mf; j++) stage[3 * (size_t)moff[f] + j] = t[j] + b;
+    }
+    stage[o_foff + F] = (uint32_t)n;
+    stage[o_moff + F] = (uint32_t)M;
+    for (int f = 0, blk = 0; f < F; f++) {
+        if (moff[f + 1] == moff[f]) continue;
+        for (uint64_t p = frame_offsets[f]; p < frame_offsets[f + 1]; p += per_block, blk++) {
+            stage[o_blk + 2 * (size_t)blk] = (uint32_t)f;
+            stage[o_blk + 2 * (size_t)blk + 1] = (uint32_t)p;
+        }
+    }
+    cudaStream_t st = ctx->stream;
+    TimeScope ts(ctx, kTagOther);
+    // scratch (b_table): staging | models float4[M] | counts u32[M] | pos u32[n + 1] | winners float4[F] | inlier offsets u32[F + 1]
+    const size_t off_models = (sizeof(uint32_t) * stage.size() + 255) & ~(size_t)255;
+    const size_t off_counts = off_models + sizeof(float4) * std::max<size_t>(M, 1);
+    const size_t off_pos = (off_counts + sizeof(uint32_t) * std::max<size_t>(M, 1) + 255) & ~(size_t)255;
+    const size_t off_best = (off_pos + sizeof(uint32_t) * (n + 1) + 255) & ~(size_t)255;
+    const size_t off_inl = off_best + sizeof(float4) * F;
+    PCR_TRY(ensure(ctx, ctx->b_table, off_inl + sizeof(uint32_t) * (F + 1)));
+    PCR_TRY(ensure_pinned(ctx, std::max<size_t>(4096, sizeof(uint32_t) * (F + 1))));
+    char *base = (char *)ctx->b_table.p;
+    const uint32_t *d_stage = (const uint32_t *)base;
+    const uint32_t *d_foff = d_stage + o_foff, *d_moff = d_stage + o_moff;
+    float4 *d_models = (float4 *)(base + off_models);
+    uint32_t *d_counts = (uint32_t *)(base + off_counts);
+    uint32_t *d_pos = (uint32_t *)(base + off_pos);
+    float4 *d_best = (float4 *)(base + off_best);
+    uint32_t *d_inl_off = (uint32_t *)(base + off_inl);
+    // (pageable source: the copy has taken the bytes when it returns)
+    PCR_CUDA(ctx, cudaMemcpyAsync(base, stage.data(), sizeof(uint32_t) * stage.size(), cudaMemcpyHostToDevice, st));
+    std::vector<float4> best(F, make_float4(0.f, 0.f, 1.f, 0.f));
+    if (M > 0) {
+        ransac_fit_kernel<<<(unsigned)((M + 255) / 256), 256, 0, st>>>(dx, dy, dz, d_stage, M, d_models, d_counts);
+        PCR_LAUNCH_CHECK(ctx);
+        ransac_count_batch_kernel<<<(unsigned)n_blocks, kRansacThreads, 0, st>>>(dx, dy, dz, (const uint2 *)(d_stage + o_blk), d_foff, d_moff,
+                                                                                 threshold, d_models, d_counts);
+        PCR_LAUNCH_CHECK(ctx);
+        std::vector<uint32_t> counts(M);
+        std::vector<float4> models(M);
+        PCR_CUDA(ctx, cudaMemcpyAsync(counts.data(), d_counts, sizeof(uint32_t) * M, cudaMemcpyDeviceToHost, st));
+        PCR_CUDA(ctx, cudaMemcpyAsync(models.data(), d_models, sizeof(float4) * M, cudaMemcpyDeviceToHost, st));
+        PCR_MARK("ransac batch: wait for counts");
+        PCR_CUDA(ctx, cudaStreamSynchronize(st));
+        for (int f = 0; f < F; f++) {
+            const size_t mf = moff[f + 1] - moff[f];
+            if (mf) best[f] = ransac_choose(counts.data() + moff[f], models.data() + moff[f], mf, frame_offsets[f + 1] - frame_offsets[f]);
+        }
+    }
+    for (int f = 0; f < F; f++) {
+        float *mo = models_out + 4 * f;
+        mo[0] = best[f].x; mo[1] = best[f].y; mo[2] = best[f].z; mo[3] = best[f].w;
+    }
+    PCR_CUDA(ctx, cudaMemcpyAsync(d_best, best.data(), sizeof(float4) * F, cudaMemcpyHostToDevice, st));
+    ransac_inlier_batch_kernel<<<(unsigned)((n + 1 + 255) / 256), 256, 0, st>>>(dx, dy, dz, n, d_foff, F, d_best, threshold, d_pos);
+    PCR_LAUNCH_CHECK(ctx);
+    PCR_TRY(exclusive_scan_u32_dev(ctx, d_pos, n + 1));
+    ransac_emit_batch_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_pos, n, d_foff, F, d_inliers);
+    PCR_LAUNCH_CHECK(ctx);
+    ransac_frame_starts_kernel<<<(F + 1 + 255) / 256, 256, 0, st>>>(d_pos, d_foff, F, d_inl_off);
+    PCR_LAUNCH_CHECK(ctx);
+    uint32_t *mail = (uint32_t *)ctx->pinned;
+    PCR_CUDA(ctx, cudaMemcpyAsync(mail, d_inl_off, sizeof(uint32_t) * (F + 1), cudaMemcpyDeviceToHost, st));
+    PCR_MARK("ransac batch: wait for inlier offsets");
+    PCR_CUDA(ctx, cudaStreamSynchronize(st));
+    for (int f = 0; f <= F; f++) inlier_offsets[f] = mail[f];
     return PCR_OK;
 }
 
