@@ -23,6 +23,8 @@
  *   pcr_ransac_plane_samples_batch / pcr_euclidean_cluster_batch
  *                               the plane fit and clustering of the obstacle pipeline, many frames per call
  *                               (examples/python/kitti_obstacle_detection.py:87-122)
+ *   pcr_radius_outlier_batch    radius_outlier_removal of many frames per call
+ *   pcr_frames_*                a batch of frames kept in HBM between those calls (the batch form of pcr_cloud_*)
  *
  * The reference calls its kd-tree once per point inside serial loops; a per-query C call would be
  * useless on a GPU, so the boundary is BATCHED and sits one level up: it replaces the bodies of the
@@ -198,6 +200,16 @@ int pcr_radius_outlier(pcr_ctx *ctx, const float *x, const float *y, const float
 
 int pcr_radius_outlier_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z, size_t n,
                            float radius, size_t min_neighbors, uint8_t *d_keep);
+/* The same for every frame of a batch (frame f = points [frame_offsets[f], frame_offsets[f+1]), HOST offsets): each point
+ * counts the points of its own frame only, and frame f's keep bytes are bit for bit pcr_radius_outlier's for the frame
+ * alone (radius <= 0 or not finite: every count is 0, a point is kept iff min_neighbors == 0).  n_kept_per_frame (may be
+ * NULL): n_frames entries.  Offsets not starting at 0 or decreasing, or a null pointer -> PCR_ERR_INVALID_ARG; N >= 2^31
+ * or more than 65535 frames -> PCR_ERR_UNSUPPORTED.  The batch never shards its queries over a communicator. */
+int pcr_radius_outlier_batch(pcr_ctx *ctx, const float *x, const float *y, const float *z, const uint64_t *frame_offsets,
+                             size_t n_frames, float radius, size_t min_neighbors, uint8_t *keep, uint64_t *n_kept_per_frame);
+/* _dev: x, y, z and keep are device pointers, frame_offsets stays on the host; enqueued on the context's stream. */
+int pcr_radius_outlier_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z, const uint64_t *frame_offsets,
+                                 size_t n_frames, float radius, size_t min_neighbors, uint8_t *d_keep);
 
 /* ---- normals ----------------------------------------------------------------------------------- */
 int pcr_estimate_normals(pcr_ctx *ctx, const float *x, const float *y, const float *z, size_t n,
@@ -470,6 +482,66 @@ int pcr_cloud_icp_point_to_point(const pcr_cloud *source, const pcr_cloud *targe
 /* the target must carry normals (crates/python/src/registration.rs:80-86) */
 int pcr_cloud_icp_point_to_plane(const pcr_cloud *source, const pcr_cloud *target,
                                  const pcr_icp_params *params, pcr_icp_result *result);              /* icp_plane.rs:20 */
+
+/* ---- device-resident frame batches ------------------------------------------------------------------
+ * F clouds back to back in one device allocation, frame f = points [offsets[f], offsets[f+1]): the batch counterpart of
+ * pcr_cloud, so that a pipeline over many frames is one upload, a chain of batch calls and one download.  The rules of
+ * pcr_cloud hold: a batch belongs to the context that made it and is freed before pcr_ctx_destroy; every function that
+ * returns a batch allocates a new handle and leaves its input unchanged; *out is set on success only (a failed call
+ * returns no handle).  Each method runs the core of the matching raw-pointer batch call, so frame f of a result is bit
+ * for bit what the pcr_cloud method returns for frame f alone, edge cases included (empty, one-point and non-finite
+ * frames).  Indices in and out are FRAME-LOCAL.  A filter ends in one compaction of all frames, which costs one host
+ * round trip (all F + 1 new offsets in one copy) on top of the round trips of its batch core.
+ * Uploads: n_frames >= 1, frame_offsets starting at 0 and never decreasing, else PCR_ERR_INVALID_ARG; N >= 2^31 or more
+ * than 65535 frames -> PCR_ERR_UNSUPPORTED.  `xyz` of the _rows form is N rows of x, y, z (see pcr_cloud_upload_rows). */
+typedef struct pcr_frames pcr_frames;
+int pcr_frames_upload(pcr_ctx *ctx, const float *x, const float *y, const float *z, const uint64_t *frame_offsets, size_t n_frames,
+                      pcr_frames **out);
+int pcr_frames_upload_rows(pcr_ctx *ctx, const float *xyz, const uint64_t *frame_offsets, size_t n_frames, pcr_frames **out);
+void pcr_frames_free(pcr_frames *frames);
+size_t pcr_frames_len(const pcr_frames *frames);    /* points of all frames */
+size_t pcr_frames_count(const pcr_frames *frames);  /* frames */
+int pcr_frames_offsets(const pcr_frames *frames, uint64_t *out /* pcr_frames_count + 1 */);
+int pcr_frames_has_normals(const pcr_frames *frames);
+int pcr_frames_device_pointers(const pcr_frames *frames, const float **d_x, const float **d_y, const float **d_z,
+                               const float **d_nx, const float **d_ny, const float **d_nz);
+/* arrays of pcr_frames_len; nx, ny, nz NULL: normals not wanted (PCR_ERR_INVALID_ARG if wanted from a batch without) */
+int pcr_frames_download(const pcr_frames *frames, float *x, float *y, float *z, float *nx, float *ny, float *nz);
+int pcr_frames_download_rows(const pcr_frames *frames, float *xyz, float *normals);
+/* frame f as a new pcr_cloud (a device copy, normals carried), for the single-frame calls; f >= count -> INVALID_ARG */
+int pcr_frames_frame(const pcr_frames *frames, size_t f, pcr_cloud **out);
+/* Per frame, list f = indices[index_offsets[f] .. index_offsets[f+1]) (HOST, index_offsets count + 1 entries).
+ * invert = 0: select (cloud.rs:103-140), the listed points in list order, duplicates kept; invert = 1: select_inverse,
+ * the unlisted points in their order.  Normals are carried.  An index >= its frame's size -> PCR_ERR_INVALID_ARG naming the
+ * frame and the index (the reference panics, cloud.rs:109), before any device work. */
+int pcr_frames_select(const pcr_frames *frames, const uint32_t *indices, const uint64_t *index_offsets, int invert, pcr_frames **out);
+/* pcr_voxel_downsample_batch: the result has no normals (voxel_downsample.rs:64) */
+int pcr_frames_voxel_downsample(const pcr_frames *frames, float voxel_size, pcr_frames **out);
+/* statistical_outlier_removal of every frame (the SOR of pcr_sor_normals_batch); k == 0 empties every frame and drops
+ * the normals, as pcr_cloud_statistical_outlier_removal does; otherwise normals are carried */
+int pcr_frames_statistical_outlier_removal(const pcr_frames *frames, size_t k, float std_mul, pcr_frames **out);
+/* pcr_radius_outlier_batch, then the compaction; normals carried */
+int pcr_frames_radius_outlier_removal(const pcr_frames *frames, float radius, size_t min_neighbors, pcr_frames **out);
+/* pcr_estimate_normals_batch / pcr_sor_normals_batch: the result carries normals (viewpoint NULL = origin; k == 0 or
+ * k_normals == 0 -> PCR_ERR_INVALID_ARG, as for pcr_cloud) */
+int pcr_frames_estimate_normals(const pcr_frames *frames, size_t k, const float viewpoint[3], pcr_frames **out);
+int pcr_frames_sor_normals(const pcr_frames *frames, size_t k_sor, float std_mul, size_t k_normals, const float viewpoint[3],
+                           pcr_frames **out);
+/* pcr_ransac_plane_samples_batch on the batch (models, inlier_offsets HOST as there; inliers HOST, may be NULL: the
+ * lists are not downloaded).  outliers non-NULL: also every frame's select_inverse(inliers), built on the device from
+ * the device inlier lists -- the ground removal of the obstacle pipeline. */
+int pcr_frames_ransac_plane_samples(const pcr_frames *frames, float distance_threshold, const uint32_t *samples,
+                                    const uint64_t *sample_offsets, float *models, uint32_t *inliers, uint64_t *inlier_offsets,
+                                    pcr_frames **outliers);
+/* pcr_euclidean_cluster_batch on the batch; host CSR as there (offsets sized len + 1, indices len) */
+int pcr_frames_euclidean_cluster(const pcr_frames *frames, float distance_threshold, size_t min_size, size_t max_size,
+                                 uint32_t *offsets, uint32_t *indices, uint64_t *cluster_offsets);
+/* pcr_icp_point_to_*_batch on the batch's frames (pairs of frame ids, HOST).  Point-to-plane reads the batch's normals:
+ * a batch without normals -> PCR_ERR_INVALID_ARG (crates/python/src/registration.rs:80-86). */
+int pcr_frames_icp_point_to_point(const pcr_frames *frames, const uint32_t *pairs, size_t n_pairs, const pcr_icp_params *params,
+                                  pcr_icp_result *results);
+int pcr_frames_icp_point_to_plane(const pcr_frames *frames, const uint32_t *pairs, size_t n_pairs, const pcr_icp_params *params,
+                                  pcr_icp_result *results);
 
 #ifdef __cplusplus
 }

@@ -17,6 +17,7 @@ and for the steps either side of it (SURVEY.md section 8f):
     euclidean_cluster(cloud, threshold, min, max)       crates/segmentation/src/euclidean_cluster.rs:96-187
     ransac_plane(cloud, threshold, iterations)          crates/segmentation/src/ransac_plane.rs:56-129 (after the sampling step)
     DeviceCloud                                         a PointCloud that stays in HBM between the steps of a pipeline
+    DeviceFrames                                        a batch of frames that stays in HBM between the batch calls
 
 Everything runs through the C ABI (include/pcr_b200.h) of lib/libpcr_b200.so: hand-written sm_100a
 CUDA, no PyTorch on the path, no CPU fallback.  Out of scope (DESIGN.md section 8): passthrough_filter and file IO.
@@ -41,6 +42,7 @@ __all__ = [
     "icp_point_to_point_batch", "icp_point_to_plane_batch", "voxel_downsample_batch", "estimate_normals_batch",
     "sor_normals_batch", "default_context", "PcrError", "euclidean_cluster", "voxel_downsample", "DeviceCloud", "ransac_plane", "PlaneResult",
     "ransac_plane_samples_batch", "ransac_plane_batch", "cluster_arrays_batch", "euclidean_cluster_batch",
+    "DeviceFrames", "radius_outlier_removal_batch",
 ]
 
 
@@ -1000,3 +1002,229 @@ def sor_normals_batch_raw(ctx: Context, x, y, z, n: int, frame_offsets: np.ndarr
                                        _p(viewpoint, _ffi.f32p), cast(keep, _ffi.u8p), cast(nx, _ffi.f32p), cast(ny, _ffi.f32p),
                                        cast(nz, _ffi.f32p), _p(kept, _ffi.u64p) if kept is not None else None)
     _ffi.check(st, ctx._h)
+
+
+def radius_outlier_removal_batch(points: np.ndarray, frame_offsets: Sequence[int], radius: float, min_neighbors: int,
+                                 ctx: Optional[Context] = None):
+    """radius_outlier_removal's mask for every frame of a batch in one call, each point counting only the points of its
+    own frame.  -> (keep u8 (N,), kept per frame (F,) u64): frame f's bytes are what ror_mask returns for the frame alone."""
+    pts, off = _batch_frames(points, frame_offsets)
+    if not math.isfinite(radius) or radius <= 0.0:  # crates/python/src/filters.rs:57-61
+        raise ValueError("radius must be > 0 and finite")
+    ctx = ctx or default_context()
+    x, y, z = _soa(pts)
+    n, nf = len(pts), len(off) - 1
+    keep = np.zeros(max(n, 1), np.uint8)
+    kept = np.zeros(max(nf, 1), np.uint64)
+    st = _ffi.load().pcr_radius_outlier_batch(ctx._h, _p(x, _ffi.f32p), _p(y, _ffi.f32p), _p(z, _ffi.f32p), _p(off, _ffi.u64p), nf,
+                                              float(radius), int(min_neighbors), _p(keep, _ffi.u8p), _p(kept, _ffi.u64p))
+    _ffi.check(st, ctx._h)
+    return keep[:n], kept[:nf]
+
+
+def _frame_lists(lists, off):
+    """Checks and stacks one frame-local index list per frame -> (indices u32, list offsets (F+1,) u64); IndexError names
+    the frame of an index outside it."""
+    nf = len(off) - 1
+    if isinstance(lists, (str, bytes)) or not hasattr(lists, "__len__") or len(lists) != nf:
+        raise ValueError(f"expected one index list per frame ({nf} frames)")
+    parts, l_off = [], np.zeros(nf + 1, np.uint64)
+    for f, lst in enumerate(lists):
+        a = np.asarray(lst)
+        if a.size == 0:
+            a = a.reshape(0).astype(np.int64)
+        if a.ndim != 1 or a.dtype.kind not in "iu":
+            raise ValueError(f"lists[{f}] must be a 1-D integer array")
+        n_f = int(off[f + 1] - off[f])
+        if len(a) and (int(a.min()) < 0 or int(a.max()) >= n_f):
+            bad = int(a.min()) if int(a.min()) < 0 else int(a.max())
+            raise IndexError(f"frame {f}: index {bad} out of bounds for a frame with {n_f} points")
+        parts.append(a.astype(np.uint32))
+        l_off[f + 1] = l_off[f] + len(a)
+    idx = np.ascontiguousarray(np.concatenate(parts) if parts else np.zeros(0, np.uint32), np.uint32)
+    return idx, l_off
+
+
+class DeviceFrames:
+    """A batch of frames that lives in HBM: the frame-batch counterpart of DeviceCloud.  Every method runs the batch core
+    of the matching *_batch call and returns a new DeviceFrames (or host results); frame f of a result is what the
+    DeviceCloud method returns for frame f alone.  Indices in and out are frame-local."""
+
+    def __init__(self, handle, ctx: Context):
+        self._h = handle
+        self._ctx = ctx
+        ctx._clouds.add(self)
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass
+
+    @staticmethod
+    def from_numpy(points, frame_offsets: Sequence[int], ctx: Optional[Context] = None) -> "DeviceFrames":
+        """points: (N, 3), frame f = rows [frame_offsets[f], frame_offsets[f+1]).  The rows cross PCIe as they are and are
+        split into SoA on the device."""
+        pts, off = _batch_frames(points, frame_offsets)
+        if len(off) < 2:
+            raise ValueError("a batch holds at least one frame")
+        ctx = ctx or default_context()
+        h = C.c_void_p()
+        _ffi.check(_ffi.load().pcr_frames_upload_rows(ctx._h, pts.ctypes.data, _p(off, _ffi.u64p), len(off) - 1, C.byref(h)), ctx._h)
+        return DeviceFrames(h, ctx)
+
+    def free(self):
+        h, self._h = getattr(self, "_h", None), None
+        if h and self._ctx._h:  # a closed context has already freed its batches
+            _ffi.load().pcr_frames_free(h)
+
+    def _new(self, fn, *args) -> "DeviceFrames":
+        h = C.c_void_p()
+        _ffi.check(fn(self._h, *args, C.byref(h)), self._ctx._h)
+        return DeviceFrames(h, self._ctx)
+
+    @property
+    def n_frames(self) -> int:
+        return int(_ffi.load().pcr_frames_count(self._h))
+
+    @property
+    def offsets(self) -> np.ndarray:
+        off = np.zeros(self.n_frames + 1, np.uint64)
+        _ffi.check(_ffi.load().pcr_frames_offsets(self._h, _p(off, _ffi.u64p)), self._ctx._h)
+        return off
+
+    def len(self) -> int:
+        return int(_ffi.load().pcr_frames_len(self._h))
+
+    __len__ = len
+
+    def has_normals(self) -> bool:
+        return bool(_ffi.load().pcr_frames_has_normals(self._h))
+
+    def __repr__(self) -> str:
+        return f"DeviceFrames(frames={self.n_frames}, n={self.len()}, normals={self.has_normals()})"
+
+    def frame(self, f: int) -> DeviceCloud:
+        """Frame f as a DeviceCloud (a device copy, normals carried)."""
+        if not 0 <= int(f) < self.n_frames:
+            raise IndexError(f"frame {f} out of range ({self.n_frames} frames)")
+        h = C.c_void_p()
+        _ffi.check(_ffi.load().pcr_frames_frame(self._h, int(f), C.byref(h)), self._ctx._h)
+        return DeviceCloud(h, self._ctx)
+
+    def to_numpy(self):
+        """-> (points (N, 3) f32, offsets (F+1,) u64), one download."""
+        out = np.empty((self.len(), 3), np.float32)
+        _ffi.check(_ffi.load().pcr_frames_download_rows(self._h, out.ctypes.data, None), self._ctx._h)
+        return out, self.offsets
+
+    def normals_to_numpy(self) -> Optional[np.ndarray]:
+        if not self.has_normals():
+            return None
+        out = np.empty((self.len(), 3), np.float32)
+        _ffi.check(_ffi.load().pcr_frames_download_rows(self._h, None, out.ctypes.data), self._ctx._h)
+        return out
+
+    def _select(self, lists, invert: int) -> "DeviceFrames":
+        idx, l_off = _frame_lists(lists, self.offsets)
+        return self._new(_ffi.load().pcr_frames_select, _p(idx, _ffi.u32p), _p(l_off, _ffi.u64p), invert)
+
+    def select(self, lists) -> "DeviceFrames":
+        """lists: one frame-local index array per frame; frame f keeps its listed points in list order (duplicates too)."""
+        return self._select(lists, 0)
+
+    def select_inverse(self, lists) -> "DeviceFrames":
+        """Frame f keeps the points its list does not name, in their order."""
+        return self._select(lists, 1)
+
+    def voxel_downsample(self, voxel_size: float) -> "DeviceFrames":
+        if not math.isfinite(voxel_size) or voxel_size <= 0.0:
+            raise ValueError("voxel_size must be > 0 and finite")
+        return self._new(_ffi.load().pcr_frames_voxel_downsample, float(voxel_size))
+
+    def statistical_outlier_removal(self, k: int, std_mul: float) -> "DeviceFrames":
+        if not math.isfinite(std_mul) or std_mul < 0.0:  # crates/python/src/filters.rs:42-46
+            raise ValueError("std_mul must be >= 0 and finite")
+        return self._new(_ffi.load().pcr_frames_statistical_outlier_removal, int(k), float(std_mul))
+
+    def radius_outlier_removal(self, radius: float, min_neighbors: int) -> "DeviceFrames":
+        if not math.isfinite(radius) or radius <= 0.0:
+            raise ValueError("radius must be > 0 and finite")
+        return self._new(_ffi.load().pcr_frames_radius_outlier_removal, float(radius), int(min_neighbors))
+
+    def estimate_normals(self, k: int, viewpoint=(0.0, 0.0, 0.0)) -> "DeviceFrames":
+        vp = np.asarray(viewpoint, np.float32).reshape(3)
+        return self._new(_ffi.load().pcr_frames_estimate_normals, int(k), _p(vp, _ffi.f32p))
+
+    def sor_normals(self, k_sor: int, std_mul: float, k_normals: int, viewpoint=(0.0, 0.0, 0.0)) -> "DeviceFrames":
+        if not math.isfinite(std_mul) or std_mul < 0.0:
+            raise ValueError("std_mul must be >= 0 and finite")
+        vp = np.asarray(viewpoint, np.float32).reshape(3)
+        return self._new(_ffi.load().pcr_frames_sor_normals, int(k_sor), float(std_mul), int(k_normals), _p(vp, _ffi.f32p))
+
+    def ransac_plane_samples(self, distance_threshold: float, samples, outliers: bool = False):
+        """samples: one (m_f, 3) array of frame-local triples per frame.  -> one PlaneResult per frame, and with
+        outliers=True also the DeviceFrames of every frame's select_inverse(inliers), built on the device."""
+        off = self.offsets
+        smp, s_off = _frame_samples(samples, off)
+        nf = len(off) - 1
+        models = np.zeros((nf, 4), np.float32)
+        inl = np.zeros(max(int(off[-1]), 1), np.uint32)
+        inl_off = np.zeros(nf + 1, np.uint64)
+        h = C.c_void_p()
+        st = _ffi.load().pcr_frames_ransac_plane_samples(self._h, float(distance_threshold), _p(smp, _ffi.u32p), _p(s_off, _ffi.u64p),
+                                                         _p(models, _ffi.f32p), _p(inl, _ffi.u32p), _p(inl_off, _ffi.u64p),
+                                                         C.byref(h) if outliers else None)
+        _ffi.check(st, self._ctx._h)
+        res = [PlaneResult(models[f, :3], models[f, 3], inl[int(inl_off[f]):int(inl_off[f + 1])].tolist()) for f in range(nf)]
+        return (res, DeviceFrames(h, self._ctx)) if outliers else res
+
+    def ransac_plane(self, distance_threshold: float, iterations: int, seed=None, outliers: bool = False):
+        """Frame f's triples are draw_plane_samples(n_f, iterations, [seed, f]), as ransac_plane_batch draws them."""
+        off = self.offsets
+        samples = [draw_plane_samples(int(off[f + 1] - off[f]), iterations, None if seed is None else [seed, f]) for f in range(len(off) - 1)]
+        return self.ransac_plane_samples(distance_threshold, samples, outliers)
+
+    def cluster_arrays(self, distance_threshold: float, min_size: int, max_size: int):
+        """-> (cluster_offsets (F+1,) u64, offsets u32, indices u32), as cluster_arrays_batch."""
+        n, nf = self.len(), self.n_frames
+        offsets = np.zeros(n + 1, np.uint32)
+        idx = np.zeros(max(n, 1), np.uint32)
+        c_off = np.zeros(nf + 1, np.uint64)
+        st = _ffi.load().pcr_frames_euclidean_cluster(self._h, float(distance_threshold), int(min_size), int(max_size), _p(offsets, _ffi.u32p),
+                                                      _p(idx, _ffi.u32p), _p(c_off, _ffi.u64p))
+        _ffi.check(st, self._ctx._h)
+        k = int(c_off[-1])
+        return c_off, offsets[:k + 1].copy(), idx[:int(offsets[k])].copy()
+
+    def euclidean_cluster(self, distance_threshold: float, min_size: int, max_size: int) -> List[List[List[int]]]:
+        """-> one list of index lists per frame, each what DeviceCloud.euclidean_cluster returns for the frame alone."""
+        c_off, offsets, idx = self.cluster_arrays(distance_threshold, min_size, max_size)
+        return [[idx[offsets[c]:offsets[c + 1]].tolist() for c in range(int(c_off[f]), int(c_off[f + 1]))] for f in range(len(c_off) - 1)]
+
+    def _icp(self, fn, pairs, max_iterations, tolerance, max_correspondence_distance) -> List[IcpResult]:
+        prm = _icp_params(max_iterations, tolerance, max_correspondence_distance)
+        nf = self.n_frames
+        pr = np.asarray(pairs)
+        if pr.size == 0:
+            pr = pr.reshape(0, 2)
+        if pr.ndim != 2 or pr.shape[1] != 2 or (len(pr) and pr.dtype.kind not in "iu"):
+            raise ValueError("pairs must be an integer array of shape (P, 2): (source frame, target frame)")
+        if len(pr) and (pr.min() < 0 or pr.max() >= nf):
+            raise ValueError(f"pairs hold a frame id outside [0, {nf})")
+        pr = np.ascontiguousarray(pr, np.uint32)
+        res = (_ffi.IcpResultC * max(len(pr), 1))()
+        _ffi.check(fn(self._h, _p(pr, _ffi.u32p), len(pr), C.byref(prm), res), self._ctx._h)
+        return [IcpResult(res[i]) for i in range(len(pr))]
+
+    def icp_point_to_point(self, pairs, max_iterations: int = 50, tolerance: float = 1e-5,
+                           max_correspondence_distance: float = math.inf) -> List[IcpResult]:
+        """pairs: (P, 2) frame ids, pair p registers frame pairs[p][0] onto frame pairs[p][1] -> one IcpResult per pair."""
+        return self._icp(_ffi.load().pcr_frames_icp_point_to_point, pairs, max_iterations, tolerance, max_correspondence_distance)
+
+    def icp_point_to_plane(self, pairs, max_iterations: int = 50, tolerance: float = 1e-5,
+                           max_correspondence_distance: float = math.inf) -> List[IcpResult]:
+        """Point-to-plane form; the batch must carry normals (estimate_normals / sor_normals)."""
+        if not self.has_normals():  # crates/python/src/registration.rs:66-71
+            raise ValueError("point-to-plane ICP needs frames with normals. Use estimate_normals first.")
+        return self._icp(_ffi.load().pcr_frames_icp_point_to_plane, pairs, max_iterations, tolerance, max_correspondence_distance)

@@ -146,6 +146,29 @@ SIGNATURES = {
     "pcr_sor_normals_batch": (C.c_int, [vp, f32p, f32p, f32p, u64p, C.c_size_t, C.c_size_t, C.c_float, C.c_size_t, f32p, u8p, f32p, f32p, f32p, u64p]),
     "pcr_sor_normals_batch_rows": (C.c_int, [vp, f32p, u64p, C.c_size_t, C.c_size_t, C.c_float, C.c_size_t, f32p, u8p, f32p, u64p]),
     "pcr_sor_normals_batch_dev": (C.c_int, [vp, vp, vp, vp, u64p, C.c_size_t, C.c_size_t, C.c_float, C.c_size_t, f32p, vp, vp, vp, vp]),
+    "pcr_radius_outlier_batch": (C.c_int, [vp, f32p, f32p, f32p, u64p, C.c_size_t, C.c_float, C.c_size_t, u8p, u64p]),
+    "pcr_radius_outlier_batch_dev": (C.c_int, [vp, vp, vp, vp, u64p, C.c_size_t, C.c_float, C.c_size_t, vp]),
+    "pcr_frames_upload": (C.c_int, [vp, vp, vp, vp, u64p, C.c_size_t, C.POINTER(vp)]),
+    "pcr_frames_upload_rows": (C.c_int, [vp, vp, u64p, C.c_size_t, C.POINTER(vp)]),
+    "pcr_frames_free": (None, [vp]),
+    "pcr_frames_len": (C.c_size_t, [vp]),
+    "pcr_frames_count": (C.c_size_t, [vp]),
+    "pcr_frames_offsets": (C.c_int, [vp, u64p]),
+    "pcr_frames_has_normals": (C.c_int, [vp]),
+    "pcr_frames_device_pointers": (C.c_int, [vp] + [C.POINTER(vp)] * 6),
+    "pcr_frames_download": (C.c_int, [vp, vp, vp, vp, vp, vp, vp]),
+    "pcr_frames_download_rows": (C.c_int, [vp, vp, vp]),
+    "pcr_frames_frame": (C.c_int, [vp, C.c_size_t, C.POINTER(vp)]),
+    "pcr_frames_select": (C.c_int, [vp, u32p, u64p, C.c_int, C.POINTER(vp)]),
+    "pcr_frames_voxel_downsample": (C.c_int, [vp, C.c_float, C.POINTER(vp)]),
+    "pcr_frames_statistical_outlier_removal": (C.c_int, [vp, C.c_size_t, C.c_float, C.POINTER(vp)]),
+    "pcr_frames_radius_outlier_removal": (C.c_int, [vp, C.c_float, C.c_size_t, C.POINTER(vp)]),
+    "pcr_frames_estimate_normals": (C.c_int, [vp, C.c_size_t, f32p, C.POINTER(vp)]),
+    "pcr_frames_sor_normals": (C.c_int, [vp, C.c_size_t, C.c_float, C.c_size_t, f32p, C.POINTER(vp)]),
+    "pcr_frames_ransac_plane_samples": (C.c_int, [vp, C.c_float, u32p, u64p, f32p, u32p, u64p, C.POINTER(vp)]),
+    "pcr_frames_euclidean_cluster": (C.c_int, [vp, C.c_float, C.c_size_t, C.c_size_t, u32p, u32p, u64p]),
+    "pcr_frames_icp_point_to_point": (C.c_int, [vp, u32p, C.c_size_t, C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
+    "pcr_frames_icp_point_to_plane": (C.c_int, [vp, u32p, C.c_size_t, C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
 }
 
 _lib = None

@@ -687,14 +687,17 @@ __global__ void ror_mask_kernel(const uint32_t *__restrict__ counts, size_t n, u
 }
 }  // namespace pcr
 
-// keep mask + kept count of radius_outlier_removal on device arrays (radius_outlier.rs:4-18)
+// keep mask + kept count of radius_outlier_removal on device arrays (radius_outlier.rs:4-18).  frame_offsets (host,
+// n_frames + 1): a batch of frames back to back, every point counted only within its own frame; a batch never shards.
 static int ror_core(Ctx *c, const float *dx, const float *dy, const float *dz, size_t n, float radius, size_t min_neighbors,
-                    uint8_t *d_keep, unsigned long long *d_kept) {
+                    uint8_t *d_keep, unsigned long long *d_kept, const uint64_t *frame_offsets = nullptr, size_t n_frames = 1) {
     // cell size = radius: the search box spans at most 3 cells per axis
     const float saved = c->forced_cell;
     if (saved == 0.f && radius > 0.f && std::isfinite(radius)) c->forced_cell = radius;
     BuildOpts bo;
     bo.transient = true;
+    bo.n_frames = (int)n_frames;
+    bo.frame_offsets = frame_offsets;
     Index *ix = nullptr;
     int s = index_build_dev(c, dx, dy, dz, n, bo, &ix);
     c->forced_cell = saved;
@@ -705,7 +708,7 @@ static int ror_core(Ctx *c, const float *dx, const float *dy, const float *dz, s
     } g{ix};
     PCR_TRY(ensure(c, c->b_misc, n * sizeof(uint32_t)));
     uint32_t *d_cnt = (uint32_t *)c->b_misc.p;
-    if (query_sharding_active(c, ix)) {
+    if (!frame_offsets && query_sharding_active(c, ix)) {
         // the count kernel takes its queries in input order: this rank counts for the input range [b, e), the counts are
         // merged like every sharded result (zero elsewhere, integer sum over NCCL), the mask is computed by every rank
         const size_t b = n * (size_t)c->rank / (size_t)c->world, e = n * (size_t)(c->rank + 1) / (size_t)c->world;
@@ -1260,7 +1263,8 @@ int pcr_ransac_plane_samples_batch_dev(pcr_ctx *ctx, const float *d_x, const flo
                               inlier_offsets);
 }
 
-static int cluster_batch_entry(pcr_ctx *ctx, bool dev, const float *x, const float *y, const float *z, const uint64_t *frame_offsets,
+// in_dev: x, y, z are device pointers; dev: offsets and indices too (in_dev alone: the CSR is downloaded)
+static int cluster_batch_entry(pcr_ctx *ctx, bool in_dev, bool dev, const float *x, const float *y, const float *z, const uint64_t *frame_offsets,
                                size_t n_frames, float distance_threshold, size_t min_size, size_t max_size, uint32_t *offsets,
                                uint32_t *indices, uint64_t *cluster_offsets) {
     if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
@@ -1286,8 +1290,12 @@ static int cluster_batch_entry(pcr_ctx *ctx, bool dev, const float *x, const flo
     if (dev)
         return euclidean_cluster_batch_dev(c, x, y, z, frame_offsets, n_frames, distance_threshold, min_size, max_size, offsets, indices,
                                            cluster_offsets, &total);
-    float *dx, *dy, *dz;
-    PCR_TRY(stage_xyz(c, c->b_in, x, y, z, n, &dx, &dy, &dz));
+    const float *dx = x, *dy = y, *dz = z;
+    if (!in_dev) {
+        float *sx, *sy, *sz;
+        PCR_TRY(stage_xyz(c, c->b_in, x, y, z, n, &sx, &sy, &sz));
+        dx = sx, dy = sy, dz = sz;
+    }
     PCR_TRY(ensure(c, c->b_out, sizeof(uint32_t) * (2 * n + 1)));
     uint32_t *d_off = (uint32_t *)c->b_out.p, *d_idx = d_off + n + 1;
     PCR_TRY(euclidean_cluster_batch_dev(c, dx, dy, dz, frame_offsets, n_frames, distance_threshold, min_size, max_size, d_off, d_idx,
@@ -1305,13 +1313,13 @@ static int cluster_batch_entry(pcr_ctx *ctx, bool dev, const float *x, const flo
 int pcr_euclidean_cluster_batch(pcr_ctx *ctx, const float *x, const float *y, const float *z, const uint64_t *frame_offsets, size_t n_frames,
                                 float distance_threshold, size_t min_size, size_t max_size, uint32_t *offsets, uint32_t *indices,
                                 uint64_t *cluster_offsets) {
-    return cluster_batch_entry(ctx, false, x, y, z, frame_offsets, n_frames, distance_threshold, min_size, max_size, offsets, indices,
+    return cluster_batch_entry(ctx, false, false, x, y, z, frame_offsets, n_frames, distance_threshold, min_size, max_size, offsets, indices,
                                cluster_offsets);
 }
 int pcr_euclidean_cluster_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z, const uint64_t *frame_offsets,
                                     size_t n_frames, float distance_threshold, size_t min_size, size_t max_size, uint32_t *d_offsets,
                                     uint32_t *d_indices, uint64_t *cluster_offsets) {
-    return cluster_batch_entry(ctx, true, d_x, d_y, d_z, frame_offsets, n_frames, distance_threshold, min_size, max_size, d_offsets, d_indices,
+    return cluster_batch_entry(ctx, true, true, d_x, d_y, d_z, frame_offsets, n_frames, distance_threshold, min_size, max_size, d_offsets, d_indices,
                                cluster_offsets);
 }
 
@@ -1329,6 +1337,51 @@ int pcr_cluster_labels_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_
     DevSetter ds(c);
     return cluster_labels_batch_dev(c, d_x, d_y, d_z, frame_offsets, n_frames, distance_threshold, d_labels);
     PCR_API_END(c)
+}
+
+/* ---- batched radius outlier removal ------------------------------------------------------------------ */
+// One index over all frames (cell = radius, as for one cloud); every point counts only the points of its own frame.
+static int ror_batch_entry(pcr_ctx *ctx, bool dev, const float *x, const float *y, const float *z, const uint64_t *frame_offsets,
+                           size_t n_frames, float radius, size_t min_neighbors, uint8_t *keep, uint64_t *n_kept_per_frame) {
+    if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
+    Ctx *c = &ctx->c;
+    PCR_TRY(batch_offsets_check(c, frame_offsets, n_frames));
+    if (n_kept_per_frame)
+        for (size_t f = 0; f < n_frames; f++) n_kept_per_frame[f] = 0;
+    const size_t n = (size_t)frame_offsets[n_frames];
+    PCR_TRY(batch_size_check(c, n, n_frames));
+    if (n && (!x || !y || !z || !keep)) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    if (n == 0) return PCR_OK;
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    if (dev) {
+        PCR_TRY(ensure(c, c->b_small, 4096));
+        return ror_core(c, x, y, z, n, radius, min_neighbors, keep, (unsigned long long *)((char *)c->b_small.p + 1024), frame_offsets,
+                        n_frames);
+    }
+    float *dx, *dy, *dz;
+    PCR_TRY(stage_xyz(c, c->b_in, x, y, z, n, &dx, &dy, &dz));
+    const size_t o_kept = (n + 255) & ~(size_t)255;
+    PCR_TRY(ensure(c, c->b_out, o_kept + 64));
+    uint8_t *d_keep = (uint8_t *)c->b_out.p;
+    PCR_TRY(ror_core(c, dx, dy, dz, n, radius, min_neighbors, d_keep, (unsigned long long *)((char *)c->b_out.p + o_kept), frame_offsets,
+                     n_frames));
+    PCR_CUDA(c, cudaMemcpyAsync(keep, d_keep, n, cudaMemcpyDeviceToHost, c->stream));
+    PCR_CUDA(c, cudaStreamSynchronize(c->stream));
+    if (n_kept_per_frame)
+        for (size_t f = 0; f < n_frames; f++)
+            for (uint64_t i = frame_offsets[f]; i < frame_offsets[f + 1]; i++) n_kept_per_frame[f] += keep[i];
+    return PCR_OK;
+    PCR_API_END(c)
+}
+
+int pcr_radius_outlier_batch(pcr_ctx *ctx, const float *x, const float *y, const float *z, const uint64_t *frame_offsets, size_t n_frames,
+                             float radius, size_t min_neighbors, uint8_t *keep, uint64_t *n_kept_per_frame) {
+    return ror_batch_entry(ctx, false, x, y, z, frame_offsets, n_frames, radius, min_neighbors, keep, n_kept_per_frame);
+}
+int pcr_radius_outlier_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z, const uint64_t *frame_offsets,
+                                 size_t n_frames, float radius, size_t min_neighbors, uint8_t *d_keep) {
+    return ror_batch_entry(ctx, true, d_x, d_y, d_z, frame_offsets, n_frames, radius, min_neighbors, d_keep, nullptr);
 }
 
 /* ---- multi-frame batch ---------------------------------------------------------------------------- */
@@ -1627,6 +1680,21 @@ __global__ void gather_kernel(const float *__restrict__ src, size_t src_stride, 
     for (int a = 0; a < n_arrays; a++) dst[(size_t)a * dst_stride + t] = src[(size_t)a * src_stride + i];
 }
 
+// The first half of every compaction (a cloud's or a frame batch's): flags of the keep mask and their exclusive scan,
+// pos[i] = kept points before point i, pos[n] = kept points.  pos lives in b_list.  Frames are contiguous and the
+// compaction keeps the order, so one scan serves every frame of a batch: frame f starts at pos[frame_offsets[f]].
+int keep_scan(Ctx *c, const uint8_t *d_keep, size_t n, uint32_t **pos_out) {
+    // (measured and dropped: flags -> tile scan -> look-back -> scatter in ONE kernel: 10-13 us against 2.5 + 6.6 + 4.4 for the
+    // three launches of a compaction -- 58 tiles of eight items per thread leave the GPU two thirds empty -- and no gain on the step)
+    PCR_TRY(ensure(c, c->b_list, sizeof(uint32_t) * (n + 1)));
+    uint32_t *pos = (uint32_t *)c->b_list.p;
+    PCR_CUDA(c, launch_chained(mask_to_u32_kernel, dim3((unsigned)((n + 1 + 255) / 256)), dim3(256), 0, c->stream, d_keep, n, pos));
+    c->launches++;
+    PCR_TRY(exclusive_scan_u32_dev(c, pos, n + 1));
+    *pos_out = pos;
+    return PCR_OK;
+}
+
 // new cloud = the points of `in` with keep != 0.  `nrm` (optional): normals of the points of `in`, three rows
 // `nrm_stride` apart, for an `in` that carries none.  `known_m`: the number of kept points if the caller
 // already has it on the host (saves the round trip), else SIZE_MAX.
@@ -1634,13 +1702,8 @@ int cloud_compact(const pcr_cloud *in, const uint8_t *d_keep, pcr_cloud **out, c
                   size_t known_m = SIZE_MAX) {
     Ctx *c = &in->owner->c;
     const size_t n = in->n;
-    // (measured and dropped: flags -> tile scan -> look-back -> scatter in ONE kernel: 10-13 us against 2.5 + 6.6 + 4.4 for the
-    // three launches below -- 58 tiles of eight items per thread leave the GPU two thirds empty -- and no gain on the step)
-    PCR_TRY(ensure(c, c->b_list, sizeof(uint32_t) * (n + 1)));
-    uint32_t *pos = (uint32_t *)c->b_list.p;
-    PCR_CUDA(c, launch_chained(mask_to_u32_kernel, dim3((unsigned)((n + 1 + 255) / 256)), dim3(256), 0, c->stream, d_keep, n, pos));
-    c->launches++;
-    PCR_TRY(exclusive_scan_u32_dev(c, pos, n + 1));
+    uint32_t *pos = nullptr;
+    PCR_TRY(keep_scan(c, d_keep, n, &pos));
     size_t m = known_m;
     if (m == SIZE_MAX) {
         uint32_t *mail = (uint32_t *)c->pinned + 96;
@@ -2151,6 +2214,590 @@ int pcr_cloud_icp_point_to_plane(const pcr_cloud *source, const pcr_cloud *targe
         return fail(c, PCR_ERR_INVALID_ARG, "target cloud must have normals (call estimate_normals first)");
     return pcr_icp_point_to_plane_dev(source->owner, source->x(), source->y(), source->z(), source->n, target->x(), target->y(), target->z(),
                                       target->n, target->nx(), target->ny(), target->nz(), target->n, params, result);
+}
+
+}  // extern "C"
+
+/* ---- device-resident frame batches ----------------------------------------------------------------------
+ * F clouds back to back in one allocation, laid out like pcr_cloud (x | y | z [| nx | ny | nz], `stride` floats apart),
+ * then the frame offsets as the kernels read them (u32[F + 1]); the host keeps them as u64[F + 1].  Every method is a
+ * batch core of the raw-pointer calls, and the filters end in ONE compaction for all frames (keep_scan, then the new
+ * frame starts read off the scan, then compact_kernel): each frame's result is what the pcr_cloud method returns for it. */
+struct pcr_frames {
+    pcr_ctx *owner;
+    size_t n, stride;
+    float *base;
+    uint32_t *d_off;
+    bool has_normals;
+    std::vector<uint64_t> off;
+    size_t count() const { return off.size() - 1; }
+    float *x() const { return base; }
+    float *y() const { return base + stride; }
+    float *z() const { return base + 2 * stride; }
+    float *nx() const { return base + 3 * stride; }
+    float *ny() const { return base + 4 * stride; }
+    float *nz() const { return base + 5 * stride; }
+};
+
+namespace pcr {
+namespace {
+
+// A new batch of n points with the given frame offsets.  d_off_src: the same offsets as u32 on the device (copied from
+// there), else they are uploaded from `off`.
+int frames_alloc(pcr_ctx *ctx, size_t n, bool normals, std::vector<uint64_t> off, pcr_frames **out, const uint32_t *d_off_src = nullptr) {
+    Ctx *c = &ctx->c;
+    pcr_frames *fr = new (std::nothrow) pcr_frames();
+    if (!fr) return fail(c, PCR_ERR_OOM, "host allocation failed");
+    fr->owner = ctx;
+    fr->n = n;
+    fr->stride = std::max<size_t>((n + 63) & ~(size_t)63, 64);
+    fr->has_normals = normals;
+    fr->off = std::move(off);
+    fr->base = nullptr;
+    const size_t F = fr->count(), arrays = sizeof(float) * fr->stride * (normals ? 6 : 3);
+    cudaError_t e = cudaMallocAsync((void **)&fr->base, arrays + sizeof(uint32_t) * (F + 1), c->stream);
+    if (e == cudaSuccess) {
+        fr->d_off = (uint32_t *)((char *)fr->base + arrays);
+        if (d_off_src) {
+            e = cudaMemcpyAsync(fr->d_off, d_off_src, sizeof(uint32_t) * (F + 1), cudaMemcpyDeviceToDevice, c->stream);
+        } else {
+            std::vector<uint32_t> h(F + 1);
+            for (size_t f = 0; f <= F; f++) h[f] = (uint32_t)fr->off[f];
+            // (pageable source: the copy has taken the bytes when it returns)
+            e = cudaMemcpyAsync(fr->d_off, h.data(), sizeof(uint32_t) * (F + 1), cudaMemcpyHostToDevice, c->stream);
+        }
+    }
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        if (fr->base) cudaFreeAsync(fr->base, c->stream);
+        delete fr;
+        return fail(c, e == cudaErrorMemoryAllocation ? PCR_ERR_OOM : PCR_ERR_CUDA, "device allocation failed: %s", cudaGetErrorString(e));
+    }
+    *out = fr;
+    return PCR_OK;
+}
+
+// the compacted batch's frame f starts where the scan stands at the old start of frame f
+__global__ void frame_starts_kernel(const uint32_t *__restrict__ pos, const uint32_t *__restrict__ frame_off, int n_frames,
+                                    uint32_t *__restrict__ new_off) {
+    const int f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f <= n_frames) new_off[f] = pos[frame_off[f]];
+}
+
+// new batch = the points of `in` with keep != 0, frame by frame.  `nrm` (optional): normals of the points of `in`, three
+// rows `nrm_stride` apart, for an `in` that carries none.  One round trip: all F + 1 new offsets in one copy.
+int frames_compact(const pcr_frames *in, const uint8_t *d_keep, pcr_frames **out, const float *nrm = nullptr, size_t nrm_stride = 0) {
+    Ctx *c = &in->owner->c;
+    const size_t n = in->n, F = in->count();
+    uint32_t *pos = nullptr;
+    PCR_TRY(keep_scan(c, d_keep, n, &pos));
+    uint32_t *d_new = nullptr;
+    PCR_CUDA(c, cudaMallocAsync((void **)&d_new, sizeof(uint32_t) * (F + 1), c->stream));
+    struct G {
+        void *p;
+        cudaStream_t s;
+        ~G() { cudaFreeAsync(p, s); }
+    } g{d_new, c->stream};
+    frame_starts_kernel<<<(unsigned)((F + 1 + 255) / 256), 256, 0, c->stream>>>(pos, in->d_off, (int)F, d_new);
+    PCR_LAUNCH_CHECK(c);
+    PCR_TRY(ensure_pinned(c, sizeof(uint32_t) * (F + 1)));
+    uint32_t *mail = (uint32_t *)c->pinned;
+    PCR_CUDA(c, cudaMemcpyAsync(mail, d_new, sizeof(uint32_t) * (F + 1), cudaMemcpyDeviceToHost, c->stream));
+    PCR_CUDA(c, cudaStreamSynchronize(c->stream));
+    std::vector<uint64_t> off(F + 1);
+    for (size_t f = 0; f <= F; f++) off[f] = mail[f];
+    const size_t m = (size_t)off[F];
+    const bool with_normals = nrm || in->has_normals;
+    pcr_frames *tmp = nullptr;  // *out is set on success only
+    PCR_TRY(frames_alloc(in->owner, m, with_normals, std::move(off), &tmp, d_new));
+    if (m) {
+        const int n_a = nrm ? 3 : (in->has_normals ? 6 : 3), n_b = nrm ? 3 : 0;
+        const cudaError_t e = launch_chained(compact_kernel, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, c->stream, in->base, in->stride, n_a,
+                                             nrm, nrm_stride, n_b, n, pos, tmp->base, tmp->stride);
+        c->launches++;
+        if (e != cudaSuccess) {
+            pcr_frames_free(tmp);
+            return fail(c, PCR_ERR_CUDA, "kernel launch failed: %s (%s:%d)", cudaGetErrorString(e), __FILE__, __LINE__);
+        }
+    }
+    *out = tmp;
+    return PCR_OK;
+}
+
+// An empty batch with in's frame count: every frame empty (the SOR rule for k == 0).
+int frames_empty(const pcr_frames *in, bool normals, pcr_frames **out) {
+    return frames_alloc(in->owner, 0, normals, std::vector<uint64_t>(in->count() + 1, 0), out);
+}
+
+// Entry t of the frame-local lists (list f = [list_off[f], list_off[f+1])) names input point frame_off[f] + idx[t].
+__device__ __forceinline__ uint32_t list_point(const uint32_t *__restrict__ idx, const uint32_t *__restrict__ list_off,
+                                               const uint32_t *__restrict__ frame_off, int n_frames, uint32_t t) {
+    return frame_off[frame_of(list_off, n_frames, t)] + idx[t];
+}
+
+__global__ void frames_gather_kernel(const float *__restrict__ src, size_t src_stride, int n_arrays, const uint32_t *__restrict__ idx,
+                                     const uint32_t *__restrict__ list_off, const uint32_t *__restrict__ frame_off, int n_frames, size_t m,
+                                     float *__restrict__ dst, size_t dst_stride) {
+    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= m) return;
+    const uint32_t i = list_point(idx, list_off, frame_off, n_frames, (uint32_t)t);
+    for (int a = 0; a < n_arrays; a++) dst[(size_t)a * dst_stride + t] = src[(size_t)a * src_stride + i];
+}
+
+// keep[listed point] = 0 (select_inverse: the mask starts all ones)
+__global__ void frames_unkeep_kernel(const uint32_t *__restrict__ idx, const uint32_t *__restrict__ list_off,
+                                     const uint32_t *__restrict__ frame_off, int n_frames, size_t m, uint8_t *__restrict__ keep) {
+    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t < m) keep[list_point(idx, list_off, frame_off, n_frames, (uint32_t)t)] = 0;
+}
+
+// select_inverse of frame-local DEVICE lists with HOST list offsets (in bounds, checked by the caller or by construction)
+int frames_select_inverse_dev(const pcr_frames *in, const uint32_t *d_idx, const std::vector<uint64_t> &list_off, pcr_frames **out) {
+    Ctx *c = &in->owner->c;
+    const size_t n = in->n, F = in->count(), m = (size_t)list_off[F];
+    // keep u8[n] (rounded up to 4 bytes) | list offsets u32[F + 1]
+    const size_t o_loff = (n + 3) & ~(size_t)3;
+    uint8_t *d_keep = nullptr;
+    PCR_CUDA(c, cudaMallocAsync((void **)&d_keep, o_loff + sizeof(uint32_t) * (F + 1), c->stream));
+    struct G {
+        void *p;
+        cudaStream_t s;
+        ~G() { cudaFreeAsync(p, s); }
+    } g{d_keep, c->stream};
+    uint32_t *d_loff = (uint32_t *)(d_keep + o_loff);
+    if (n) PCR_CUDA(c, cudaMemsetAsync(d_keep, 1, n, c->stream));
+    if (m) {
+        std::vector<uint32_t> h(F + 1);
+        for (size_t f = 0; f <= F; f++) h[f] = (uint32_t)list_off[f];
+        PCR_CUDA(c, cudaMemcpyAsync(d_loff, h.data(), sizeof(uint32_t) * (F + 1), cudaMemcpyHostToDevice, c->stream));
+        frames_unkeep_kernel<<<(unsigned)((m + 255) / 256), 256, 0, c->stream>>>(d_idx, d_loff, in->d_off, (int)F, m, d_keep);
+        PCR_LAUNCH_CHECK(c);
+    }
+    return frames_compact(in, d_keep, out);
+}
+
+}  // namespace
+}  // namespace pcr
+
+extern "C" {
+
+#define PCR_FRAMES_CHECK(fr)                                                                  \
+    if (!(fr) || !(fr)->owner) return fail(nullptr, PCR_ERR_INVALID_ARG, "frames is NULL");   \
+    Ctx *c = &(fr)->owner->c;
+
+// offsets, sizes and the output handle of an upload; n receives the point count
+static int frames_upload_check(Ctx *c, const uint64_t *frame_offsets, size_t n_frames, pcr_frames **out, size_t *n) {
+    if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    *out = nullptr;
+    if (n_frames == 0) return fail(c, PCR_ERR_INVALID_ARG, "a batch holds at least one frame");
+    PCR_TRY(batch_offsets_check(c, frame_offsets, n_frames));
+    *n = (size_t)frame_offsets[n_frames];
+    return batch_size_check(c, *n, n_frames);
+}
+
+int pcr_frames_upload(pcr_ctx *ctx, const float *x, const float *y, const float *z, const uint64_t *frame_offsets, size_t n_frames,
+                      pcr_frames **out) {
+    if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
+    Ctx *c = &ctx->c;
+    size_t n = 0;
+    PCR_TRY(frames_upload_check(c, frame_offsets, n_frames, out, &n));
+    if (n && (!x || !y || !z)) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    pcr_frames *fr = nullptr;
+    PCR_TRY(frames_alloc(ctx, n, false, std::vector<uint64_t>(frame_offsets, frame_offsets + n_frames + 1), &fr));
+    cudaError_t e = cudaSuccess;
+    if (n) {
+        e = cudaMemcpyAsync(fr->x(), x, sizeof(float) * n, cudaMemcpyHostToDevice, c->stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(fr->y(), y, sizeof(float) * n, cudaMemcpyHostToDevice, c->stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(fr->z(), z, sizeof(float) * n, cudaMemcpyHostToDevice, c->stream);
+    }
+    const cudaError_t es = cudaStreamSynchronize(c->stream);  // the caller's buffers are free again on return
+    if (e == cudaSuccess) e = es;
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        pcr_frames_free(fr);
+        return fail(c, PCR_ERR_CUDA, "upload failed: %s", cudaGetErrorString(e));
+    }
+    *out = fr;
+    return PCR_OK;
+    PCR_API_END(c)
+}
+
+// row-major (N, 3): one contiguous transfer, split on the device (as pcr_cloud_upload_rows)
+int pcr_frames_upload_rows(pcr_ctx *ctx, const float *xyz, const uint64_t *frame_offsets, size_t n_frames, pcr_frames **out) {
+    if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
+    Ctx *c = &ctx->c;
+    size_t n = 0;
+    PCR_TRY(frames_upload_check(c, frame_offsets, n_frames, out, &n));
+    if (n && !xyz) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    pcr_frames *fr = nullptr;
+    PCR_TRY(frames_alloc(ctx, n, false, std::vector<uint64_t>(frame_offsets, frame_offsets + n_frames + 1), &fr));
+    cudaError_t e = cudaSuccess;
+    if (n) {
+        if (ensure(c, c->b_in, sizeof(float) * 3 * n) != PCR_OK) {
+            pcr_frames_free(fr);
+            return PCR_ERR_CUDA;
+        }
+        e = cudaMemcpyAsync(c->b_in.p, xyz, sizeof(float) * 3 * n, cudaMemcpyHostToDevice, c->stream);
+        if (e == cudaSuccess) {
+            rows_to_soa_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>((const float *)c->b_in.p, n, fr->base, fr->stride);
+            c->launches++;
+            e = cudaGetLastError();
+        }
+    }
+    const cudaError_t es = cudaStreamSynchronize(c->stream);
+    if (e == cudaSuccess) e = es;
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        pcr_frames_free(fr);
+        return fail(c, PCR_ERR_CUDA, "upload failed: %s", cudaGetErrorString(e));
+    }
+    *out = fr;
+    return PCR_OK;
+    PCR_API_END(c)
+}
+
+void pcr_frames_free(pcr_frames *frames) {
+    if (!frames) return;
+    if (frames->base && frames->owner) {
+        DevSetter ds(&frames->owner->c);
+        cudaFreeAsync(frames->base, frames->owner->c.stream);
+    }
+    delete frames;
+}
+
+size_t pcr_frames_len(const pcr_frames *frames) { return frames ? frames->n : 0; }
+size_t pcr_frames_count(const pcr_frames *frames) { return frames ? frames->count() : 0; }
+int pcr_frames_has_normals(const pcr_frames *frames) { return frames && frames->has_normals ? 1 : 0; }
+
+int pcr_frames_offsets(const pcr_frames *frames, uint64_t *out) {
+    PCR_FRAMES_CHECK(frames)
+    if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    std::copy(frames->off.begin(), frames->off.end(), out);
+    return PCR_OK;
+}
+
+int pcr_frames_device_pointers(const pcr_frames *frames, const float **d_x, const float **d_y, const float **d_z, const float **d_nx,
+                               const float **d_ny, const float **d_nz) {
+    PCR_FRAMES_CHECK(frames)
+    (void)c;
+    if (d_x) *d_x = frames->x();
+    if (d_y) *d_y = frames->y();
+    if (d_z) *d_z = frames->z();
+    if (d_nx) *d_nx = frames->has_normals ? frames->nx() : nullptr;
+    if (d_ny) *d_ny = frames->has_normals ? frames->ny() : nullptr;
+    if (d_nz) *d_nz = frames->has_normals ? frames->nz() : nullptr;
+    return PCR_OK;
+}
+
+int pcr_frames_download(const pcr_frames *frames, float *x, float *y, float *z, float *nx, float *ny, float *nz) {
+    PCR_FRAMES_CHECK(frames)
+    const bool want_n = nx || ny || nz;
+    if (want_n && !frames->has_normals) return fail(c, PCR_ERR_INVALID_ARG, "the frames have no normals");
+    const size_t n = frames->n;
+    if (n && (!x || !y || !z || (want_n && (!nx || !ny || !nz)))) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    if (!n) return PCR_OK;
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    float *dst[6] = {x, y, z, nx, ny, nz};
+    for (int a = 0; a < (want_n ? 6 : 3); a++)
+        PCR_CUDA(c, cudaMemcpyAsync(dst[a], frames->base + (size_t)a * frames->stride, sizeof(float) * n, cudaMemcpyDeviceToHost, c->stream));
+    PCR_CUDA(c, cudaStreamSynchronize(c->stream));
+    return PCR_OK;
+    PCR_API_END(c)
+}
+
+int pcr_frames_download_rows(const pcr_frames *frames, float *xyz, float *normals) {
+    PCR_FRAMES_CHECK(frames)
+    if (normals && !frames->has_normals) return fail(c, PCR_ERR_INVALID_ARG, "the frames have no normals");
+    if (frames->n && !xyz && !normals) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    if (!frames->n) return PCR_OK;
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    const size_t n = frames->n, row = sizeof(float) * 3 * n;
+    PCR_TRY(ensure(c, c->b_out, 2 * row));
+    float *d_xyz = (float *)c->b_out.p, *d_nrm = d_xyz + 3 * n;
+    const unsigned blocks = (unsigned)((n + 255) / 256);
+    if (xyz) {
+        soa_to_rows_kernel<<<blocks, 256, 0, c->stream>>>(frames->base, frames->stride, n, d_xyz);
+        PCR_LAUNCH_CHECK(c);
+        PCR_CUDA(c, cudaMemcpyAsync(xyz, d_xyz, row, cudaMemcpyDeviceToHost, c->stream));
+    }
+    if (normals) {
+        soa_to_rows_kernel<<<blocks, 256, 0, c->stream>>>(frames->nx(), frames->stride, n, d_nrm);
+        PCR_LAUNCH_CHECK(c);
+        PCR_CUDA(c, cudaMemcpyAsync(normals, d_nrm, row, cudaMemcpyDeviceToHost, c->stream));
+    }
+    PCR_CUDA(c, cudaStreamSynchronize(c->stream));
+    return PCR_OK;
+    PCR_API_END(c)
+}
+
+int pcr_frames_frame(const pcr_frames *frames, size_t f, pcr_cloud **out) {
+    PCR_FRAMES_CHECK(frames)
+    if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    *out = nullptr;
+    if (f >= frames->count()) return fail(c, PCR_ERR_INVALID_ARG, "frame %zu out of range (%zu frames)", f, frames->count());
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    const size_t b = (size_t)frames->off[f], m = (size_t)frames->off[f + 1] - b;
+    pcr_cloud *cl = nullptr;
+    PCR_TRY(cloud_alloc(frames->owner, m, frames->has_normals, &cl));
+    for (int a = 0; m && a < (frames->has_normals ? 6 : 3); a++) {
+        const cudaError_t e = cudaMemcpyAsync(cl->base + (size_t)a * cl->stride, frames->base + (size_t)a * frames->stride + b, sizeof(float) * m,
+                                              cudaMemcpyDeviceToDevice, c->stream);
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            pcr_cloud_free(cl);
+            return fail(c, PCR_ERR_CUDA, "copy failed: %s", cudaGetErrorString(e));
+        }
+    }
+    *out = cl;
+    return PCR_OK;
+    PCR_API_END(c)
+}
+
+int pcr_frames_select(const pcr_frames *frames, const uint32_t *indices, const uint64_t *index_offsets, int invert, pcr_frames **out) {
+    PCR_FRAMES_CHECK(frames)
+    if (!out || !index_offsets) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    *out = nullptr;
+    const size_t F = frames->count();
+    if (index_offsets[0] != 0) return fail(c, PCR_ERR_INVALID_ARG, "index_offsets must start at 0");
+    for (size_t f = 0; f < F; f++)
+        if (index_offsets[f + 1] < index_offsets[f]) return fail(c, PCR_ERR_INVALID_ARG, "index_offsets must be non-decreasing");
+    const size_t m = (size_t)index_offsets[F];
+    if (m && !indices) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    if (m > 0x7fffffffull) return fail(c, PCR_ERR_UNSUPPORTED, "at most 2^31 - 1 listed indices per call");
+    for (size_t f = 0; f < F; f++) {  // cloud.rs:109: select panics on an out-of-bounds index
+        const uint64_t n_f = frames->off[f + 1] - frames->off[f];
+        for (uint64_t t = index_offsets[f]; t < index_offsets[f + 1]; t++)
+            if (indices[t] >= n_f)
+                return fail(c, PCR_ERR_INVALID_ARG, "frame %zu: index %u out of bounds for a frame with %llu points", f, indices[t],
+                            (unsigned long long)n_f);
+    }
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    std::vector<uint64_t> loff(index_offsets, index_offsets + F + 1);
+    uint32_t *d_idx = nullptr;
+    PCR_CUDA(c, cudaMallocAsync((void **)&d_idx, sizeof(uint32_t) * std::max<size_t>(m, 1), c->stream));
+    struct G {
+        void *p;
+        cudaStream_t s;
+        ~G() { cudaFreeAsync(p, s); }
+    } g{d_idx, c->stream};
+    if (m) PCR_CUDA(c, cudaMemcpyAsync(d_idx, indices, sizeof(uint32_t) * m, cudaMemcpyHostToDevice, c->stream));
+    if (invert) return frames_select_inverse_dev(frames, d_idx, loff, out);
+    pcr_frames *tmp = nullptr;
+    PCR_TRY(frames_alloc(frames->owner, m, frames->has_normals, loff, &tmp));
+    if (m) {
+        // the gather reads the list offsets as u32: the new batch's own device offsets are exactly those
+        frames_gather_kernel<<<(unsigned)((m + 255) / 256), 256, 0, c->stream>>>(frames->base, frames->stride, frames->has_normals ? 6 : 3, d_idx,
+                                                                                 tmp->d_off, frames->d_off, (int)F, m, tmp->base, tmp->stride);
+        const cudaError_t e = cudaGetLastError();
+        c->launches++;
+        if (e != cudaSuccess) {
+            pcr_frames_free(tmp);
+            return fail(c, PCR_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(e));
+        }
+    }
+    // the caller's index array is free again on return (a pinned one is read by the copy while it runs)
+    const cudaError_t es = cudaStreamSynchronize(c->stream);
+    if (es != cudaSuccess) {
+        cudaGetLastError();
+        pcr_frames_free(tmp);
+        return fail(c, PCR_ERR_CUDA, "select failed: %s", cudaGetErrorString(es));
+    }
+    *out = tmp;
+    return PCR_OK;
+    PCR_API_END(c)
+}
+
+int pcr_frames_voxel_downsample(const pcr_frames *frames, float voxel_size, pcr_frames **out) {
+    PCR_FRAMES_CHECK(frames)
+    if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    *out = nullptr;
+    if (!std::isfinite(voxel_size) || !(voxel_size > 0.f)) return fail(c, PCR_ERR_INVALID_ARG, "voxel_size must be > 0 and finite");
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    const size_t F = frames->count();
+    pcr_frames *tmp = nullptr;  // voxel_downsample.rs:64: xyz only; sized for the input, then shrunk to the voxels
+    PCR_TRY(frames_alloc(frames->owner, frames->n, false, std::vector<uint64_t>(F + 1, 0), &tmp));
+    std::vector<uint64_t> out_off(F + 1, 0);
+    const int s = voxel_batch_entry(frames->owner, true, frames->x(), frames->y(), frames->z(), frames->off.data(), F, voxel_size, tmp->x(),
+                                    tmp->y(), tmp->z(), out_off.data());
+    if (s != PCR_OK) {
+        pcr_frames_free(tmp);
+        return s;
+    }
+    std::vector<uint32_t> h(F + 1);
+    for (size_t f = 0; f <= F; f++) h[f] = (uint32_t)out_off[f];
+    const cudaError_t e = cudaMemcpyAsync(tmp->d_off, h.data(), sizeof(uint32_t) * (F + 1), cudaMemcpyHostToDevice, c->stream);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        pcr_frames_free(tmp);
+        return fail(c, PCR_ERR_CUDA, "copy failed: %s", cudaGetErrorString(e));
+    }
+    tmp->n = (size_t)out_off[F];  // (the allocation keeps its original stride)
+    tmp->off = std::move(out_off);
+    *out = tmp;
+    return PCR_OK;
+    PCR_API_END(c)
+}
+
+int pcr_frames_statistical_outlier_removal(const pcr_frames *frames, size_t k, float std_mul, pcr_frames **out) {
+    PCR_FRAMES_CHECK(frames)
+    if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    *out = nullptr;
+    if (!std::isfinite(std_mul) || std_mul < 0.f) return fail(c, PCR_ERR_INVALID_ARG, "std_mul must be >= 0 and finite");
+    if (k + 1 > PCR_MAX_K) return fail(c, PCR_ERR_UNSUPPORTED, "k = %zu exceeds PCR_MAX_K - 1", k);
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    const size_t n = frames->n;
+    if (n == 0 || k == 0) return frames_empty(frames, false, out);  // statistical_outlier.rs:5-7: PointCloud::new()
+    uint8_t *d_keep = nullptr;
+    PCR_CUDA(c, cudaMallocAsync((void **)&d_keep, n, c->stream));
+    struct G {
+        void *p;
+        cudaStream_t s;
+        ~G() { cudaFreeAsync(p, s); }
+    } g{d_keep, c->stream};
+    const float vp0[3] = {0.f, 0.f, 0.f};
+    PCR_TRY(pcr_sor_normals_batch_dev(frames->owner, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(), k, std_mul, 0,
+                                      vp0, d_keep, nullptr, nullptr, nullptr));
+    return frames_compact(frames, d_keep, out);  // :68 select
+    PCR_API_END(c)
+}
+
+int pcr_frames_radius_outlier_removal(const pcr_frames *frames, float radius, size_t min_neighbors, pcr_frames **out) {
+    PCR_FRAMES_CHECK(frames)
+    if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    *out = nullptr;
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    const size_t n = frames->n;
+    if (n == 0) return frames_empty(frames, frames->has_normals, out);
+    uint8_t *d_keep = nullptr;
+    PCR_CUDA(c, cudaMallocAsync((void **)&d_keep, n, c->stream));
+    struct G {
+        void *p;
+        cudaStream_t s;
+        ~G() { cudaFreeAsync(p, s); }
+    } g{d_keep, c->stream};
+    PCR_TRY(pcr_radius_outlier_batch_dev(frames->owner, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(), radius,
+                                         min_neighbors, d_keep));
+    return frames_compact(frames, d_keep, out);
+    PCR_API_END(c)
+}
+
+int pcr_frames_estimate_normals(const pcr_frames *frames, size_t k, const float viewpoint[3], pcr_frames **out) {
+    PCR_FRAMES_CHECK(frames)
+    if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    *out = nullptr;
+    if (k == 0) return fail(c, PCR_ERR_INVALID_ARG, "k must be > 0");  // as pcr_cloud_estimate_normals
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    const size_t n = frames->n;
+    pcr_frames *res = nullptr;
+    PCR_TRY(frames_alloc(frames->owner, n, true, frames->off, &res, frames->d_off));
+    if (n) {
+        for (int a = 0; a < 3; a++)
+            cudaMemcpyAsync(res->base + (size_t)a * res->stride, frames->base + (size_t)a * frames->stride, sizeof(float) * n, cudaMemcpyDeviceToDevice,
+                            c->stream);
+        const float vp0[3] = {0.f, 0.f, 0.f};  // estimate.rs:13-15
+        const int s = pcr_estimate_normals_batch_dev(frames->owner, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(), k,
+                                                     viewpoint ? viewpoint : vp0, res->nx(), res->ny(), res->nz());
+        if (s != PCR_OK) {
+            pcr_frames_free(res);
+            return s;
+        }
+    }
+    *out = res;
+    return PCR_OK;
+    PCR_API_END(c)
+}
+
+int pcr_frames_sor_normals(const pcr_frames *frames, size_t k_sor, float std_mul, size_t k_normals, const float viewpoint[3],
+                           pcr_frames **out) {
+    PCR_FRAMES_CHECK(frames)
+    if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    *out = nullptr;
+    if (k_normals == 0) return fail(c, PCR_ERR_INVALID_ARG, "k_normals must be > 0");
+    if (!std::isfinite(std_mul) || std_mul < 0.f) return fail(c, PCR_ERR_INVALID_ARG, "std_mul must be >= 0 and finite");
+    if (k_sor + 1 > PCR_MAX_K || k_normals > PCR_MAX_K) return fail(c, PCR_ERR_UNSUPPORTED, "k exceeds PCR_MAX_K");
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    const size_t n = frames->n;
+    if (n == 0 || k_sor == 0) return frames_empty(frames, true, out);  // statistical_outlier.rs:5-7
+    // normals by input index go to a scratch block; the kept points and their normals are compacted together
+    const size_t stride = (n + 63) & ~(size_t)63;
+    float *d_nrm = nullptr;
+    PCR_CUDA(c, cudaMallocAsync((void **)&d_nrm, sizeof(float) * 3 * stride + n, c->stream));
+    struct G {
+        void *p;
+        cudaStream_t s;
+        ~G() { cudaFreeAsync(p, s); }
+    } g{d_nrm, c->stream};
+    uint8_t *d_keep = (uint8_t *)(d_nrm + 3 * stride);
+    const float vp0[3] = {0.f, 0.f, 0.f};
+    PCR_TRY(pcr_sor_normals_batch_dev(frames->owner, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(), k_sor, std_mul,
+                                      k_normals, viewpoint ? viewpoint : vp0, d_keep, d_nrm, d_nrm + stride, d_nrm + 2 * stride));
+    return frames_compact(frames, d_keep, out, d_nrm, stride);
+    PCR_API_END(c)
+}
+
+int pcr_frames_ransac_plane_samples(const pcr_frames *frames, float distance_threshold, const uint32_t *samples, const uint64_t *sample_offsets,
+                                    float *models, uint32_t *inliers, uint64_t *inlier_offsets, pcr_frames **outliers) {
+    PCR_FRAMES_CHECK(frames)
+    if (outliers) *outliers = nullptr;
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    const size_t n = frames->n, F = frames->count();
+    uint32_t *d_inl = nullptr;
+    PCR_CUDA(c, cudaMallocAsync((void **)&d_inl, sizeof(uint32_t) * std::max<size_t>(n, 1), c->stream));
+    struct G {
+        void *p;
+        cudaStream_t s;
+        ~G() { cudaFreeAsync(p, s); }
+    } g{d_inl, c->stream};
+    PCR_TRY(ransac_batch_entry(frames->owner, true, frames->x(), frames->y(), frames->z(), frames->off.data(), F, distance_threshold, samples,
+                               sample_offsets, models, d_inl, inlier_offsets));
+    const size_t k = (size_t)inlier_offsets[F];
+    if (inliers && k) {
+        PCR_CUDA(c, cudaMemcpyAsync(inliers, d_inl, sizeof(uint32_t) * k, cudaMemcpyDeviceToHost, c->stream));
+        PCR_CUDA(c, cudaStreamSynchronize(c->stream));
+    }
+    if (outliers)  // ransac_plane.rs's inliers are in bounds by construction: straight to the device select_inverse
+        return frames_select_inverse_dev(frames, d_inl, std::vector<uint64_t>(inlier_offsets, inlier_offsets + F + 1), outliers);
+    return PCR_OK;
+    PCR_API_END(c)
+}
+
+int pcr_frames_euclidean_cluster(const pcr_frames *frames, float distance_threshold, size_t min_size, size_t max_size, uint32_t *offsets,
+                                 uint32_t *indices, uint64_t *cluster_offsets) {
+    PCR_FRAMES_CHECK(frames)
+    (void)c;
+    return cluster_batch_entry(frames->owner, true, false, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(),
+                               distance_threshold, min_size, max_size, offsets, indices, cluster_offsets);
+}
+
+int pcr_frames_icp_point_to_point(const pcr_frames *frames, const uint32_t *pairs, size_t n_pairs, const pcr_icp_params *params,
+                                  pcr_icp_result *results) {
+    PCR_FRAMES_CHECK(frames)
+    (void)c;
+    return icp_batch_entry(frames->owner, true, false, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(), nullptr, nullptr,
+                           nullptr, 0, pairs, n_pairs, params, results);
+}
+
+int pcr_frames_icp_point_to_plane(const pcr_frames *frames, const uint32_t *pairs, size_t n_pairs, const pcr_icp_params *params,
+                                  pcr_icp_result *results) {
+    PCR_FRAMES_CHECK(frames)
+    if (!frames->has_normals)  // crates/python/src/registration.rs:80-86
+        return fail(c, PCR_ERR_INVALID_ARG, "point-to-plane ICP needs frames with normals (call estimate_normals first)");
+    return icp_batch_entry(frames->owner, true, true, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(), frames->nx(),
+                           frames->ny(), frames->nz(), frames->n, pairs, n_pairs, params, results);
 }
 
 }  // extern "C"

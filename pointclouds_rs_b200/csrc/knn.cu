@@ -1091,16 +1091,19 @@ __global__ void fill_f32_kernel(float *__restrict__ p, size_t n, float v) {
 // d^2 <= r*r with r*r rounded in f32 (kdtree.rs:114,127).  Cells are taken from the box
 // [q - r', q + r'] with r' = sqrt(r2) * (1 + 1e-6): a point that passes the f32 test is at most a
 // few ulp further than sqrt(r2) on any axis.
-template <bool kFill>
+// kFrames (batch): the queries are the input points of a multi-frame index, query i = point i, and each is searched
+// only in the grid of its own frame.  The single-frame calls leave frame_in_off / n_frames unset.
+template <bool kFill, bool kFrames = false>
 __global__ void __launch_bounds__(256) radius_kernel(const GridDesc *__restrict__ grids,
                                                      const uint32_t *__restrict__ cell_start,
                                                      const float4 *__restrict__ sorted, const float *__restrict__ qx,
                                                      const float *__restrict__ qy, const float *__restrict__ qz, size_t nq,
                                                      float radius, uint32_t *__restrict__ counts,
-                                                     const uint64_t *__restrict__ offsets, uint32_t *__restrict__ out_idx) {
+                                                     const uint64_t *__restrict__ offsets, uint32_t *__restrict__ out_idx,
+                                                     const uint32_t *__restrict__ frame_in_off = nullptr, int n_frames = 1) {
     size_t qi = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (qi >= nq) return;
-    const GridDesc g = grids[0];
+    const GridDesc g = grids[kFrames ? frame_of(frame_in_off, n_frames, (uint32_t)qi) : 0];
     float x = qx[qi], y = qy[qi], z = qz[qi];
     uint32_t cnt = 0;
     uint32_t *dst = kFill ? out_idx + offsets[qi] : nullptr;
@@ -2036,7 +2039,14 @@ int radius_count_dev(Index *ix, const float *dqx, const float *dqy, const float 
                      uint32_t *d_counts) {
     Ctx *ctx = ix->ctx;
     if (nq == 0) return PCR_OK;
-    if (ix->n_frames != 1) return fail(ctx, PCR_ERR_UNSUPPORTED, "radius queries need a single-frame index");
+    if (ix->n_frames != 1) {  // a batch: every indexed point counts its neighbours inside its own frame
+        if (nq != ix->n) return fail(ctx, PCR_ERR_UNSUPPORTED, "radius queries on a multi-frame index must be its own points");
+        radius_kernel<false, true><<<(unsigned)((nq + 255) / 256), 256, 0, ctx->stream>>>(ix->grids, ix->cell_start, ix->sorted, dqx, dqy, dqz, nq,
+                                                                                          radius, d_counts, nullptr, nullptr, ix->frame_in_off,
+                                                                                          ix->n_frames);
+        PCR_LAUNCH_CHECK(ctx);
+        return PCR_OK;
+    }
     radius_kernel<false><<<(unsigned)((nq + 255) / 256), 256, 0, ctx->stream>>>(ix->grids, ix->cell_start, ix->sorted, dqx, dqy,
                                                                                 dqz, nq, radius, d_counts, nullptr, nullptr);
     PCR_LAUNCH_CHECK(ctx);

@@ -291,6 +291,8 @@ int index_shard_queries(Index *ix);
 // coordinates become NaN) and makes later-built levels skip them: the index of the SOR pass is
 // reused for the normals of the kept points without a rebuild.
 int index_apply_mask_dev(Index *ix, const uint8_t *d_keep);
+// On a multi-frame index the queries must be the indexed points themselves (query i = input point i), each counted in
+// its own frame only.
 int radius_count_dev(Index *ix, const float *dqx, const float *dqy, const float *dqz, size_t nq,
                      float radius, uint32_t *d_counts);
 int radius_fill_dev(Index *ix, const float *dqx, const float *dqy, const float *dqz, size_t nq,
