@@ -25,6 +25,8 @@
  *                               (examples/python/kitti_obstacle_detection.py:87-122)
  *   pcr_radius_outlier_batch    radius_outlier_removal of many frames per call
  *   pcr_frames_*                a batch of frames kept in HBM between those calls (the batch form of pcr_cloud_*)
+ *   pcr_index_build_batch / pcr_knn_batch / pcr_radius_*_batch / pcr_find_correspondences_batch
+ *                               the KdTree queries of many frames per call, each frame searched alone
  *
  * The reference calls its kd-tree once per point inside serial loops; a per-query C call would be
  * useless on a GPU, so the boundary is BATCHED and sits one level up: it replaces the bodies of the
@@ -183,6 +185,55 @@ int pcr_radius_count(pcr_index *index, const float *qx, const float *qy, const f
  * PCR_ERR_CAPACITY is returned (call again with a larger buffer). */
 int pcr_radius_search(pcr_index *index, const float *qx, const float *qy, const float *qz, size_t nq,
                       float radius, uint64_t *offsets, uint32_t *idx, size_t cap, size_t *total);
+
+/* Batch index: the KdTree queries of many frames per call.  The index is built over F frames back to back, frame f =
+ * points [frame_offsets[f], frame_offsets[f+1]) (HOST, n_frames + 1 entries, as in the other batch calls), and queried
+ * with frames of queries back to back, query frame f = queries [query_offsets[f], query_offsets[f+1]) (HOST, the index's
+ * n_frames + 1 entries).  Query frame f is searched in index frame f only, and its results are bit for bit what the
+ * single call returns for index frame f alone (pcr_index_build on that frame) and the queries of frame f: KNN rows
+ * (indices, distances, counts, padding), radius counts, ascending radius CSR rows, correspondences in source order.
+ * Indices in and out are FRAME-LOCAL.  Edge cases follow the single calls (k == 0, non-finite queries, r <= 0 or
+ * non-finite r, k above a frame's indexed count); an index frame that is empty or holds only non-finite points gives
+ * every query of its frame count 0, and a query frame may be empty.
+ * Unlike the transient indexes inside the batch consumers, a batch index is persistent: it owns its cell table and its
+ * coarser and finer grid levels (a 100-frame table can take hundreds of MB), so other calls on the same context and
+ * other batch indexes leave it unchanged.  pcr_index_len returns N; pcr_index_info describes frame 0's grid and the
+ * indexed count of all frames.  The single-cloud queries (pcr_knn[_dev], pcr_radius_count, pcr_radius_search,
+ * pcr_find_correspondences) on a batch index of more than one frame -> PCR_ERR_INVALID_ARG naming the _batch form; the
+ * _batch queries on a single-cloud index are a batch of one.
+ * Errors: frame or query offsets not starting at 0 or decreasing, n_frames == 0 at build, a query frame count other
+ * than the index's, or a null pointer -> PCR_ERR_INVALID_ARG; N >= 2^31, more than 65535 frames, more than 0xfffffff0
+ * queries or k > PCR_MAX_K -> PCR_ERR_UNSUPPORTED.  The batch never shards its queries: on a context with a communicator
+ * every rank queries the frames it was given. */
+int pcr_index_build_batch(pcr_ctx *ctx, const float *x, const float *y, const float *z,
+                          const uint64_t *frame_offsets, size_t n_frames, size_t k_hint, pcr_index **out);
+/* _dev: x, y, z are device pointers (e.g. pcr_frames_device_pointers); frame_offsets stays on the host. */
+int pcr_index_build_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z,
+                              const uint64_t *frame_offsets /* HOST */, size_t n_frames, size_t k_hint, pcr_index **out);
+/* pcr_knn per query frame: idx, dist row-major nq x k (nq = query_offsets[n_frames], nq * k in 64 bits), counts nq;
+ * dist and counts may be NULL. */
+int pcr_knn_batch(pcr_index *index, const float *qx, const float *qy, const float *qz,
+                  const uint64_t *query_offsets, size_t n_frames, size_t k, uint32_t *idx, float *dist, uint32_t *counts);
+/* _dev: queries and outputs are device pointers, query_offsets stays on the host; enqueued like pcr_knn_dev. */
+int pcr_knn_batch_dev(pcr_index *index, const float *d_qx, const float *d_qy, const float *d_qz,
+                      const uint64_t *query_offsets /* HOST */, size_t n_frames, size_t k, uint32_t *d_idx,
+                      float *d_dist, uint32_t *d_counts);
+/* pcr_radius_count per query frame (counts: nq entries). */
+int pcr_radius_count_batch(pcr_index *index, const float *qx, const float *qy, const float *qz,
+                           const uint64_t *query_offsets, size_t n_frames, float radius, uint32_t *counts);
+int pcr_radius_count_batch_dev(pcr_index *index, const float *d_qx, const float *d_qy, const float *d_qz,
+                               const uint64_t *query_offsets /* HOST */, size_t n_frames, float radius,
+                               uint32_t *d_counts);
+/* pcr_radius_search per query frame: offsets[nq + 1] over all queries, row q frame-local and ascending; the
+ * PCR_ERR_CAPACITY protocol of pcr_radius_search. */
+int pcr_radius_search_batch(pcr_index *index, const float *qx, const float *qy, const float *qz,
+                            const uint64_t *query_offsets, size_t n_frames, float radius, uint64_t *offsets,
+                            uint32_t *idx, size_t cap, size_t *total);
+/* pcr_find_correspondences per query frame: frame f's pairs are [corr_offsets[f], corr_offsets[f+1]) of src_idx,
+ * tgt_idx and dist (each sized nq; corr_offsets HOST, n_frames + 1), in source order, both indices frame-local. */
+int pcr_find_correspondences_batch(pcr_index *target, const float *sx, const float *sy, const float *sz,
+                                   const uint64_t *query_offsets, size_t n_frames, float max_distance,
+                                   uint32_t *src_idx, uint32_t *tgt_idx, float *dist, uint64_t *corr_offsets);
 
 /* ---- filters ----------------------------------------------------------------------------------- */
 /* statistical_outlier_removal up to (not including) cloud.select(): keep[i] = 1 iff point i

@@ -10,6 +10,7 @@ The module mirrors the names and argument meaning of the reference's PyO3 module
     icp_point_to_point / icp_point_to_plane / apply_transform / IcpResult
                                                         crates/python/src/registration.rs:4-109
     KdTree (batched)                                    crates/spatial/src/kdtree.rs:14-164
+    KdTreeBatch                                         KdTree over many frames per call, each frame searched alone
 
 and for the steps either side of it (SURVEY.md section 8f):
 
@@ -42,7 +43,7 @@ __all__ = [
     "icp_point_to_point_batch", "icp_point_to_plane_batch", "voxel_downsample_batch", "estimate_normals_batch",
     "sor_normals_batch", "default_context", "PcrError", "euclidean_cluster", "voxel_downsample", "DeviceCloud", "ransac_plane", "PlaneResult",
     "ransac_plane_samples_batch", "ransac_plane_batch", "cluster_arrays_batch", "euclidean_cluster_batch",
-    "DeviceFrames", "radius_outlier_removal_batch",
+    "DeviceFrames", "radius_outlier_removal_batch", "KdTreeBatch",
 ]
 
 
@@ -1228,3 +1229,134 @@ class DeviceFrames:
         if not self.has_normals():  # crates/python/src/registration.rs:66-71
             raise ValueError("point-to-plane ICP needs frames with normals. Use estimate_normals first.")
         return self._icp(_ffi.load().pcr_frames_icp_point_to_plane, pairs, max_iterations, tolerance, max_correspondence_distance)
+
+
+def _query_frames(queries, query_offsets, n_frames: int):
+    """Checks and converts the queries of a KdTreeBatch call: (nq,3) rows, frames back to back, one frame per index frame."""
+    q, off = _batch_frames(queries, query_offsets)
+    if len(off) - 1 != n_frames:
+        raise ValueError(f"query_offsets describe {len(off) - 1} frames, the index holds {n_frames}")
+    return _soa(q), off
+
+
+class KdTreeBatch:
+    """KdTree over many frames at once: frame f = rows [frame_offsets[f], frame_offsets[f+1]) of the points, queried with
+    frames of queries back to back, query frame f searched in index frame f only.  Frame f's results are what
+    KdTree(frame f).<method>(queries of frame f) returns; indices in and out are frame-local.  The index stays in HBM
+    (cell table and grid levels included) until the object is freed."""
+
+    def __init__(self, points, frame_offsets: Sequence[int], k_hint: int = 0, ctx: Optional[Context] = None, _handle=None):
+        if _handle is not None:
+            self._ctx = ctx
+            self._h, self._off = _handle, np.ascontiguousarray(frame_offsets, np.uint64)
+        else:
+            pts, off = _batch_frames(points, frame_offsets)
+            if len(off) < 2:
+                raise ValueError("a batch index holds at least one frame")
+            self._ctx = ctx or default_context()
+            x, y, z = _soa(pts)
+            h = C.c_void_p()
+            _ffi.check(_ffi.load().pcr_index_build_batch(self._ctx._h, _p(x, _ffi.f32p), _p(y, _ffi.f32p), _p(z, _ffi.f32p), _p(off, _ffi.u64p),
+                                                         len(off) - 1, int(k_hint), C.byref(h)), self._ctx._h)
+            self._h, self._off = h, off
+        self._ctx._clouds.add(self)
+
+    @staticmethod
+    def from_device_frames(frames: "DeviceFrames", k_hint: int = 0) -> "KdTreeBatch":
+        """The index of a DeviceFrames batch, built from its device arrays (no host copy of the points)."""
+        off = frames.offsets
+        ptrs = [C.c_void_p() for _ in range(6)]
+        lib = _ffi.load()
+        _ffi.check(lib.pcr_frames_device_pointers(frames._h, *(C.byref(p) for p in ptrs)), frames._ctx._h)
+        h = C.c_void_p()
+        _ffi.check(lib.pcr_index_build_batch_dev(frames._ctx._h, ptrs[0], ptrs[1], ptrs[2], _p(off, _ffi.u64p), len(off) - 1, int(k_hint),
+                                                 C.byref(h)), frames._ctx._h)
+        return KdTreeBatch(None, off, ctx=frames._ctx, _handle=h)
+
+    def free(self):
+        h, self._h = getattr(self, "_h", None), None
+        if h and self._ctx._h:  # a closed context has already freed its indexes
+            _ffi.load().pcr_index_free(h)
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass
+
+    @property
+    def n_frames(self) -> int:
+        return len(self._off) - 1
+
+    @property
+    def offsets(self) -> np.ndarray:
+        return self._off.copy()
+
+    def len(self) -> int:
+        return int(_ffi.load().pcr_index_len(self._h))
+
+    __len__ = len
+
+    def __repr__(self) -> str:
+        return f"KdTreeBatch(frames={self.n_frames}, n={self.len()})"
+
+    def _knn(self, queries, query_offsets, k: int, want_dist: bool):
+        (qx, qy, qz), off = _query_frames(queries, query_offsets, self.n_frames)
+        nq = len(qx)
+        idx = np.full((nq, max(k, 0)), 0xFFFFFFFF, np.uint32)
+        dist = np.full((nq, max(k, 0)), np.inf, np.float32) if want_dist else None
+        cnt = np.zeros(nq, np.uint32)
+        st = _ffi.load().pcr_knn_batch(self._h, _p(qx, _ffi.f32p), _p(qy, _ffi.f32p), _p(qz, _ffi.f32p), _p(off, _ffi.u64p), self.n_frames,
+                                       int(k), _p(idx, _ffi.u32p), _p(dist, _ffi.f32p), _p(cnt, _ffi.u32p))
+        _ffi.check(st, self._ctx._h)
+        return idx, dist, cnt
+
+    def knn(self, queries, query_offsets: Sequence[int], k: int):
+        """-> (idx (nq,k) u32, dist (nq,k) f32, counts (nq,) u32), rows as KdTree.knn, indices frame-local."""
+        return self._knn(queries, query_offsets, k, True)
+
+    def knn_indices(self, queries, query_offsets: Sequence[int], k: int):
+        idx, _, cnt = self._knn(queries, query_offsets, k, False)
+        return idx, cnt
+
+    def radius_count(self, queries, query_offsets: Sequence[int], radius: float) -> np.ndarray:
+        (qx, qy, qz), off = _query_frames(queries, query_offsets, self.n_frames)
+        cnt = np.zeros(len(qx), np.uint32)
+        st = _ffi.load().pcr_radius_count_batch(self._h, _p(qx, _ffi.f32p), _p(qy, _ffi.f32p), _p(qz, _ffi.f32p), _p(off, _ffi.u64p),
+                                                self.n_frames, float(radius), _p(cnt, _ffi.u32p))
+        _ffi.check(st, self._ctx._h)
+        return cnt
+
+    def radius_search(self, queries, query_offsets: Sequence[int], radius: float):
+        """CSR over all queries: (offsets (nq+1,) u64, idx u32), every row frame-local and ascending (kdtree.rs:132)."""
+        (qx, qy, qz), off = _query_frames(queries, query_offsets, self.n_frames)
+        nq = len(qx)
+        r_off = np.zeros(nq + 1, np.uint64)
+        total = C.c_size_t()
+        cap = max(16 * nq, 1024)
+        lib = _ffi.load()
+        for _ in range(2):
+            idx = np.empty(cap, np.uint32)
+            st = lib.pcr_radius_search_batch(self._h, _p(qx, _ffi.f32p), _p(qy, _ffi.f32p), _p(qz, _ffi.f32p), _p(off, _ffi.u64p), self.n_frames,
+                                             float(radius), _p(r_off, _ffi.u64p), _p(idx, _ffi.u32p), cap, C.byref(total))
+            if st == _ffi.PCR_ERR_CAPACITY:
+                cap = int(total.value)
+                continue
+            _ffi.check(st, self._ctx._h)
+            return r_off, idx[: total.value].copy()
+        raise PcrError(_ffi.PCR_ERR_CAPACITY, "radius_search: capacity retry failed")
+
+    def find_correspondences(self, queries, query_offsets: Sequence[int], max_distance: float = math.inf):
+        """-> (src_idx u32, tgt_idx u32, dist f32, corr_offsets (F+1,) u64): frame f's pairs are [corr_offsets[f],
+        corr_offsets[f+1]), as KdTree(frame f).find_correspondences(queries of frame f) returns them."""
+        (qx, qy, qz), off = _query_frames(queries, query_offsets, self.n_frames)
+        ns = len(qx)
+        si, ti = np.empty(max(ns, 1), np.uint32), np.empty(max(ns, 1), np.uint32)
+        dd = np.empty(max(ns, 1), np.float32)
+        c_off = np.zeros(self.n_frames + 1, np.uint64)
+        st = _ffi.load().pcr_find_correspondences_batch(self._h, _p(qx, _ffi.f32p), _p(qy, _ffi.f32p), _p(qz, _ffi.f32p), _p(off, _ffi.u64p),
+                                                        self.n_frames, float(max_distance), _p(si, _ffi.u32p), _p(ti, _ffi.u32p),
+                                                        _p(dd, _ffi.f32p), _p(c_off, _ffi.u64p))
+        _ffi.check(st, self._ctx._h)
+        m = int(c_off[-1])
+        return si[:m].copy(), ti[:m].copy(), dd[:m].copy(), c_off

@@ -88,6 +88,14 @@ SIGNATURES = {
     "pcr_knn_dev": (C.c_int, [vp, vp, vp, vp, C.c_size_t, C.c_size_t, vp, vp, vp]),
     "pcr_radius_count": (C.c_int, [vp, f32p, f32p, f32p, C.c_size_t, C.c_float, u32p]),
     "pcr_radius_search": (C.c_int, [vp, f32p, f32p, f32p, C.c_size_t, C.c_float, u64p, u32p, C.c_size_t, szp]),
+    "pcr_index_build_batch": (C.c_int, [vp, f32p, f32p, f32p, u64p, C.c_size_t, C.c_size_t, C.POINTER(vp)]),
+    "pcr_index_build_batch_dev": (C.c_int, [vp, vp, vp, vp, u64p, C.c_size_t, C.c_size_t, C.POINTER(vp)]),
+    "pcr_knn_batch": (C.c_int, [vp, f32p, f32p, f32p, u64p, C.c_size_t, C.c_size_t, u32p, f32p, u32p]),
+    "pcr_knn_batch_dev": (C.c_int, [vp, vp, vp, vp, u64p, C.c_size_t, C.c_size_t, vp, vp, vp]),
+    "pcr_radius_count_batch": (C.c_int, [vp, f32p, f32p, f32p, u64p, C.c_size_t, C.c_float, u32p]),
+    "pcr_radius_count_batch_dev": (C.c_int, [vp, vp, vp, vp, u64p, C.c_size_t, C.c_float, vp]),
+    "pcr_radius_search_batch": (C.c_int, [vp, f32p, f32p, f32p, u64p, C.c_size_t, C.c_float, u64p, u32p, C.c_size_t, szp]),
+    "pcr_find_correspondences_batch": (C.c_int, [vp, f32p, f32p, f32p, u64p, C.c_size_t, C.c_float, u32p, u32p, f32p, u64p]),
     "pcr_sor": (C.c_int, [vp, f32p, f32p, f32p, C.c_size_t, C.c_size_t, C.c_float, u8p, szp, f32p, f32p]),
     "pcr_sor_dev": (C.c_int, [vp, vp, vp, vp, C.c_size_t, C.c_size_t, C.c_float, vp, vp]),
     "pcr_radius_outlier": (C.c_int, [vp, f32p, f32p, f32p, C.c_size_t, C.c_float, C.c_size_t, u8p, szp]),

@@ -271,6 +271,7 @@ void pcr_ctx_destroy(pcr_ctx *ctx) {
     free_buf(c, c->b_fine_misc);
     free_buf(c, c->b_fine_scan);
     free_buf(c, c->b_list);
+    free_buf(c, c->b_qoff);
     for (auto &b : c->b_cells) free_buf(c, b);
     for (auto &b : c->b_lsorted) free_buf(c, b);
     for (auto &b : c->b_lgrids) free_buf(c, b);
@@ -480,10 +481,17 @@ int pcr_index_info(const pcr_index *index, float *cell_size, int32_t dims[3], si
     return PCR_OK;
 }
 
+// The single-cloud queries would mix the frames of a batch index (pcr_index_build_batch): they name the batch form instead.
+static int single_cloud_check(const Index *ix, const char *batch_call) {
+    if (ix->n_frames == 1) return PCR_OK;
+    return fail(ix->ctx, PCR_ERR_INVALID_ARG, "the index holds %d frames: query it with %s", ix->n_frames, batch_call);
+}
+
 int pcr_knn_dev(pcr_index *index, const float *d_qx, const float *d_qy, const float *d_qz, size_t nq, size_t k, uint32_t *d_idx,
                 float *d_dist, uint32_t *d_counts) {
     if (!index || !index->ix) return fail(nullptr, PCR_ERR_INVALID_ARG, "index is NULL");
     Ctx *c = index->ix->ctx;
+    PCR_TRY(single_cloud_check(index->ix, "pcr_knn_batch_dev"));
     if (nq && k && (!d_qx || !d_qy || !d_qz || !d_idx)) return fail(c, PCR_ERR_INVALID_ARG, "null query/output pointer");
     PCR_API_BEGIN
     DevSetter ds(c);
@@ -496,6 +504,7 @@ int pcr_knn(pcr_index *index, const float *qx, const float *qy, const float *qz,
             uint32_t *counts) {
     if (!index || !index->ix) return fail(nullptr, PCR_ERR_INVALID_ARG, "index is NULL");
     Ctx *c = index->ix->ctx;
+    PCR_TRY(single_cloud_check(index->ix, "pcr_knn_batch"));
     if (nq == 0) return PCR_OK;
     if (!qx || !qy || !qz) return fail(c, PCR_ERR_INVALID_ARG, "null query pointer");
     if (k == 0) {  // kdtree.rs:65
@@ -527,6 +536,7 @@ int pcr_radius_count(pcr_index *index, const float *qx, const float *qy, const f
                      uint32_t *counts) {
     if (!index || !index->ix) return fail(nullptr, PCR_ERR_INVALID_ARG, "index is NULL");
     Ctx *c = index->ix->ctx;
+    PCR_TRY(single_cloud_check(index->ix, "pcr_radius_count_batch"));
     if (nq == 0) return PCR_OK;
     if (!qx || !qy || !qz || !counts) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     PCR_API_BEGIN
@@ -545,6 +555,7 @@ int pcr_radius_search(pcr_index *index, const float *qx, const float *qy, const 
                       uint64_t *offsets, uint32_t *idx, size_t cap, size_t *total) {
     if (!index || !index->ix) return fail(nullptr, PCR_ERR_INVALID_ARG, "index is NULL");
     Ctx *c = index->ix->ctx;
+    PCR_TRY(single_cloud_check(index->ix, "pcr_radius_search_batch"));
     if (!offsets || !total) return fail(c, PCR_ERR_INVALID_ARG, "offsets/total is NULL");
     *total = 0;
     offsets[0] = 0;
@@ -902,6 +913,7 @@ int pcr_find_correspondences(pcr_index *target, const float *sx, const float *sy
                              uint32_t *src_idx, uint32_t *tgt_idx, float *dist, size_t *count) {
     if (!target || !target->ix) return fail(nullptr, PCR_ERR_INVALID_ARG, "target is NULL");
     Ctx *c = target->ix->ctx;
+    PCR_TRY(single_cloud_check(target->ix, "pcr_find_correspondences_batch"));
     if (!count) return fail(c, PCR_ERR_INVALID_ARG, "count is NULL");
     *count = 0;
     if (ns == 0) return PCR_OK;
@@ -1204,6 +1216,212 @@ int pcr_estimate_normals_batch(pcr_ctx *ctx, const float *x, const float *y, con
 int pcr_estimate_normals_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z, const uint64_t *frame_offsets,
                                    size_t n_frames, size_t k, const float viewpoint[3], float *d_nx, float *d_ny, float *d_nz) {
     return normals_batch_entry(ctx, true, d_x, d_y, d_z, frame_offsets, n_frames, k, viewpoint, d_nx, d_ny, d_nz);
+}
+
+/* ---- batch index: the KdTree queries of many frames per call ----------------------------------------------- */
+// A persistent index over frames back to back (it owns every level it builds: no context slot is borrowed), queried with
+// frames of queries back to back, query frame f searched in index frame f only, indices frame-local.
+static int index_build_batch_entry(pcr_ctx *ctx, bool dev, const float *x, const float *y, const float *z, const uint64_t *frame_offsets,
+                                   size_t n_frames, size_t k_hint, pcr_index **out) {
+    if (!ctx || !out) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx/out is NULL");
+    *out = nullptr;
+    Ctx *c = &ctx->c;
+    if (n_frames == 0) return fail(c, PCR_ERR_INVALID_ARG, "a batch index holds at least one frame");
+    PCR_TRY(batch_offsets_check(c, frame_offsets, n_frames));
+    const size_t n = (size_t)frame_offsets[n_frames];
+    PCR_TRY(batch_size_check(c, n, n_frames));
+    if (n && (!x || !y || !z)) return fail(c, PCR_ERR_INVALID_ARG, "x/y/z is NULL");
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    const float *dx = x, *dy = y, *dz = z;
+    if (!dev) {
+        float *sx, *sy, *sz;
+        PCR_TRY(stage_xyz(c, c->b_in, x, y, z, n, &sx, &sy, &sz));
+        dx = sx; dy = sy; dz = sz;
+    }
+    BuildOpts bo;
+    bo.k_hint = k_hint;
+    bo.n_frames = (int)n_frames;
+    bo.frame_offsets = frame_offsets;
+    Index *ix = nullptr;
+    PCR_TRY(index_build_dev(c, dx, dy, dz, n, bo, &ix));
+    if (!dev) PCR_CUDA(c, cudaStreamSynchronize(c->stream));
+    return wrap_index(ctx, ix, out);
+    PCR_API_END(c)
+}
+
+int pcr_index_build_batch(pcr_ctx *ctx, const float *x, const float *y, const float *z, const uint64_t *frame_offsets, size_t n_frames,
+                          size_t k_hint, pcr_index **out) {
+    return index_build_batch_entry(ctx, false, x, y, z, frame_offsets, n_frames, k_hint, out);
+}
+int pcr_index_build_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z, const uint64_t *frame_offsets,
+                              size_t n_frames, size_t k_hint, pcr_index **out) {
+    return index_build_batch_entry(ctx, true, d_x, d_y, d_z, frame_offsets, n_frames, k_hint, out);
+}
+
+// The query side of a batch call: offsets as batch_offsets_check, as many frames as the index, at most 0xfffffff0 queries.
+static int batch_query_check(const Index *ix, const uint64_t *query_offsets, size_t n_frames, size_t *nq) {
+    Ctx *c = ix->ctx;
+    PCR_TRY(batch_offsets_check(c, query_offsets, n_frames));
+    if (n_frames != (size_t)ix->n_frames)
+        return fail(c, PCR_ERR_INVALID_ARG, "%zu query frames for an index of %d frames", n_frames, ix->n_frames);
+    *nq = (size_t)query_offsets[n_frames];
+    if (*nq > 0xfffffff0ull) return fail(c, PCR_ERR_UNSUPPORTED, "too many queries");
+    return PCR_OK;
+}
+
+static int knn_batch_entry(pcr_index *index, bool dev, const float *qx, const float *qy, const float *qz, const uint64_t *query_offsets,
+                           size_t n_frames, size_t k, uint32_t *idx, float *dist, uint32_t *counts) {
+    if (!index || !index->ix) return fail(nullptr, PCR_ERR_INVALID_ARG, "index is NULL");
+    Ctx *c = index->ix->ctx;
+    size_t nq = 0;
+    PCR_TRY(batch_query_check(index->ix, query_offsets, n_frames, &nq));
+    if (nq == 0) return PCR_OK;
+    if (!qx || !qy || !qz) return fail(c, PCR_ERR_INVALID_ARG, "null query pointer");
+    if (k > PCR_MAX_K) return fail(c, PCR_ERR_UNSUPPORTED, "k = %zu exceeds PCR_MAX_K = %d", k, PCR_MAX_K);
+    if (k && !idx) return fail(c, PCR_ERR_INVALID_ARG, "idx is NULL");
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    const QueryFrames qf = {query_offsets, n_frames};
+    if (k == 0) {  // kdtree.rs:65
+        if (counts && dev) PCR_CUDA(c, cudaMemsetAsync(counts, 0, sizeof(uint32_t) * nq, c->stream));
+        if (counts && !dev) memset(counts, 0, sizeof(uint32_t) * nq);
+        return PCR_OK;
+    }
+    if (dev) return knn_queries_dev(index->ix, qx, qy, qz, nq, k, idx, dist, counts, &qf);
+    float *dx, *dy, *dz;
+    PCR_TRY(stage_xyz(c, c->b_in2, qx, qy, qz, nq, &dx, &dy, &dz));
+    const size_t rows = nq * k;
+    PCR_TRY(ensure(c, c->b_out, rows * sizeof(uint32_t) + (dist ? rows * sizeof(float) : 0) + nq * sizeof(uint32_t) + 512));
+    uint32_t *d_idx = (uint32_t *)c->b_out.p;
+    float *d_dist = dist ? (float *)(d_idx + rows) : nullptr;
+    uint32_t *d_cnt = (uint32_t *)((char *)c->b_out.p + rows * sizeof(uint32_t) + (dist ? rows * sizeof(float) : 0));
+    PCR_TRY(knn_queries_dev(index->ix, dx, dy, dz, nq, k, d_idx, d_dist, d_cnt, &qf));
+    PCR_CUDA(c, cudaMemcpyAsync(idx, d_idx, rows * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+    if (dist) PCR_CUDA(c, cudaMemcpyAsync(dist, d_dist, rows * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    if (counts) PCR_CUDA(c, cudaMemcpyAsync(counts, d_cnt, nq * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+    PCR_CUDA(c, cudaStreamSynchronize(c->stream));
+    return PCR_OK;
+    PCR_API_END(c)
+}
+
+int pcr_knn_batch(pcr_index *index, const float *qx, const float *qy, const float *qz, const uint64_t *query_offsets, size_t n_frames,
+                  size_t k, uint32_t *idx, float *dist, uint32_t *counts) {
+    return knn_batch_entry(index, false, qx, qy, qz, query_offsets, n_frames, k, idx, dist, counts);
+}
+int pcr_knn_batch_dev(pcr_index *index, const float *d_qx, const float *d_qy, const float *d_qz, const uint64_t *query_offsets,
+                      size_t n_frames, size_t k, uint32_t *d_idx, float *d_dist, uint32_t *d_counts) {
+    return knn_batch_entry(index, true, d_qx, d_qy, d_qz, query_offsets, n_frames, k, d_idx, d_dist, d_counts);
+}
+
+static int radius_count_batch_entry(pcr_index *index, bool dev, const float *qx, const float *qy, const float *qz,
+                                    const uint64_t *query_offsets, size_t n_frames, float radius, uint32_t *counts) {
+    if (!index || !index->ix) return fail(nullptr, PCR_ERR_INVALID_ARG, "index is NULL");
+    Ctx *c = index->ix->ctx;
+    size_t nq = 0;
+    PCR_TRY(batch_query_check(index->ix, query_offsets, n_frames, &nq));
+    if (nq == 0) return PCR_OK;
+    if (!qx || !qy || !qz || !counts) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    const QueryFrames qf = {query_offsets, n_frames};
+    if (dev) return radius_count_dev(index->ix, qx, qy, qz, nq, radius, counts, &qf);
+    float *dx, *dy, *dz;
+    PCR_TRY(stage_xyz(c, c->b_in2, qx, qy, qz, nq, &dx, &dy, &dz));
+    PCR_TRY(ensure(c, c->b_out, nq * sizeof(uint32_t)));
+    PCR_TRY(radius_count_dev(index->ix, dx, dy, dz, nq, radius, (uint32_t *)c->b_out.p, &qf));
+    PCR_CUDA(c, cudaMemcpyAsync(counts, c->b_out.p, nq * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+    PCR_CUDA(c, cudaStreamSynchronize(c->stream));
+    return PCR_OK;
+    PCR_API_END(c)
+}
+
+int pcr_radius_count_batch(pcr_index *index, const float *qx, const float *qy, const float *qz, const uint64_t *query_offsets,
+                           size_t n_frames, float radius, uint32_t *counts) {
+    return radius_count_batch_entry(index, false, qx, qy, qz, query_offsets, n_frames, radius, counts);
+}
+int pcr_radius_count_batch_dev(pcr_index *index, const float *d_qx, const float *d_qy, const float *d_qz, const uint64_t *query_offsets,
+                               size_t n_frames, float radius, uint32_t *d_counts) {
+    return radius_count_batch_entry(index, true, d_qx, d_qy, d_qz, query_offsets, n_frames, radius, d_counts);
+}
+
+int pcr_radius_search_batch(pcr_index *index, const float *qx, const float *qy, const float *qz, const uint64_t *query_offsets,
+                            size_t n_frames, float radius, uint64_t *offsets, uint32_t *idx, size_t cap, size_t *total) {
+    if (!index || !index->ix) return fail(nullptr, PCR_ERR_INVALID_ARG, "index is NULL");
+    Ctx *c = index->ix->ctx;
+    if (!offsets || !total) return fail(c, PCR_ERR_INVALID_ARG, "offsets/total is NULL");
+    *total = 0;
+    offsets[0] = 0;
+    size_t nq = 0;
+    PCR_TRY(batch_query_check(index->ix, query_offsets, n_frames, &nq));
+    if (nq == 0) return PCR_OK;
+    if (!qx || !qy || !qz) return fail(c, PCR_ERR_INVALID_ARG, "null query pointer");
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    const QueryFrames qf = {query_offsets, n_frames};
+    float *dx, *dy, *dz;
+    PCR_TRY(stage_xyz(c, c->b_in2, qx, qy, qz, nq, &dx, &dy, &dz));
+    // counts (u32) | offsets (u64, nq+1), as pcr_radius_search
+    size_t off_bytes = ((nq * sizeof(uint32_t) + 255) & ~(size_t)255);
+    PCR_TRY(ensure(c, c->b_out, off_bytes + (nq + 1) * sizeof(uint64_t)));
+    uint32_t *d_cnt = (uint32_t *)c->b_out.p;
+    uint64_t *d_off = (uint64_t *)((char *)c->b_out.p + off_bytes);
+    PCR_TRY(radius_count_dev(index->ix, dx, dy, dz, nq, radius, d_cnt, &qf));
+    PCR_TRY(exclusive_scan_u64_from_u32_dev(c, d_cnt, d_off, nq));
+    PCR_CUDA(c, cudaMemcpyAsync(offsets, d_off, (nq + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, c->stream));
+    PCR_CUDA(c, cudaStreamSynchronize(c->stream));
+    *total = (size_t)offsets[nq];
+    if (*total > cap) return fail(c, PCR_ERR_CAPACITY, "radius_search needs room for %zu indices, cap is %zu", *total, cap);
+    if (*total == 0) return PCR_OK;
+    if (!idx) return fail(c, PCR_ERR_INVALID_ARG, "idx is NULL");
+    PCR_TRY(ensure(c, c->b_misc, *total * sizeof(uint32_t)));
+    PCR_TRY(radius_fill_dev(index->ix, dx, dy, dz, nq, radius, d_off, (uint32_t *)c->b_misc.p, &qf));
+    PCR_CUDA(c, cudaMemcpyAsync(idx, c->b_misc.p, *total * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+    PCR_CUDA(c, cudaStreamSynchronize(c->stream));
+    return PCR_OK;
+    PCR_API_END(c)
+}
+
+int pcr_find_correspondences_batch(pcr_index *target, const float *sx, const float *sy, const float *sz, const uint64_t *query_offsets,
+                                   size_t n_frames, float max_distance, uint32_t *src_idx, uint32_t *tgt_idx, float *dist,
+                                   uint64_t *corr_offsets) {
+    if (!target || !target->ix) return fail(nullptr, PCR_ERR_INVALID_ARG, "target is NULL");
+    Ctx *c = target->ix->ctx;
+    if (!corr_offsets) return fail(c, PCR_ERR_INVALID_ARG, "corr_offsets is NULL");
+    size_t ns = 0;
+    PCR_TRY(batch_query_check(target->ix, query_offsets, n_frames, &ns));
+    for (size_t f = 0; f <= n_frames; f++) corr_offsets[f] = 0;
+    if (ns == 0) return PCR_OK;
+    if (!sx || !sy || !sz || !src_idx || !tgt_idx || !dist) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    const QueryFrames qf = {query_offsets, n_frames};
+    float *dx, *dy, *dz;
+    PCR_TRY(stage_xyz(c, c->b_in2, sx, sy, sz, ns, &dx, &dy, &dz));
+    PCR_TRY(ensure(c, c->b_out, ns * 8));
+    uint32_t *d_t = (uint32_t *)c->b_out.p;
+    float *d_d = (float *)(d_t + ns);
+    PCR_TRY(find_correspondences_dev(target->ix, dx, dy, dz, ns, max_distance, d_t, d_d, &qf));
+    // compact on the host, frame by frame in source order (correspondence.rs:23-36); source indices frame-local
+    std::vector<uint32_t> ht(ns);
+    std::vector<float> hd(ns);
+    PCR_CUDA(c, cudaMemcpyAsync(ht.data(), d_t, ns * 4, cudaMemcpyDeviceToHost, c->stream));
+    PCR_CUDA(c, cudaMemcpyAsync(hd.data(), d_d, ns * 4, cudaMemcpyDeviceToHost, c->stream));
+    PCR_CUDA(c, cudaStreamSynchronize(c->stream));
+    size_t m = 0;
+    for (size_t f = 0; f < n_frames; f++) {
+        corr_offsets[f] = m;
+        for (size_t i = (size_t)query_offsets[f]; i < (size_t)query_offsets[f + 1]; i++)
+            if (ht[i] != 0xffffffffu) {
+                src_idx[m] = (uint32_t)(i - (size_t)query_offsets[f]);
+                tgt_idx[m] = ht[i];
+                dist[m] = hd[i];
+                m++;
+            }
+    }
+    corr_offsets[n_frames] = m;
+    return PCR_OK;
+    PCR_API_END(c)
 }
 
 /* ---- batched RANSAC plane fit and euclidean_cluster ------------------------------------------------- */

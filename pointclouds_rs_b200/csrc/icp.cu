@@ -855,13 +855,13 @@ int apply_transform_dev(Ctx *ctx, const float *dx, const float *dy, const float 
 }
 
 int find_correspondences_dev(Index *target, const float *dsx, const float *dsy, const float *dsz, size_t ns,
-                             float max_distance, uint32_t *d_tgt, float *d_dist) {
+                             float max_distance, uint32_t *d_tgt, float *d_dist, const QueryFrames *qf) {
     Ctx *ctx = target->ctx;
     if (ns == 0) return PCR_OK;
     PCR_TRY(ensure(ctx, ctx->b_misc2, ns * sizeof(uint32_t)));
     uint32_t *d_cnt = (uint32_t *)ctx->b_misc2.p;
     PCR_CUDA(ctx, cudaMemsetAsync(d_cnt, 0, ns * sizeof(uint32_t), ctx->stream));
-    PCR_TRY(knn_queries_dev(target, dsx, dsy, dsz, ns, 1, d_tgt, d_dist, d_cnt));  // correspondence.rs:25
+    PCR_TRY(knn_queries_dev(target, dsx, dsy, dsz, ns, 1, d_tgt, d_dist, d_cnt, qf));  // correspondence.rs:25
     correspond_filter_kernel<<<(unsigned)((ns + 255) / 256), 256, 0, ctx->stream>>>(ns, max_distance, d_tgt, d_dist, d_cnt);
     PCR_LAUNCH_CHECK(ctx);
     return PCR_OK;

@@ -78,39 +78,44 @@ __device__ __forceinline__ int frame_of_sorted(const GridDesc *__restrict__ grid
 }
 
 // ---- external queries -----------------------------------------------------------------------------
+// base: subtracted from every emitted index (a batch index: the query's frame's first input point -> frame-local indices)
 template <class TopK>
 __device__ __forceinline__ void emit_row(const TopK &tk, int cnt, size_t k, size_t qi, uint32_t *__restrict__ idx,
-                                         float *__restrict__ dist);
+                                         float *__restrict__ dist, uint32_t base);
 
 template <>
 __device__ __forceinline__ void emit_row<RegTopK>(const RegTopK &tk, int cnt, size_t k, size_t qi,
-                                                  uint32_t *__restrict__ idx, float *__restrict__ dist) {
+                                                  uint32_t *__restrict__ idx, float *__restrict__ dist, uint32_t base) {
     if ((size_t)tk.lane < k) {
         bool v = tk.lane < cnt;
-        idx[qi * k + tk.lane] = v ? key_idx(tk.K) : 0xffffffffu;
+        idx[qi * k + tk.lane] = v ? key_idx(tk.K) - base : 0xffffffffu;
         if (dist) dist[qi * k + tk.lane] = v ? __fsqrt_rn(key_d2(tk.K)) : INFINITY;  // kdtree.rs:76
     }
 }
 template <>
 __device__ __forceinline__ void emit_row<SmemTopK>(const SmemTopK &tk, int cnt, size_t k, size_t qi,
-                                                   uint32_t *__restrict__ idx, float *__restrict__ dist) {
+                                                   uint32_t *__restrict__ idx, float *__restrict__ dist, uint32_t base) {
     for (size_t j = tk.lane; j < k; j += 32) {
         bool v = j < (size_t)cnt;
         unsigned long long key = v ? tk.s[j] : 0ull;
-        idx[qi * k + j] = v ? key_idx(key) : 0xffffffffu;
+        idx[qi * k + j] = v ? key_idx(key) - base : 0xffffffffu;
         if (dist) dist[qi * k + j] = v ? __fsqrt_rn(key_d2(key)) : INFINITY;
     }
 }
 
-template <bool kSmem, int QPW>
-__global__ void __launch_bounds__(kThreads, (!kSmem && QPW == kQPWS) ? 8 : 1) knn_queries_kernel(LevelArgs a, const float *__restrict__ qx,
+// kQFrames (batch index): query qi belongs to query frame f = frame_of(qoff, a.n_frames, qi) and is searched in grid f of
+// the level only; indices come back frame-local.  The single-frame calls pass no qoff.
+// (kQFrames, warp per query: the frame's grid stays live through the search; 7 blocks per SM instead of 8 keep its spills below
+// the single-frame form's)
+template <bool kSmem, int QPW, bool kQFrames = false>
+__global__ void __launch_bounds__(kThreads, (!kSmem && QPW == kQPWS) ? (kQFrames ? 7 : 8) : 1) knn_queries_kernel(LevelArgs a, const float *__restrict__ qx,
                                                                const float *__restrict__ qy, const float *__restrict__ qz,
                                                                int kk, uint32_t *__restrict__ idx, float *__restrict__ dist,
-                                                               uint32_t *__restrict__ counts) {
+                                                               uint32_t *__restrict__ counts, const uint32_t *__restrict__ qoff = nullptr) {
     extern __shared__ unsigned long long smem_keys[];
     __shared__ WarpSelScratch s_sel[kWarps];
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    const GridDesc g = a.grids[0];
+    GridDesc g = a.grids[0];
     typename std::conditional<kSmem, SmemTopK, RegTopK>::type tk;
     tk.kk = kk;
     tk.lane = lane;
@@ -123,14 +128,19 @@ __global__ void __launch_bounds__(kThreads, (!kSmem && QPW == kQPWS) ? 8 : 1) kn
         float x = __ldg(&qx[qi]), y = __ldg(&qy[qi]), z = __ldg(&qz[qi]);
         int cnt = 0;
         tk.reset(PCR_EMPTY_KEY);
-        if (finite3(x, y, z)) {  // kdtree.rs:65
+        bool searchable = finite3(x, y, z);  // kdtree.rs:65
+        if constexpr (kQFrames) {
+            g = a.grids[frame_of(qoff, a.n_frames, qi)];
+            searchable = searchable && g.pt_end > g.pt_begin;  // (an empty index frame: no neighbours)
+        }
+        if (searchable) {
             if (!warp_knn_search(tk, g, a.cell_start, a.pts, x, y, z, a.max_rings, a.last_level != 0, PCR_EMPTY_KEY, (QPW == kQPWS || a.no_tile) ? &s_sel[w] : nullptr)) {
                 defer_query(a, qi, lane);
                 continue;
             }
             cnt = tk.count();
         }
-        emit_row(tk, cnt, (size_t)kk, (size_t)qi, idx, dist);
+        emit_row(tk, cnt, (size_t)kk, (size_t)qi, idx, dist, kQFrames ? g.in_begin : 0u);
         if (counts && lane == 0) counts[qi] = (uint32_t)cnt;
         if constexpr (kSmem) __syncwarp();
     }
@@ -431,6 +441,8 @@ struct ThreadArgs {
     uint8_t *list_cnt;   // [list_stride]: valid entries (0xff = no list: the query was deferred)
     size_t list_stride;
     int kk_sor;          // k_sor + 1 <= kk: the SOR statistic uses the first kk_sor entries
+    // MODE 0 on a batch index (kQFrames): device query offsets [n_frames + 1], query frame f searched in index frame f only
+    const uint32_t *qoff;
 };
 
 constexpr int kTQThreads = 128;
@@ -486,7 +498,7 @@ __device__ __forceinline__ void normal_from_topk(const ThreadTopK<KC> &acc, int 
     nx = ex; ny = ey; nz = ez;
 }
 
-template <int KC, int MODE>
+template <int KC, int MODE, bool kQFrames = false>
 __global__ void __launch_bounds__(kTQThreads) knn_thread_kernel(LevelArgs a, ThreadArgs t) {
     const uint32_t q = a.q_offset + blockIdx.x * kTQThreads + threadIdx.x;
     const int lane = threadIdx.x & 31;
@@ -505,6 +517,10 @@ __global__ void __launch_bounds__(kTQThreads) knn_thread_kernel(LevelArgs a, Thr
             py = __ldg(&t.qy[q]);
             pz = __ldg(&t.qz[q]);
             searchable = finite3(px, py, pz);  // kdtree.rs:65
+            if constexpr (kQFrames) {
+                f = frame_of(t.qoff, a.n_frames, q);
+                searchable = searchable && a.grids[f].pt_end > a.grids[f].pt_begin;  // (an empty index frame: no neighbours)
+            }
         } else {
             float4 p = __ldg(&a.qpts[q]);
             px = p.x; py = p.y; pz = p.z;
@@ -538,11 +554,13 @@ __global__ void __launch_bounds__(kTQThreads) knn_thread_kernel(LevelArgs a, Thr
     if (MODE == 0) {
         uint32_t *ri = t.idx + (size_t)q * t.kk;
         float *rd = t.dist ? t.dist + (size_t)q * t.kk : nullptr;
+        // (frame-local indices; the frame is looked up again rather than kept live through the search)
+        const uint32_t base = kQFrames ? a.grids[frame_of(t.qoff, a.n_frames, q)].in_begin : 0u;
 #pragma unroll
         for (int j = 0; j < KC; j++)
             if (j < t.kk) {
                 bool v = j < cnt;
-                ri[j] = v ? key_idx(acc.K[j]) : 0xffffffffu;
+                ri[j] = v ? key_idx(acc.K[j]) - base : 0xffffffffu;
                 if (rd) rd[j] = v ? __fsqrt_rn(key_d2(acc.K[j])) : INFINITY;  // kdtree.rs:76
             }
         if (t.counts) t.counts[q] = (uint32_t)cnt;
@@ -580,20 +598,20 @@ __global__ void __launch_bounds__(kTQThreads) knn_thread_kernel(LevelArgs a, Thr
     }
 }
 
-template <int MODE>
+template <int MODE, bool kQFrames = false>
 int launch_sel_kernel(Ctx *ctx, const LevelArgs &a, const ThreadArgs &t);
 inline bool use_select(int kk);
 template <class Kern>
 int set_smem(Ctx *ctx, Kern kern, size_t bytes);
 
-template <int MODE>
+template <int MODE, bool kQFrames = false>
 int launch_thread_kernel(Ctx *ctx, const LevelArgs &a, const ThreadArgs &t) {
-    if (use_select(t.kk)) return launch_sel_kernel<MODE>(ctx, a, t);
+    if (use_select(t.kk)) return launch_sel_kernel<MODE, kQFrames>(ctx, a, t);
     const unsigned blocks = (a.nq + kTQThreads - 1) / kTQThreads;
     const int kk = t.kk;
 #define PCR_TQ(KC)                                                                          \
     if (kk <= KC) {                                                                         \
-        knn_thread_kernel<KC, MODE><<<blocks, kTQThreads, 0, ctx->stream>>>(a, t);          \
+        knn_thread_kernel<KC, MODE, kQFrames><<<blocks, kTQThreads, 0, ctx->stream>>>(a, t); \
         PCR_LAUNCH_CHECK(ctx);                                                              \
         return PCR_OK;                                                                      \
     }
@@ -615,8 +633,9 @@ __device__ __forceinline__ void push_list(bool mine, uint32_t *__restrict__ list
     if (mine) list[base + __popc(mask & ((1u << lane) - 1u))] = q;
 }
 
-template <int MODE>
-__global__ void __launch_bounds__(kTQThreads, 6) knn_sel_kernel(LevelArgs a, ThreadArgs t) {
+// (kQFrames: the query's grid pointer stays live through the search; 5 blocks per SM instead of 6 keep it free of spills)
+template <int MODE, bool kQFrames = false>
+__global__ void __launch_bounds__(kTQThreads, kQFrames ? 5 : 6) knn_sel_kernel(LevelArgs a, ThreadArgs t) {
     static_assert(kTQThreads == kSelStride, "one buffer column per thread");
     const uint32_t nq = a.nq_dev ? min(a.nq, *a.nq_dev) : a.nq;
     if (blockIdx.x * kTQThreads >= nq) return;  // (block-uniform: the follow-up pass is launched for a capacity)
@@ -636,6 +655,10 @@ __global__ void __launch_bounds__(kTQThreads, 6) knn_sel_kernel(LevelArgs a, Thr
             py = __ldg(&t.qy[q]);
             pz = __ldg(&t.qz[q]);
             searchable = finite3(px, py, pz);  // kdtree.rs:65
+            if constexpr (kQFrames) {
+                f = frame_of(t.qoff, a.n_frames, q);
+                searchable = searchable && a.grids[f].pt_end > a.grids[f].pt_begin;  // (an empty index frame: no neighbours)
+            }
         } else {
             const float4 p = __ldg(&a.qpts[q]);
             px = p.x; py = p.y; pz = p.z;
@@ -661,12 +684,14 @@ __global__ void __launch_bounds__(kTQThreads, 6) knn_sel_kernel(LevelArgs a, Thr
     if (MODE == 0) {
         uint32_t *ri = t.idx + (size_t)q * t.kk;
         float *rd = t.dist ? t.dist + (size_t)q * t.kk : nullptr;
+        // (frame-local indices; the frame is looked up again rather than kept live through the search)
+        const uint32_t base = kQFrames ? a.grids[frame_of(t.qoff, a.n_frames, q)].in_begin : 0u;
 #pragma unroll
         for (int j = 0; j < kSelMaxK; j++)
             if (j < t.kk) {
                 const bool v = j < cnt;
                 const unsigned long long key = v ? acc.key_at(acc.ord[j]) : 0ull;
-                ri[j] = v ? key_idx(key) : 0xffffffffu;
+                ri[j] = v ? key_idx(key) - base : 0xffffffffu;
                 if (rd) rd[j] = v ? __fsqrt_rn(key_d2(key)) : INFINITY;  // kdtree.rs:76
             }
         if (t.counts) t.counts[q] = (uint32_t)cnt;
@@ -1013,7 +1038,7 @@ inline bool use_tile(int kk) {
     return on && kk > 0 && kk <= kTileMaxK;
 }
 
-template <int MODE>
+template <int MODE, bool kQFrames>
 int launch_sel_kernel(Ctx *ctx, const LevelArgs &a, const ThreadArgs &t) {
     const unsigned blocks = (a.nq + kTQThreads - 1) / kTQThreads;
     if constexpr (MODE != 0) {
@@ -1062,7 +1087,7 @@ int launch_sel_kernel(Ctx *ctx, const LevelArgs &a, const ThreadArgs &t) {
             return PCR_OK;  // (run_levels launches a warp-per-query pass over what the tiles handed back)
         }
     }
-    knn_sel_kernel<MODE><<<blocks, kTQThreads, 0, ctx->stream>>>(a, t);
+    knn_sel_kernel<MODE, kQFrames><<<blocks, kTQThreads, 0, ctx->stream>>>(a, t);
     PCR_LAUNCH_CHECK(ctx);
     return PCR_OK;
 }
@@ -1091,8 +1116,10 @@ __global__ void fill_f32_kernel(float *__restrict__ p, size_t n, float v) {
 // d^2 <= r*r with r*r rounded in f32 (kdtree.rs:114,127).  Cells are taken from the box
 // [q - r', q + r'] with r' = sqrt(r2) * (1 + 1e-6): a point that passes the f32 test is at most a
 // few ulp further than sqrt(r2) on any axis.
-// kFrames (batch): the queries are the input points of a multi-frame index, query i = point i, and each is searched
-// only in the grid of its own frame.  The single-frame calls leave frame_in_off / n_frames unset.
+// kFrames (batch): query i belongs to frame frame_of(frame_in_off, n_frames, i) and is searched only in the grid of that frame
+// -- the input points of a multi-frame index themselves (frame_in_off = its input offsets), or the external queries of a
+// batch (frame_in_off = the query offsets; the filled indices are then frame-local).  The single-frame calls leave
+// frame_in_off / n_frames unset.
 template <bool kFill, bool kFrames = false>
 __global__ void __launch_bounds__(256) radius_kernel(const GridDesc *__restrict__ grids,
                                                      const uint32_t *__restrict__ cell_start,
@@ -1129,7 +1156,7 @@ __global__ void __launch_bounds__(256) radius_kernel(const GridDesc *__restrict_
                     for (uint32_t i = b; i < e; i++) {
                         float4 p = __ldg(&sorted[i]);
                         if (dist2_exact(x, y, z, p.x, p.y, p.z) <= r2) {
-                            if (kFill) dst[cnt] = __float_as_uint(p.w);
+                            if (kFill) dst[cnt] = __float_as_uint(p.w) - (kFrames ? g.in_begin : 0u);
                             cnt++;
                         }
                     }
@@ -1203,7 +1230,10 @@ struct ClassArgs {
     uint32_t heavy_n;  // more than this: heavy normal (0: no such class)
 };
 
-__global__ void __launch_bounds__(kClsThreads) classify_kernel(LevelArgs a, ClassArgs c) {
+// kQFrames: external queries of a batch index, qoff their device offsets (frame f searched in grid f).  (qoff is a parameter
+// of its own: the kernel copies ClassArgs to local memory, and a longer struct would change the single-frame SASS.)
+template <bool kQFrames = false>
+__global__ void __launch_bounds__(kClsThreads) classify_kernel(LevelArgs a, ClassArgs c, const uint32_t *__restrict__ qoff) {
     PCR_GRID_DEP_SYNC();
     const uint32_t slot = blockIdx.x * kClsThreads + threadIdx.x;
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
@@ -1218,6 +1248,7 @@ __global__ void __launch_bounds__(kClsThreads) classify_kernel(LevelArgs a, Clas
             py = __ldg(&c.qy[q]);
             pz = __ldg(&c.qz[q]);
             searchable = finite3(px, py, pz);
+            if constexpr (kQFrames) f = frame_of(qoff, a.n_frames, q);
         } else {
             const float4 p = __ldg(&a.qpts[q]);
             px = p.x; py = p.y; pz = p.z;
@@ -1288,7 +1319,8 @@ int run_levels(Index *ix, uint32_t nq, int tag0, Launch launch, const uint32_t *
                int sel_kk = 0 /* > 0: level 0 is a thread-per-query launch for this many neighbours */,
                uint32_t q_offset = 0 /* level 0 takes the queries q_offset .. q_offset + nq (a rank's shard) */,
                const float *eqx = nullptr, const float *eqy = nullptr, const float *eqz = nullptr /* external queries (device) */,
-               bool tile_ok = false /* level 0 may run as the cell-tile kernel (self-queries with a fused consumer) */) {
+               bool tile_ok = false /* level 0 may run as the cell-tile kernel (self-queries with a fused consumer) */,
+               const uint32_t *eq_off = nullptr /* external queries of a batch index: device query offsets [n_frames + 1] */) {
     // init_list: level 0 runs over these nq query ids only (warp kernels) instead of over all queries
     // nq_dev:    the length of init_list is still on the device; nq is the capacity level 0 is launched for
     Ctx *ctx = ix->ctx;
@@ -1380,7 +1412,8 @@ int run_levels(Index *ix, uint32_t nq, int tag0, Launch launch, const uint32_t *
             ca.heavy_n = a.ovf_list ? heavy_n : 0u;
             {
                 TimeScope ts(ctx, kTagKnnDeferred);
-                PCR_CUDA(ctx, launch_chained(classify_kernel, dim3((n_cur + kClsThreads - 1) / kClsThreads), dim3(kClsThreads), 0, ctx->stream, a, ca));
+                PCR_CUDA(ctx, launch_chained(eq_off ? classify_kernel<true> : classify_kernel<false>, dim3((n_cur + kClsThreads - 1) / kClsThreads),
+                                             dim3(kClsThreads), 0, ctx->stream, a, ca, eq_off));
                 ctx->launches++;
             }
             PCR_CUDA(ctx, cudaEventRecord(ctx->ev_fork, ctx->stream));
@@ -1627,39 +1660,64 @@ int index_shard_queries(Index *ix) {
     return PCR_OK;
 }
 
-int knn_queries_dev(Index *ix, const float *dqx, const float *dqy, const float *dqz, size_t nq, size_t k, uint32_t *d_idx,
-                    float *d_dist, uint32_t *d_counts) {
+namespace {
+// Device u32 copy of the query offsets of a batch (in ctx->b_qoff, valid until the next batch query on the context).
+int upload_query_offsets(Ctx *ctx, const QueryFrames &qf, const uint32_t **d_off) {
+    std::vector<uint32_t> h(qf.n_frames + 1);
+    for (size_t f = 0; f <= qf.n_frames; f++) h[f] = (uint32_t)qf.offsets[f];
+    PCR_TRY(ensure(ctx, ctx->b_qoff, sizeof(uint32_t) * h.size()));
+    PCR_CUDA(ctx, cudaMemcpyAsync(ctx->b_qoff.p, h.data(), sizeof(uint32_t) * h.size(), cudaMemcpyHostToDevice, ctx->stream));
+    *d_off = (const uint32_t *)ctx->b_qoff.p;
+    return PCR_OK;
+}
+
+// kQFrames: the queries of a batch index, d_qoff their device offsets (see knn_queries_kernel)
+template <bool kQFrames>
+int knn_queries_run(Index *ix, const float *dqx, const float *dqy, const float *dqz, size_t nq, size_t k, uint32_t *d_idx,
+                    float *d_dist, uint32_t *d_counts, const uint32_t *d_qoff) {
     Ctx *ctx = ix->ctx;
-    if (nq == 0 || k == 0) return PCR_OK;
-    if (ix->n_frames != 1) return fail(ctx, PCR_ERR_UNSUPPORTED, "external queries need a single-frame index");
-    if (k > PCR_MAX_K) return fail(ctx, PCR_ERR_UNSUPPORTED, "k = %zu exceeds PCR_MAX_K = %d", k, PCR_MAX_K);
-    if (nq > 0xfffffff0ull) return fail(ctx, PCR_ERR_UNSUPPORTED, "too many queries");
     const int kk = (int)k;
-    if (k > 32) PCR_TRY(set_smem(ctx, knn_queries_kernel<true, kQPW0>, sizeof(unsigned long long) * k * kWarps));
-    if (k > 32) PCR_TRY(set_smem(ctx, knn_queries_kernel<true, kQPWL>, sizeof(unsigned long long) * k * kWarps));
+    if (k > 32) PCR_TRY(set_smem(ctx, knn_queries_kernel<true, kQPW0, kQFrames>, sizeof(unsigned long long) * k * kWarps));
+    if (k > 32) PCR_TRY(set_smem(ctx, knn_queries_kernel<true, kQPWL, kQFrames>, sizeof(unsigned long long) * k * kWarps));
     ThreadArgs ta = {};
     ta.qx = dqx; ta.qy = dqy; ta.qz = dqz;
     ta.idx = d_idx; ta.dist = d_dist; ta.counts = d_counts;
     ta.kk = kk;
+    ta.qoff = d_qoff;
     return run_levels(ix, (uint32_t)nq, kTagKnn, [&](const LevelArgs &a, int qpw) -> int {
-        if (qpw == kQPW0 && k <= 32) return launch_thread_kernel<0>(ctx, a, ta);
+        if (qpw == kQPW0 && k <= 32) return launch_thread_kernel<0, kQFrames>(ctx, a, ta);
         unsigned blocks = blocks_for(ctx, a, qpw);
         if (qpw == kQPWS) {
-            knn_queries_kernel<false, kQPWS><<<blocks, kThreads, 0, ctx->stream>>>(a, dqx, dqy, dqz, kk, d_idx, d_dist, d_counts);
+            knn_queries_kernel<false, kQPWS, kQFrames><<<blocks, kThreads, 0, ctx->stream>>>(a, dqx, dqy, dqz, kk, d_idx, d_dist, d_counts, d_qoff);
             PCR_LAUNCH_CHECK(ctx);
             return PCR_OK;
         }
         size_t smem = k <= 32 ? 0 : sizeof(unsigned long long) * k * kWarps;
         if (k <= 32) {
-            if (qpw == kQPW0) knn_queries_kernel<false, kQPW0><<<blocks, kThreads, 0, ctx->stream>>>(a, dqx, dqy, dqz, kk, d_idx, d_dist, d_counts);
-            else knn_queries_kernel<false, kQPWL><<<blocks, kThreads, 0, ctx->stream>>>(a, dqx, dqy, dqz, kk, d_idx, d_dist, d_counts);
+            if (qpw == kQPW0) knn_queries_kernel<false, kQPW0, kQFrames><<<blocks, kThreads, 0, ctx->stream>>>(a, dqx, dqy, dqz, kk, d_idx, d_dist, d_counts, d_qoff);
+            else knn_queries_kernel<false, kQPWL, kQFrames><<<blocks, kThreads, 0, ctx->stream>>>(a, dqx, dqy, dqz, kk, d_idx, d_dist, d_counts, d_qoff);
         } else {
-            if (qpw == kQPW0) knn_queries_kernel<true, kQPW0><<<blocks, kThreads, smem, ctx->stream>>>(a, dqx, dqy, dqz, kk, d_idx, d_dist, d_counts);
-            else knn_queries_kernel<true, kQPWL><<<blocks, kThreads, smem, ctx->stream>>>(a, dqx, dqy, dqz, kk, d_idx, d_dist, d_counts);
+            if (qpw == kQPW0) knn_queries_kernel<true, kQPW0, kQFrames><<<blocks, kThreads, smem, ctx->stream>>>(a, dqx, dqy, dqz, kk, d_idx, d_dist, d_counts, d_qoff);
+            else knn_queries_kernel<true, kQPWL, kQFrames><<<blocks, kThreads, smem, ctx->stream>>>(a, dqx, dqy, dqz, kk, d_idx, d_dist, d_counts, d_qoff);
         }
         PCR_LAUNCH_CHECK(ctx);
         return PCR_OK;
-    }, nullptr, nullptr, k <= 32 ? kk : 0, 0, dqx, dqy, dqz);
+    }, nullptr, nullptr, k <= 32 ? kk : 0, 0, dqx, dqy, dqz, false, d_qoff);
+}
+}  // namespace
+
+int knn_queries_dev(Index *ix, const float *dqx, const float *dqy, const float *dqz, size_t nq, size_t k, uint32_t *d_idx,
+                    float *d_dist, uint32_t *d_counts, const QueryFrames *qf) {
+    Ctx *ctx = ix->ctx;
+    if (nq == 0 || k == 0) return PCR_OK;
+    if (k > PCR_MAX_K) return fail(ctx, PCR_ERR_UNSUPPORTED, "k = %zu exceeds PCR_MAX_K = %d", k, PCR_MAX_K);
+    if (nq > 0xfffffff0ull) return fail(ctx, PCR_ERR_UNSUPPORTED, "too many queries");
+    if (ix->n_frames == 1) return knn_queries_run<false>(ix, dqx, dqy, dqz, nq, k, d_idx, d_dist, d_counts, nullptr);  // (a batch of one)
+    if (!qf || qf->n_frames != (size_t)ix->n_frames)
+        return fail(ctx, PCR_ERR_INVALID_ARG, "queries on a batch index of %d frames need query offsets of as many frames (pcr_knn_batch)", ix->n_frames);
+    const uint32_t *d_qoff = nullptr;
+    PCR_TRY(upload_query_offsets(ctx, *qf, &d_qoff));
+    return knn_queries_run<true>(ix, dqx, dqy, dqz, nq, k, d_idx, d_dist, d_counts, d_qoff);
 }
 
 int sor_mean_dist_dev(Index *ix, size_t k, float *d_mean_d, const SorLists *keep_lists, bool allow_shard) {
@@ -2036,9 +2094,19 @@ int normals_from_lists_dev(Index *ix, size_t k, const float vp[3], const SorList
 }
 
 int radius_count_dev(Index *ix, const float *dqx, const float *dqy, const float *dqz, size_t nq, float radius,
-                     uint32_t *d_counts) {
+                     uint32_t *d_counts, const QueryFrames *qf) {
     Ctx *ctx = ix->ctx;
     if (nq == 0) return PCR_OK;
+    if (ix->n_frames != 1 && qf) {  // external queries of a batch: query frame f counts in index frame f
+        if (qf->n_frames != (size_t)ix->n_frames)
+            return fail(ctx, PCR_ERR_INVALID_ARG, "queries on a batch index of %d frames need query offsets of as many frames", ix->n_frames);
+        const uint32_t *d_qoff = nullptr;
+        PCR_TRY(upload_query_offsets(ctx, *qf, &d_qoff));
+        radius_kernel<false, true><<<(unsigned)((nq + 255) / 256), 256, 0, ctx->stream>>>(ix->grids, ix->cell_start, ix->sorted, dqx, dqy, dqz, nq,
+                                                                                          radius, d_counts, nullptr, nullptr, d_qoff, ix->n_frames);
+        PCR_LAUNCH_CHECK(ctx);
+        return PCR_OK;
+    }
     if (ix->n_frames != 1) {  // a batch: every indexed point counts its neighbours inside its own frame
         if (nq != ix->n) return fail(ctx, PCR_ERR_UNSUPPORTED, "radius queries on a multi-frame index must be its own points");
         radius_kernel<false, true><<<(unsigned)((nq + 255) / 256), 256, 0, ctx->stream>>>(ix->grids, ix->cell_start, ix->sorted, dqx, dqy, dqz, nq,
@@ -2054,9 +2122,19 @@ int radius_count_dev(Index *ix, const float *dqx, const float *dqy, const float 
 }
 
 int radius_fill_dev(Index *ix, const float *dqx, const float *dqy, const float *dqz, size_t nq, float radius,
-                    const uint64_t *d_offsets, uint32_t *d_idx) {
+                    const uint64_t *d_offsets, uint32_t *d_idx, const QueryFrames *qf) {
     Ctx *ctx = ix->ctx;
     if (nq == 0) return PCR_OK;
+    if (ix->n_frames != 1) {  // external queries of a batch: frame-local indices
+        if (!qf || qf->n_frames != (size_t)ix->n_frames)
+            return fail(ctx, PCR_ERR_INVALID_ARG, "queries on a batch index of %d frames need query offsets of as many frames", ix->n_frames);
+        const uint32_t *d_qoff = nullptr;
+        PCR_TRY(upload_query_offsets(ctx, *qf, &d_qoff));
+        radius_kernel<true, true><<<(unsigned)((nq + 255) / 256), 256, 0, ctx->stream>>>(ix->grids, ix->cell_start, ix->sorted, dqx, dqy, dqz, nq,
+                                                                                         radius, nullptr, d_offsets, d_idx, d_qoff, ix->n_frames);
+        PCR_LAUNCH_CHECK(ctx);
+        return PCR_OK;
+    }
     radius_kernel<true><<<(unsigned)((nq + 255) / 256), 256, 0, ctx->stream>>>(ix->grids, ix->cell_start, ix->sorted, dqx, dqy,
                                                                                dqz, nq, radius, nullptr, d_offsets, d_idx);
     PCR_LAUNCH_CHECK(ctx);

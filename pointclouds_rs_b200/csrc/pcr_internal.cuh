@@ -141,6 +141,7 @@ struct Ctx {
     DevBuf b_scan;     // single-pass scan: ticket + one state word per tile (tagged with scan_epoch, never cleared between scans)
     uint32_t scan_epoch = 0;
     DevBuf b_list;     // deferred-query lists of the level loop
+    DevBuf b_qoff;     // u32 query offsets of the external queries of a batch index (knn.cu upload_query_offsets)
     // cell tables of TRANSIENT indices (the ones an entry point builds and frees itself), one per grid
     // level.  A 100-frame batch needs a 280 MB table: taking it from the stream-ordered pool on every
     // call cost 4-16 ms (the pool had just carved the freed block up for the smaller arrays).
@@ -260,9 +261,16 @@ int index_coarser_level(Index *ix, Index **out);
 // The finer level of `ix` (cell size / 2, or as fine as the cell-table cap allows), built on first use and owned by `ix`.
 int index_finer_level(Index *ix, Index **out);
 
-// KNN over external queries (n_frames == 1).  d_idx/d_dist row-major nq x k.
+// External queries of a batch index (pcr_*_batch): query frame f = queries [offsets[f], offsets[f+1]) (HOST, n_frames + 1
+// entries, checked by the caller) is searched in index frame f only, and the indices come back frame-local.
+struct QueryFrames {
+    const uint64_t *offsets;
+    size_t n_frames;
+};
+// KNN over external queries.  d_idx/d_dist row-major nq x k.  A multi-frame index needs qf (with its frame count); on a
+// single-frame index qf is ignored (a batch of one).
 int knn_queries_dev(Index *ix, const float *dqx, const float *dqy, const float *dqz, size_t nq,
-                    size_t k, uint32_t *d_idx, float *d_dist, uint32_t *d_counts);
+                    size_t k, uint32_t *d_idx, float *d_dist, uint32_t *d_counts, const QueryFrames *qf = nullptr);
 // mean neighbour distance of every point of the indexed cloud(s) (SOR, k+1 neighbours, drop self)
 // Neighbour lists a fused SOR -> normals pipeline keeps from its SOR pass (knn.cu): entry j of the query at
 // cell-sorted position q is lists[j * stride + q]; cnt[q] = valid entries, 0xff = no list.
@@ -291,12 +299,12 @@ int index_shard_queries(Index *ix);
 // coordinates become NaN) and makes later-built levels skip them: the index of the SOR pass is
 // reused for the normals of the kept points without a rebuild.
 int index_apply_mask_dev(Index *ix, const uint8_t *d_keep);
-// On a multi-frame index the queries must be the indexed points themselves (query i = input point i), each counted in
-// its own frame only.
+// On a multi-frame index without qf the queries must be the indexed points themselves (query i = input point i), each
+// counted in its own frame only; with qf they are external queries as in knn_queries_dev (radius_fill_dev needs qf there).
 int radius_count_dev(Index *ix, const float *dqx, const float *dqy, const float *dqz, size_t nq,
-                     float radius, uint32_t *d_counts);
+                     float radius, uint32_t *d_counts, const QueryFrames *qf = nullptr);
 int radius_fill_dev(Index *ix, const float *dqx, const float *dqy, const float *dqz, size_t nq,
-                    float radius, const uint64_t *d_offsets, uint32_t *d_idx);
+                    float radius, const uint64_t *d_offsets, uint32_t *d_idx, const QueryFrames *qf = nullptr);
 
 // SOR statistics + mask (statistical_outlier.rs:43-66), one segment per frame.  d_stats receives
 // per frame {mean, stddev, threshold, n_finite(as float bits)}; d_kept per-frame kept counts.
@@ -329,7 +337,7 @@ struct IcpBatchArgs {
 };
 int icp_batch_dev(Ctx *ctx, const IcpBatchArgs &a, pcr_icp_result *results);
 int find_correspondences_dev(Index *target, const float *dsx, const float *dsy, const float *dsz,
-                             size_t ns, float max_distance, uint32_t *d_tgt, float *d_dist);
+                             size_t ns, float max_distance, uint32_t *d_tgt, float *d_dist, const QueryFrames *qf = nullptr);
 int apply_transform_dev(Ctx *ctx, const float *dx, const float *dy, const float *dz, size_t n,
                         const float R[9], const float t[3], float *ox, float *oy, float *oz);
 
