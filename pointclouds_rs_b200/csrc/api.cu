@@ -596,12 +596,11 @@ static int sor_core(Ctx *c, const float *dx, const float *dy, const float *dz, s
     bo.transient = true;
     Index *ix = nullptr;
     PCR_TRY(index_build_dev(c, dx, dy, dz, n, bo, &ix));
+    const IndexPtr guard(ix);
     // (a query-sharded context: every rank searches its share, the mean distances are merged, and every rank runs the
     // same exact fold over all of them -- the statistics and the mask do not depend on the number of ranks)
-    int s = sor_mean_dist_dev(ix, k, d_mean, nullptr, c->shard_queries);
-    if (s == PCR_OK) s = sor_threshold_mask_dev(c, d_mean, nullptr, 1, n, std_mul, d_keep, d_stats, d_kept);
-    index_free(ix);
-    return s;
+    PCR_TRY(sor_mean_dist_dev(ix, k, d_mean, nullptr, c->shard_queries));
+    return sor_threshold_mask_dev(c, d_mean, nullptr, 1, n, std_mul, d_keep, d_stats, d_kept);
 }
 
 int pcr_sor_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z, size_t n, size_t k, float std_mul,
@@ -713,10 +712,7 @@ static int ror_core(Ctx *c, const float *dx, const float *dy, const float *dz, s
     int s = index_build_dev(c, dx, dy, dz, n, bo, &ix);
     c->forced_cell = saved;
     PCR_TRY(s);
-    struct G {
-        Index *ix;
-        ~G() { index_free(ix); }
-    } g{ix};
+    const IndexPtr guard(ix);
     PCR_TRY(ensure(c, c->b_misc, n * sizeof(uint32_t)));
     uint32_t *d_cnt = (uint32_t *)c->b_misc.p;
     if (!frame_offsets && query_sharding_active(c, ix)) {
@@ -871,9 +867,8 @@ int pcr_estimate_normals_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, c
     bo.transient = true;
     Index *ix = nullptr;
     PCR_TRY(index_build_dev(c, d_x, d_y, d_z, n, bo, &ix));
-    int s = normals_dev(ix, k, viewpoint, d_nx, d_ny, d_nz, nullptr, c->shard_queries);
-    index_free(ix);
-    return s;
+    const IndexPtr guard(ix);
+    return normals_dev(ix, k, viewpoint, d_nx, d_ny, d_nz, nullptr, c->shard_queries);
     PCR_API_END(c)
 }
 
@@ -897,9 +892,7 @@ int pcr_estimate_normals(pcr_ctx *ctx, const float *x, const float *y, const flo
     bo.transient = true;
     Index *ix = nullptr;
     PCR_TRY(index_build_dev(c, dx, dy, dz, n, bo, &ix));
-    int s = normals_dev(ix, k, viewpoint, dnx, dny, dnz, nullptr, c->shard_queries);
-    index_free(ix);
-    PCR_TRY(s);
+    PCR_TRY(normals_dev(IndexPtr(ix).get(), k, viewpoint, dnx, dny, dnz, nullptr, c->shard_queries));  // (freed before the copies)
     PCR_CUDA(c, cudaMemcpyAsync(nx, dnx, n * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
     PCR_CUDA(c, cudaMemcpyAsync(ny, dny, n * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
     PCR_CUDA(c, cudaMemcpyAsync(nz, dnz, n * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
@@ -1040,13 +1033,13 @@ int pcr_icp_point_to_plane_dev(pcr_ctx *ctx, const float *sx, const float *sy, c
     return icp_entry(ctx, true, true, sx, sy, sz, ns, tx, ty, tz, nt, nx, ny, nz, n_normals, params, result);
 }
 
-// Frame offsets of a batch call (ICP, voxel_downsample, estimate_normals, RANSAC and clustering batches): frame f = points
-// [frame_offsets[f], frame_offsets[f+1]), starting at 0, never decreasing.
-static int batch_offsets_check(Ctx *c, const uint64_t *frame_offsets, size_t n_frames) {
-    if (!frame_offsets) return fail(c, PCR_ERR_INVALID_ARG, "frame_offsets is NULL");
-    if (frame_offsets[0] != 0) return fail(c, PCR_ERR_INVALID_ARG, "frame_offsets must start at 0");
+// Offsets of a batch argument (frame, query, sample or index offsets; `name` names it in the message): frame f = entries
+// [offsets[f], offsets[f+1]), starting at 0, never decreasing.
+static int offsets_check(Ctx *c, const char *name, const uint64_t *offsets, size_t n_frames) {
+    if (!offsets) return fail(c, PCR_ERR_INVALID_ARG, "%s is NULL", name);
+    if (offsets[0] != 0) return fail(c, PCR_ERR_INVALID_ARG, "%s must start at 0", name);
     for (size_t f = 0; f < n_frames; f++)
-        if (frame_offsets[f + 1] < frame_offsets[f]) return fail(c, PCR_ERR_INVALID_ARG, "frame_offsets must be non-decreasing");
+        if (offsets[f + 1] < offsets[f]) return fail(c, PCR_ERR_INVALID_ARG, "%s must be non-decreasing", name);
     return PCR_OK;
 }
 // ... and the sizes their kernels are built for: u32 point indices, one grid row per frame
@@ -1065,7 +1058,7 @@ static int icp_batch_entry(pcr_ctx *ctx, bool dev, bool plane, const float *x, c
     PCR_TRY(icp_check(c, params, results));
     for (size_t p = 0; p < n_pairs; p++) icp_identity(&results[p]);
     if (n_pairs && !pairs) return fail(c, PCR_ERR_INVALID_ARG, "pairs is NULL");
-    PCR_TRY(batch_offsets_check(c, frame_offsets, n_frames));
+    PCR_TRY(offsets_check(c, "frame_offsets", frame_offsets, n_frames));
     const size_t n = (size_t)frame_offsets[n_frames];
     if (plane && n_normals != n)  // icp_plane.rs:27-32, for the whole buffer
         return fail(c, PCR_ERR_NORMALS_MISMATCH, "normals length (%zu) does not match the number of points (%zu)", n_normals, n);
@@ -1129,7 +1122,7 @@ static int voxel_batch_entry(pcr_ctx *ctx, bool dev, const float *x, const float
     Ctx *c = &ctx->c;
     if (!out_offsets) return fail(c, PCR_ERR_INVALID_ARG, "out_offsets is NULL");
     out_offsets[0] = 0;
-    PCR_TRY(batch_offsets_check(c, frame_offsets, n_frames));
+    PCR_TRY(offsets_check(c, "frame_offsets", frame_offsets, n_frames));
     for (size_t f = 1; f <= n_frames; f++) out_offsets[f] = 0;
     const size_t n = (size_t)frame_offsets[n_frames];
     PCR_TRY(batch_size_check(c, n, n_frames));
@@ -1177,16 +1170,15 @@ static int normals_batch_core(Ctx *c, const float *dx, const float *dy, const fl
     bo.transient = true;
     Index *ix = nullptr;
     PCR_TRY(index_build_dev(c, dx, dy, dz, n, bo, &ix));
-    const int s = normals_dev(ix, k, vp, d_nx, d_ny, d_nz, nullptr, /*allow_shard=*/false);
-    index_free(ix);
-    return s;
+    const IndexPtr guard(ix);
+    return normals_dev(ix, k, vp, d_nx, d_ny, d_nz, nullptr, /*allow_shard=*/false);
 }
 
 static int normals_batch_entry(pcr_ctx *ctx, bool dev, const float *x, const float *y, const float *z, const uint64_t *frame_offsets,
                                size_t n_frames, size_t k, const float viewpoint[3], float *nx, float *ny, float *nz) {
     if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
     Ctx *c = &ctx->c;
-    PCR_TRY(batch_offsets_check(c, frame_offsets, n_frames));
+    PCR_TRY(offsets_check(c, "frame_offsets", frame_offsets, n_frames));
     const size_t n = (size_t)frame_offsets[n_frames];
     PCR_TRY(batch_size_check(c, n, n_frames));
     if (n == 0 || k == 0) return PCR_OK;  // estimate.rs:25-31, as the single call
@@ -1227,7 +1219,7 @@ static int index_build_batch_entry(pcr_ctx *ctx, bool dev, const float *x, const
     *out = nullptr;
     Ctx *c = &ctx->c;
     if (n_frames == 0) return fail(c, PCR_ERR_INVALID_ARG, "a batch index holds at least one frame");
-    PCR_TRY(batch_offsets_check(c, frame_offsets, n_frames));
+    PCR_TRY(offsets_check(c, "frame_offsets", frame_offsets, n_frames));
     const size_t n = (size_t)frame_offsets[n_frames];
     PCR_TRY(batch_size_check(c, n, n_frames));
     if (n && (!x || !y || !z)) return fail(c, PCR_ERR_INVALID_ARG, "x/y/z is NULL");
@@ -1259,10 +1251,10 @@ int pcr_index_build_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, 
     return index_build_batch_entry(ctx, true, d_x, d_y, d_z, frame_offsets, n_frames, k_hint, out);
 }
 
-// The query side of a batch call: offsets as batch_offsets_check, as many frames as the index, at most 0xfffffff0 queries.
+// The query side of a batch call: offsets as offsets_check, as many frames as the index, at most 0xfffffff0 queries.
 static int batch_query_check(const Index *ix, const uint64_t *query_offsets, size_t n_frames, size_t *nq) {
     Ctx *c = ix->ctx;
-    PCR_TRY(batch_offsets_check(c, query_offsets, n_frames));
+    PCR_TRY(offsets_check(c, "query_offsets", query_offsets, n_frames));
     if (n_frames != (size_t)ix->n_frames)
         return fail(c, PCR_ERR_INVALID_ARG, "%zu query frames for an index of %d frames", n_frames, ix->n_frames);
     *nq = (size_t)query_offsets[n_frames];
@@ -1434,14 +1426,12 @@ static int ransac_batch_entry(pcr_ctx *ctx, bool dev, const float *x, const floa
     Ctx *c = &ctx->c;
     if (!models || !inlier_offsets) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     inlier_offsets[0] = 0;
-    PCR_TRY(batch_offsets_check(c, frame_offsets, n_frames));
+    PCR_TRY(offsets_check(c, "frame_offsets", frame_offsets, n_frames));
     for (size_t f = 1; f <= n_frames; f++) inlier_offsets[f] = 0;
     const size_t n = (size_t)frame_offsets[n_frames];
     PCR_TRY(batch_size_check(c, n, n_frames));
     if (sample_offsets) {
-        if (sample_offsets[0] != 0) return fail(c, PCR_ERR_INVALID_ARG, "sample_offsets must start at 0");
-        for (size_t f = 0; f < n_frames; f++)
-            if (sample_offsets[f + 1] < sample_offsets[f]) return fail(c, PCR_ERR_INVALID_ARG, "sample_offsets must be non-decreasing");
+        PCR_TRY(offsets_check(c, "sample_offsets", sample_offsets, n_frames));
         if (sample_offsets[n_frames] && !samples) return fail(c, PCR_ERR_INVALID_ARG, "samples is NULL");
         if (sample_offsets[n_frames] > 0x7fffffffull) return fail(c, PCR_ERR_UNSUPPORTED, "at most 2^31 - 1 sample triples per batch");
     } else if (samples) {
@@ -1490,7 +1480,7 @@ static int cluster_batch_entry(pcr_ctx *ctx, bool in_dev, bool dev, const float 
     if (!offsets || !cluster_offsets) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     cluster_offsets[0] = 0;
     if (!dev) offsets[0] = 0;
-    PCR_TRY(batch_offsets_check(c, frame_offsets, n_frames));
+    PCR_TRY(offsets_check(c, "frame_offsets", frame_offsets, n_frames));
     for (size_t f = 1; f <= n_frames; f++) cluster_offsets[f] = 0;
     const size_t n = (size_t)frame_offsets[n_frames];
     PCR_TRY(batch_size_check(c, n, n_frames));
@@ -1545,7 +1535,7 @@ int pcr_cluster_labels_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_
                                  size_t n_frames, float distance_threshold, uint32_t *d_labels) {
     if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
     Ctx *c = &ctx->c;
-    PCR_TRY(batch_offsets_check(c, frame_offsets, n_frames));
+    PCR_TRY(offsets_check(c, "frame_offsets", frame_offsets, n_frames));
     const size_t n = (size_t)frame_offsets[n_frames];
     PCR_TRY(batch_size_check(c, n, n_frames));
     if (n && (!d_x || !d_y || !d_z || !d_labels)) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
@@ -1563,7 +1553,7 @@ static int ror_batch_entry(pcr_ctx *ctx, bool dev, const float *x, const float *
                            size_t n_frames, float radius, size_t min_neighbors, uint8_t *keep, uint64_t *n_kept_per_frame) {
     if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
     Ctx *c = &ctx->c;
-    PCR_TRY(batch_offsets_check(c, frame_offsets, n_frames));
+    PCR_TRY(offsets_check(c, "frame_offsets", frame_offsets, n_frames));
     if (n_kept_per_frame)
         for (size_t f = 0; f < n_frames; f++) n_kept_per_frame[f] = 0;
     const size_t n = (size_t)frame_offsets[n_frames];
@@ -1625,17 +1615,10 @@ static int batch_core(Ctx *c, const float *dx, const float *dy, const float *dz,
                       const CloudStats *known_stats = nullptr /* single frame: its box and finite count, if already measured */,
                       bool allow_nowait = true /* false: the redo of a call whose unawaited deferred counts were not zero */) {
     const int F = (int)n_frames;
-    float *d_mean = nullptr, *d_stats = nullptr;
-    PCR_CUDA(c, cudaMallocAsync((void **)&d_mean, sizeof(float) * std::max<size_t>(n, 1), c->stream));
-    struct FreeLater {
-        void *p;
-        cudaStream_t s;
-        ~FreeLater() {
-            if (p) cudaFreeAsync(p, s);
-        }
-    } f1{d_mean, c->stream};
-    PCR_CUDA(c, cudaMallocAsync((void **)&d_stats, sizeof(float) * 4 * F, c->stream));
-    FreeLater f2{d_stats, c->stream};
+    StreamAlloc<float> mean_mem(c->stream), stats_mem(c->stream);
+    PCR_CUDA(c, mean_mem.alloc(sizeof(float) * std::max<size_t>(n, 1)));
+    PCR_CUDA(c, stats_mem.alloc(sizeof(float) * 4 * F));
+    float *d_mean = mean_mem.p, *d_stats = stats_mem.p;
 
     // ONE index serves both stages: built for the larger k, then the points SOR removes are
     // tombstoned in place (NaN coordinates) and the normals of the kept points run on the same grid.
@@ -1651,15 +1634,13 @@ static int batch_core(Ctx *c, const float *dx, const float *dy, const float *dz,
     const bool may_fuse = !no_fuse && k_sor > 0 && k_normals > 0 && K <= 32 && n > 1;
     SorLists sl;
     bool early = false;
-    void *list_mem = nullptr;
-    FreeLater f3{nullptr, c->stream};
+    StreamAlloc<uint32_t> list_mem(c->stream);
     if (may_fuse) {
         sl.K = K;
         sl.stride = (n + 63) & ~(size_t)63;  // (>= the indexed points, whose number the build has yet to report)
         const size_t bytes = sizeof(uint32_t) * (K * sl.stride + sl.stride + 64) + sl.stride;
-        PCR_CUDA(c, cudaMallocAsync(&list_mem, bytes, c->stream));
-        f3.p = list_mem;
-        sl.lists = (uint32_t *)list_mem;
+        PCR_CUDA(c, list_mem.alloc(bytes));
+        sl.lists = list_mem.p;
         sl.fallback = sl.lists + K * sl.stride;
         sl.cnt = (uint8_t *)(sl.fallback + sl.stride + 64);
         PCR_CUDA(c, cudaMemsetAsync(sl.fallback + sl.stride, 0, 64 * sizeof(uint32_t), c->stream));  // the fallback counter (and its padding)
@@ -1680,10 +1661,7 @@ static int batch_core(Ctx *c, const float *dx, const float *dy, const float *dz,
     PCR_MARK("core: build begin");
     PCR_TRY(index_build_dev(c, dx, dy, dz, n, bo, &ix));
     PCR_MARK("core: build queued");
-    struct IxGuard {
-        Index *ix;
-        ~IxGuard() { index_free(ix); }
-    } g{ix};
+    const IndexPtr guard(ix);
     const bool fused = may_fuse && ix->n_indexed > 0;
     struct EarlyJoin {  // an error return between the early normals pass and its join: the lists are freed in stream order
         Ctx *c;
@@ -1736,6 +1714,12 @@ static int batch_core(Ctx *c, const float *dx, const float *dy, const float *dz,
     return normals_dev(ix, k_normals, vp, d_nx, d_ny, d_nz, d_keep);
 }
 
+// The parameters the three pcr_sor_normals_batch forms check after their offsets and pointers
+static int sor_normals_batch_check(Ctx *c, size_t n, size_t n_frames, size_t k_sor, float std_mul, size_t k_normals) {
+    if (!std::isfinite(std_mul) || std_mul < 0.f) return fail(c, PCR_ERR_INVALID_ARG, "std_mul must be >= 0 and finite");
+    if (k_sor + 1 > PCR_MAX_K || k_normals > PCR_MAX_K) return fail(c, PCR_ERR_UNSUPPORTED, "k exceeds PCR_MAX_K");
+    return batch_size_check(c, n, n_frames);
+}
 
 int pcr_sor_normals_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z, const uint64_t *frame_offsets,
                               size_t n_frames, size_t k_sor, float std_mul, size_t k_normals, const float viewpoint[3],
@@ -1743,22 +1727,19 @@ int pcr_sor_normals_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, 
     if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
     Ctx *c = &ctx->c;
     if (n_frames == 0) return PCR_OK;
-    if (!frame_offsets) return fail(c, PCR_ERR_INVALID_ARG, "frame_offsets is NULL");
+    PCR_TRY(offsets_check(c, "frame_offsets", frame_offsets, n_frames));
     const size_t n = (size_t)frame_offsets[n_frames];
     if (n == 0) return PCR_OK;
     if (!d_x || !d_y || !d_z || !d_keep || !viewpoint || (k_normals && (!d_nx || !d_ny || !d_nz)))
         return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
-    if (!std::isfinite(std_mul) || std_mul < 0.f) return fail(c, PCR_ERR_INVALID_ARG, "std_mul must be >= 0 and finite");
-    if (k_sor + 1 > PCR_MAX_K || k_normals > PCR_MAX_K) return fail(c, PCR_ERR_UNSUPPORTED, "k exceeds PCR_MAX_K");
-    if (n_frames > 65535) return fail(c, PCR_ERR_UNSUPPORTED, "at most 65535 frames per batch");
+    PCR_TRY(sor_normals_batch_check(c, n, n_frames, k_sor, std_mul, k_normals));
     PCR_API_BEGIN
     DevSetter ds(c);
     PCR_MARK("batch_dev: enter");
-    unsigned long long *d_kept = nullptr;
-    PCR_CUDA(c, cudaMallocAsync((void **)&d_kept, sizeof(unsigned long long) * n_frames, c->stream));
-    int s = batch_core(c, d_x, d_y, d_z, frame_offsets, n_frames, n, k_sor, std_mul, k_normals, viewpoint, d_keep, d_nx, d_ny, d_nz,
-                       d_kept);
-    cudaFreeAsync(d_kept, c->stream);
+    StreamAlloc<unsigned long long> d_kept(c->stream);
+    PCR_CUDA(c, d_kept.alloc(sizeof(unsigned long long) * n_frames));
+    const int s = batch_core(c, d_x, d_y, d_z, frame_offsets, n_frames, n, k_sor, std_mul, k_normals, viewpoint, d_keep, d_nx, d_ny, d_nz,
+                             d_kept.p);
     if (g_trace_on) {  // (tracing only: the entry point itself is asynchronous)
         cudaStreamSynchronize(c->stream);
         PCR_MARK("batch_dev: synced, exit");
@@ -1773,14 +1754,12 @@ int pcr_sor_normals_batch(pcr_ctx *ctx, const float *x, const float *y, const fl
     if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
     Ctx *c = &ctx->c;
     if (n_frames == 0) return PCR_OK;
-    if (!frame_offsets) return fail(c, PCR_ERR_INVALID_ARG, "frame_offsets is NULL");
+    PCR_TRY(offsets_check(c, "frame_offsets", frame_offsets, n_frames));
     const size_t n = (size_t)frame_offsets[n_frames];
     if (n_kept_per_frame) memset(n_kept_per_frame, 0, sizeof(uint64_t) * n_frames);
     if (n == 0) return PCR_OK;
     if (!x || !y || !z || !keep || !viewpoint || (k_normals && (!nx || !ny || !nz))) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
-    if (!std::isfinite(std_mul) || std_mul < 0.f) return fail(c, PCR_ERR_INVALID_ARG, "std_mul must be >= 0 and finite");
-    if (k_sor + 1 > PCR_MAX_K || k_normals > PCR_MAX_K) return fail(c, PCR_ERR_UNSUPPORTED, "k exceeds PCR_MAX_K");
-    if (n_frames > 65535) return fail(c, PCR_ERR_UNSUPPORTED, "at most 65535 frames per batch");
+    PCR_TRY(sor_normals_batch_check(c, n, n_frames, k_sor, std_mul, k_normals));
     PCR_API_BEGIN
     DevSetter ds(c);
     float *dx, *dy, *dz;
@@ -1813,13 +1792,14 @@ int pcr_sor_normals_batch(pcr_ctx *ctx, const float *x, const float *y, const fl
 /* ---- device-resident clouds (SURVEY 8f-3) -------------------------------------------------------------
  * PointCloud (crates/core/src/cloud.rs:4-18) kept in HBM between the steps of a pipeline
  * (voxel -> SOR -> normals -> cluster / ICP): one upload, one download, `select` as a device
- * compaction.  Layout: one allocation, x | y | z | (nx | ny | nz), every array 256 B aligned. */
-struct pcr_cloud {
-    pcr_ctx *owner;
-    size_t n, stride;
-    float *base;
-    bool has_normals;
-    pcr::CloudStats stats;  // bounding box + finite count if the step that wrote the cloud measured them (stats.valid)
+ * compaction.  DevPoints is the storage of both handles (pcr_cloud and the frame batch pcr_frames):
+ * one allocation, x | y | z | (nx | ny | nz), every array `stride` floats apart and 256 B aligned. */
+struct DevPoints {
+    pcr_ctx *owner = nullptr;
+    size_t n = 0, stride = 0;
+    float *base = nullptr;
+    bool has_normals = false;
+    int arrays() const { return has_normals ? 6 : 3; }
     float *x() const { return base; }
     float *y() const { return base + stride; }
     float *z() const { return base + 2 * stride; }
@@ -1828,26 +1808,44 @@ struct pcr_cloud {
     float *nz() const { return base + 5 * stride; }
 };
 
+struct pcr_cloud : DevPoints {
+    pcr::CloudStats stats;  // bounding box + finite count if the step that wrote the cloud measured them (stats.valid)
+};
+
 namespace pcr {
 namespace {
 
-int cloud_alloc(pcr_ctx *ctx, size_t n, bool normals, pcr_cloud **out) {
-    Ctx *c = &ctx->c;
-    pcr_cloud *cl = new (std::nothrow) pcr_cloud();
-    if (!cl) return fail(c, PCR_ERR_OOM, "host allocation failed");
-    cl->owner = ctx;
-    cl->n = n;
-    cl->stride = std::max<size_t>((n + 63) & ~(size_t)63, 64);
-    cl->has_normals = normals;
-    cl->base = nullptr;
-    cudaError_t e = cudaMallocAsync((void **)&cl->base, sizeof(float) * cl->stride * (normals ? 6 : 3), c->stream);
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        delete cl;
-        return fail(c, PCR_ERR_OOM, "device allocation failed: %s", cudaGetErrorString(e));
-    }
-    *out = cl;
+// Owning handles: a failed call frees what it built, and `*out = h.release()` is the only place a handle is handed out.
+struct HandleFree {
+    void operator()(pcr_cloud *h) const { pcr_cloud_free(h); }
+    void operator()(pcr_frames *h) const { pcr_frames_free(h); }
+};
+using CloudPtr = std::unique_ptr<pcr_cloud, HandleFree>;
+using FramesPtr = std::unique_ptr<pcr_frames, HandleFree>;
+
+// A new handle of n points on ctx, `tail` more bytes after its arrays (a frame batch keeps its offsets there).
+template <class H>
+int points_alloc(pcr_ctx *ctx, size_t n, bool normals, std::unique_ptr<H, HandleFree> &out, size_t tail = 0) {
+    std::unique_ptr<H, HandleFree> h(new H());
+    h->owner = ctx;
+    h->n = n;
+    h->stride = std::max<size_t>((n + 63) & ~(size_t)63, 64);
+    h->has_normals = normals;
+    float *base = nullptr;
+    PCR_CUDA(&ctx->c, cudaMallocAsync((void **)&base, sizeof(float) * h->stride * h->arrays() + tail, ctx->c.stream));
+    h->base = base;
+    out = std::move(h);
     return PCR_OK;
+}
+
+template <class H>
+void handle_free(H *h) {
+    if (!h) return;
+    if (h->base && h->owner) {
+        DevSetter ds(&h->owner->c);
+        cudaFreeAsync(h->base, h->owner->c.stream);
+    }
+    delete h;
 }
 
 __global__ void mask_to_u32_kernel(const uint8_t *__restrict__ keep, size_t n, uint32_t *__restrict__ flag) {
@@ -1913,37 +1911,122 @@ int keep_scan(Ctx *c, const uint8_t *d_keep, size_t n, uint32_t **pos_out) {
     return PCR_OK;
 }
 
-// new cloud = the points of `in` with keep != 0.  `nrm` (optional): normals of the points of `in`, three rows
-// `nrm_stride` apart, for an `in` that carries none.  `known_m`: the number of kept points if the caller
+// The second half of every compaction: the points of `in` whose pos[i + 1] != pos[i] go to row pos[i] of `out`, in order,
+// normals along.  `nrm` (optional): normals of the points of `in`, three rows `nrm_stride` apart, for an `in` that
+// carries none.
+int compact_into(const DevPoints *in, const uint32_t *pos, const float *nrm, size_t nrm_stride, const DevPoints *out) {
+    if (!out->n) return PCR_OK;
+    Ctx *c = &in->owner->c;
+    const int n_a = nrm ? 3 : in->arrays(), n_b = nrm ? 3 : 0;
+    c->launches++;
+    PCR_CUDA(c, launch_chained(compact_kernel, dim3((unsigned)((in->n + 255) / 256)), dim3(256), 0, c->stream, in->base, in->stride, n_a, nrm,
+                               nrm_stride, n_b, in->n, pos, out->base, out->stride));
+    return PCR_OK;
+}
+
+// new cloud = the points of `in` with keep != 0 (see compact_into).  `known_m`: the number of kept points if the caller
 // already has it on the host (saves the round trip), else SIZE_MAX.
-int cloud_compact(const pcr_cloud *in, const uint8_t *d_keep, pcr_cloud **out, const float *nrm = nullptr, size_t nrm_stride = 0,
+int cloud_compact(const pcr_cloud *in, const uint8_t *d_keep, CloudPtr &out, const float *nrm = nullptr, size_t nrm_stride = 0,
                   size_t known_m = SIZE_MAX) {
     Ctx *c = &in->owner->c;
-    const size_t n = in->n;
     uint32_t *pos = nullptr;
-    PCR_TRY(keep_scan(c, d_keep, n, &pos));
+    PCR_TRY(keep_scan(c, d_keep, in->n, &pos));
     size_t m = known_m;
     if (m == SIZE_MAX) {
         uint32_t *mail = (uint32_t *)c->pinned + 96;
-        PCR_CUDA(c, cudaMemcpyAsync(mail, pos + n, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+        PCR_CUDA(c, cudaMemcpyAsync(mail, pos + in->n, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
         PCR_CUDA(c, cudaStreamSynchronize(c->stream));
         m = *mail;
     }
-    const bool with_normals = nrm || in->has_normals;
-    pcr_cloud *tmp = nullptr;  // *out is set on success only: a failed call hands the caller no live handle
-    PCR_TRY(cloud_alloc(in->owner, m, with_normals, &tmp));
-    if (m) {
-        const int n_a = nrm ? 3 : (in->has_normals ? 6 : 3), n_b = nrm ? 3 : 0;
-        const cudaError_t e = launch_chained(compact_kernel, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, c->stream, in->base, in->stride, n_a, nrm,
-                                             nrm_stride, n_b, n, pos, tmp->base, tmp->stride);
-        c->launches++;
-        if (e != cudaSuccess) {
-            pcr_cloud_free(tmp);
-            return fail(c, PCR_ERR_CUDA, "kernel launch failed: %s (%s:%d)", cudaGetErrorString(e), __FILE__, __LINE__);
+    PCR_TRY(points_alloc(in->owner, m, nrm || in->has_normals, out));
+    return compact_into(in, pos, nrm, nrm_stride, out.get());
+}
+
+// the first `arrays` arrays of dst <- those of src from point `first` on, dst->n points each
+int copy_arrays(const DevPoints *src, size_t first, int arrays, const DevPoints *dst) {
+    Ctx *c = &src->owner->c;
+    for (int a = 0; dst->n && a < arrays; a++)
+        PCR_CUDA(c, cudaMemcpyAsync(dst->base + (size_t)a * dst->stride, src->base + (size_t)a * src->stride + first, sizeof(float) * dst->n,
+                                    cudaMemcpyDeviceToDevice, c->stream));
+    return PCR_OK;
+}
+
+// The end of an upload: wait, so that the caller's buffers are free again on return, then report the first error.
+int upload_wait(Ctx *c, cudaError_t upload) {
+    const cudaError_t sync = cudaStreamSynchronize(c->stream);
+    PCR_CUDA(c, upload);
+    PCR_CUDA(c, sync);
+    return PCR_OK;
+}
+
+// host x, y, z (n floats each) into the first three arrays of p
+int points_upload(const DevPoints *p, const float *x, const float *y, const float *z) {
+    Ctx *c = &p->owner->c;
+    const float *src[3] = {x, y, z};
+    cudaError_t upload = cudaSuccess;
+    for (int a = 0; p->n && a < 3 && upload == cudaSuccess; a++)
+        upload = cudaMemcpyAsync(p->base + (size_t)a * p->stride, src[a], sizeof(float) * p->n, cudaMemcpyHostToDevice, c->stream);
+    return upload_wait(c, upload);
+}
+
+// Row-major (N, 3) in and out (the PyO3 surface's layout): one contiguous transfer, (de)interleaved on the device.
+int points_upload_rows(const DevPoints *p, const float *xyz) {
+    Ctx *c = &p->owner->c;
+    const size_t n = p->n;
+    cudaError_t upload = cudaSuccess;
+    if (n) {
+        PCR_TRY(ensure(c, c->b_in, sizeof(float) * 3 * n));
+        upload = cudaMemcpyAsync(c->b_in.p, xyz, sizeof(float) * 3 * n, cudaMemcpyHostToDevice, c->stream);
+        if (upload == cudaSuccess) {
+            rows_to_soa_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>((const float *)c->b_in.p, n, p->base, p->stride);
+            c->launches++;
+            upload = cudaGetLastError();
         }
     }
-    *out = tmp;
+    return upload_wait(c, upload);
+}
+
+int points_download_rows(const DevPoints *p, float *xyz, float *normals) {
+    Ctx *c = &p->owner->c;
+    const size_t n = p->n, row = sizeof(float) * 3 * n;
+    PCR_TRY(ensure(c, c->b_out, 2 * row));
+    float *d_xyz = (float *)c->b_out.p, *d_nrm = d_xyz + 3 * n;
+    const unsigned blocks = (unsigned)((n + 255) / 256);
+    if (xyz) {
+        soa_to_rows_kernel<<<blocks, 256, 0, c->stream>>>(p->base, p->stride, n, d_xyz);
+        PCR_LAUNCH_CHECK(c);
+        PCR_CUDA(c, cudaMemcpyAsync(xyz, d_xyz, row, cudaMemcpyDeviceToHost, c->stream));
+    }
+    if (normals) {
+        soa_to_rows_kernel<<<blocks, 256, 0, c->stream>>>(p->nx(), p->stride, n, d_nrm);
+        PCR_LAUNCH_CHECK(c);
+        PCR_CUDA(c, cudaMemcpyAsync(normals, d_nrm, row, cudaMemcpyDeviceToHost, c->stream));
+    }
+    PCR_CUDA(c, cudaStreamSynchronize(c->stream));
     return PCR_OK;
+}
+
+// any of the six arrays to the host (n floats each): a NULL destination is skipped
+int points_download(const DevPoints *p, float *x, float *y, float *z, float *nx, float *ny, float *nz) {
+    Ctx *c = &p->owner->c;
+    float *const dst[6] = {x, y, z, nx, ny, nz};
+    for (int a = 0; a < 6; a++)
+        if (dst[a]) PCR_CUDA(c, cudaMemcpyAsync(dst[a], p->base + (size_t)a * p->stride, sizeof(float) * p->n, cudaMemcpyDeviceToHost, c->stream));
+    PCR_CUDA(c, cudaStreamSynchronize(c->stream));
+    return PCR_OK;
+}
+
+void points_device_pointers(const DevPoints *p, const float **d_x, const float **d_y, const float **d_z, const float **d_nx, const float **d_ny,
+                            const float **d_nz) {
+    const float **const dst[6] = {d_x, d_y, d_z, d_nx, d_ny, d_nz};
+    for (int a = 0; a < 6; a++)
+        if (dst[a]) *dst[a] = a < p->arrays() ? p->base + (size_t)a * p->stride : nullptr;
+}
+
+// a handle argument of a pcr_cloud_* / pcr_frames_* call: `what` names it
+int handle_check(const DevPoints *h, const char *what) {
+    if (h && h->owner) return PCR_OK;
+    return fail(nullptr, PCR_ERR_INVALID_ARG, "%s is NULL", what);
 }
 
 }  // namespace
@@ -1952,10 +2035,6 @@ int cloud_compact(const pcr_cloud *in, const uint8_t *d_keep, pcr_cloud **out, c
 
 extern "C" {
 
-#define PCR_CLOUD_CHECK(cl)                                                             \
-    if (!(cl) || !(cl)->owner) return fail(nullptr, PCR_ERR_INVALID_ARG, "cloud is NULL"); \
-    Ctx *c = &(cl)->owner->c;
-
 int pcr_cloud_upload(pcr_ctx *ctx, const float *x, const float *y, const float *z, size_t n, pcr_cloud **out) {
     if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
     Ctx *c = &ctx->c;
@@ -1963,80 +2042,49 @@ int pcr_cloud_upload(pcr_ctx *ctx, const float *x, const float *y, const float *
     *out = nullptr;
     PCR_API_BEGIN
     DevSetter ds(c);
-    pcr_cloud *cl = nullptr;
-    PCR_TRY(cloud_alloc(ctx, n, false, &cl));
-    cudaError_t e = cudaSuccess;
-    if (n) {
-        e = cudaMemcpyAsync(cl->x(), x, sizeof(float) * n, cudaMemcpyHostToDevice, c->stream);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(cl->y(), y, sizeof(float) * n, cudaMemcpyHostToDevice, c->stream);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(cl->z(), z, sizeof(float) * n, cudaMemcpyHostToDevice, c->stream);
-    }
-    const cudaError_t es = cudaStreamSynchronize(c->stream);  // the caller's buffers are free again on return
-    if (e == cudaSuccess) e = es;
-    if (e != cudaSuccess) {
-        pcr_cloud_free(cl);
-        return fail(c, PCR_ERR_CUDA, "upload failed: %s", cudaGetErrorString(e));
-    }
-    *out = cl;
+    CloudPtr res;
+    PCR_TRY(points_alloc(ctx, n, false, res));
+    PCR_TRY(points_upload(res.get(), x, y, z));
+    *out = res.release();
     return PCR_OK;
     PCR_API_END(c)
 }
 
-void pcr_cloud_free(pcr_cloud *cloud) {
-    if (!cloud) return;
-    if (cloud->base && cloud->owner) {
-        DevSetter ds(&cloud->owner->c);
-        cudaFreeAsync(cloud->base, cloud->owner->c.stream);
-    }
-    delete cloud;
-}
+void pcr_cloud_free(pcr_cloud *cloud) { handle_free(cloud); }
 
 size_t pcr_cloud_len(const pcr_cloud *cloud) { return cloud ? cloud->n : 0; }
 int pcr_cloud_has_normals(const pcr_cloud *cloud) { return cloud && cloud->has_normals ? 1 : 0; }
 
 int pcr_cloud_device_pointers(const pcr_cloud *cloud, const float **d_x, const float **d_y, const float **d_z, const float **d_nx,
                               const float **d_ny, const float **d_nz) {
-    PCR_CLOUD_CHECK(cloud)
-    (void)c;
-    if (d_x) *d_x = cloud->x();
-    if (d_y) *d_y = cloud->y();
-    if (d_z) *d_z = cloud->z();
-    if (d_nx) *d_nx = cloud->has_normals ? cloud->nx() : nullptr;
-    if (d_ny) *d_ny = cloud->has_normals ? cloud->ny() : nullptr;
-    if (d_nz) *d_nz = cloud->has_normals ? cloud->nz() : nullptr;
+    PCR_TRY(handle_check(cloud, "cloud"));
+    points_device_pointers(cloud, d_x, d_y, d_z, d_nx, d_ny, d_nz);
     return PCR_OK;
 }
 
 int pcr_cloud_download(const pcr_cloud *cloud, float *x, float *y, float *z) {
-    PCR_CLOUD_CHECK(cloud)
+    PCR_TRY(handle_check(cloud, "cloud"));
+    Ctx *c = &cloud->owner->c;
     if (cloud->n && (!x || !y || !z)) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     if (!cloud->n) return PCR_OK;
     PCR_API_BEGIN
     DevSetter ds(c);
-    PCR_CUDA(c, cudaMemcpyAsync(x, cloud->x(), sizeof(float) * cloud->n, cudaMemcpyDeviceToHost, c->stream));
-    PCR_CUDA(c, cudaMemcpyAsync(y, cloud->y(), sizeof(float) * cloud->n, cudaMemcpyDeviceToHost, c->stream));
-    PCR_CUDA(c, cudaMemcpyAsync(z, cloud->z(), sizeof(float) * cloud->n, cudaMemcpyDeviceToHost, c->stream));
-    PCR_CUDA(c, cudaStreamSynchronize(c->stream));
-    return PCR_OK;
+    return points_download(cloud, x, y, z, nullptr, nullptr, nullptr);
     PCR_API_END(c)
 }
 
 int pcr_cloud_download_normals(const pcr_cloud *cloud, float *nx, float *ny, float *nz) {
-    PCR_CLOUD_CHECK(cloud)
+    PCR_TRY(handle_check(cloud, "cloud"));
+    Ctx *c = &cloud->owner->c;
     if (!cloud->has_normals) return fail(c, PCR_ERR_INVALID_ARG, "the cloud has no normals");
     if (cloud->n && (!nx || !ny || !nz)) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     if (!cloud->n) return PCR_OK;
     PCR_API_BEGIN
     DevSetter ds(c);
-    PCR_CUDA(c, cudaMemcpyAsync(nx, cloud->nx(), sizeof(float) * cloud->n, cudaMemcpyDeviceToHost, c->stream));
-    PCR_CUDA(c, cudaMemcpyAsync(ny, cloud->ny(), sizeof(float) * cloud->n, cudaMemcpyDeviceToHost, c->stream));
-    PCR_CUDA(c, cudaMemcpyAsync(nz, cloud->nz(), sizeof(float) * cloud->n, cudaMemcpyDeviceToHost, c->stream));
-    PCR_CUDA(c, cudaStreamSynchronize(c->stream));
-    return PCR_OK;
+    return points_download(cloud, nullptr, nullptr, nullptr, nx, ny, nz);
     PCR_API_END(c)
 }
 
-// Row-major (N, 3) in and out (the PyO3 surface's layout): one contiguous transfer, (de)interleaved on the device.
 int pcr_cloud_upload_rows(pcr_ctx *ctx, const float *xyz, size_t n, pcr_cloud **out) {
     if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
     Ctx *c = &ctx->c;
@@ -2044,55 +2092,23 @@ int pcr_cloud_upload_rows(pcr_ctx *ctx, const float *xyz, size_t n, pcr_cloud **
     *out = nullptr;
     PCR_API_BEGIN
     DevSetter ds(c);
-    pcr_cloud *cl = nullptr;
-    PCR_TRY(cloud_alloc(ctx, n, false, &cl));
-    cudaError_t e = cudaSuccess;
-    if (n) {
-        if (ensure(c, c->b_in, sizeof(float) * 3 * n) != PCR_OK) {
-            pcr_cloud_free(cl);
-            return PCR_ERR_CUDA;
-        }
-        e = cudaMemcpyAsync(c->b_in.p, xyz, sizeof(float) * 3 * n, cudaMemcpyHostToDevice, c->stream);
-        if (e == cudaSuccess) {
-            rows_to_soa_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>((const float *)c->b_in.p, n, cl->base, cl->stride);
-            c->launches++;
-            e = cudaGetLastError();
-        }
-    }
-    const cudaError_t es = cudaStreamSynchronize(c->stream);  // the caller's buffer is free again on return
-    if (e == cudaSuccess) e = es;
-    if (e != cudaSuccess) {
-        pcr_cloud_free(cl);
-        return fail(c, PCR_ERR_CUDA, "upload failed: %s", cudaGetErrorString(e));
-    }
-    *out = cl;
+    CloudPtr res;
+    PCR_TRY(points_alloc(ctx, n, false, res));
+    PCR_TRY(points_upload_rows(res.get(), xyz));
+    *out = res.release();
     return PCR_OK;
     PCR_API_END(c)
 }
 
 int pcr_cloud_download_rows(const pcr_cloud *cloud, float *xyz, float *normals) {
-    PCR_CLOUD_CHECK(cloud)
+    PCR_TRY(handle_check(cloud, "cloud"));
+    Ctx *c = &cloud->owner->c;
     if (normals && !cloud->has_normals) return fail(c, PCR_ERR_INVALID_ARG, "the cloud has no normals");
     if (cloud->n && !xyz && !normals) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     if (!cloud->n) return PCR_OK;
     PCR_API_BEGIN
     DevSetter ds(c);
-    const size_t n = cloud->n, row = sizeof(float) * 3 * n;
-    PCR_TRY(ensure(c, c->b_out, 2 * row));
-    float *d_xyz = (float *)c->b_out.p, *d_nrm = d_xyz + 3 * n;
-    const unsigned blocks = (unsigned)((n + 255) / 256);
-    if (xyz) {
-        soa_to_rows_kernel<<<blocks, 256, 0, c->stream>>>(cloud->base, cloud->stride, n, d_xyz);
-        PCR_LAUNCH_CHECK(c);
-        PCR_CUDA(c, cudaMemcpyAsync(xyz, d_xyz, row, cudaMemcpyDeviceToHost, c->stream));
-    }
-    if (normals) {
-        soa_to_rows_kernel<<<blocks, 256, 0, c->stream>>>(cloud->nx(), cloud->stride, n, d_nrm);
-        PCR_LAUNCH_CHECK(c);
-        PCR_CUDA(c, cudaMemcpyAsync(normals, d_nrm, row, cudaMemcpyDeviceToHost, c->stream));
-    }
-    PCR_CUDA(c, cudaStreamSynchronize(c->stream));
-    return PCR_OK;
+    return points_download_rows(cloud, xyz, normals);
     PCR_API_END(c)
 }
 
@@ -2101,14 +2117,12 @@ int pcr_sor_normals_batch_rows(pcr_ctx *ctx, const float *xyz, const uint64_t *f
     if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
     Ctx *c = &ctx->c;
     if (n_frames == 0) return PCR_OK;
-    if (!frame_offsets) return fail(c, PCR_ERR_INVALID_ARG, "frame_offsets is NULL");
+    PCR_TRY(offsets_check(c, "frame_offsets", frame_offsets, n_frames));
     const size_t n = (size_t)frame_offsets[n_frames];
     if (n_kept_per_frame) memset(n_kept_per_frame, 0, sizeof(uint64_t) * n_frames);
     if (n == 0) return PCR_OK;
     if (!xyz || !keep || !viewpoint || (k_normals && !normals)) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
-    if (!std::isfinite(std_mul) || std_mul < 0.f) return fail(c, PCR_ERR_INVALID_ARG, "std_mul must be >= 0 and finite");
-    if (k_sor + 1 > PCR_MAX_K || k_normals > PCR_MAX_K) return fail(c, PCR_ERR_UNSUPPORTED, "k exceeds PCR_MAX_K");
-    if (n_frames > 65535) return fail(c, PCR_ERR_UNSUPPORTED, "at most 65535 frames per batch");
+    PCR_TRY(sor_normals_batch_check(c, n, n_frames, k_sor, std_mul, k_normals));
     PCR_API_BEGIN
     DevSetter ds(c);
     const size_t stride = (n + 63) & ~(size_t)63;
@@ -2160,23 +2174,23 @@ static int upload_block(pcr_ctx *ctx, const float *xyz, size_t stride, size_t n,
     *out = nullptr;
     PCR_API_BEGIN
     DevSetter ds(c);
-    pcr_cloud *cl = nullptr;
-    PCR_TRY(cloud_alloc(ctx, n, false, &cl));
+    CloudPtr res;
+    PCR_TRY(points_alloc(ctx, n, false, res));
     cudaError_t e = cudaSuccess;
-    if (n) e = cudaMemcpy2DAsync(cl->base, cl->stride * sizeof(float), xyz, stride * sizeof(float), n * sizeof(float), 3, cudaMemcpyHostToDevice, c->stream);
+    if (n) e = cudaMemcpy2DAsync(res->base, res->stride * sizeof(float), xyz, stride * sizeof(float), n * sizeof(float), 3, cudaMemcpyHostToDevice, c->stream);
     if (e == cudaSuccess && wait) e = cudaStreamSynchronize(c->stream);  // the caller's buffer is free again on return
     if (e != cudaSuccess) {
         cudaGetLastError();
-        pcr_cloud_free(cl);
         return fail(c, PCR_ERR_CUDA, "upload failed: %s", cudaGetErrorString(e));
     }
-    *out = cl;
+    *out = res.release();
     return PCR_OK;
     PCR_API_END(c)
 }
 
 int pcr_cloud_download_block(const pcr_cloud *cloud, float *dst, size_t stride, int with_normals) {
-    PCR_CLOUD_CHECK(cloud)
+    PCR_TRY(handle_check(cloud, "cloud"));
+    Ctx *c = &cloud->owner->c;
     if (with_normals && !cloud->has_normals) return fail(c, PCR_ERR_INVALID_ARG, "the cloud has no normals");
     if ((cloud->n && !dst) || stride < cloud->n) return fail(c, PCR_ERR_INVALID_ARG, "null pointer or stride < len");
     if (!cloud->n) return PCR_OK;
@@ -2190,111 +2204,109 @@ int pcr_cloud_download_block(const pcr_cloud *cloud, float *dst, size_t stride, 
 }
 
 int pcr_cloud_select(const pcr_cloud *cloud, const uint32_t *indices, size_t m, pcr_cloud **out) {
-    PCR_CLOUD_CHECK(cloud)
+    PCR_TRY(handle_check(cloud, "cloud"));
+    Ctx *c = &cloud->owner->c;
     if (!out || (m && !indices)) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     *out = nullptr;
     for (size_t t = 0; t < m; t++)  // cloud.rs:109: select panics on an out-of-bounds index
         if (indices[t] >= cloud->n) return fail(c, PCR_ERR_INVALID_ARG, "index %u out of bounds for cloud with %zu points", indices[t], cloud->n);
     PCR_API_BEGIN
     DevSetter ds(c);
-    pcr_cloud *tmp = nullptr;  // *out is set on success only
-    PCR_TRY(cloud_alloc(cloud->owner, m, cloud->has_normals, &tmp));
-    const int rc = [&]() -> int {
-        if (!m) return PCR_OK;
+    CloudPtr res;
+    PCR_TRY(points_alloc(cloud->owner, m, cloud->has_normals, res));
+    if (m) {
         PCR_TRY(ensure(c, c->b_list, sizeof(uint32_t) * m));
         PCR_CUDA(c, cudaMemcpyAsync(c->b_list.p, indices, sizeof(uint32_t) * m, cudaMemcpyHostToDevice, c->stream));
-        gather_kernel<<<(unsigned)((m + 255) / 256), 256, 0, c->stream>>>(cloud->base, cloud->stride, cloud->has_normals ? 6 : 3,
-                                                                          (const uint32_t *)c->b_list.p, m, tmp->base, tmp->stride);
+        gather_kernel<<<(unsigned)((m + 255) / 256), 256, 0, c->stream>>>(cloud->base, cloud->stride, cloud->arrays(), (const uint32_t *)c->b_list.p,
+                                                                          m, res->base, res->stride);
         PCR_LAUNCH_CHECK(c);
         PCR_CUDA(c, cudaStreamSynchronize(c->stream));
-        return PCR_OK;
-    }();
-    if (rc != PCR_OK) {
-        pcr_cloud_free(tmp);
-        return rc;
     }
-    *out = tmp;
+    *out = res.release();
     return PCR_OK;
     PCR_API_END(c)
 }
 
 int pcr_cloud_voxel_downsample(const pcr_cloud *cloud, float voxel_size, pcr_cloud **out) {
-    PCR_CLOUD_CHECK(cloud)
+    PCR_TRY(handle_check(cloud, "cloud"));
+    Ctx *c = &cloud->owner->c;
     if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     *out = nullptr;
     if (!std::isfinite(voxel_size) || !(voxel_size > 0.f)) return fail(c, PCR_ERR_INVALID_ARG, "voxel_size must be > 0 and finite");
     PCR_API_BEGIN
     DevSetter ds(c);
     PCR_MARK("voxel: enter");
-    pcr_cloud *tmp = nullptr;
-    PCR_TRY(cloud_alloc(cloud->owner, cloud->n, false, &tmp));  // voxel_downsample.rs:64: xyz only
+    CloudPtr res;
+    PCR_TRY(points_alloc(cloud->owner, cloud->n, false, res));  // voxel_downsample.rs:64: xyz only
     size_t m = 0;
-    int s = voxel_downsample_dev(c, cloud->x(), cloud->y(), cloud->z(), cloud->n, voxel_size, tmp->x(), tmp->y(), tmp->z(), &m, &tmp->stats);
-    if (s != PCR_OK) {
-        pcr_cloud_free(tmp);
-        return s;
-    }
-    tmp->n = m;  // (the allocation keeps its original stride)
-    *out = tmp;
+    PCR_TRY(voxel_downsample_dev(c, cloud->x(), cloud->y(), cloud->z(), cloud->n, voxel_size, res->x(), res->y(), res->z(), &m, &res->stats));
+    res->n = m;  // (the allocation keeps its original stride)
+    *out = res.release();
     PCR_MARK("voxel: exit");
     return PCR_OK;
     PCR_API_END(c)
 }
 
 int pcr_cloud_statistical_outlier_removal(const pcr_cloud *cloud, size_t k, float std_mul, pcr_cloud **out) {
-    PCR_CLOUD_CHECK(cloud)
+    PCR_TRY(handle_check(cloud, "cloud"));
+    Ctx *c = &cloud->owner->c;
     if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     *out = nullptr;
     PCR_API_BEGIN
     DevSetter ds(c);
     const size_t n = cloud->n;
-    if (n == 0 || k == 0) return cloud_alloc(cloud->owner, 0, false, out);  // statistical_outlier.rs:5-7: PointCloud::new()
-    PCR_TRY(ensure(c, c->b_in2, n + 256));
-    uint8_t *d_keep = (uint8_t *)c->b_in2.p;
-    PCR_TRY(pcr_sor_dev(cloud->owner, cloud->x(), cloud->y(), cloud->z(), n, k, std_mul, d_keep, nullptr));
-    return cloud_compact(cloud, d_keep, out);  // :68 select
+    CloudPtr res;
+    if (n == 0 || k == 0) {  // statistical_outlier.rs:5-7: PointCloud::new()
+        PCR_TRY(points_alloc(cloud->owner, 0, false, res));
+    } else {
+        PCR_TRY(ensure(c, c->b_in2, n + 256));
+        uint8_t *d_keep = (uint8_t *)c->b_in2.p;
+        PCR_TRY(pcr_sor_dev(cloud->owner, cloud->x(), cloud->y(), cloud->z(), n, k, std_mul, d_keep, nullptr));
+        PCR_TRY(cloud_compact(cloud, d_keep, res));  // :68 select
+    }
+    *out = res.release();
+    return PCR_OK;
     PCR_API_END(c)
 }
 
 int pcr_cloud_radius_outlier_removal(const pcr_cloud *cloud, float radius, size_t min_neighbors, pcr_cloud **out) {
-    PCR_CLOUD_CHECK(cloud)
+    PCR_TRY(handle_check(cloud, "cloud"));
+    Ctx *c = &cloud->owner->c;
     if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     *out = nullptr;
     PCR_API_BEGIN
     DevSetter ds(c);
     const size_t n = cloud->n;
-    if (n == 0) return cloud_alloc(cloud->owner, 0, cloud->has_normals, out);
-    PCR_TRY(ensure(c, c->b_in2, n + 256));
-    uint8_t *d_keep = (uint8_t *)c->b_in2.p;
-    PCR_TRY(pcr_radius_outlier_dev(cloud->owner, cloud->x(), cloud->y(), cloud->z(), n, radius, min_neighbors, d_keep));
-    return cloud_compact(cloud, d_keep, out);
+    CloudPtr res;
+    if (n == 0) {
+        PCR_TRY(points_alloc(cloud->owner, 0, cloud->has_normals, res));
+    } else {
+        PCR_TRY(ensure(c, c->b_in2, n + 256));
+        uint8_t *d_keep = (uint8_t *)c->b_in2.p;
+        PCR_TRY(pcr_radius_outlier_dev(cloud->owner, cloud->x(), cloud->y(), cloud->z(), n, radius, min_neighbors, d_keep));
+        PCR_TRY(cloud_compact(cloud, d_keep, res));
+    }
+    *out = res.release();
+    return PCR_OK;
     PCR_API_END(c)
 }
 
 int pcr_cloud_estimate_normals(const pcr_cloud *cloud, size_t k, const float viewpoint[3], pcr_cloud **out) {
-    PCR_CLOUD_CHECK(cloud)
+    PCR_TRY(handle_check(cloud, "cloud"));
+    Ctx *c = &cloud->owner->c;
     if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     *out = nullptr;
     // estimate.rs:25-31 returns EMPTY normals for k == 0, which no consumer accepts (icp_plane.rs:27-32): reported here
     if (k == 0) return fail(c, PCR_ERR_INVALID_ARG, "k must be > 0");
     PCR_API_BEGIN
     DevSetter ds(c);
-    const size_t n = cloud->n;
-    pcr_cloud *res = nullptr;
-    PCR_TRY(cloud_alloc(cloud->owner, n, true, &res));
-    if (n) {
-        cudaMemcpyAsync(res->x(), cloud->x(), sizeof(float) * n, cudaMemcpyDeviceToDevice, c->stream);
-        cudaMemcpyAsync(res->y(), cloud->y(), sizeof(float) * n, cudaMemcpyDeviceToDevice, c->stream);
-        cudaMemcpyAsync(res->z(), cloud->z(), sizeof(float) * n, cudaMemcpyDeviceToDevice, c->stream);
-        const float vp0[3] = {0.f, 0.f, 0.f};  // estimate.rs:13-15
-        int s = pcr_estimate_normals_dev(cloud->owner, cloud->x(), cloud->y(), cloud->z(), n, k, viewpoint ? viewpoint : vp0, res->nx(),
-                                     res->ny(), res->nz());
-        if (s != PCR_OK) {
-            pcr_cloud_free(res);
-            return s;
-        }
-    }
-    *out = res;
+    CloudPtr res;
+    PCR_TRY(points_alloc(cloud->owner, cloud->n, true, res));
+    PCR_TRY(copy_arrays(cloud, 0, 3, res.get()));
+    const float vp0[3] = {0.f, 0.f, 0.f};  // estimate.rs:13-15
+    PCR_TRY(pcr_estimate_normals_dev(cloud->owner, cloud->x(), cloud->y(), cloud->z(), cloud->n, k, viewpoint ? viewpoint : vp0, res->nx(),
+                                     res->ny(), res->nz()));
+    *out = res.release();
     return PCR_OK;
     PCR_API_END(c)
 }
@@ -2303,7 +2315,8 @@ int pcr_cloud_estimate_normals(const pcr_cloud *cloud, size_t k, const float vie
 // SOR removes are tombstoned in place, see batch_core): the fused form of the two calls above
 int pcr_cloud_sor_normals(const pcr_cloud *cloud, size_t k_sor, float std_mul, size_t k_normals, const float viewpoint[3],
                           pcr_cloud **out) {
-    PCR_CLOUD_CHECK(cloud)
+    PCR_TRY(handle_check(cloud, "cloud"));
+    Ctx *c = &cloud->owner->c;
     if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     *out = nullptr;
     if (k_normals == 0) return fail(c, PCR_ERR_INVALID_ARG, "k_normals must be > 0");
@@ -2312,18 +2325,19 @@ int pcr_cloud_sor_normals(const pcr_cloud *cloud, size_t k_sor, float std_mul, s
     PCR_API_BEGIN
     DevSetter ds(c);
     const size_t n = cloud->n;
-    if (n == 0 || k_sor == 0) return cloud_alloc(cloud->owner, 0, true, out);  // statistical_outlier.rs:5-7
+    CloudPtr res;
+    if (n == 0 || k_sor == 0) {  // statistical_outlier.rs:5-7
+        PCR_TRY(points_alloc(cloud->owner, 0, true, res));
+        *out = res.release();
+        return PCR_OK;
+    }
     PCR_MARK("sor_normals: enter");
     // normals by original index go to a scratch block; the kept points and their normals are compacted from the
     // input cloud and that block in one pass
     const size_t stride = (n + 63) & ~(size_t)63;
-    float *d_nrm = nullptr;
-    PCR_CUDA(c, cudaMallocAsync((void **)&d_nrm, sizeof(float) * 3 * stride, c->stream));
-    struct G {
-        float *p;
-        cudaStream_t s;
-        ~G() { cudaFreeAsync(p, s); }
-    } g{d_nrm, c->stream};
+    StreamAlloc<float> nrm_mem(c->stream);
+    PCR_CUDA(c, nrm_mem.alloc(sizeof(float) * 3 * stride));
+    float *d_nrm = nrm_mem.p;
     PCR_TRY(ensure(c, c->b_in2, n + 512));
     uint8_t *d_keep = (uint8_t *)c->b_in2.p;
     unsigned long long *d_kept = (unsigned long long *)((char *)c->b_in2.p + ((n + 255) & ~(size_t)255));
@@ -2333,15 +2347,17 @@ int pcr_cloud_sor_normals(const pcr_cloud *cloud, size_t k_sor, float std_mul, s
     PCR_TRY(batch_core(c, cloud->x(), cloud->y(), cloud->z(), offs, 1, n, k_sor, std_mul, k_normals, viewpoint ? viewpoint : vp0, d_keep,
                        d_nrm, d_nrm + stride, d_nrm + 2 * stride, d_kept, &h_kept, cloud->stats.valid ? &cloud->stats : nullptr));
     PCR_MARK("sor_normals: core done");
-    const int rc = cloud_compact(cloud, d_keep, out, d_nrm, stride, h_kept == ~0ull ? SIZE_MAX : (size_t)h_kept);
+    PCR_TRY(cloud_compact(cloud, d_keep, res, d_nrm, stride, h_kept == ~0ull ? SIZE_MAX : (size_t)h_kept));
     PCR_MARK("sor_normals: exit");
-    return rc;
+    *out = res.release();
+    return PCR_OK;
     PCR_API_END(c)
 }
 
 int pcr_cloud_euclidean_cluster(const pcr_cloud *cloud, float distance_threshold, size_t min_size, size_t max_size, uint32_t *offsets,
                                 uint32_t *indices, size_t *n_clusters) {
-    PCR_CLOUD_CHECK(cloud)
+    PCR_TRY(handle_check(cloud, "cloud"));
+    Ctx *c = &cloud->owner->c;
     if (n_clusters) *n_clusters = 0;
     if (!offsets || !n_clusters) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     offsets[0] = 0;
@@ -2390,7 +2406,8 @@ int pcr_ransac_plane_samples(pcr_ctx *ctx, const float *x, const float *y, const
 
 int pcr_cloud_ransac_plane_samples(const pcr_cloud *cloud, float distance_threshold, const uint32_t *samples, size_t m, float model[4],
                                    uint32_t *inliers, size_t *n_inliers) {
-    PCR_CLOUD_CHECK(cloud)
+    PCR_TRY(handle_check(cloud, "cloud"));
+    Ctx *c = &cloud->owner->c;
     if (!model || !n_inliers || (m && !samples) || (cloud->n && !inliers)) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     PCR_API_BEGIN
     DevSetter ds(c);
@@ -2399,34 +2416,31 @@ int pcr_cloud_ransac_plane_samples(const pcr_cloud *cloud, float distance_thresh
 }
 
 int pcr_cloud_apply_transform(const pcr_cloud *cloud, const float rotation[9], const float translation[3], pcr_cloud **out) {
-    PCR_CLOUD_CHECK(cloud)
+    PCR_TRY(handle_check(cloud, "cloud"));
+    Ctx *c = &cloud->owner->c;
     if (!out || !rotation || !translation) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     *out = nullptr;
     PCR_API_BEGIN
     DevSetter ds(c);
-    pcr_cloud *res = nullptr;
-    PCR_TRY(cloud_alloc(cloud->owner, cloud->n, false, &res));  // icp.rs:91: xyz only
-    if (cloud->n) {
-        int s = apply_transform_dev(c, cloud->x(), cloud->y(), cloud->z(), cloud->n, rotation, translation, res->x(), res->y(), res->z());
-        if (s != PCR_OK) {
-            pcr_cloud_free(res);
-            return s;
-        }
-    }
-    *out = res;
+    CloudPtr res;
+    PCR_TRY(points_alloc(cloud->owner, cloud->n, false, res));  // icp.rs:91: xyz only
+    if (cloud->n) PCR_TRY(apply_transform_dev(c, cloud->x(), cloud->y(), cloud->z(), cloud->n, rotation, translation, res->x(), res->y(), res->z()));
+    *out = res.release();
     return PCR_OK;
     PCR_API_END(c)
 }
 
 int pcr_cloud_icp_point_to_point(const pcr_cloud *source, const pcr_cloud *target, const pcr_icp_params *params, pcr_icp_result *result) {
-    PCR_CLOUD_CHECK(source)
+    PCR_TRY(handle_check(source, "cloud"));
+    Ctx *c = &source->owner->c;
     if (!target || target->owner != source->owner) return fail(c, PCR_ERR_INVALID_ARG, "source and target must live on the same context");
     return pcr_icp_point_to_point_dev(source->owner, source->x(), source->y(), source->z(), source->n, target->x(), target->y(), target->z(),
                                       target->n, params, result);
 }
 
 int pcr_cloud_icp_point_to_plane(const pcr_cloud *source, const pcr_cloud *target, const pcr_icp_params *params, pcr_icp_result *result) {
-    PCR_CLOUD_CHECK(source)
+    PCR_TRY(handle_check(source, "cloud"));
+    Ctx *c = &source->owner->c;
     if (!target || target->owner != source->owner) return fail(c, PCR_ERR_INVALID_ARG, "source and target must live on the same context");
     if (!target->has_normals)  // crates/python/src/registration.rs:80-86
         return fail(c, PCR_ERR_INVALID_ARG, "target cloud must have normals (call estimate_normals first)");
@@ -2441,57 +2455,35 @@ int pcr_cloud_icp_point_to_plane(const pcr_cloud *source, const pcr_cloud *targe
  * then the frame offsets as the kernels read them (u32[F + 1]); the host keeps them as u64[F + 1].  Every method is a
  * batch core of the raw-pointer calls, and the filters end in ONE compaction for all frames (keep_scan, then the new
  * frame starts read off the scan, then compact_kernel): each frame's result is what the pcr_cloud method returns for it. */
-struct pcr_frames {
-    pcr_ctx *owner;
-    size_t n, stride;
-    float *base;
-    uint32_t *d_off;
-    bool has_normals;
+struct pcr_frames : DevPoints {
+    uint32_t *d_off = nullptr;
     std::vector<uint64_t> off;
     size_t count() const { return off.size() - 1; }
-    float *x() const { return base; }
-    float *y() const { return base + stride; }
-    float *z() const { return base + 2 * stride; }
-    float *nx() const { return base + 3 * stride; }
-    float *ny() const { return base + 4 * stride; }
-    float *nz() const { return base + 5 * stride; }
 };
 
 namespace pcr {
 namespace {
 
+// host offsets (u64[F + 1]) to the u32 copy the kernels read (pageable source: the copy has taken the bytes when it returns)
+int offsets_upload(Ctx *c, const std::vector<uint64_t> &off, uint32_t *d_off) {
+    const std::vector<uint32_t> h(off.begin(), off.end());
+    PCR_CUDA(c, cudaMemcpyAsync(d_off, h.data(), sizeof(uint32_t) * h.size(), cudaMemcpyHostToDevice, c->stream));
+    return PCR_OK;
+}
+
 // A new batch of n points with the given frame offsets.  d_off_src: the same offsets as u32 on the device (copied from
 // there), else they are uploaded from `off`.
-int frames_alloc(pcr_ctx *ctx, size_t n, bool normals, std::vector<uint64_t> off, pcr_frames **out, const uint32_t *d_off_src = nullptr) {
+int frames_alloc(pcr_ctx *ctx, size_t n, bool normals, std::vector<uint64_t> off, FramesPtr &out, const uint32_t *d_off_src = nullptr) {
     Ctx *c = &ctx->c;
-    pcr_frames *fr = new (std::nothrow) pcr_frames();
-    if (!fr) return fail(c, PCR_ERR_OOM, "host allocation failed");
-    fr->owner = ctx;
-    fr->n = n;
-    fr->stride = std::max<size_t>((n + 63) & ~(size_t)63, 64);
-    fr->has_normals = normals;
+    FramesPtr fr;
+    PCR_TRY(points_alloc(ctx, n, normals, fr, sizeof(uint32_t) * off.size()));
     fr->off = std::move(off);
-    fr->base = nullptr;
-    const size_t F = fr->count(), arrays = sizeof(float) * fr->stride * (normals ? 6 : 3);
-    cudaError_t e = cudaMallocAsync((void **)&fr->base, arrays + sizeof(uint32_t) * (F + 1), c->stream);
-    if (e == cudaSuccess) {
-        fr->d_off = (uint32_t *)((char *)fr->base + arrays);
-        if (d_off_src) {
-            e = cudaMemcpyAsync(fr->d_off, d_off_src, sizeof(uint32_t) * (F + 1), cudaMemcpyDeviceToDevice, c->stream);
-        } else {
-            std::vector<uint32_t> h(F + 1);
-            for (size_t f = 0; f <= F; f++) h[f] = (uint32_t)fr->off[f];
-            // (pageable source: the copy has taken the bytes when it returns)
-            e = cudaMemcpyAsync(fr->d_off, h.data(), sizeof(uint32_t) * (F + 1), cudaMemcpyHostToDevice, c->stream);
-        }
-    }
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        if (fr->base) cudaFreeAsync(fr->base, c->stream);
-        delete fr;
-        return fail(c, e == cudaErrorMemoryAllocation ? PCR_ERR_OOM : PCR_ERR_CUDA, "device allocation failed: %s", cudaGetErrorString(e));
-    }
-    *out = fr;
+    fr->d_off = (uint32_t *)(fr->base + fr->stride * fr->arrays());
+    if (d_off_src)
+        PCR_CUDA(c, cudaMemcpyAsync(fr->d_off, d_off_src, sizeof(uint32_t) * fr->off.size(), cudaMemcpyDeviceToDevice, c->stream));
+    else
+        PCR_TRY(offsets_upload(c, fr->off, fr->d_off));
+    out = std::move(fr);
     return PCR_OK;
 }
 
@@ -2504,18 +2496,14 @@ __global__ void frame_starts_kernel(const uint32_t *__restrict__ pos, const uint
 
 // new batch = the points of `in` with keep != 0, frame by frame.  `nrm` (optional): normals of the points of `in`, three
 // rows `nrm_stride` apart, for an `in` that carries none.  One round trip: all F + 1 new offsets in one copy.
-int frames_compact(const pcr_frames *in, const uint8_t *d_keep, pcr_frames **out, const float *nrm = nullptr, size_t nrm_stride = 0) {
+int frames_compact(const pcr_frames *in, const uint8_t *d_keep, FramesPtr &out, const float *nrm = nullptr, size_t nrm_stride = 0) {
     Ctx *c = &in->owner->c;
-    const size_t n = in->n, F = in->count();
+    const size_t F = in->count();
     uint32_t *pos = nullptr;
-    PCR_TRY(keep_scan(c, d_keep, n, &pos));
-    uint32_t *d_new = nullptr;
-    PCR_CUDA(c, cudaMallocAsync((void **)&d_new, sizeof(uint32_t) * (F + 1), c->stream));
-    struct G {
-        void *p;
-        cudaStream_t s;
-        ~G() { cudaFreeAsync(p, s); }
-    } g{d_new, c->stream};
+    PCR_TRY(keep_scan(c, d_keep, in->n, &pos));
+    StreamAlloc<uint32_t> new_off(c->stream);
+    PCR_CUDA(c, new_off.alloc(sizeof(uint32_t) * (F + 1)));
+    uint32_t *d_new = new_off.p;
     frame_starts_kernel<<<(unsigned)((F + 1 + 255) / 256), 256, 0, c->stream>>>(pos, in->d_off, (int)F, d_new);
     PCR_LAUNCH_CHECK(c);
     PCR_TRY(ensure_pinned(c, sizeof(uint32_t) * (F + 1)));
@@ -2525,25 +2513,12 @@ int frames_compact(const pcr_frames *in, const uint8_t *d_keep, pcr_frames **out
     std::vector<uint64_t> off(F + 1);
     for (size_t f = 0; f <= F; f++) off[f] = mail[f];
     const size_t m = (size_t)off[F];
-    const bool with_normals = nrm || in->has_normals;
-    pcr_frames *tmp = nullptr;  // *out is set on success only
-    PCR_TRY(frames_alloc(in->owner, m, with_normals, std::move(off), &tmp, d_new));
-    if (m) {
-        const int n_a = nrm ? 3 : (in->has_normals ? 6 : 3), n_b = nrm ? 3 : 0;
-        const cudaError_t e = launch_chained(compact_kernel, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, c->stream, in->base, in->stride, n_a,
-                                             nrm, nrm_stride, n_b, n, pos, tmp->base, tmp->stride);
-        c->launches++;
-        if (e != cudaSuccess) {
-            pcr_frames_free(tmp);
-            return fail(c, PCR_ERR_CUDA, "kernel launch failed: %s (%s:%d)", cudaGetErrorString(e), __FILE__, __LINE__);
-        }
-    }
-    *out = tmp;
-    return PCR_OK;
+    PCR_TRY(frames_alloc(in->owner, m, nrm || in->has_normals, std::move(off), out, d_new));
+    return compact_into(in, pos, nrm, nrm_stride, out.get());
 }
 
 // An empty batch with in's frame count: every frame empty (the SOR rule for k == 0).
-int frames_empty(const pcr_frames *in, bool normals, pcr_frames **out) {
+int frames_empty(const pcr_frames *in, bool normals, FramesPtr &out) {
     return frames_alloc(in->owner, 0, normals, std::vector<uint64_t>(in->count() + 1, 0), out);
 }
 
@@ -2570,24 +2545,18 @@ __global__ void frames_unkeep_kernel(const uint32_t *__restrict__ idx, const uin
 }
 
 // select_inverse of frame-local DEVICE lists with HOST list offsets (in bounds, checked by the caller or by construction)
-int frames_select_inverse_dev(const pcr_frames *in, const uint32_t *d_idx, const std::vector<uint64_t> &list_off, pcr_frames **out) {
+int frames_select_inverse_dev(const pcr_frames *in, const uint32_t *d_idx, const std::vector<uint64_t> &list_off, FramesPtr &out) {
     Ctx *c = &in->owner->c;
     const size_t n = in->n, F = in->count(), m = (size_t)list_off[F];
     // keep u8[n] (rounded up to 4 bytes) | list offsets u32[F + 1]
     const size_t o_loff = (n + 3) & ~(size_t)3;
-    uint8_t *d_keep = nullptr;
-    PCR_CUDA(c, cudaMallocAsync((void **)&d_keep, o_loff + sizeof(uint32_t) * (F + 1), c->stream));
-    struct G {
-        void *p;
-        cudaStream_t s;
-        ~G() { cudaFreeAsync(p, s); }
-    } g{d_keep, c->stream};
+    StreamAlloc<uint8_t> keep_mem(c->stream);
+    PCR_CUDA(c, keep_mem.alloc(o_loff + sizeof(uint32_t) * (F + 1)));
+    uint8_t *d_keep = keep_mem.p;
     uint32_t *d_loff = (uint32_t *)(d_keep + o_loff);
     if (n) PCR_CUDA(c, cudaMemsetAsync(d_keep, 1, n, c->stream));
     if (m) {
-        std::vector<uint32_t> h(F + 1);
-        for (size_t f = 0; f <= F; f++) h[f] = (uint32_t)list_off[f];
-        PCR_CUDA(c, cudaMemcpyAsync(d_loff, h.data(), sizeof(uint32_t) * (F + 1), cudaMemcpyHostToDevice, c->stream));
+        PCR_TRY(offsets_upload(c, list_off, d_loff));
         frames_unkeep_kernel<<<(unsigned)((m + 255) / 256), 256, 0, c->stream>>>(d_idx, d_loff, in->d_off, (int)F, m, d_keep);
         PCR_LAUNCH_CHECK(c);
     }
@@ -2599,16 +2568,12 @@ int frames_select_inverse_dev(const pcr_frames *in, const uint32_t *d_idx, const
 
 extern "C" {
 
-#define PCR_FRAMES_CHECK(fr)                                                                  \
-    if (!(fr) || !(fr)->owner) return fail(nullptr, PCR_ERR_INVALID_ARG, "frames is NULL");   \
-    Ctx *c = &(fr)->owner->c;
-
 // offsets, sizes and the output handle of an upload; n receives the point count
 static int frames_upload_check(Ctx *c, const uint64_t *frame_offsets, size_t n_frames, pcr_frames **out, size_t *n) {
     if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     *out = nullptr;
     if (n_frames == 0) return fail(c, PCR_ERR_INVALID_ARG, "a batch holds at least one frame");
-    PCR_TRY(batch_offsets_check(c, frame_offsets, n_frames));
+    PCR_TRY(offsets_check(c, "frame_offsets", frame_offsets, n_frames));
     *n = (size_t)frame_offsets[n_frames];
     return batch_size_check(c, *n, n_frames);
 }
@@ -2622,27 +2587,14 @@ int pcr_frames_upload(pcr_ctx *ctx, const float *x, const float *y, const float 
     if (n && (!x || !y || !z)) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     PCR_API_BEGIN
     DevSetter ds(c);
-    pcr_frames *fr = nullptr;
-    PCR_TRY(frames_alloc(ctx, n, false, std::vector<uint64_t>(frame_offsets, frame_offsets + n_frames + 1), &fr));
-    cudaError_t e = cudaSuccess;
-    if (n) {
-        e = cudaMemcpyAsync(fr->x(), x, sizeof(float) * n, cudaMemcpyHostToDevice, c->stream);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(fr->y(), y, sizeof(float) * n, cudaMemcpyHostToDevice, c->stream);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(fr->z(), z, sizeof(float) * n, cudaMemcpyHostToDevice, c->stream);
-    }
-    const cudaError_t es = cudaStreamSynchronize(c->stream);  // the caller's buffers are free again on return
-    if (e == cudaSuccess) e = es;
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        pcr_frames_free(fr);
-        return fail(c, PCR_ERR_CUDA, "upload failed: %s", cudaGetErrorString(e));
-    }
-    *out = fr;
+    FramesPtr res;
+    PCR_TRY(frames_alloc(ctx, n, false, std::vector<uint64_t>(frame_offsets, frame_offsets + n_frames + 1), res));
+    PCR_TRY(points_upload(res.get(), x, y, z));
+    *out = res.release();
     return PCR_OK;
     PCR_API_END(c)
 }
 
-// row-major (N, 3): one contiguous transfer, split on the device (as pcr_cloud_upload_rows)
 int pcr_frames_upload_rows(pcr_ctx *ctx, const float *xyz, const uint64_t *frame_offsets, size_t n_frames, pcr_frames **out) {
     if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
     Ctx *c = &ctx->c;
@@ -2651,68 +2603,37 @@ int pcr_frames_upload_rows(pcr_ctx *ctx, const float *xyz, const uint64_t *frame
     if (n && !xyz) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     PCR_API_BEGIN
     DevSetter ds(c);
-    pcr_frames *fr = nullptr;
-    PCR_TRY(frames_alloc(ctx, n, false, std::vector<uint64_t>(frame_offsets, frame_offsets + n_frames + 1), &fr));
-    cudaError_t e = cudaSuccess;
-    if (n) {
-        if (ensure(c, c->b_in, sizeof(float) * 3 * n) != PCR_OK) {
-            pcr_frames_free(fr);
-            return PCR_ERR_CUDA;
-        }
-        e = cudaMemcpyAsync(c->b_in.p, xyz, sizeof(float) * 3 * n, cudaMemcpyHostToDevice, c->stream);
-        if (e == cudaSuccess) {
-            rows_to_soa_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>((const float *)c->b_in.p, n, fr->base, fr->stride);
-            c->launches++;
-            e = cudaGetLastError();
-        }
-    }
-    const cudaError_t es = cudaStreamSynchronize(c->stream);
-    if (e == cudaSuccess) e = es;
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        pcr_frames_free(fr);
-        return fail(c, PCR_ERR_CUDA, "upload failed: %s", cudaGetErrorString(e));
-    }
-    *out = fr;
+    FramesPtr res;
+    PCR_TRY(frames_alloc(ctx, n, false, std::vector<uint64_t>(frame_offsets, frame_offsets + n_frames + 1), res));
+    PCR_TRY(points_upload_rows(res.get(), xyz));
+    *out = res.release();
     return PCR_OK;
     PCR_API_END(c)
 }
 
-void pcr_frames_free(pcr_frames *frames) {
-    if (!frames) return;
-    if (frames->base && frames->owner) {
-        DevSetter ds(&frames->owner->c);
-        cudaFreeAsync(frames->base, frames->owner->c.stream);
-    }
-    delete frames;
-}
+void pcr_frames_free(pcr_frames *frames) { handle_free(frames); }
 
 size_t pcr_frames_len(const pcr_frames *frames) { return frames ? frames->n : 0; }
 size_t pcr_frames_count(const pcr_frames *frames) { return frames ? frames->count() : 0; }
 int pcr_frames_has_normals(const pcr_frames *frames) { return frames && frames->has_normals ? 1 : 0; }
 
 int pcr_frames_offsets(const pcr_frames *frames, uint64_t *out) {
-    PCR_FRAMES_CHECK(frames)
-    if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    PCR_TRY(handle_check(frames, "frames"));
+    if (!out) return fail(&frames->owner->c, PCR_ERR_INVALID_ARG, "null pointer");
     std::copy(frames->off.begin(), frames->off.end(), out);
     return PCR_OK;
 }
 
 int pcr_frames_device_pointers(const pcr_frames *frames, const float **d_x, const float **d_y, const float **d_z, const float **d_nx,
                                const float **d_ny, const float **d_nz) {
-    PCR_FRAMES_CHECK(frames)
-    (void)c;
-    if (d_x) *d_x = frames->x();
-    if (d_y) *d_y = frames->y();
-    if (d_z) *d_z = frames->z();
-    if (d_nx) *d_nx = frames->has_normals ? frames->nx() : nullptr;
-    if (d_ny) *d_ny = frames->has_normals ? frames->ny() : nullptr;
-    if (d_nz) *d_nz = frames->has_normals ? frames->nz() : nullptr;
+    PCR_TRY(handle_check(frames, "frames"));
+    points_device_pointers(frames, d_x, d_y, d_z, d_nx, d_ny, d_nz);
     return PCR_OK;
 }
 
 int pcr_frames_download(const pcr_frames *frames, float *x, float *y, float *z, float *nx, float *ny, float *nz) {
-    PCR_FRAMES_CHECK(frames)
+    PCR_TRY(handle_check(frames, "frames"));
+    Ctx *c = &frames->owner->c;
     const bool want_n = nx || ny || nz;
     if (want_n && !frames->has_normals) return fail(c, PCR_ERR_INVALID_ARG, "the frames have no normals");
     const size_t n = frames->n;
@@ -2720,72 +2641,45 @@ int pcr_frames_download(const pcr_frames *frames, float *x, float *y, float *z, 
     if (!n) return PCR_OK;
     PCR_API_BEGIN
     DevSetter ds(c);
-    float *dst[6] = {x, y, z, nx, ny, nz};
-    for (int a = 0; a < (want_n ? 6 : 3); a++)
-        PCR_CUDA(c, cudaMemcpyAsync(dst[a], frames->base + (size_t)a * frames->stride, sizeof(float) * n, cudaMemcpyDeviceToHost, c->stream));
-    PCR_CUDA(c, cudaStreamSynchronize(c->stream));
-    return PCR_OK;
+    return points_download(frames, x, y, z, nx, ny, nz);
     PCR_API_END(c)
 }
 
 int pcr_frames_download_rows(const pcr_frames *frames, float *xyz, float *normals) {
-    PCR_FRAMES_CHECK(frames)
+    PCR_TRY(handle_check(frames, "frames"));
+    Ctx *c = &frames->owner->c;
     if (normals && !frames->has_normals) return fail(c, PCR_ERR_INVALID_ARG, "the frames have no normals");
     if (frames->n && !xyz && !normals) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     if (!frames->n) return PCR_OK;
     PCR_API_BEGIN
     DevSetter ds(c);
-    const size_t n = frames->n, row = sizeof(float) * 3 * n;
-    PCR_TRY(ensure(c, c->b_out, 2 * row));
-    float *d_xyz = (float *)c->b_out.p, *d_nrm = d_xyz + 3 * n;
-    const unsigned blocks = (unsigned)((n + 255) / 256);
-    if (xyz) {
-        soa_to_rows_kernel<<<blocks, 256, 0, c->stream>>>(frames->base, frames->stride, n, d_xyz);
-        PCR_LAUNCH_CHECK(c);
-        PCR_CUDA(c, cudaMemcpyAsync(xyz, d_xyz, row, cudaMemcpyDeviceToHost, c->stream));
-    }
-    if (normals) {
-        soa_to_rows_kernel<<<blocks, 256, 0, c->stream>>>(frames->nx(), frames->stride, n, d_nrm);
-        PCR_LAUNCH_CHECK(c);
-        PCR_CUDA(c, cudaMemcpyAsync(normals, d_nrm, row, cudaMemcpyDeviceToHost, c->stream));
-    }
-    PCR_CUDA(c, cudaStreamSynchronize(c->stream));
-    return PCR_OK;
+    return points_download_rows(frames, xyz, normals);
     PCR_API_END(c)
 }
 
 int pcr_frames_frame(const pcr_frames *frames, size_t f, pcr_cloud **out) {
-    PCR_FRAMES_CHECK(frames)
+    PCR_TRY(handle_check(frames, "frames"));
+    Ctx *c = &frames->owner->c;
     if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     *out = nullptr;
     if (f >= frames->count()) return fail(c, PCR_ERR_INVALID_ARG, "frame %zu out of range (%zu frames)", f, frames->count());
     PCR_API_BEGIN
     DevSetter ds(c);
-    const size_t b = (size_t)frames->off[f], m = (size_t)frames->off[f + 1] - b;
-    pcr_cloud *cl = nullptr;
-    PCR_TRY(cloud_alloc(frames->owner, m, frames->has_normals, &cl));
-    for (int a = 0; m && a < (frames->has_normals ? 6 : 3); a++) {
-        const cudaError_t e = cudaMemcpyAsync(cl->base + (size_t)a * cl->stride, frames->base + (size_t)a * frames->stride + b, sizeof(float) * m,
-                                              cudaMemcpyDeviceToDevice, c->stream);
-        if (e != cudaSuccess) {
-            cudaGetLastError();
-            pcr_cloud_free(cl);
-            return fail(c, PCR_ERR_CUDA, "copy failed: %s", cudaGetErrorString(e));
-        }
-    }
-    *out = cl;
+    CloudPtr res;
+    PCR_TRY(points_alloc(frames->owner, (size_t)(frames->off[f + 1] - frames->off[f]), frames->has_normals, res));
+    PCR_TRY(copy_arrays(frames, (size_t)frames->off[f], frames->arrays(), res.get()));
+    *out = res.release();
     return PCR_OK;
     PCR_API_END(c)
 }
 
 int pcr_frames_select(const pcr_frames *frames, const uint32_t *indices, const uint64_t *index_offsets, int invert, pcr_frames **out) {
-    PCR_FRAMES_CHECK(frames)
-    if (!out || !index_offsets) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    PCR_TRY(handle_check(frames, "frames"));
+    Ctx *c = &frames->owner->c;
+    if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     *out = nullptr;
     const size_t F = frames->count();
-    if (index_offsets[0] != 0) return fail(c, PCR_ERR_INVALID_ARG, "index_offsets must start at 0");
-    for (size_t f = 0; f < F; f++)
-        if (index_offsets[f + 1] < index_offsets[f]) return fail(c, PCR_ERR_INVALID_ARG, "index_offsets must be non-decreasing");
+    PCR_TRY(offsets_check(c, "index_offsets", index_offsets, F));
     const size_t m = (size_t)index_offsets[F];
     if (m && !indices) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     if (m > 0x7fffffffull) return fail(c, PCR_ERR_UNSUPPORTED, "at most 2^31 - 1 listed indices per call");
@@ -2799,74 +2693,54 @@ int pcr_frames_select(const pcr_frames *frames, const uint32_t *indices, const u
     PCR_API_BEGIN
     DevSetter ds(c);
     std::vector<uint64_t> loff(index_offsets, index_offsets + F + 1);
-    uint32_t *d_idx = nullptr;
-    PCR_CUDA(c, cudaMallocAsync((void **)&d_idx, sizeof(uint32_t) * std::max<size_t>(m, 1), c->stream));
-    struct G {
-        void *p;
-        cudaStream_t s;
-        ~G() { cudaFreeAsync(p, s); }
-    } g{d_idx, c->stream};
-    if (m) PCR_CUDA(c, cudaMemcpyAsync(d_idx, indices, sizeof(uint32_t) * m, cudaMemcpyHostToDevice, c->stream));
-    if (invert) return frames_select_inverse_dev(frames, d_idx, loff, out);
-    pcr_frames *tmp = nullptr;
-    PCR_TRY(frames_alloc(frames->owner, m, frames->has_normals, loff, &tmp));
+    StreamAlloc<uint32_t> d_idx(c->stream);
+    PCR_CUDA(c, d_idx.alloc(sizeof(uint32_t) * std::max<size_t>(m, 1)));
+    if (m) PCR_CUDA(c, cudaMemcpyAsync(d_idx.p, indices, sizeof(uint32_t) * m, cudaMemcpyHostToDevice, c->stream));
+    FramesPtr res;
+    if (invert) {
+        PCR_TRY(frames_select_inverse_dev(frames, d_idx.p, loff, res));
+        *out = res.release();
+        return PCR_OK;
+    }
+    PCR_TRY(frames_alloc(frames->owner, m, frames->has_normals, loff, res));
     if (m) {
         // the gather reads the list offsets as u32: the new batch's own device offsets are exactly those
-        frames_gather_kernel<<<(unsigned)((m + 255) / 256), 256, 0, c->stream>>>(frames->base, frames->stride, frames->has_normals ? 6 : 3, d_idx,
-                                                                                 tmp->d_off, frames->d_off, (int)F, m, tmp->base, tmp->stride);
-        const cudaError_t e = cudaGetLastError();
-        c->launches++;
-        if (e != cudaSuccess) {
-            pcr_frames_free(tmp);
-            return fail(c, PCR_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(e));
-        }
+        frames_gather_kernel<<<(unsigned)((m + 255) / 256), 256, 0, c->stream>>>(frames->base, frames->stride, frames->arrays(), d_idx.p,
+                                                                                 res->d_off, frames->d_off, (int)F, m, res->base, res->stride);
+        PCR_LAUNCH_CHECK(c);
     }
     // the caller's index array is free again on return (a pinned one is read by the copy while it runs)
-    const cudaError_t es = cudaStreamSynchronize(c->stream);
-    if (es != cudaSuccess) {
-        cudaGetLastError();
-        pcr_frames_free(tmp);
-        return fail(c, PCR_ERR_CUDA, "select failed: %s", cudaGetErrorString(es));
-    }
-    *out = tmp;
+    PCR_CUDA(c, cudaStreamSynchronize(c->stream));
+    *out = res.release();
     return PCR_OK;
     PCR_API_END(c)
 }
 
 int pcr_frames_voxel_downsample(const pcr_frames *frames, float voxel_size, pcr_frames **out) {
-    PCR_FRAMES_CHECK(frames)
+    PCR_TRY(handle_check(frames, "frames"));
+    Ctx *c = &frames->owner->c;
     if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     *out = nullptr;
     if (!std::isfinite(voxel_size) || !(voxel_size > 0.f)) return fail(c, PCR_ERR_INVALID_ARG, "voxel_size must be > 0 and finite");
     PCR_API_BEGIN
     DevSetter ds(c);
     const size_t F = frames->count();
-    pcr_frames *tmp = nullptr;  // voxel_downsample.rs:64: xyz only; sized for the input, then shrunk to the voxels
-    PCR_TRY(frames_alloc(frames->owner, frames->n, false, std::vector<uint64_t>(F + 1, 0), &tmp));
+    FramesPtr res;  // voxel_downsample.rs:64: xyz only; sized for the input, then shrunk to the voxels
+    PCR_TRY(frames_alloc(frames->owner, frames->n, false, std::vector<uint64_t>(F + 1, 0), res));
     std::vector<uint64_t> out_off(F + 1, 0);
-    const int s = voxel_batch_entry(frames->owner, true, frames->x(), frames->y(), frames->z(), frames->off.data(), F, voxel_size, tmp->x(),
-                                    tmp->y(), tmp->z(), out_off.data());
-    if (s != PCR_OK) {
-        pcr_frames_free(tmp);
-        return s;
-    }
-    std::vector<uint32_t> h(F + 1);
-    for (size_t f = 0; f <= F; f++) h[f] = (uint32_t)out_off[f];
-    const cudaError_t e = cudaMemcpyAsync(tmp->d_off, h.data(), sizeof(uint32_t) * (F + 1), cudaMemcpyHostToDevice, c->stream);
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        pcr_frames_free(tmp);
-        return fail(c, PCR_ERR_CUDA, "copy failed: %s", cudaGetErrorString(e));
-    }
-    tmp->n = (size_t)out_off[F];  // (the allocation keeps its original stride)
-    tmp->off = std::move(out_off);
-    *out = tmp;
+    PCR_TRY(voxel_batch_entry(frames->owner, true, frames->x(), frames->y(), frames->z(), frames->off.data(), F, voxel_size, res->x(), res->y(),
+                              res->z(), out_off.data()));
+    PCR_TRY(offsets_upload(c, out_off, res->d_off));
+    res->n = (size_t)out_off[F];  // (the allocation keeps its original stride)
+    res->off = std::move(out_off);
+    *out = res.release();
     return PCR_OK;
     PCR_API_END(c)
 }
 
 int pcr_frames_statistical_outlier_removal(const pcr_frames *frames, size_t k, float std_mul, pcr_frames **out) {
-    PCR_FRAMES_CHECK(frames)
+    PCR_TRY(handle_check(frames, "frames"));
+    Ctx *c = &frames->owner->c;
     if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     *out = nullptr;
     if (!std::isfinite(std_mul) || std_mul < 0.f) return fail(c, PCR_ERR_INVALID_ARG, "std_mul must be >= 0 and finite");
@@ -2874,72 +2748,68 @@ int pcr_frames_statistical_outlier_removal(const pcr_frames *frames, size_t k, f
     PCR_API_BEGIN
     DevSetter ds(c);
     const size_t n = frames->n;
-    if (n == 0 || k == 0) return frames_empty(frames, false, out);  // statistical_outlier.rs:5-7: PointCloud::new()
-    uint8_t *d_keep = nullptr;
-    PCR_CUDA(c, cudaMallocAsync((void **)&d_keep, n, c->stream));
-    struct G {
-        void *p;
-        cudaStream_t s;
-        ~G() { cudaFreeAsync(p, s); }
-    } g{d_keep, c->stream};
-    const float vp0[3] = {0.f, 0.f, 0.f};
-    PCR_TRY(pcr_sor_normals_batch_dev(frames->owner, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(), k, std_mul, 0,
-                                      vp0, d_keep, nullptr, nullptr, nullptr));
-    return frames_compact(frames, d_keep, out);  // :68 select
+    FramesPtr res;
+    if (n == 0 || k == 0) {  // statistical_outlier.rs:5-7: PointCloud::new()
+        PCR_TRY(frames_empty(frames, false, res));
+    } else {
+        StreamAlloc<uint8_t> d_keep(c->stream);
+        PCR_CUDA(c, d_keep.alloc(n));
+        const float vp0[3] = {0.f, 0.f, 0.f};
+        PCR_TRY(pcr_sor_normals_batch_dev(frames->owner, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(), k, std_mul, 0,
+                                          vp0, d_keep.p, nullptr, nullptr, nullptr));
+        PCR_TRY(frames_compact(frames, d_keep.p, res));  // :68 select
+    }
+    *out = res.release();
+    return PCR_OK;
     PCR_API_END(c)
 }
 
 int pcr_frames_radius_outlier_removal(const pcr_frames *frames, float radius, size_t min_neighbors, pcr_frames **out) {
-    PCR_FRAMES_CHECK(frames)
+    PCR_TRY(handle_check(frames, "frames"));
+    Ctx *c = &frames->owner->c;
     if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     *out = nullptr;
     PCR_API_BEGIN
     DevSetter ds(c);
     const size_t n = frames->n;
-    if (n == 0) return frames_empty(frames, frames->has_normals, out);
-    uint8_t *d_keep = nullptr;
-    PCR_CUDA(c, cudaMallocAsync((void **)&d_keep, n, c->stream));
-    struct G {
-        void *p;
-        cudaStream_t s;
-        ~G() { cudaFreeAsync(p, s); }
-    } g{d_keep, c->stream};
-    PCR_TRY(pcr_radius_outlier_batch_dev(frames->owner, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(), radius,
-                                         min_neighbors, d_keep));
-    return frames_compact(frames, d_keep, out);
+    FramesPtr res;
+    if (n == 0) {
+        PCR_TRY(frames_empty(frames, frames->has_normals, res));
+    } else {
+        StreamAlloc<uint8_t> d_keep(c->stream);
+        PCR_CUDA(c, d_keep.alloc(n));
+        PCR_TRY(pcr_radius_outlier_batch_dev(frames->owner, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(), radius,
+                                             min_neighbors, d_keep.p));
+        PCR_TRY(frames_compact(frames, d_keep.p, res));
+    }
+    *out = res.release();
+    return PCR_OK;
     PCR_API_END(c)
 }
 
 int pcr_frames_estimate_normals(const pcr_frames *frames, size_t k, const float viewpoint[3], pcr_frames **out) {
-    PCR_FRAMES_CHECK(frames)
+    PCR_TRY(handle_check(frames, "frames"));
+    Ctx *c = &frames->owner->c;
     if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     *out = nullptr;
     if (k == 0) return fail(c, PCR_ERR_INVALID_ARG, "k must be > 0");  // as pcr_cloud_estimate_normals
     PCR_API_BEGIN
     DevSetter ds(c);
-    const size_t n = frames->n;
-    pcr_frames *res = nullptr;
-    PCR_TRY(frames_alloc(frames->owner, n, true, frames->off, &res, frames->d_off));
-    if (n) {
-        for (int a = 0; a < 3; a++)
-            cudaMemcpyAsync(res->base + (size_t)a * res->stride, frames->base + (size_t)a * frames->stride, sizeof(float) * n, cudaMemcpyDeviceToDevice,
-                            c->stream);
-        const float vp0[3] = {0.f, 0.f, 0.f};  // estimate.rs:13-15
-        const int s = pcr_estimate_normals_batch_dev(frames->owner, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(), k,
-                                                     viewpoint ? viewpoint : vp0, res->nx(), res->ny(), res->nz());
-        if (s != PCR_OK) {
-            pcr_frames_free(res);
-            return s;
-        }
-    }
-    *out = res;
+    FramesPtr res;
+    PCR_TRY(frames_alloc(frames->owner, frames->n, true, frames->off, res, frames->d_off));
+    PCR_TRY(copy_arrays(frames, 0, 3, res.get()));
+    const float vp0[3] = {0.f, 0.f, 0.f};  // estimate.rs:13-15
+    PCR_TRY(pcr_estimate_normals_batch_dev(frames->owner, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(), k,
+                                           viewpoint ? viewpoint : vp0, res->nx(), res->ny(), res->nz()));
+    *out = res.release();
     return PCR_OK;
     PCR_API_END(c)
 }
 
 int pcr_frames_sor_normals(const pcr_frames *frames, size_t k_sor, float std_mul, size_t k_normals, const float viewpoint[3],
                            pcr_frames **out) {
-    PCR_FRAMES_CHECK(frames)
+    PCR_TRY(handle_check(frames, "frames"));
+    Ctx *c = &frames->owner->c;
     if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     *out = nullptr;
     if (k_normals == 0) return fail(c, PCR_ERR_INVALID_ARG, "k_normals must be > 0");
@@ -2948,72 +2818,71 @@ int pcr_frames_sor_normals(const pcr_frames *frames, size_t k_sor, float std_mul
     PCR_API_BEGIN
     DevSetter ds(c);
     const size_t n = frames->n;
-    if (n == 0 || k_sor == 0) return frames_empty(frames, true, out);  // statistical_outlier.rs:5-7
-    // normals by input index go to a scratch block; the kept points and their normals are compacted together
-    const size_t stride = (n + 63) & ~(size_t)63;
-    float *d_nrm = nullptr;
-    PCR_CUDA(c, cudaMallocAsync((void **)&d_nrm, sizeof(float) * 3 * stride + n, c->stream));
-    struct G {
-        void *p;
-        cudaStream_t s;
-        ~G() { cudaFreeAsync(p, s); }
-    } g{d_nrm, c->stream};
-    uint8_t *d_keep = (uint8_t *)(d_nrm + 3 * stride);
-    const float vp0[3] = {0.f, 0.f, 0.f};
-    PCR_TRY(pcr_sor_normals_batch_dev(frames->owner, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(), k_sor, std_mul,
-                                      k_normals, viewpoint ? viewpoint : vp0, d_keep, d_nrm, d_nrm + stride, d_nrm + 2 * stride));
-    return frames_compact(frames, d_keep, out, d_nrm, stride);
+    FramesPtr res;
+    if (n == 0 || k_sor == 0) {  // statistical_outlier.rs:5-7
+        PCR_TRY(frames_empty(frames, true, res));
+    } else {
+        // normals by input index go to a scratch block; the kept points and their normals are compacted together
+        const size_t stride = (n + 63) & ~(size_t)63;
+        StreamAlloc<float> nrm_mem(c->stream);
+        PCR_CUDA(c, nrm_mem.alloc(sizeof(float) * 3 * stride + n));
+        float *d_nrm = nrm_mem.p;
+        uint8_t *d_keep = (uint8_t *)(d_nrm + 3 * stride);
+        const float vp0[3] = {0.f, 0.f, 0.f};
+        PCR_TRY(pcr_sor_normals_batch_dev(frames->owner, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(), k_sor, std_mul,
+                                          k_normals, viewpoint ? viewpoint : vp0, d_keep, d_nrm, d_nrm + stride, d_nrm + 2 * stride));
+        PCR_TRY(frames_compact(frames, d_keep, res, d_nrm, stride));
+    }
+    *out = res.release();
+    return PCR_OK;
     PCR_API_END(c)
 }
 
 int pcr_frames_ransac_plane_samples(const pcr_frames *frames, float distance_threshold, const uint32_t *samples, const uint64_t *sample_offsets,
                                     float *models, uint32_t *inliers, uint64_t *inlier_offsets, pcr_frames **outliers) {
-    PCR_FRAMES_CHECK(frames)
+    PCR_TRY(handle_check(frames, "frames"));
+    Ctx *c = &frames->owner->c;
     if (outliers) *outliers = nullptr;
     PCR_API_BEGIN
     DevSetter ds(c);
     const size_t n = frames->n, F = frames->count();
-    uint32_t *d_inl = nullptr;
-    PCR_CUDA(c, cudaMallocAsync((void **)&d_inl, sizeof(uint32_t) * std::max<size_t>(n, 1), c->stream));
-    struct G {
-        void *p;
-        cudaStream_t s;
-        ~G() { cudaFreeAsync(p, s); }
-    } g{d_inl, c->stream};
+    StreamAlloc<uint32_t> d_inl(c->stream);
+    PCR_CUDA(c, d_inl.alloc(sizeof(uint32_t) * std::max<size_t>(n, 1)));
     PCR_TRY(ransac_batch_entry(frames->owner, true, frames->x(), frames->y(), frames->z(), frames->off.data(), F, distance_threshold, samples,
-                               sample_offsets, models, d_inl, inlier_offsets));
+                               sample_offsets, models, d_inl.p, inlier_offsets));
     const size_t k = (size_t)inlier_offsets[F];
     if (inliers && k) {
-        PCR_CUDA(c, cudaMemcpyAsync(inliers, d_inl, sizeof(uint32_t) * k, cudaMemcpyDeviceToHost, c->stream));
+        PCR_CUDA(c, cudaMemcpyAsync(inliers, d_inl.p, sizeof(uint32_t) * k, cudaMemcpyDeviceToHost, c->stream));
         PCR_CUDA(c, cudaStreamSynchronize(c->stream));
     }
-    if (outliers)  // ransac_plane.rs's inliers are in bounds by construction: straight to the device select_inverse
-        return frames_select_inverse_dev(frames, d_inl, std::vector<uint64_t>(inlier_offsets, inlier_offsets + F + 1), outliers);
+    if (outliers) {  // ransac_plane.rs's inliers are in bounds by construction: straight to the device select_inverse
+        FramesPtr res;
+        PCR_TRY(frames_select_inverse_dev(frames, d_inl.p, std::vector<uint64_t>(inlier_offsets, inlier_offsets + F + 1), res));
+        *outliers = res.release();
+    }
     return PCR_OK;
     PCR_API_END(c)
 }
 
 int pcr_frames_euclidean_cluster(const pcr_frames *frames, float distance_threshold, size_t min_size, size_t max_size, uint32_t *offsets,
                                  uint32_t *indices, uint64_t *cluster_offsets) {
-    PCR_FRAMES_CHECK(frames)
-    (void)c;
+    PCR_TRY(handle_check(frames, "frames"));
     return cluster_batch_entry(frames->owner, true, false, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(),
                                distance_threshold, min_size, max_size, offsets, indices, cluster_offsets);
 }
 
 int pcr_frames_icp_point_to_point(const pcr_frames *frames, const uint32_t *pairs, size_t n_pairs, const pcr_icp_params *params,
                                   pcr_icp_result *results) {
-    PCR_FRAMES_CHECK(frames)
-    (void)c;
+    PCR_TRY(handle_check(frames, "frames"));
     return icp_batch_entry(frames->owner, true, false, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(), nullptr, nullptr,
                            nullptr, 0, pairs, n_pairs, params, results);
 }
 
 int pcr_frames_icp_point_to_plane(const pcr_frames *frames, const uint32_t *pairs, size_t n_pairs, const pcr_icp_params *params,
                                   pcr_icp_result *results) {
-    PCR_FRAMES_CHECK(frames)
+    PCR_TRY(handle_check(frames, "frames"));
     if (!frames->has_normals)  // crates/python/src/registration.rs:80-86
-        return fail(c, PCR_ERR_INVALID_ARG, "point-to-plane ICP needs frames with normals (call estimate_normals first)");
+        return fail(&frames->owner->c, PCR_ERR_INVALID_ARG, "point-to-plane ICP needs frames with normals (call estimate_normals first)");
     return icp_batch_entry(frames->owner, true, true, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(), frames->nx(),
                            frames->ny(), frames->nz(), frames->n, pairs, n_pairs, params, results);
 }

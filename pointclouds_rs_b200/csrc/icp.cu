@@ -876,26 +876,16 @@ int icp_dev(Ctx *ctx, const IcpArgs &a, pcr_icp_result *result) {
     bo.k_hint = 1;
     bo.transient = true;
     PCR_TRY(index_build_dev(ctx, a.d_tx, a.d_ty, a.d_tz, a.nt, bo, &tgt));
-    struct Guard {
-        Index *ix;
-        ~Guard() { index_free(ix); }
-    } guard{tgt};
+    const IndexPtr guard(tgt);
 
     const size_t ns = a.ns;
     // working copy of the source, binned by target cell
-    float4 *cur = nullptr, *nrm4 = nullptr;
-    PCR_CUDA(ctx, cudaMallocAsync((void **)&cur, sizeof(float4) * std::max<size_t>(ns, 1), st));
-    struct FreeLater {
-        void *p;
-        cudaStream_t s;
-        ~FreeLater() {
-            if (p) cudaFreeAsync(p, s);
-        }
-    } f1{cur, st};
-    FreeLater f2{nullptr, st};
+    StreamAlloc<float4> cur_mem(st), nrm4_mem(st);
+    PCR_CUDA(ctx, cur_mem.alloc(sizeof(float4) * std::max<size_t>(ns, 1)));
+    float4 *cur = cur_mem.p, *nrm4 = nullptr;
     if (plane) {
-        PCR_CUDA(ctx, cudaMallocAsync((void **)&nrm4, sizeof(float4) * a.nt, st));
-        f2.p = nrm4;
+        PCR_CUDA(ctx, nrm4_mem.alloc(sizeof(float4) * a.nt));
+        nrm4 = nrm4_mem.p;
         pack_normals_kernel<<<(unsigned)((a.nt + 255) / 256), 256, 0, st>>>(a.d_nx, a.d_ny, a.d_nz, a.nt, nrm4);
         PCR_LAUNCH_CHECK(ctx);
     }
@@ -916,12 +906,12 @@ int icp_dev(Ctx *ctx, const IcpArgs &a, pcr_icp_result *result) {
     // coarser levels of the target grid for deferred source points (built once, reused every iteration)
     Index *levels[kMaxLevels] = {tgt, nullptr, nullptr, nullptr};
     for (int l = 1; l < kMaxLevels; l++) PCR_TRY(index_coarser_level(levels[l - 1], &levels[l]));
-    unsigned long long *nn = nullptr;
-    uint32_t *dlist = nullptr;  // 2 ping-pong lists of ns entries + counters
-    PCR_CUDA(ctx, cudaMallocAsync((void **)&nn, sizeof(unsigned long long) * std::max<size_t>(ns, 1), st));
-    FreeLater f3{nn, st};
-    PCR_CUDA(ctx, cudaMallocAsync((void **)&dlist, sizeof(uint32_t) * (2 * std::max<size_t>(ns, 1) + 64), st));
-    FreeLater f4{dlist, st};
+    StreamAlloc<unsigned long long> nn_mem(st);
+    PCR_CUDA(ctx, nn_mem.alloc(sizeof(unsigned long long) * std::max<size_t>(ns, 1)));
+    StreamAlloc<uint32_t> dlist_mem(st);  // 2 ping-pong lists of ns entries + counters
+    PCR_CUDA(ctx, dlist_mem.alloc(sizeof(uint32_t) * (2 * std::max<size_t>(ns, 1) + 64)));
+    unsigned long long *nn = nn_mem.p;
+    uint32_t *dlist = dlist_mem.p;
     uint32_t *dcount = dlist;  // [kMaxLevels]
     uint32_t *dl[2] = {dlist + 64, dlist + 64 + std::max<size_t>(ns, 1)};
 
@@ -1053,10 +1043,7 @@ int icp_batch_dev(Ctx *ctx, const IcpBatchArgs &a, pcr_icp_result *results) {
     bo.n_frames = (int)a.n_frames;
     bo.frame_offsets = a.frame_offsets;
     PCR_TRY(index_build_dev(ctx, a.d_x, a.d_y, a.d_z, a.n, bo, &tgt));
-    struct Guard {
-        Index *ix;
-        ~Guard() { index_free(ix); }
-    } guard{tgt};
+    const IndexPtr guard(tgt);
     Index *levels[kMaxLevels] = {tgt, nullptr, nullptr, nullptr};
     for (int l = 1; l < kMaxLevels; l++) PCR_TRY(index_coarser_level(levels[l - 1], &levels[l]));
 
@@ -1071,15 +1058,9 @@ int icp_batch_dev(Ctx *ctx, const IcpBatchArgs &a, pcr_icp_result *results) {
     const size_t tab_words = 4 * (size_t)Q + 2;
     const size_t o_nrm = o_tab + up(sizeof(uint32_t) * tab_words);
     const size_t bytes = o_nrm + (plane ? sizeof(float4) * a.n : 0);
-    char *mem = nullptr;
-    PCR_CUDA(ctx, cudaMallocAsync((void **)&mem, bytes, st));
-    struct FreeLater {
-        void *p;
-        cudaStream_t s;
-        ~FreeLater() {
-            if (p) cudaFreeAsync(p, s);
-        }
-    } f1{mem, st};
+    StreamAlloc<char> mem_alloc(st);
+    PCR_CUDA(ctx, mem_alloc.alloc(bytes));
+    char *mem = mem_alloc.p;
     float4 *cur = (float4 *)mem;
     unsigned long long *nn = (unsigned long long *)(mem + o_nn);
     uint32_t *dcount = (uint32_t *)(mem + o_dl);  // [kMaxLevels]
@@ -1119,10 +1100,9 @@ int icp_batch_dev(Ctx *ctx, const IcpBatchArgs &a, pcr_icp_result *results) {
         const int cell_bits = bits_for(max_cells);
         const int key_bits = cell_bits + bits_for((uint64_t)Q);
         const size_t hist_words = radix_sort_hist_words(total);
-        char *sm = nullptr;
-        PCR_CUDA(ctx, cudaMallocAsync((void **)&sm, up(2 * sizeof(unsigned long long) * total) + up(2 * sizeof(uint32_t) * total) +
-                                                        sizeof(uint32_t) * hist_words, st));
-        FreeLater f2{sm, st};
+        StreamAlloc<char> sm_alloc(st);
+        PCR_CUDA(ctx, sm_alloc.alloc(up(2 * sizeof(unsigned long long) * total) + up(2 * sizeof(uint32_t) * total) + sizeof(uint32_t) * hist_words));
+        char *sm = sm_alloc.p;
         unsigned long long *kA = (unsigned long long *)sm, *kB = kA + total;
         uint32_t *vA = (uint32_t *)(sm + up(2 * sizeof(unsigned long long) * total)), *vB = vA + total;
         uint32_t *hist = (uint32_t *)((char *)vA + up(2 * sizeof(uint32_t) * total));

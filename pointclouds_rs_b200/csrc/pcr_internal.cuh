@@ -8,6 +8,7 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -233,6 +234,25 @@ struct TimeScope {  // records an event pair around a stage when timing is enabl
 int ensure(Ctx *ctx, DevBuf &b, size_t bytes);
 int ensure_pinned(Ctx *ctx, size_t bytes);
 
+// A device allocation owned by a scope: cudaMallocAsync in alloc(), cudaFreeAsync on the same stream at scope exit,
+// so an error return frees it in stream order after the work already queued.
+template <class T = void>
+struct StreamAlloc {
+    T *p = nullptr;
+    cudaStream_t s;
+    explicit StreamAlloc(cudaStream_t stream) : s(stream) {}
+    StreamAlloc(const StreamAlloc &) = delete;
+    StreamAlloc &operator=(const StreamAlloc &) = delete;
+    ~StreamAlloc() {
+        if (p) cudaFreeAsync(p, s);
+    }
+    cudaError_t alloc(size_t bytes) {
+        const cudaError_t e = cudaMallocAsync((void **)&p, bytes, s);
+        if (e != cudaSuccess) p = nullptr;
+        return e;
+    }
+};
+
 // ------------------------------------------------------------------------------------------------
 // host entry points implemented across the .cu files (all asynchronous on ctx->stream)
 // ------------------------------------------------------------------------------------------------
@@ -256,6 +276,10 @@ struct BuildOpts {
 int index_build_dev(Ctx *ctx, const float *dx, const float *dy, const float *dz, size_t n,
                     const BuildOpts &opts, Index **out);
 void index_free(Index *ix);
+struct IndexFree {
+    void operator()(Index *ix) const { index_free(ix); }
+};
+using IndexPtr = std::unique_ptr<Index, IndexFree>;  // an index owned by a scope
 // The next-coarser level of `ix` (cell size x kLevelFactor), built on first use and owned by `ix`.
 int index_coarser_level(Index *ix, Index **out);
 // The finer level of `ix` (cell size / 2, or as fine as the cell-table cap allows), built on first use and owned by `ix`.

@@ -359,6 +359,19 @@ def test_errors(pcr):
         cl = C.c_void_p(1234)
         assert lib.pcr_frames_frame(fr, 2, C.byref(cl)) == _ffi.PCR_ERR_INVALID_ARG and cl.value is None
         assert lib.pcr_frames_frame(None, 0, C.byref(cl)) == _ffi.PCR_ERR_INVALID_ARG
+        # the pcr_cloud filters hand out no handle on failure either
+        assert lib.pcr_frames_frame(fr, 0, C.byref(cl)) == _ffi.PCR_OK
+        try:
+            outside = np.array([300], np.uint32)
+            for call in (lambda o: lib.pcr_cloud_select(cl, u32(outside), 1, o),
+                         lambda o: lib.pcr_cloud_voxel_downsample(cl, 0.0, o),
+                         lambda o: lib.pcr_cloud_statistical_outlier_removal(cl, 10, -1.0, o),
+                         lambda o: lib.pcr_cloud_estimate_normals(cl, 0, None, o),
+                         lambda o: lib.pcr_cloud_sor_normals(cl, 10, 1.0, 0, None, o)):
+                o = C.c_void_p(1234)
+                assert call(C.byref(o)) == _ffi.PCR_ERR_INVALID_ARG and o.value is None
+        finally:
+            lib.pcr_cloud_free(cl)
         # ICP: a pair outside [0, F), point-to-plane without normals
         prm = _ffi.IcpParams(10, 1e-5, float("inf"))
         res = (_ffi.IcpResultC * 1)()

@@ -326,6 +326,7 @@ def test_c_error_codes(mixed):
     bad = q_off.copy()
     bad[0] = 1
     assert knn(off=bad) == _ffi.PCR_ERR_INVALID_ARG
+    assert "query_offsets" in _ffi.last_error(ctx._h)
     bad = q_off.copy()
     bad[2], bad[3] = bad[3], bad[2] - 1
     assert knn(off=bad) == _ffi.PCR_ERR_INVALID_ARG

@@ -343,3 +343,24 @@ def test_errors(pcr):
     # 65535 frames are accepted (all empty but the last, which holds every point)
     assert vox(f(x), u64(many[1:]), 65535, outp=u64(big_out)) == _ffi.PCR_OK
     assert not big_out[:65535].any() and int(big_out[65535]) == len(pcr.voxel_downsample(_cloud(pts), 0.1))
+    # SOR + normals batch, all three forms: bad frame offsets are rejected before any device work and named in the
+    # message, also for one frame; no frames is nothing to do
+    import torch
+
+    d = [torch.from_numpy(a).cuda() for a in (x, y, z)]
+    d_out = [torch.zeros(len(pts), dtype=dt, device="cuda") for dt in (torch.uint8, torch.float32, torch.float32, torch.float32)]
+    torch.cuda.synchronize()
+    keep, kept = np.zeros(len(pts), np.uint8), np.zeros(2, np.uint64)
+    rows, nrm_rows = np.ascontiguousarray(pts, np.float32), np.zeros((len(pts), 3), np.float32)
+    u8 = lambda a: a.ctypes.data_as(_ffi.u8p)
+    forms = (lambda offp, nf: lib.pcr_sor_normals_batch(h, f(x), f(y), f(z), offp, nf, 10, 1.0, 20, f(vp), u8(keep), f(o[0]), f(o[1]), f(o[2]),
+                                                        u64(kept)),
+             lambda offp, nf: lib.pcr_sor_normals_batch_dev(h, *(t.data_ptr() for t in d), offp, nf, 10, 1.0, 20, f(vp),
+                                                            *(t.data_ptr() for t in d_out)),
+             lambda offp, nf: lib.pcr_sor_normals_batch_rows(h, f(rows), offp, nf, 10, 1.0, 20, f(vp), u8(keep), f(nrm_rows), u64(kept)))
+    for call in forms:
+        for bad in ([0, 400, 300], [1, 300, 600], [1, 300]):
+            b = np.array(bad, np.uint64)
+            assert call(u64(b), len(bad) - 1) == _ffi.PCR_ERR_INVALID_ARG
+            assert "frame_offsets" in _ffi.last_error(h)
+        assert call(u64(off), 0) == _ffi.PCR_OK
