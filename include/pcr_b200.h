@@ -27,6 +27,10 @@
  *   pcr_frames_*                a batch of frames kept in HBM between those calls (the batch form of pcr_cloud_*)
  *   pcr_index_build_batch / pcr_knn_batch / pcr_radius_*_batch / pcr_find_correspondences_batch
  *                               the KdTree queries of many frames per call, each frame searched alone
+ *   pcr_apply_transform_batch / pcr_frames_apply_transform / pcr_transform_compose / pcr_frames_merge
+ *                               apply_transform of many frames per call, RigidTransform::compose
+ *                               (crates/registration/src/icp.rs:39-92), and the frames joined into one cloud: the
+ *                               map of an odometry chain assembled on the device
  *
  * The reference calls its kd-tree once per point inside serial loops; a per-query C call would be
  * useless on a GPU, so the boundary is BATCHED and sits one level up: it replaces the bodies of the
@@ -292,6 +296,22 @@ int pcr_find_correspondences(pcr_index *target, const float *sx, const float *sy
 int pcr_apply_transform(pcr_ctx *ctx, const float *x, const float *y, const float *z, size_t n,
                         const float rotation[9], const float translation[3], float *ox, float *oy,
                         float *oz);
+/* apply_transform of every frame of a batch: frame f = points [frame_offsets[f], frame_offsets[f+1]) (HOST offsets) is
+ * moved by transforms[12f .. 12f+12) (HOST: row-major rotation[9], then translation[3]); frame f's output is bit for bit
+ * what pcr_apply_transform returns for frame f alone with that transform.  Offsets that do not start at 0 or decrease, or a
+ * NULL pointer -> PCR_ERR_INVALID_ARG; N >= 2^31 or more than 65535 frames -> PCR_ERR_UNSUPPORTED; n_frames == 0 -> PCR_OK.
+ * The transform values are not checked, as in pcr_apply_transform.  _dev: device points, host offsets and transforms
+ * (free for reuse on return), enqueued on the context's stream. */
+int pcr_apply_transform_batch(pcr_ctx *ctx, const float *x, const float *y, const float *z,
+                              const uint64_t *frame_offsets, size_t n_frames, const float *transforms,
+                              float *ox, float *oy, float *oz);
+int pcr_apply_transform_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z,
+                                  const uint64_t *frame_offsets, size_t n_frames, const float *transforms,
+                                  float *d_ox, float *d_oy, float *d_oz);
+/* RigidTransform::compose (icp.rs:52-73): apply `first`, then `then`.  R = then.R * first.R,
+ * t = then.R * first.t + then.t, f32 in the reference's operation order, no FMA; 12-float layout as above.  Host only:
+ * needs no context or device.  out may alias first or then. */
+int pcr_transform_compose(const float first[12], const float then[12], float out[12]);
 int pcr_icp_point_to_point(pcr_ctx *ctx, const float *sx, const float *sy, const float *sz, size_t ns,
                            const float *tx, const float *ty, const float *tz, size_t nt,
                            const pcr_icp_params *params, pcr_icp_result *result);
@@ -561,6 +581,11 @@ int pcr_frames_download(const pcr_frames *frames, float *x, float *y, float *z, 
 int pcr_frames_download_rows(const pcr_frames *frames, float *xyz, float *normals);
 /* frame f as a new pcr_cloud (a device copy, normals carried), for the single-frame calls; f >= count -> INVALID_ARG */
 int pcr_frames_frame(const pcr_frames *frames, size_t f, pcr_cloud **out);
+/* all frames as one pcr_cloud, in frame order, normals carried (the map that pcr_cloud_voxel_downsample then thins) */
+int pcr_frames_merge(const pcr_frames *frames, pcr_cloud **out);
+/* pcr_apply_transform_batch on the batch: frame f moved by transforms[12f .. 12f+12) (HOST, count x 12 floats).  The
+ * result holds xyz only (icp.rs:91, as pcr_cloud_apply_transform); the offsets are unchanged. */
+int pcr_frames_apply_transform(const pcr_frames *frames, const float *transforms, pcr_frames **out);
 /* Per frame, list f = indices[index_offsets[f] .. index_offsets[f+1]) (HOST, index_offsets count + 1 entries).
  * invert = 0: select (cloud.rs:103-140), the listed points in list order, duplicates kept; invert = 1: select_inverse,
  * the unlisted points in their order.  Normals are carried.  An index >= its frame's size -> PCR_ERR_INVALID_ARG naming the

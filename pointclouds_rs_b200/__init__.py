@@ -19,6 +19,8 @@ and for the steps either side of it (SURVEY.md section 8f):
     ransac_plane(cloud, threshold, iterations)          crates/segmentation/src/ransac_plane.rs:56-129 (after the sampling step)
     DeviceCloud                                         a PointCloud that stays in HBM between the steps of a pipeline
     DeviceFrames                                        a batch of frames that stays in HBM between the batch calls
+    apply_transform_batch / compose / chain_poses       apply_transform of many frames per call, RigidTransform::compose
+                                                        (icp.rs:39-92), and the poses of an odometry chain
 
 Everything runs through the C ABI (include/pcr_b200.h) of lib/libpcr_b200.so: hand-written sm_100a
 CUDA, no PyTorch on the path, no CPU fallback.  Out of scope (DESIGN.md section 8): passthrough_filter and file IO.
@@ -43,7 +45,7 @@ __all__ = [
     "icp_point_to_point_batch", "icp_point_to_plane_batch", "voxel_downsample_batch", "estimate_normals_batch",
     "sor_normals_batch", "default_context", "PcrError", "euclidean_cluster", "voxel_downsample", "DeviceCloud", "ransac_plane", "PlaneResult",
     "ransac_plane_samples_batch", "ransac_plane_batch", "cluster_arrays_batch", "euclidean_cluster_batch",
-    "DeviceFrames", "radius_outlier_removal_batch", "KdTreeBatch",
+    "DeviceFrames", "radius_outlier_removal_batch", "KdTreeBatch", "apply_transform_batch", "compose", "chain_poses",
 ]
 
 
@@ -605,6 +607,68 @@ def _batch_frames(points, frame_offsets):
     return np.ascontiguousarray(pts, np.float32), np.ascontiguousarray(off, np.uint64)
 
 
+def _frame_transforms(transforms, n_frames: int) -> np.ndarray:
+    """Checks and converts one rigid transform per frame -> (F, 12) f32 rows: row-major rotation, then translation.
+    (F, 3, 4) is read as [R | t] per frame."""
+    t = np.asarray(transforms)
+    if t.ndim == 3 and t.shape[1:] == (3, 4):
+        t = np.concatenate([t[:, :, :3].reshape(-1, 9), t[:, :, 3]], axis=1)
+    if t.ndim != 2 or t.shape[1] != 12 or t.dtype.kind not in "iuf":
+        raise ValueError(f"transforms must have shape (F, 12) or (F, 3, 4); got {t.shape}")
+    if len(t) != n_frames:
+        raise ValueError(f"expected one transform per frame ({n_frames} frames), got {len(t)}")
+    return np.ascontiguousarray(t, np.float32)
+
+
+def _transform12(rotation, translation) -> np.ndarray:
+    return np.concatenate([np.asarray(rotation, np.float32).reshape(9), np.asarray(translation, np.float32).reshape(3)])
+
+
+def compose(first, then):
+    """RigidTransform::compose (icp.rs:52-73): the transform that applies `first`, then `then`.  Args: (R, t) pairs;
+    -> (R (3,3) f32, t (3,) f32) with R = then.R @ first.R and t = then.R @ first.t + then.t, in the reference's f32
+    operation order (no FMA)."""
+    a, b, out = _transform12(*first), _transform12(*then), np.empty(12, np.float32)
+    _ffi.check(_ffi.load().pcr_transform_compose(_p(a, _ffi.f32p), _p(b, _ffi.f32p), _p(out, _ffi.f32p)))
+    return out[:9].reshape(3, 3), out[9:].copy()
+
+
+def chain_poses(relative) -> np.ndarray:
+    """Poses of an odometry chain -> (n + 1, 12) f32, the layout apply_transform_batch takes.  `relative`: the n
+    IcpResults of the CONSECUTIVE pairs (i + 1, i) in order (relative[i] takes frame i + 1 into frame i's coordinates),
+    or their transforms as apply_transform_batch takes them: (n, 12) rows (row-major R, then t) or (n, 3, 4) [R | t].
+    pose[0] is the identity and pose[i + 1] = compose(relative[i], pose[i]): the transform that takes frame i + 1 into
+    frame 0's coordinates.  Other pairings are not chains and give meaningless poses."""
+    if isinstance(relative, np.ndarray):
+        rel = relative
+    else:
+        rel = [_transform12(r.rotation, r.translation) if isinstance(r, IcpResult) else r for r in relative]
+        rel = np.asarray(rel) if rel else np.zeros((0, 12), np.float32)
+    rel = _frame_transforms(rel, len(rel) if rel.ndim else 0)
+    poses = np.zeros((len(rel) + 1, 12), np.float32)
+    poses[0, [0, 4, 8]] = 1.0
+    lib = _ffi.load()
+    for i in range(len(rel)):
+        _ffi.check(lib.pcr_transform_compose(_p(rel[i], _ffi.f32p), _p(poses[i], _ffi.f32p), _p(poses[i + 1], _ffi.f32p)))
+    return poses
+
+
+def apply_transform_batch(points: np.ndarray, frame_offsets: Sequence[int], transforms, ctx: Optional[Context] = None) -> np.ndarray:
+    """apply_transform of every frame of a batch in one call.  points: (N,3), frame f = rows [frame_offsets[f],
+    frame_offsets[f+1]); transforms: (F, 12) (row-major R, then t) or (F, 3, 4) [R | t], one per frame.  -> (N,3) f32,
+    frame f's rows bit for bit what apply_transform returns for the frame alone with transform f."""
+    pts, off = _batch_frames(points, frame_offsets)
+    tr = _frame_transforms(transforms, len(off) - 1)
+    ctx = ctx or default_context()
+    x, y, z = _soa(pts)
+    n = len(pts)
+    ox, oy, oz = (np.empty(max(n, 1), np.float32) for _ in range(3))
+    st = _ffi.load().pcr_apply_transform_batch(ctx._h, _p(x, _ffi.f32p), _p(y, _ffi.f32p), _p(z, _ffi.f32p), _p(off, _ffi.u64p), len(off) - 1,
+                                               _p(tr, _ffi.f32p), _p(ox, _ffi.f32p), _p(oy, _ffi.f32p), _p(oz, _ffi.f32p))
+    _ffi.check(st, ctx._h)
+    return np.stack([ox[:n], oy[:n], oz[:n]], axis=1)
+
+
 def _icp_batch_arrays(points, frame_offsets, pairs):
     """Checks and converts the frame buffer of a batched ICP: (N,3) f32 rows, u64 offsets, (P,2) u32 pairs."""
     pts, off = _batch_frames(points, frame_offsets)
@@ -1112,6 +1176,19 @@ class DeviceFrames:
         h = C.c_void_p()
         _ffi.check(_ffi.load().pcr_frames_frame(self._h, int(f), C.byref(h)), self._ctx._h)
         return DeviceCloud(h, self._ctx)
+
+    def merge(self) -> DeviceCloud:
+        """All frames as one DeviceCloud, in frame order, normals carried (a device copy): the map of an odometry chain
+        once every frame is in one frame's coordinates (apply_transform), ready for voxel_downsample."""
+        h = C.c_void_p()
+        _ffi.check(_ffi.load().pcr_frames_merge(self._h, C.byref(h)), self._ctx._h)
+        return DeviceCloud(h, self._ctx)
+
+    def apply_transform(self, transforms) -> "DeviceFrames":
+        """Frame f moved by transforms[f]: (F, 12) (row-major R, then t, as chain_poses returns them) or (F, 3, 4) [R | t].
+        The result carries xyz only (icp.rs:91) and the same offsets."""
+        tr = _frame_transforms(transforms, self.n_frames)
+        return self._new(_ffi.load().pcr_frames_apply_transform, _p(tr, _ffi.f32p))
 
     def to_numpy(self):
         """-> (points (N, 3) f32, offsets (F+1,) u64), one download."""

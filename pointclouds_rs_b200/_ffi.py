@@ -167,6 +167,11 @@ SIGNATURES = {
     "pcr_frames_download": (C.c_int, [vp, vp, vp, vp, vp, vp, vp]),
     "pcr_frames_download_rows": (C.c_int, [vp, vp, vp]),
     "pcr_frames_frame": (C.c_int, [vp, C.c_size_t, C.POINTER(vp)]),
+    "pcr_frames_merge": (C.c_int, [vp, C.POINTER(vp)]),
+    "pcr_frames_apply_transform": (C.c_int, [vp, f32p, C.POINTER(vp)]),
+    "pcr_apply_transform_batch": (C.c_int, [vp, f32p, f32p, f32p, u64p, C.c_size_t, f32p, f32p, f32p, f32p]),
+    "pcr_apply_transform_batch_dev": (C.c_int, [vp, vp, vp, vp, u64p, C.c_size_t, f32p, vp, vp, vp]),
+    "pcr_transform_compose": (C.c_int, [f32p, f32p, f32p]),
     "pcr_frames_select": (C.c_int, [vp, u32p, u64p, C.c_int, C.POINTER(vp)]),
     "pcr_frames_voxel_downsample": (C.c_int, [vp, C.c_float, C.POINTER(vp)]),
     "pcr_frames_statistical_outlier_removal": (C.c_int, [vp, C.c_size_t, C.c_float, C.POINTER(vp)]),

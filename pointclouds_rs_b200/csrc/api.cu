@@ -1592,6 +1592,57 @@ int pcr_radius_outlier_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_
     return ror_batch_entry(ctx, true, d_x, d_y, d_z, frame_offsets, n_frames, radius, min_neighbors, d_keep, nullptr);
 }
 
+/* ---- batched apply_transform --------------------------------------------------------------------------- */
+// Frame f moved by transform f; the transform values are not checked (pcr_apply_transform does not check them either).
+static int apply_transform_batch_entry(pcr_ctx *ctx, bool dev, const float *x, const float *y, const float *z, const uint64_t *frame_offsets,
+                                       size_t n_frames, const float *transforms, float *ox, float *oy, float *oz) {
+    if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
+    Ctx *c = &ctx->c;
+    PCR_TRY(offsets_check(c, "frame_offsets", frame_offsets, n_frames));
+    const size_t n = (size_t)frame_offsets[n_frames];
+    PCR_TRY(batch_size_check(c, n, n_frames));
+    if ((n_frames && !transforms) || (n && (!x || !y || !z || !ox || !oy || !oz))) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    if (n == 0) return PCR_OK;
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    if (dev) return apply_transform_batch_dev(c, x, y, z, frame_offsets, n_frames, nullptr, transforms, ox, oy, oz);
+    float *dx, *dy, *dz;
+    PCR_TRY(stage_xyz(c, c->b_in, x, y, z, n, &dx, &dy, &dz));
+    const size_t stride = (n + 63) & ~(size_t)63;
+    PCR_TRY(ensure(c, c->b_out, sizeof(float) * 3 * stride));
+    float *o0 = (float *)c->b_out.p, *o1 = o0 + stride, *o2 = o1 + stride;
+    PCR_TRY(apply_transform_batch_dev(c, dx, dy, dz, frame_offsets, n_frames, nullptr, transforms, o0, o1, o2));
+    PCR_CUDA(c, cudaMemcpyAsync(ox, o0, n * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    PCR_CUDA(c, cudaMemcpyAsync(oy, o1, n * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    PCR_CUDA(c, cudaMemcpyAsync(oz, o2, n * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    PCR_CUDA(c, cudaStreamSynchronize(c->stream));
+    return PCR_OK;
+    PCR_API_END(c)
+}
+
+int pcr_apply_transform_batch(pcr_ctx *ctx, const float *x, const float *y, const float *z, const uint64_t *frame_offsets, size_t n_frames,
+                              const float *transforms, float *ox, float *oy, float *oz) {
+    return apply_transform_batch_entry(ctx, false, x, y, z, frame_offsets, n_frames, transforms, ox, oy, oz);
+}
+int pcr_apply_transform_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z, const uint64_t *frame_offsets,
+                                  size_t n_frames, const float *transforms, float *d_ox, float *d_oy, float *d_oz) {
+    return apply_transform_batch_entry(ctx, true, d_x, d_y, d_z, frame_offsets, n_frames, transforms, d_ox, d_oy, d_oz);
+}
+
+// icp.rs:52-73 (RigidTransform::compose), the operation order of icp_step's compose (icp.cu): host code, built with
+// -ffp-contract=off (Makefile) so that no product is fused into a sum.
+int pcr_transform_compose(const float first[12], const float then[12], float out[12]) {
+    if (!first || !then || !out) return fail(nullptr, PCR_ERR_INVALID_ARG, "null pointer");
+    const float *A = then, *B = first;  // R = then.R * first.R, t = then.R * first.t + then.t
+    float r[12];
+    for (int i = 0; i < 3; i++) {
+        for (int j = 0; j < 3; j++) r[i * 3 + j] = (A[i * 3 + 0] * B[0 * 3 + j] + A[i * 3 + 1] * B[1 * 3 + j]) + A[i * 3 + 2] * B[2 * 3 + j];
+        r[9 + i] = ((A[i * 3 + 0] * B[9] + A[i * 3 + 1] * B[10]) + A[i * 3 + 2] * B[11]) + A[9 + i];
+    }
+    memcpy(out, r, sizeof(r));  // out may be first or then
+    return PCR_OK;
+}
+
 /* ---- multi-frame batch ---------------------------------------------------------------------------- */
 namespace pcr {
 // frames of exactly one point are returned unchanged by the reference (statistical_outlier.rs:10-12)
@@ -2668,6 +2719,37 @@ int pcr_frames_frame(const pcr_frames *frames, size_t f, pcr_cloud **out) {
     CloudPtr res;
     PCR_TRY(points_alloc(frames->owner, (size_t)(frames->off[f + 1] - frames->off[f]), frames->has_normals, res));
     PCR_TRY(copy_arrays(frames, (size_t)frames->off[f], frames->arrays(), res.get()));
+    *out = res.release();
+    return PCR_OK;
+    PCR_API_END(c)
+}
+
+int pcr_frames_merge(const pcr_frames *frames, pcr_cloud **out) {
+    if (out) *out = nullptr;
+    PCR_TRY(handle_check(frames, "frames"));
+    Ctx *c = &frames->owner->c;
+    if (!out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    CloudPtr res;  // pcr_frames_frame over all frames: the arrays hold the frames back to back already
+    PCR_TRY(points_alloc(frames->owner, frames->n, frames->has_normals, res));
+    PCR_TRY(copy_arrays(frames, 0, frames->arrays(), res.get()));
+    *out = res.release();
+    return PCR_OK;
+    PCR_API_END(c)
+}
+
+int pcr_frames_apply_transform(const pcr_frames *frames, const float *transforms, pcr_frames **out) {
+    if (out) *out = nullptr;
+    PCR_TRY(handle_check(frames, "frames"));
+    Ctx *c = &frames->owner->c;
+    if (!out || !transforms) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    FramesPtr res;  // icp.rs:91: xyz only; the offsets are the input's
+    PCR_TRY(frames_alloc(frames->owner, frames->n, false, frames->off, res, frames->d_off));
+    PCR_TRY(apply_transform_batch_dev(c, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(), frames->d_off, transforms,
+                                      res->x(), res->y(), res->z()));
     *out = res.release();
     return PCR_OK;
     PCR_API_END(c)

@@ -63,6 +63,27 @@ __global__ void apply_transform_kernel(const float *__restrict__ x, const float 
     oz[i] = c;
 }
 
+// Every frame of a batch by its own transform: one thread per point over all N points, so the grid does not depend on
+// how uneven the frames are; point i finds its frame in the u32 offsets and reads that frame's 12 floats.
+__global__ void apply_transform_batch_kernel(const float *__restrict__ x, const float *__restrict__ y, const float *__restrict__ z,
+                                             size_t n, const float *__restrict__ Rt /* 12 per frame */,
+                                             const uint32_t *__restrict__ frame_off, int n_frames, float *__restrict__ ox,
+                                             float *__restrict__ oy, float *__restrict__ oz) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const float *rt = Rt + 12 * frame_of(frame_off, n_frames, (uint32_t)i);
+    float R[9], t[3];
+#pragma unroll
+    for (int j = 0; j < 9; j++) R[j] = rt[j];
+#pragma unroll
+    for (int j = 0; j < 3; j++) t[j] = rt[9 + j];
+    float a, b, c;
+    apply_point(R, t, x[i], y[i], z[i], a, b, c);
+    ox[i] = a;
+    oy[i] = b;
+    oz[i] = c;
+}
+
 // ---- plain correspondences (C ABI pcr_find_correspondences): k = 1 KNN + the distance test ------
 __global__ void correspond_filter_kernel(size_t ns, float max_distance, uint32_t *__restrict__ tgt, float *__restrict__ dist,
                                          const uint32_t *__restrict__ counts) {
@@ -850,6 +871,26 @@ int apply_transform_dev(Ctx *ctx, const float *dx, const float *dy, const float 
     memcpy((char *)ctx->pinned + 2048, h, sizeof(h));
     PCR_CUDA(ctx, cudaMemcpyAsync(d_rt, (char *)ctx->pinned + 2048, sizeof(h), cudaMemcpyHostToDevice, ctx->stream));
     apply_transform_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(dx, dy, dz, n, d_rt, ox, oy, oz);
+    PCR_LAUNCH_CHECK(ctx);
+    return PCR_OK;
+}
+
+int apply_transform_batch_dev(Ctx *ctx, const float *dx, const float *dy, const float *dz, const uint64_t *frame_offsets, size_t n_frames,
+                              const uint32_t *d_frame_off, const float *transforms, float *ox, float *oy, float *oz) {
+    const size_t n = (size_t)frame_offsets[n_frames];
+    if (n == 0) return PCR_OK;
+    // transforms (12 f32 per frame), then the u32 offsets unless the caller has them on the device: one pageable staging
+    // copy, so the caller's arrays are free again when the call returns
+    std::vector<uint32_t> h(12 * n_frames + (d_frame_off ? 0 : n_frames + 1));
+    memcpy(h.data(), transforms, sizeof(float) * 12 * n_frames);
+    if (!d_frame_off)
+        for (size_t f = 0; f <= n_frames; f++) h[12 * n_frames + f] = (uint32_t)frame_offsets[f];
+    StreamAlloc<uint32_t> mem(ctx->stream);
+    PCR_CUDA(ctx, mem.alloc(sizeof(uint32_t) * h.size()));
+    PCR_CUDA(ctx, cudaMemcpyAsync(mem.p, h.data(), sizeof(uint32_t) * h.size(), cudaMemcpyHostToDevice, ctx->stream));
+    const float *d_rt = (const float *)mem.p;
+    const uint32_t *d_off = d_frame_off ? d_frame_off : mem.p + 12 * n_frames;
+    apply_transform_batch_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(dx, dy, dz, n, d_rt, d_off, (int)n_frames, ox, oy, oz);
     PCR_LAUNCH_CHECK(ctx);
     return PCR_OK;
 }

@@ -364,6 +364,11 @@ int find_correspondences_dev(Index *target, const float *dsx, const float *dsy, 
                              size_t ns, float max_distance, uint32_t *d_tgt, float *d_dist, const QueryFrames *qf = nullptr);
 int apply_transform_dev(Ctx *ctx, const float *dx, const float *dy, const float *dz, size_t n,
                         const float R[9], const float t[3], float *ox, float *oy, float *oz);
+// every frame of a batch (pcr_apply_transform_batch, arguments checked by the caller): frame f = points [frame_offsets[f],
+// frame_offsets[f+1]) (host) moved by transforms[12f .. 12f+12) (host: row-major R, then t).  d_frame_off: the same offsets
+// as u32 on the device if the caller holds them (a pcr_frames batch), else nullptr and they are uploaded with the transforms.
+int apply_transform_batch_dev(Ctx *ctx, const float *dx, const float *dy, const float *dz, const uint64_t *frame_offsets, size_t n_frames,
+                              const uint32_t *d_frame_off, const float *transforms, float *ox, float *oy, float *oz);
 
 // euclidean_cluster (cluster.cu): labels[i] = smallest index of the component of point i
 // (d_frame_off: device frame offsets of a batch, no component crosses a frame; labels stay global indices)
