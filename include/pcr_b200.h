@@ -31,6 +31,10 @@
  *                               apply_transform of many frames per call, RigidTransform::compose
  *                               (crates/registration/src/icp.rs:39-92), and the frames joined into one cloud: the
  *                               map of an odometry chain assembled on the device
+ *   pcr_icp_point_to_*_init[_dev] / pcr_icp_point_to_*_batch_init[_dev] / pcr_cloud_icp_point_to_*_init /
+ *   pcr_frames_icp_point_to_*_init
+ *                               ICP started from a guess (Open3D's registration_icp(init), PCL's align(guess)):
+ *                               coarse-to-fine, priors, multi-start, and with max_iterations == 0 the metrics at a pose
  *
  * The reference calls its kd-tree once per point inside serial loops; a per-query C call would be
  * useless on a GPU, so the boundary is BATCHED and sits one level up: it replaces the bodies of the
@@ -329,6 +333,30 @@ int pcr_icp_point_to_plane_dev(pcr_ctx *ctx, const float *d_sx, const float *d_s
                                size_t ns, const float *d_tx, const float *d_ty, const float *d_tz,
                                size_t nt, const float *d_nx, const float *d_ny, const float *d_nz,
                                size_t n_normals, const pcr_icp_params *params, pcr_icp_result *result);
+/* ICP started from a guess: init is 12 floats (row-major rotation[9], then translation[3], the layout of
+ * pcr_apply_transform_batch).  The loop is the reference loop seeded with init: current = apply_transform(source, init),
+ * bit for bit what pcr_apply_transform returns, and cumulative = init; every increment is then composed onto it as in the
+ * plain call, so the result's transform includes init.  max_iterations == 0: the transform is init and fitness / rmse are
+ * measured at init (Open3D's evaluate_registration).  An empty source or target: the transform is init, converged as in
+ * the plain call.  An identity init gives what the plain call gives, within its rounding (the single-pair call orders the
+ * points of a grid cell by atomics).  init NULL, or a NaN / Inf in it -> PCR_ERR_INVALID_ARG before any device work;
+ * orthonormality is not checked, as in pcr_apply_transform.  A failing call leaves *result untouched.  Sharded (a
+ * communicator): every rank passes the same init and moves its own shard. */
+int pcr_icp_point_to_point_init(pcr_ctx *ctx, const float *sx, const float *sy, const float *sz, size_t ns,
+                                const float *tx, const float *ty, const float *tz, size_t nt, const float init[12],
+                                const pcr_icp_params *params, pcr_icp_result *result);
+int pcr_icp_point_to_plane_init(pcr_ctx *ctx, const float *sx, const float *sy, const float *sz, size_t ns,
+                                const float *tx, const float *ty, const float *tz, size_t nt,
+                                const float *nx, const float *ny, const float *nz, size_t n_normals, const float init[12],
+                                const pcr_icp_params *params, pcr_icp_result *result);
+int pcr_icp_point_to_point_init_dev(pcr_ctx *ctx, const float *d_sx, const float *d_sy, const float *d_sz,
+                                    size_t ns, const float *d_tx, const float *d_ty, const float *d_tz,
+                                    size_t nt, const float init[12], const pcr_icp_params *params, pcr_icp_result *result);
+int pcr_icp_point_to_plane_init_dev(pcr_ctx *ctx, const float *d_sx, const float *d_sy, const float *d_sz,
+                                    size_t ns, const float *d_tx, const float *d_ty, const float *d_tz,
+                                    size_t nt, const float *d_nx, const float *d_ny, const float *d_nz,
+                                    size_t n_normals, const float init[12], const pcr_icp_params *params,
+                                    pcr_icp_result *result);
 
 /* Batched ICP: many (source, target) pairs of frames in one call.  The frames sit back to back in one buffer, frame f =
  * points [frame_offsets[f], frame_offsets[f+1]) (as in pcr_sor_normals_batch), N = frame_offsets[n_frames].  Pair p
@@ -364,6 +392,30 @@ int pcr_icp_point_to_plane_batch_dev(pcr_ctx *ctx, const float *d_x, const float
                                      const float *d_nx, const float *d_ny, const float *d_nz, size_t n_normals,
                                      const uint32_t *pairs, size_t n_pairs,
                                      const pcr_icp_params *params, pcr_icp_result *results);
+/* The batch started from guesses: pair p from inits[12p .. 12p+12) (HOST, n_pairs x 12 floats, the layout of
+ * pcr_icp_point_to_point_init, free for reuse on return; NULL = every pair from the identity), with that call's rules.
+ * Every pair is the reference loop seeded with its guess, and an identity guess gives bit for bit what the plain batch
+ * gives.  A pair may be listed many times with different guesses (multi-start): each result is bit for bit that pair
+ * alone with that guess.  A NaN / Inf in a guess -> PCR_ERR_INVALID_ARG naming the pair, before any device work.  A
+ * failing call leaves *results untouched. */
+int pcr_icp_point_to_point_batch_init(pcr_ctx *ctx, const float *x, const float *y, const float *z,
+                                      const uint64_t *frame_offsets, size_t n_frames,
+                                      const uint32_t *pairs, size_t n_pairs, const float *inits,
+                                      const pcr_icp_params *params, pcr_icp_result *results);
+int pcr_icp_point_to_plane_batch_init(pcr_ctx *ctx, const float *x, const float *y, const float *z,
+                                      const uint64_t *frame_offsets, size_t n_frames,
+                                      const float *nx, const float *ny, const float *nz, size_t n_normals,
+                                      const uint32_t *pairs, size_t n_pairs, const float *inits,
+                                      const pcr_icp_params *params, pcr_icp_result *results);
+int pcr_icp_point_to_point_batch_init_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z,
+                                          const uint64_t *frame_offsets, size_t n_frames,
+                                          const uint32_t *pairs, size_t n_pairs, const float *inits,
+                                          const pcr_icp_params *params, pcr_icp_result *results);
+int pcr_icp_point_to_plane_batch_init_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z,
+                                          const uint64_t *frame_offsets, size_t n_frames,
+                                          const float *d_nx, const float *d_ny, const float *d_nz, size_t n_normals,
+                                          const uint32_t *pairs, size_t n_pairs, const float *inits,
+                                          const pcr_icp_params *params, pcr_icp_result *results);
 
 /* ---- voxel grid filter (SURVEY 8f-2) ---------------------------------------------------------------
  * voxel_downsample (crates/filters/src/voxel_downsample.rs:12-65): one point per occupied voxel
@@ -553,6 +605,11 @@ int pcr_cloud_icp_point_to_point(const pcr_cloud *source, const pcr_cloud *targe
 /* the target must carry normals (crates/python/src/registration.rs:80-86) */
 int pcr_cloud_icp_point_to_plane(const pcr_cloud *source, const pcr_cloud *target,
                                  const pcr_icp_params *params, pcr_icp_result *result);              /* icp_plane.rs:20 */
+/* the same from a guess (init as in pcr_icp_point_to_point_init) */
+int pcr_cloud_icp_point_to_point_init(const pcr_cloud *source, const pcr_cloud *target, const float init[12],
+                                      const pcr_icp_params *params, pcr_icp_result *result);
+int pcr_cloud_icp_point_to_plane_init(const pcr_cloud *source, const pcr_cloud *target, const float init[12],
+                                      const pcr_icp_params *params, pcr_icp_result *result);
 
 /* ---- device-resident frame batches ------------------------------------------------------------------
  * F clouds back to back in one device allocation, frame f = points [offsets[f], offsets[f+1]): the batch counterpart of
@@ -618,6 +675,11 @@ int pcr_frames_icp_point_to_point(const pcr_frames *frames, const uint32_t *pair
                                   pcr_icp_result *results);
 int pcr_frames_icp_point_to_plane(const pcr_frames *frames, const uint32_t *pairs, size_t n_pairs, const pcr_icp_params *params,
                                   pcr_icp_result *results);
+/* the same from guesses (inits as in pcr_icp_point_to_point_batch_init: HOST, n_pairs x 12, NULL = identity) */
+int pcr_frames_icp_point_to_point_init(const pcr_frames *frames, const uint32_t *pairs, size_t n_pairs, const float *inits,
+                                       const pcr_icp_params *params, pcr_icp_result *results);
+int pcr_frames_icp_point_to_plane_init(const pcr_frames *frames, const uint32_t *pairs, size_t n_pairs, const float *inits,
+                                       const pcr_icp_params *params, pcr_icp_result *results);
 
 #ifdef __cplusplus
 }

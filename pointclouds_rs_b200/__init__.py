@@ -550,30 +550,76 @@ def _icp_params(max_iterations, tolerance, max_correspondence_distance):
     return _ffi.IcpParams(int(max_iterations), float(tolerance), float(max_correspondence_distance))
 
 
+def _icp_init(init) -> np.ndarray:
+    """Checks and converts the starting pose of an ICP call -> (12,) f32: row-major rotation, then translation.  Takes an
+    (R, t) pair, a (3, 4) [R | t] array, 12 floats or an IcpResult (a coarse stage's result)."""
+    if isinstance(init, IcpResult):
+        init = (init.rotation, init.translation)
+    if isinstance(init, (tuple, list)) and len(init) == 2:
+        r, t = (np.asarray(v) for v in init)
+        if r.shape != (3, 3) or t.shape != (3,):
+            raise ValueError(f"init (R, t) must be a (3, 3) rotation and a (3,) translation; got {r.shape} and {t.shape}")
+        a = np.concatenate([r.reshape(9), t])
+    else:
+        a = np.asarray(init)
+        if a.shape == (3, 4):
+            a = np.concatenate([a[:, :3].reshape(9), a[:, 3]])
+        if a.shape != (12,):
+            raise ValueError(f"init must be (R, t), a (3, 4) [R | t] array, 12 floats or an IcpResult; got shape {a.shape}")
+    if a.dtype.kind not in "iuf" or not np.all(np.isfinite(a)):
+        raise ValueError("init must hold 12 finite numbers")
+    return np.ascontiguousarray(a, np.float32)
+
+
+def _icp_inits(inits, n_pairs: int) -> np.ndarray:
+    """Starting poses of a batched ICP, one per pair -> (P, 12) f32 (see _frame_transforms; also a list of IcpResults)."""
+    if not isinstance(inits, np.ndarray):
+        inits = [_transform12(r.rotation, r.translation) if isinstance(r, IcpResult) else r for r in inits]
+        inits = np.asarray(inits) if inits else np.zeros((0, 12), np.float32)
+    try:
+        a = _frame_transforms(inits, n_pairs)
+    except ValueError as e:
+        raise ValueError(f"init: one transform per pair; {e}") from None
+    bad = np.flatnonzero(~np.all(np.isfinite(a), axis=1))
+    if len(bad):
+        raise ValueError(f"init of pair {int(bad[0])} is not finite")
+    return a
+
+
 def icp_point_to_point(source: PointCloud, target: PointCloud, max_iterations: int = 50, tolerance: float = 1e-5,
-                       max_correspondence_distance: float = math.inf, ctx: Optional[Context] = None) -> IcpResult:
-    ctx = ctx or default_context()
+                       max_correspondence_distance: float = math.inf, ctx: Optional[Context] = None, init=None) -> IcpResult:
+    """init: the starting pose ((R, t), a (3, 4) array, 12 floats or an IcpResult; None = identity).  ICP from init is the
+    reference loop seeded with it: the source is moved by init first and the result's transform includes init."""
     p = _icp_params(max_iterations, tolerance, max_correspondence_distance)
+    g = None if init is None else _icp_init(init)
+    ctx = ctx or default_context()
     res = _ffi.IcpResultC()
-    st = _ffi.load().pcr_icp_point_to_point(ctx._h, _p(source.x, _ffi.f32p), _p(source.y, _ffi.f32p), _p(source.z, _ffi.f32p),
-                                            len(source), _p(target.x, _ffi.f32p), _p(target.y, _ffi.f32p), _p(target.z, _ffi.f32p),
-                                            len(target), C.byref(p), C.byref(res))
+    args = (ctx._h, _p(source.x, _ffi.f32p), _p(source.y, _ffi.f32p), _p(source.z, _ffi.f32p), len(source), _p(target.x, _ffi.f32p),
+            _p(target.y, _ffi.f32p), _p(target.z, _ffi.f32p), len(target))
+    if g is None:
+        st = _ffi.load().pcr_icp_point_to_point(*args, C.byref(p), C.byref(res))
+    else:
+        st = _ffi.load().pcr_icp_point_to_point_init(*args, _p(g, _ffi.f32p), C.byref(p), C.byref(res))
     _ffi.check(st, ctx._h)
     return IcpResult(res)
 
 
 def icp_point_to_plane(source: PointCloud, target: PointCloud, max_iterations: int = 50, tolerance: float = 1e-5,
-                       max_correspondence_distance: float = math.inf, ctx: Optional[Context] = None) -> IcpResult:
+                       max_correspondence_distance: float = math.inf, ctx: Optional[Context] = None, init=None) -> IcpResult:
+    """init: as for icp_point_to_point."""
+    g = None if init is None else _icp_init(init)
     ctx = ctx or default_context()
     if target.normals is None:  # crates/python/src/registration.rs:66-71
         raise ValueError("target cloud must have normals for point-to-plane ICP. Use estimate_normals(target, k) first.")
     p = _icp_params(max_iterations, tolerance, max_correspondence_distance)
     nx, ny, nz = target._normals_soa()
     res = _ffi.IcpResultC()
-    st = _ffi.load().pcr_icp_point_to_plane(ctx._h, _p(source.x, _ffi.f32p), _p(source.y, _ffi.f32p), _p(source.z, _ffi.f32p),
-                                            len(source), _p(target.x, _ffi.f32p), _p(target.y, _ffi.f32p), _p(target.z, _ffi.f32p),
-                                            len(target), _p(nx, _ffi.f32p), _p(ny, _ffi.f32p), _p(nz, _ffi.f32p), len(nx),
-                                            C.byref(p), C.byref(res))
+    args = (ctx._h, _p(source.x, _ffi.f32p), _p(source.y, _ffi.f32p), _p(source.z, _ffi.f32p), len(source), _p(target.x, _ffi.f32p),
+            _p(target.y, _ffi.f32p), _p(target.z, _ffi.f32p), len(target), _p(nx, _ffi.f32p), _p(ny, _ffi.f32p), _p(nz, _ffi.f32p), len(nx))
+    if g is None:
+        st = _ffi.load().pcr_icp_point_to_plane(*args, C.byref(p), C.byref(res))
+    else:
+        st = _ffi.load().pcr_icp_point_to_plane_init(*args, _p(g, _ffi.f32p), C.byref(p), C.byref(res))
     _ffi.check(st, ctx._h)
     return IcpResult(res)
 
@@ -685,24 +731,30 @@ def _icp_batch_arrays(points, frame_offsets, pairs):
 
 def icp_point_to_point_batch(points: np.ndarray, frame_offsets: Sequence[int], pairs, max_iterations: int = 50,
                              tolerance: float = 1e-5, max_correspondence_distance: float = math.inf,
-                             ctx: Optional[Context] = None) -> List[IcpResult]:
+                             ctx: Optional[Context] = None, init=None) -> List[IcpResult]:
     """Point-to-point ICP of many frame pairs in one call.  points: (N,3), every frame back to back, frame f = rows
     [frame_offsets[f], frame_offsets[f+1]); pairs: (P,2), pair p registers frame pairs[p][0] (source) onto frame
-    pairs[p][1] (target).  -> one IcpResult per pair, each what icp_point_to_point returns for those two clouds."""
+    pairs[p][1] (target).  -> one IcpResult per pair, each what icp_point_to_point returns for those two clouds.
+    init: one starting pose per pair ((P, 12) rows, (P, 3, 4) [R | t] or a list of P IcpResults; None = identity), each
+    as icp_point_to_point's init.  A pair listed several times with different poses is a multi-start."""
     p = _icp_params(max_iterations, tolerance, max_correspondence_distance)
     pts, off, pr = _icp_batch_arrays(points, frame_offsets, pairs)
+    g = None if init is None else _icp_inits(init, len(pr))
     ctx = ctx or default_context()
     x, y, z = _soa(pts)
     res = (_ffi.IcpResultC * max(len(pr), 1))()
-    st = _ffi.load().pcr_icp_point_to_point_batch(ctx._h, _p(x, _ffi.f32p), _p(y, _ffi.f32p), _p(z, _ffi.f32p), _p(off, _ffi.u64p),
-                                                  len(off) - 1, _p(pr, _ffi.u32p), len(pr), C.byref(p), res)
+    args = (ctx._h, _p(x, _ffi.f32p), _p(y, _ffi.f32p), _p(z, _ffi.f32p), _p(off, _ffi.u64p), len(off) - 1, _p(pr, _ffi.u32p), len(pr))
+    if g is None:
+        st = _ffi.load().pcr_icp_point_to_point_batch(*args, C.byref(p), res)
+    else:
+        st = _ffi.load().pcr_icp_point_to_point_batch_init(*args, _p(g, _ffi.f32p), C.byref(p), res)
     _ffi.check(st, ctx._h)
     return [IcpResult(res[i]) for i in range(len(pr))]
 
 
 def icp_point_to_plane_batch(points: np.ndarray, frame_offsets: Sequence[int], pairs, normals: Optional[np.ndarray],
                              max_iterations: int = 50, tolerance: float = 1e-5, max_correspondence_distance: float = math.inf,
-                             ctx: Optional[Context] = None) -> List[IcpResult]:
+                             ctx: Optional[Context] = None, init=None) -> List[IcpResult]:
     """Point-to-plane form of icp_point_to_point_batch.  normals: (N,3), one per row of `points` (only the rows of
     target frames are read)."""
     if normals is None:  # crates/python/src/registration.rs:66-71
@@ -712,13 +764,17 @@ def icp_point_to_plane_batch(points: np.ndarray, frame_offsets: Sequence[int], p
     nrm = np.asarray(normals)
     if nrm.ndim != 2 or nrm.shape[1] != 3 or len(nrm) != len(pts):
         raise ValueError(f"normals must have shape ({len(pts)}, 3), one per point; got {nrm.shape}")
+    g = None if init is None else _icp_inits(init, len(pr))
     ctx = ctx or default_context()
     x, y, z = _soa(pts)
     nx, ny, nz = _soa(np.ascontiguousarray(nrm, np.float32))
     res = (_ffi.IcpResultC * max(len(pr), 1))()
-    st = _ffi.load().pcr_icp_point_to_plane_batch(ctx._h, _p(x, _ffi.f32p), _p(y, _ffi.f32p), _p(z, _ffi.f32p), _p(off, _ffi.u64p),
-                                                  len(off) - 1, _p(nx, _ffi.f32p), _p(ny, _ffi.f32p), _p(nz, _ffi.f32p), len(nx),
-                                                  _p(pr, _ffi.u32p), len(pr), C.byref(p), res)
+    args = (ctx._h, _p(x, _ffi.f32p), _p(y, _ffi.f32p), _p(z, _ffi.f32p), _p(off, _ffi.u64p), len(off) - 1, _p(nx, _ffi.f32p),
+            _p(ny, _ffi.f32p), _p(nz, _ffi.f32p), len(nx), _p(pr, _ffi.u32p), len(pr))
+    if g is None:
+        st = _ffi.load().pcr_icp_point_to_plane_batch(*args, C.byref(p), res)
+    else:
+        st = _ffi.load().pcr_icp_point_to_plane_batch_init(*args, _p(g, _ffi.f32p), C.byref(p), res)
     _ffi.check(st, ctx._h)
     return [IcpResult(res[i]) for i in range(len(pr))]
 
@@ -896,19 +952,29 @@ class DeviceCloud:
         t = np.ascontiguousarray(np.asarray(translation, np.float32).reshape(3))
         return self._new(_ffi.load().pcr_cloud_apply_transform, _p(r, _ffi.f32p), _p(t, _ffi.f32p))
 
-    def icp_point_to_point(self, target: "DeviceCloud", max_iterations: int = 50, tolerance: float = 1e-5,
-                           max_correspondence_distance: float = math.inf) -> "IcpResult":
+    def _icp(self, plain, seeded, target, max_iterations, tolerance, max_correspondence_distance, init) -> "IcpResult":
         prm = _icp_params(max_iterations, tolerance, max_correspondence_distance)
         res = _ffi.IcpResultC()
-        _ffi.check(_ffi.load().pcr_cloud_icp_point_to_point(self._h, target._h, C.byref(prm), C.byref(res)), self._ctx._h)
+        if init is None:
+            st = plain(self._h, target._h, C.byref(prm), C.byref(res))
+        else:
+            g = _icp_init(init)
+            st = seeded(self._h, target._h, _p(g, _ffi.f32p), C.byref(prm), C.byref(res))
+        _ffi.check(st, self._ctx._h)
         return IcpResult(res)
 
+    def icp_point_to_point(self, target: "DeviceCloud", max_iterations: int = 50, tolerance: float = 1e-5,
+                           max_correspondence_distance: float = math.inf, init=None) -> "IcpResult":
+        """init: the starting pose, as for the module's icp_point_to_point."""
+        lib = _ffi.load()
+        return self._icp(lib.pcr_cloud_icp_point_to_point, lib.pcr_cloud_icp_point_to_point_init, target, max_iterations, tolerance,
+                         max_correspondence_distance, init)
+
     def icp_point_to_plane(self, target: "DeviceCloud", max_iterations: int = 50, tolerance: float = 1e-5,
-                           max_correspondence_distance: float = math.inf) -> "IcpResult":
-        prm = _icp_params(max_iterations, tolerance, max_correspondence_distance)
-        res = _ffi.IcpResultC()
-        _ffi.check(_ffi.load().pcr_cloud_icp_point_to_plane(self._h, target._h, C.byref(prm), C.byref(res)), self._ctx._h)
-        return IcpResult(res)
+                           max_correspondence_distance: float = math.inf, init=None) -> "IcpResult":
+        lib = _ffi.load()
+        return self._icp(lib.pcr_cloud_icp_point_to_plane, lib.pcr_cloud_icp_point_to_plane_init, target, max_iterations, tolerance,
+                         max_correspondence_distance, init)
 
 # ---------------------------------------------------------------------------------------------------
 # multi-frame batch (BASELINE config 5)
@@ -1280,7 +1346,7 @@ class DeviceFrames:
         c_off, offsets, idx = self.cluster_arrays(distance_threshold, min_size, max_size)
         return [[idx[offsets[c]:offsets[c + 1]].tolist() for c in range(int(c_off[f]), int(c_off[f + 1]))] for f in range(len(c_off) - 1)]
 
-    def _icp(self, fn, pairs, max_iterations, tolerance, max_correspondence_distance) -> List[IcpResult]:
+    def _icp(self, fn, seeded, pairs, max_iterations, tolerance, max_correspondence_distance, init) -> List[IcpResult]:
         prm = _icp_params(max_iterations, tolerance, max_correspondence_distance)
         nf = self.n_frames
         pr = np.asarray(pairs)
@@ -1291,21 +1357,31 @@ class DeviceFrames:
         if len(pr) and (pr.min() < 0 or pr.max() >= nf):
             raise ValueError(f"pairs hold a frame id outside [0, {nf})")
         pr = np.ascontiguousarray(pr, np.uint32)
+        g = None if init is None else _icp_inits(init, len(pr))
         res = (_ffi.IcpResultC * max(len(pr), 1))()
-        _ffi.check(fn(self._h, _p(pr, _ffi.u32p), len(pr), C.byref(prm), res), self._ctx._h)
+        if g is None:
+            st = fn(self._h, _p(pr, _ffi.u32p), len(pr), C.byref(prm), res)
+        else:
+            st = seeded(self._h, _p(pr, _ffi.u32p), len(pr), _p(g, _ffi.f32p), C.byref(prm), res)
+        _ffi.check(st, self._ctx._h)
         return [IcpResult(res[i]) for i in range(len(pr))]
 
     def icp_point_to_point(self, pairs, max_iterations: int = 50, tolerance: float = 1e-5,
-                           max_correspondence_distance: float = math.inf) -> List[IcpResult]:
-        """pairs: (P, 2) frame ids, pair p registers frame pairs[p][0] onto frame pairs[p][1] -> one IcpResult per pair."""
-        return self._icp(_ffi.load().pcr_frames_icp_point_to_point, pairs, max_iterations, tolerance, max_correspondence_distance)
+                           max_correspondence_distance: float = math.inf, init=None) -> List[IcpResult]:
+        """pairs: (P, 2) frame ids, pair p registers frame pairs[p][0] onto frame pairs[p][1] -> one IcpResult per pair.
+        init: one starting pose per pair, as for icp_point_to_point_batch."""
+        lib = _ffi.load()
+        return self._icp(lib.pcr_frames_icp_point_to_point, lib.pcr_frames_icp_point_to_point_init, pairs, max_iterations, tolerance,
+                         max_correspondence_distance, init)
 
     def icp_point_to_plane(self, pairs, max_iterations: int = 50, tolerance: float = 1e-5,
-                           max_correspondence_distance: float = math.inf) -> List[IcpResult]:
+                           max_correspondence_distance: float = math.inf, init=None) -> List[IcpResult]:
         """Point-to-plane form; the batch must carry normals (estimate_normals / sor_normals)."""
         if not self.has_normals():  # crates/python/src/registration.rs:66-71
             raise ValueError("point-to-plane ICP needs frames with normals. Use estimate_normals first.")
-        return self._icp(_ffi.load().pcr_frames_icp_point_to_plane, pairs, max_iterations, tolerance, max_correspondence_distance)
+        lib = _ffi.load()
+        return self._icp(lib.pcr_frames_icp_point_to_plane, lib.pcr_frames_icp_point_to_plane_init, pairs, max_iterations, tolerance,
+                         max_correspondence_distance, init)
 
 
 def _query_frames(queries, query_offsets, n_frames: int):

@@ -113,6 +113,20 @@ SIGNATURES = {
     "pcr_icp_point_to_point_batch_dev": (C.c_int, [vp, vp, vp, vp, u64p, C.c_size_t, u32p, C.c_size_t, C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
     "pcr_icp_point_to_plane_batch_dev": (C.c_int, [vp, vp, vp, vp, u64p, C.c_size_t, vp, vp, vp, C.c_size_t, u32p, C.c_size_t,
                                                    C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
+    "pcr_icp_point_to_point_init": (C.c_int, [vp, f32p, f32p, f32p, C.c_size_t, f32p, f32p, f32p, C.c_size_t, f32p, C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
+    "pcr_icp_point_to_plane_init": (C.c_int, [vp, f32p, f32p, f32p, C.c_size_t, f32p, f32p, f32p, C.c_size_t, f32p, f32p, f32p, C.c_size_t, f32p,
+                                              C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
+    "pcr_icp_point_to_point_init_dev": (C.c_int, [vp, vp, vp, vp, C.c_size_t, vp, vp, vp, C.c_size_t, f32p, C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
+    "pcr_icp_point_to_plane_init_dev": (C.c_int, [vp, vp, vp, vp, C.c_size_t, vp, vp, vp, C.c_size_t, vp, vp, vp, C.c_size_t, f32p,
+                                                  C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
+    "pcr_icp_point_to_point_batch_init": (C.c_int, [vp, f32p, f32p, f32p, u64p, C.c_size_t, u32p, C.c_size_t, f32p, C.POINTER(IcpParams),
+                                                    C.POINTER(IcpResultC)]),
+    "pcr_icp_point_to_plane_batch_init": (C.c_int, [vp, f32p, f32p, f32p, u64p, C.c_size_t, f32p, f32p, f32p, C.c_size_t, u32p, C.c_size_t, f32p,
+                                                    C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
+    "pcr_icp_point_to_point_batch_init_dev": (C.c_int, [vp, vp, vp, vp, u64p, C.c_size_t, u32p, C.c_size_t, f32p, C.POINTER(IcpParams),
+                                                        C.POINTER(IcpResultC)]),
+    "pcr_icp_point_to_plane_batch_init_dev": (C.c_int, [vp, vp, vp, vp, u64p, C.c_size_t, vp, vp, vp, C.c_size_t, u32p, C.c_size_t, f32p,
+                                                        C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
     "pcr_voxel_downsample": (C.c_int, [vp, f32p, f32p, f32p, C.c_size_t, C.c_float, f32p, f32p, f32p, szp]),
     "pcr_voxel_downsample_dev": (C.c_int, [vp, vp, vp, vp, C.c_size_t, C.c_float, vp, vp, vp, szp]),
     "pcr_voxel_downsample_batch": (C.c_int, [vp, f32p, f32p, f32p, u64p, C.c_size_t, C.c_float, f32p, f32p, f32p, u64p]),
@@ -144,6 +158,8 @@ SIGNATURES = {
     "pcr_cloud_apply_transform": (C.c_int, [vp, f32p, f32p, C.POINTER(vp)]),
     "pcr_cloud_icp_point_to_point": (C.c_int, [vp, vp, C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
     "pcr_cloud_icp_point_to_plane": (C.c_int, [vp, vp, C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
+    "pcr_cloud_icp_point_to_point_init": (C.c_int, [vp, vp, f32p, C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
+    "pcr_cloud_icp_point_to_plane_init": (C.c_int, [vp, vp, f32p, C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
     "pcr_ransac_plane_samples": (C.c_int, [vp, f32p, f32p, f32p, C.c_size_t, C.c_float, u32p, C.c_size_t, f32p, u32p, szp]),
     "pcr_cloud_ransac_plane_samples": (C.c_int, [vp, C.c_float, u32p, C.c_size_t, f32p, u32p, szp]),
     "pcr_ransac_plane_samples_batch": (C.c_int, [vp, f32p, f32p, f32p, u64p, C.c_size_t, C.c_float, u32p, u64p, f32p, u32p, u64p]),
@@ -182,6 +198,8 @@ SIGNATURES = {
     "pcr_frames_euclidean_cluster": (C.c_int, [vp, C.c_float, C.c_size_t, C.c_size_t, u32p, u32p, u64p]),
     "pcr_frames_icp_point_to_point": (C.c_int, [vp, u32p, C.c_size_t, C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
     "pcr_frames_icp_point_to_plane": (C.c_int, [vp, u32p, C.c_size_t, C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
+    "pcr_frames_icp_point_to_point_init": (C.c_int, [vp, u32p, C.c_size_t, f32p, C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
+    "pcr_frames_icp_point_to_plane_init": (C.c_int, [vp, u32p, C.c_size_t, f32p, C.POINTER(IcpParams), C.POINTER(IcpResultC)]),
 }
 
 _lib = None

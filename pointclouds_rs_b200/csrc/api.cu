@@ -965,14 +965,31 @@ static void icp_identity(pcr_icp_result *r) {
     r->rotation[0] = r->rotation[4] = r->rotation[8] = 1.f;
 }
 
+// the result before the loop runs: the transform is the guess (12 floats, row-major R then t)
+static void icp_seed(pcr_icp_result *r, const float *init) {
+    icp_identity(r);
+    memcpy(r->rotation, init, sizeof(float) * 9);
+    memcpy(r->translation, init + 9, sizeof(float) * 3);
+}
+
+// guesses of the _init calls: 12 finite floats per pair (orthonormality is not checked, as in pcr_apply_transform)
+static int inits_check(Ctx *c, const char *name, const float *inits, size_t n_pairs) {
+    if (!inits) return fail(c, PCR_ERR_INVALID_ARG, "%s is NULL", name);
+    for (size_t p = 0; p < n_pairs; p++)
+        for (int j = 0; j < 12; j++)
+            if (!std::isfinite(inits[12 * p + j])) return fail(c, PCR_ERR_INVALID_ARG, "%s: pair %zu has a non-finite value", name, p);
+    return PCR_OK;
+}
+
 static int icp_common_dev(Ctx *c, const float *dsx, const float *dsy, const float *dsz, size_t ns, const float *dtx, const float *dty,
-                          const float *dtz, size_t nt, const float *dnx, const float *dny, const float *dnz,
+                          const float *dtz, size_t nt, const float *dnx, const float *dny, const float *dnz, const float *init,
                           const pcr_icp_params *params, pcr_icp_result *result) {
     IcpArgs a;
     a.d_sx = dsx; a.d_sy = dsy; a.d_sz = dsz; a.ns = ns;
     a.d_tx = dtx; a.d_ty = dty; a.d_tz = dtz; a.nt = nt;
     a.d_nx = dnx; a.d_ny = dny; a.d_nz = dnz;
     a.params = *params;
+    a.init = init;
     return icp_dev(c, a, result);
 }
 
@@ -985,52 +1002,75 @@ static int icp_check(Ctx *c, const pcr_icp_params *params, pcr_icp_result *resul
     return PCR_OK;
 }
 
+// seeded: the _init calls (init: 12 floats).  They check every argument before they write *result; the plain calls
+// preset the identity first, as they always have.
 static int icp_entry(pcr_ctx *ctx, bool dev, bool plane, const float *sx, const float *sy, const float *sz, size_t ns, const float *tx,
                      const float *ty, const float *tz, size_t nt, const float *nx, const float *ny, const float *nz, size_t nn,
-                     const pcr_icp_params *params, pcr_icp_result *result) {
+                     bool seeded, const float *init, const pcr_icp_params *params, pcr_icp_result *result) {
     if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
     Ctx *c = &ctx->c;
     PCR_TRY(icp_check(c, params, result));
-    icp_identity(result);
+    if (seeded) PCR_TRY(inits_check(c, "init", init, 1));
+    else icp_identity(result);
     if (plane && nn != nt)  // icp_plane.rs:27-32
         return fail(c, PCR_ERR_NORMALS_MISMATCH, "target_normals length (%zu) does not match target cloud length (%zu)", nn, nt);
-    if (c->world == 1 && (ns == 0 || nt == 0)) {  // icp.rs:131-139
-        result->converged = (ns == 0 && nt == 0) ? 1 : 0;
+    // icp.rs:131-139 (with a communicator a rank may hold no source points and still takes part)
+    const bool empty = nt == 0 || (c->world == 1 && ns == 0);
+    if (!empty && ((ns && (!sx || !sy || !sz)) || !tx || !ty || !tz || (plane && (!nx || !ny || !nz))))
+        return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    if (seeded) icp_seed(result, init);
+    if (empty) {
+        result->converged = (c->world == 1 && ns == 0 && nt == 0) ? 1 : 0;
         return PCR_OK;
     }
-    if (nt == 0) {
-        result->converged = 0;
-        return PCR_OK;
-    }
-    if ((ns && (!sx || !sy || !sz)) || !tx || !ty || !tz || (plane && (!nx || !ny || !nz))) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
     PCR_API_BEGIN
     DevSetter ds(c);
-    if (dev) return icp_common_dev(c, sx, sy, sz, ns, tx, ty, tz, nt, plane ? nx : nullptr, ny, nz, params, result);
+    if (dev) return icp_common_dev(c, sx, sy, sz, ns, tx, ty, tz, nt, plane ? nx : nullptr, ny, nz, init, params, result);
     float *dsx, *dsy, *dsz, *dtx, *dty, *dtz, *dnx = nullptr, *dny = nullptr, *dnz = nullptr;
     PCR_TRY(stage_xyz(c, c->b_in2, sx, sy, sz, ns, &dsx, &dsy, &dsz));
     PCR_TRY(stage_xyz(c, c->b_in, tx, ty, tz, nt, &dtx, &dty, &dtz));
     if (plane) PCR_TRY(stage_xyz(c, c->b_out, nx, ny, nz, nt, &dnx, &dny, &dnz));
-    return icp_common_dev(c, dsx, dsy, dsz, ns, dtx, dty, dtz, nt, dnx, dny, dnz, params, result);
+    return icp_common_dev(c, dsx, dsy, dsz, ns, dtx, dty, dtz, nt, dnx, dny, dnz, init, params, result);
     PCR_API_END(c)
 }
 
 int pcr_icp_point_to_point(pcr_ctx *ctx, const float *sx, const float *sy, const float *sz, size_t ns, const float *tx,
                            const float *ty, const float *tz, size_t nt, const pcr_icp_params *params, pcr_icp_result *result) {
-    return icp_entry(ctx, false, false, sx, sy, sz, ns, tx, ty, tz, nt, nullptr, nullptr, nullptr, nt, params, result);
+    return icp_entry(ctx, false, false, sx, sy, sz, ns, tx, ty, tz, nt, nullptr, nullptr, nullptr, nt, false, nullptr, params, result);
 }
 int pcr_icp_point_to_plane(pcr_ctx *ctx, const float *sx, const float *sy, const float *sz, size_t ns, const float *tx,
                            const float *ty, const float *tz, size_t nt, const float *nx, const float *ny, const float *nz,
                            size_t n_normals, const pcr_icp_params *params, pcr_icp_result *result) {
-    return icp_entry(ctx, false, true, sx, sy, sz, ns, tx, ty, tz, nt, nx, ny, nz, n_normals, params, result);
+    return icp_entry(ctx, false, true, sx, sy, sz, ns, tx, ty, tz, nt, nx, ny, nz, n_normals, false, nullptr, params, result);
 }
 int pcr_icp_point_to_point_dev(pcr_ctx *ctx, const float *sx, const float *sy, const float *sz, size_t ns, const float *tx,
                                const float *ty, const float *tz, size_t nt, const pcr_icp_params *params, pcr_icp_result *result) {
-    return icp_entry(ctx, true, false, sx, sy, sz, ns, tx, ty, tz, nt, nullptr, nullptr, nullptr, nt, params, result);
+    return icp_entry(ctx, true, false, sx, sy, sz, ns, tx, ty, tz, nt, nullptr, nullptr, nullptr, nt, false, nullptr, params, result);
 }
 int pcr_icp_point_to_plane_dev(pcr_ctx *ctx, const float *sx, const float *sy, const float *sz, size_t ns, const float *tx,
                                const float *ty, const float *tz, size_t nt, const float *nx, const float *ny, const float *nz,
                                size_t n_normals, const pcr_icp_params *params, pcr_icp_result *result) {
-    return icp_entry(ctx, true, true, sx, sy, sz, ns, tx, ty, tz, nt, nx, ny, nz, n_normals, params, result);
+    return icp_entry(ctx, true, true, sx, sy, sz, ns, tx, ty, tz, nt, nx, ny, nz, n_normals, false, nullptr, params, result);
+}
+int pcr_icp_point_to_point_init(pcr_ctx *ctx, const float *sx, const float *sy, const float *sz, size_t ns, const float *tx,
+                                const float *ty, const float *tz, size_t nt, const float init[12], const pcr_icp_params *params,
+                                pcr_icp_result *result) {
+    return icp_entry(ctx, false, false, sx, sy, sz, ns, tx, ty, tz, nt, nullptr, nullptr, nullptr, nt, true, init, params, result);
+}
+int pcr_icp_point_to_plane_init(pcr_ctx *ctx, const float *sx, const float *sy, const float *sz, size_t ns, const float *tx,
+                                const float *ty, const float *tz, size_t nt, const float *nx, const float *ny, const float *nz,
+                                size_t n_normals, const float init[12], const pcr_icp_params *params, pcr_icp_result *result) {
+    return icp_entry(ctx, false, true, sx, sy, sz, ns, tx, ty, tz, nt, nx, ny, nz, n_normals, true, init, params, result);
+}
+int pcr_icp_point_to_point_init_dev(pcr_ctx *ctx, const float *sx, const float *sy, const float *sz, size_t ns, const float *tx,
+                                    const float *ty, const float *tz, size_t nt, const float init[12], const pcr_icp_params *params,
+                                    pcr_icp_result *result) {
+    return icp_entry(ctx, true, false, sx, sy, sz, ns, tx, ty, tz, nt, nullptr, nullptr, nullptr, nt, true, init, params, result);
+}
+int pcr_icp_point_to_plane_init_dev(pcr_ctx *ctx, const float *sx, const float *sy, const float *sz, size_t ns, const float *tx,
+                                    const float *ty, const float *tz, size_t nt, const float *nx, const float *ny, const float *nz,
+                                    size_t n_normals, const float init[12], const pcr_icp_params *params, pcr_icp_result *result) {
+    return icp_entry(ctx, true, true, sx, sy, sz, ns, tx, ty, tz, nt, nx, ny, nz, n_normals, true, init, params, result);
 }
 
 // Offsets of a batch argument (frame, query, sample or index offsets; `name` names it in the message): frame f = entries
@@ -1050,13 +1090,15 @@ static int batch_size_check(Ctx *c, size_t n, size_t n_frames) {
 }
 
 // Pairs of frames of one buffer: every pair is checked and answered as the single-pair call would (icp_entry).
+// seeded: the _init calls (inits: 12 floats per pair, NULL = identity), which write *results after every check.
 static int icp_batch_entry(pcr_ctx *ctx, bool dev, bool plane, const float *x, const float *y, const float *z, const uint64_t *frame_offsets,
                            size_t n_frames, const float *nx, const float *ny, const float *nz, size_t n_normals, const uint32_t *pairs,
-                           size_t n_pairs, const pcr_icp_params *params, pcr_icp_result *results) {
+                           size_t n_pairs, bool seeded, const float *inits, const pcr_icp_params *params, pcr_icp_result *results) {
     if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
     Ctx *c = &ctx->c;
     PCR_TRY(icp_check(c, params, results));
-    for (size_t p = 0; p < n_pairs; p++) icp_identity(&results[p]);
+    if (!seeded)
+        for (size_t p = 0; p < n_pairs; p++) icp_identity(&results[p]);
     if (n_pairs && !pairs) return fail(c, PCR_ERR_INVALID_ARG, "pairs is NULL");
     PCR_TRY(offsets_check(c, "frame_offsets", frame_offsets, n_frames));
     const size_t n = (size_t)frame_offsets[n_frames];
@@ -1071,6 +1113,12 @@ static int icp_batch_entry(pcr_ctx *ctx, bool dev, bool plane, const float *x, c
     if (src_points >= (1ull << 31)) return fail(c, PCR_ERR_UNSUPPORTED, "the source frames of one batch must hold fewer than 2^31 points");
     PCR_TRY(batch_size_check(c, n, n_frames));
     if (n && (!x || !y || !z || (plane && (!nx || !ny || !nz)))) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    if (inits) PCR_TRY(inits_check(c, "inits", inits, n_pairs));
+    if (seeded)
+        for (size_t p = 0; p < n_pairs; p++) {
+            if (inits) icp_seed(&results[p], inits + 12 * p);
+            else icp_identity(&results[p]);
+        }
     PCR_API_BEGIN
     DevSetter ds(c);
     IcpBatchArgs a;
@@ -1079,6 +1127,7 @@ static int icp_batch_entry(pcr_ctx *ctx, bool dev, bool plane, const float *x, c
     a.d_nx = a.d_ny = a.d_nz = nullptr;
     a.pairs = pairs; a.n_pairs = n_pairs;
     a.params = *params;
+    a.inits = inits;
     if (dev) {
         if (plane) { a.d_nx = nx; a.d_ny = ny; a.d_nz = nz; }
         return icp_batch_dev(c, a, results);
@@ -1094,22 +1143,46 @@ static int icp_batch_entry(pcr_ctx *ctx, bool dev, bool plane, const float *x, c
 
 int pcr_icp_point_to_point_batch(pcr_ctx *ctx, const float *x, const float *y, const float *z, const uint64_t *frame_offsets, size_t n_frames,
                                  const uint32_t *pairs, size_t n_pairs, const pcr_icp_params *params, pcr_icp_result *results) {
-    return icp_batch_entry(ctx, false, false, x, y, z, frame_offsets, n_frames, nullptr, nullptr, nullptr, 0, pairs, n_pairs, params, results);
+    return icp_batch_entry(ctx, false, false, x, y, z, frame_offsets, n_frames, nullptr, nullptr, nullptr, 0, pairs, n_pairs, false, nullptr, params, results);
 }
 int pcr_icp_point_to_plane_batch(pcr_ctx *ctx, const float *x, const float *y, const float *z, const uint64_t *frame_offsets, size_t n_frames,
                                  const float *nx, const float *ny, const float *nz, size_t n_normals, const uint32_t *pairs, size_t n_pairs,
                                  const pcr_icp_params *params, pcr_icp_result *results) {
-    return icp_batch_entry(ctx, false, true, x, y, z, frame_offsets, n_frames, nx, ny, nz, n_normals, pairs, n_pairs, params, results);
+    return icp_batch_entry(ctx, false, true, x, y, z, frame_offsets, n_frames, nx, ny, nz, n_normals, pairs, n_pairs, false, nullptr, params, results);
 }
 int pcr_icp_point_to_point_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z, const uint64_t *frame_offsets,
                                      size_t n_frames, const uint32_t *pairs, size_t n_pairs, const pcr_icp_params *params,
                                      pcr_icp_result *results) {
-    return icp_batch_entry(ctx, true, false, d_x, d_y, d_z, frame_offsets, n_frames, nullptr, nullptr, nullptr, 0, pairs, n_pairs, params, results);
+    return icp_batch_entry(ctx, true, false, d_x, d_y, d_z, frame_offsets, n_frames, nullptr, nullptr, nullptr, 0, pairs, n_pairs, false, nullptr, params, results);
 }
 int pcr_icp_point_to_plane_batch_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z, const uint64_t *frame_offsets,
                                      size_t n_frames, const float *d_nx, const float *d_ny, const float *d_nz, size_t n_normals,
                                      const uint32_t *pairs, size_t n_pairs, const pcr_icp_params *params, pcr_icp_result *results) {
-    return icp_batch_entry(ctx, true, true, d_x, d_y, d_z, frame_offsets, n_frames, d_nx, d_ny, d_nz, n_normals, pairs, n_pairs, params,
+    return icp_batch_entry(ctx, true, true, d_x, d_y, d_z, frame_offsets, n_frames, d_nx, d_ny, d_nz, n_normals, pairs, n_pairs, false, nullptr, params,
+                           results);
+}
+int pcr_icp_point_to_point_batch_init(pcr_ctx *ctx, const float *x, const float *y, const float *z, const uint64_t *frame_offsets,
+                                      size_t n_frames, const uint32_t *pairs, size_t n_pairs, const float *inits, const pcr_icp_params *params,
+                                      pcr_icp_result *results) {
+    return icp_batch_entry(ctx, false, false, x, y, z, frame_offsets, n_frames, nullptr, nullptr, nullptr, 0, pairs, n_pairs, true, inits, params,
+                           results);
+}
+int pcr_icp_point_to_plane_batch_init(pcr_ctx *ctx, const float *x, const float *y, const float *z, const uint64_t *frame_offsets,
+                                      size_t n_frames, const float *nx, const float *ny, const float *nz, size_t n_normals, const uint32_t *pairs,
+                                      size_t n_pairs, const float *inits, const pcr_icp_params *params, pcr_icp_result *results) {
+    return icp_batch_entry(ctx, false, true, x, y, z, frame_offsets, n_frames, nx, ny, nz, n_normals, pairs, n_pairs, true, inits, params, results);
+}
+int pcr_icp_point_to_point_batch_init_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z, const uint64_t *frame_offsets,
+                                          size_t n_frames, const uint32_t *pairs, size_t n_pairs, const float *inits,
+                                          const pcr_icp_params *params, pcr_icp_result *results) {
+    return icp_batch_entry(ctx, true, false, d_x, d_y, d_z, frame_offsets, n_frames, nullptr, nullptr, nullptr, 0, pairs, n_pairs, true, inits, params,
+                           results);
+}
+int pcr_icp_point_to_plane_batch_init_dev(pcr_ctx *ctx, const float *d_x, const float *d_y, const float *d_z, const uint64_t *frame_offsets,
+                                          size_t n_frames, const float *d_nx, const float *d_ny, const float *d_nz, size_t n_normals,
+                                          const uint32_t *pairs, size_t n_pairs, const float *inits, const pcr_icp_params *params,
+                                          pcr_icp_result *results) {
+    return icp_batch_entry(ctx, true, true, d_x, d_y, d_z, frame_offsets, n_frames, d_nx, d_ny, d_nz, n_normals, pairs, n_pairs, true, inits, params,
                            results);
 }
 
@@ -2499,6 +2572,27 @@ int pcr_cloud_icp_point_to_plane(const pcr_cloud *source, const pcr_cloud *targe
                                       target->n, target->nx(), target->ny(), target->nz(), target->n, params, result);
 }
 
+int pcr_cloud_icp_point_to_point_init(const pcr_cloud *source, const pcr_cloud *target, const float init[12], const pcr_icp_params *params,
+                                      pcr_icp_result *result) {
+    PCR_TRY(handle_check(source, "cloud"));
+    Ctx *c = &source->owner->c;
+    if (!target || target->owner != source->owner) return fail(c, PCR_ERR_INVALID_ARG, "source and target must live on the same context");
+    return pcr_icp_point_to_point_init_dev(source->owner, source->x(), source->y(), source->z(), source->n, target->x(), target->y(),
+                                           target->z(), target->n, init, params, result);
+}
+
+int pcr_cloud_icp_point_to_plane_init(const pcr_cloud *source, const pcr_cloud *target, const float init[12], const pcr_icp_params *params,
+                                      pcr_icp_result *result) {
+    PCR_TRY(handle_check(source, "cloud"));
+    Ctx *c = &source->owner->c;
+    if (!target || target->owner != source->owner) return fail(c, PCR_ERR_INVALID_ARG, "source and target must live on the same context");
+    if (!target->has_normals)  // crates/python/src/registration.rs:80-86
+        return fail(c, PCR_ERR_INVALID_ARG, "target cloud must have normals (call estimate_normals first)");
+    return pcr_icp_point_to_plane_init_dev(source->owner, source->x(), source->y(), source->z(), source->n, target->x(), target->y(),
+                                           target->z(), target->n, target->nx(), target->ny(), target->nz(), target->n, init, params,
+                                           result);
+}
+
 }  // extern "C"
 
 /* ---- device-resident frame batches ----------------------------------------------------------------------
@@ -2957,7 +3051,7 @@ int pcr_frames_icp_point_to_point(const pcr_frames *frames, const uint32_t *pair
                                   pcr_icp_result *results) {
     PCR_TRY(handle_check(frames, "frames"));
     return icp_batch_entry(frames->owner, true, false, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(), nullptr, nullptr,
-                           nullptr, 0, pairs, n_pairs, params, results);
+                           nullptr, 0, pairs, n_pairs, false, nullptr, params, results);
 }
 
 int pcr_frames_icp_point_to_plane(const pcr_frames *frames, const uint32_t *pairs, size_t n_pairs, const pcr_icp_params *params,
@@ -2966,7 +3060,23 @@ int pcr_frames_icp_point_to_plane(const pcr_frames *frames, const uint32_t *pair
     if (!frames->has_normals)  // crates/python/src/registration.rs:80-86
         return fail(&frames->owner->c, PCR_ERR_INVALID_ARG, "point-to-plane ICP needs frames with normals (call estimate_normals first)");
     return icp_batch_entry(frames->owner, true, true, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(), frames->nx(),
-                           frames->ny(), frames->nz(), frames->n, pairs, n_pairs, params, results);
+                           frames->ny(), frames->nz(), frames->n, pairs, n_pairs, false, nullptr, params, results);
+}
+
+int pcr_frames_icp_point_to_point_init(const pcr_frames *frames, const uint32_t *pairs, size_t n_pairs, const float *inits,
+                                       const pcr_icp_params *params, pcr_icp_result *results) {
+    PCR_TRY(handle_check(frames, "frames"));
+    return icp_batch_entry(frames->owner, true, false, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(), nullptr, nullptr,
+                           nullptr, 0, pairs, n_pairs, true, inits, params, results);
+}
+
+int pcr_frames_icp_point_to_plane_init(const pcr_frames *frames, const uint32_t *pairs, size_t n_pairs, const float *inits,
+                                       const pcr_icp_params *params, pcr_icp_result *results) {
+    PCR_TRY(handle_check(frames, "frames"));
+    if (!frames->has_normals)  // crates/python/src/registration.rs:80-86
+        return fail(&frames->owner->c, PCR_ERR_INVALID_ARG, "point-to-plane ICP needs frames with normals (call estimate_normals first)");
+    return icp_batch_entry(frames->owner, true, true, frames->x(), frames->y(), frames->z(), frames->off.data(), frames->count(), frames->nx(),
+                           frames->ny(), frames->nz(), frames->n, pairs, n_pairs, true, inits, params, results);
 }
 
 }  // extern "C"

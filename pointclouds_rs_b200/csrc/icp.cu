@@ -97,14 +97,23 @@ __global__ void correspond_filter_kernel(size_t ns, float max_distance, uint32_t
 }
 
 // ---- binning of the source by target cell ---------------------------------------------------------
+// kInit: the loop starts from a guess, and the working copy holds apply_point(init, p) from the start.  The moved point
+// is what the first pass searches, so it is also what gets binned: binning the unmoved source would scatter the
+// threads of one target cell over the whole source when the guess moves it by metres.
+struct Xform {
+    float R[9], t[3];  // row-major R, then t (the 12 floats of pcr_apply_transform_batch)
+};
+
+template <bool kInit>
 __global__ void __launch_bounds__(256) src_count_kernel(const float *__restrict__ sx, const float *__restrict__ sy,
                                                         const float *__restrict__ sz, size_t ns,
                                                         const GridDesc *__restrict__ grids, uint32_t *__restrict__ table,
-                                                        uint32_t *__restrict__ cell_id, uint32_t *__restrict__ rank) {
+                                                        uint32_t *__restrict__ cell_id, uint32_t *__restrict__ rank, Xform init) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= ns) return;
     const GridDesc g = grids[0];
     float x = sx[i], y = sy[i], z = sz[i];
+    if (kInit) apply_point(init.R, init.t, x, y, z, x, y, z);
     uint32_t cid = 0;
     if (finite3(x, y, z) && g.n_cells > 0) {
         int c0 = cell_coord(g, 0, pick_axis(g.ax[0], x, y, z), nullptr);
@@ -116,14 +125,17 @@ __global__ void __launch_bounds__(256) src_count_kernel(const float *__restrict_
     rank[i] = atomicAdd(&table[cid], 1u);
 }
 
+template <bool kInit>
 __global__ void __launch_bounds__(256) src_scatter_kernel(const float *__restrict__ sx, const float *__restrict__ sy,
                                                           const float *__restrict__ sz, size_t ns,
                                                           const uint32_t *__restrict__ table,
                                                           const uint32_t *__restrict__ cell_id,
-                                                          const uint32_t *__restrict__ rank, float4 *__restrict__ cur) {
+                                                          const uint32_t *__restrict__ rank, float4 *__restrict__ cur, Xform init) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= ns) return;
-    cur[table[cell_id[i]] + rank[i]] = make_float4(sx[i], sy[i], sz[i], __uint_as_float((uint32_t)i));
+    float x = sx[i], y = sy[i], z = sz[i];
+    if (kInit) apply_point(init.R, init.t, x, y, z, x, y, z);
+    cur[table[cell_id[i]] + rank[i]] = make_float4(x, y, z, __uint_as_float((uint32_t)i));
 }
 
 // ---- per-iteration kernels ---------------------------------------------------------------------------
@@ -713,9 +725,17 @@ __device__ __forceinline__ void icp_init_state(IcpState *s) {
     for (int i = 0; i < NP; i++) s->sums[i] = 0.0;
 }
 
-__global__ void icp_init_state_kernel(IcpState *s) {
+// kInit: cumulative = init, no increment pending (the working copy was moved by init when it was binned)
+__device__ __forceinline__ void icp_seed_state(IcpState *s, const float *R, const float *t) {
+    for (int i = 0; i < 9; i++) s->cum_R[i] = R[i];
+    for (int i = 0; i < 3; i++) s->cum_t[i] = t[i];
+}
+
+template <bool kInit>
+__global__ void icp_init_state_kernel(IcpState *s, Xform init) {
     if (threadIdx.x != 0) return;
     icp_init_state(s);
+    if (kInit) icp_seed_state(s, init.R, init.t);
 }
 
 __global__ void pack_normals_kernel(const float *__restrict__ nx, const float *__restrict__ ny, const float *__restrict__ nz,
@@ -741,16 +761,20 @@ struct IcpBatchPairs {
 
 // Binning, deterministic: key (pair, target cell) for every working-copy point, in working-copy order, then the stable
 // radix sort; a cell's points end up in source order.  Non-finite points go to cell 0, as in src_count_kernel.
+// kInit: pair q's points are moved by inits[12q .. 12q + 12) before they are binned and stored (see src_count_kernel).
+template <bool kInit>
 __global__ void __launch_bounds__(256) icp_batch_bin_key_kernel(const float *__restrict__ x, const float *__restrict__ y,
                                                                 const float *__restrict__ z, IcpBatchPairs bp, uint32_t total,
                                                                 const GridDesc *__restrict__ grids, int cell_bits,
-                                                                unsigned long long *__restrict__ keys, uint32_t *__restrict__ vals) {
+                                                                unsigned long long *__restrict__ keys, uint32_t *__restrict__ vals,
+                                                                const float *__restrict__ inits) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= total) return;
     const int q = frame_of(bp.cur_off, bp.n_pairs, i);
     const uint32_t gi = bp.src_begin[q] + (i - bp.cur_off[q]);
     const GridDesc g = grids[bp.tgt_frame[q]];
-    const float px = x[gi], py = y[gi], pz = z[gi];
+    float px = x[gi], py = y[gi], pz = z[gi];
+    if (kInit) apply_point(inits + 12 * q, inits + 12 * q + 9, px, py, pz, px, py, pz);
     uint32_t cid = 0;
     if (finite3(px, py, pz) && g.n_cells > 0) {
         const int c0 = cell_coord(g, 0, pick_axis(g.ax[0], px, py, pz), nullptr);
@@ -762,19 +786,27 @@ __global__ void __launch_bounds__(256) icp_batch_bin_key_kernel(const float *__r
     vals[i] = gi;
 }
 
+template <bool kInit>
 __global__ void __launch_bounds__(256) icp_batch_bin_gather_kernel(const float *__restrict__ x, const float *__restrict__ y,
                                                                    const float *__restrict__ z, IcpBatchPairs bp, uint32_t total,
                                                                    int cell_bits, const unsigned long long *__restrict__ keys,
-                                                                   const uint32_t *__restrict__ vals, float4 *__restrict__ cur) {
+                                                                   const uint32_t *__restrict__ vals, float4 *__restrict__ cur,
+                                                                   const float *__restrict__ inits) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= total) return;
     const uint32_t q = (uint32_t)(keys[i] >> cell_bits), gi = vals[i];
-    cur[i] = make_float4(x[gi], y[gi], z[gi], __uint_as_float(gi - bp.src_begin[q]));
+    float px = x[gi], py = y[gi], pz = z[gi];
+    if (kInit) apply_point(inits + 12 * q, inits + 12 * q + 9, px, py, pz, px, py, pz);
+    cur[i] = make_float4(px, py, pz, __uint_as_float(gi - bp.src_begin[q]));
 }
 
-__global__ void icp_batch_init_kernel(IcpState *states, int n_pairs, unsigned *active) {
+template <bool kInit>
+__global__ void icp_batch_init_kernel(IcpState *states, int n_pairs, unsigned *active, const float *__restrict__ inits) {
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
-    if (q < n_pairs) icp_init_state(states + q);
+    if (q < n_pairs) {
+        icp_init_state(states + q);
+        if (kInit) icp_seed_state(states + q, inits + 12 * q, inits + 12 * q + 9);
+    }
     if (q == 0) *active = (unsigned)n_pairs;
 }
 
@@ -911,7 +943,7 @@ int find_correspondences_dev(Index *target, const float *dsx, const float *dsy, 
 int icp_dev(Ctx *ctx, const IcpArgs &a, pcr_icp_result *result) {
     cudaStream_t st = ctx->stream;
     const bool plane = a.d_nx != nullptr;
-    // identity / empty handling is done by the caller (api.cu); here ns > 0 and nt > 0
+    // the start (identity or init) and the empty cases are handled by the caller (api.cu); here nt > 0
     Index *tgt = nullptr;
     BuildOpts bo;
     bo.k_hint = 1;
@@ -920,7 +952,9 @@ int icp_dev(Ctx *ctx, const IcpArgs &a, pcr_icp_result *result) {
     const IndexPtr guard(tgt);
 
     const size_t ns = a.ns;
-    // working copy of the source, binned by target cell
+    Xform init = {};
+    if (a.init) memcpy(&init, a.init, sizeof(init));
+    // working copy of the source (moved by init), binned by target cell
     StreamAlloc<float4> cur_mem(st), nrm4_mem(st);
     PCR_CUDA(ctx, cur_mem.alloc(sizeof(float4) * std::max<size_t>(ns, 1)));
     float4 *cur = cur_mem.p, *nrm4 = nullptr;
@@ -937,10 +971,12 @@ int icp_dev(Ctx *ctx, const IcpArgs &a, pcr_icp_result *result) {
         uint32_t *table = (uint32_t *)ctx->b_table.p;
         uint32_t *cid = (uint32_t *)ctx->b_misc.p, *rank = cid + ns;
         PCR_CUDA(ctx, cudaMemsetAsync(table, 0, sizeof(uint32_t) * cells, st));
-        src_count_kernel<<<(unsigned)((ns + 255) / 256), 256, 0, st>>>(a.d_sx, a.d_sy, a.d_sz, ns, tgt->grids, table, cid, rank);
+        (a.init ? src_count_kernel<true> : src_count_kernel<false>)<<<(unsigned)((ns + 255) / 256), 256, 0, st>>>(
+            a.d_sx, a.d_sy, a.d_sz, ns, tgt->grids, table, cid, rank, init);
         PCR_LAUNCH_CHECK(ctx);
         PCR_TRY(exclusive_scan_u32_dev(ctx, table, cells));
-        src_scatter_kernel<<<(unsigned)((ns + 255) / 256), 256, 0, st>>>(a.d_sx, a.d_sy, a.d_sz, ns, table, cid, rank, cur);
+        (a.init ? src_scatter_kernel<true> : src_scatter_kernel<false>)<<<(unsigned)((ns + 255) / 256), 256, 0, st>>>(
+            a.d_sx, a.d_sy, a.d_sz, ns, table, cid, rank, cur, init);
         PCR_LAUNCH_CHECK(ctx);
     }
 
@@ -965,7 +1001,7 @@ int icp_dev(Ctx *ctx, const IcpArgs &a, pcr_icp_result *result) {
     volatile int *h_done = (volatile int *)ctx->pinned;  // device-visible through UVA
     *h_done = 0;
     double *partials = (double *)ctx->b_misc2.p;
-    icp_init_state_kernel<<<1, 32, 0, st>>>(d_state);
+    (a.init ? icp_init_state_kernel<true> : icp_init_state_kernel<false>)<<<1, 32, 0, st>>>(d_state, init);
     PCR_LAUNCH_CHECK(ctx);
 
     auto one_pass = [&](int metrics_only) -> int {
@@ -1056,7 +1092,7 @@ int icp_batch_dev(Ctx *ctx, const IcpBatchArgs &a, pcr_icp_result *results) {
     cudaStream_t st = ctx->stream;
     const bool plane = a.d_nx != nullptr;
     const uint64_t *off = a.frame_offsets;
-    // pairs with an empty side are answered here (icp.rs:131-139: the identity the caller stored, 0 iterations); the
+    // pairs with an empty side are answered here (icp.rs:131-139: the guess the caller stored, 0 iterations); the
     // others are numbered q = 0 .. Q - 1
     std::vector<uint32_t> act, cur_off(1, 0), blk_off(1, 0), tgt_frame, src_begin;
     const uint64_t blk_cap = (uint64_t)ctx->sm_count * 4;
@@ -1096,7 +1132,7 @@ int icp_batch_dev(Ctx *ctx, const IcpBatchArgs &a, pcr_icp_result *results) {
     const size_t o_part = o_dl + up(sizeof(uint32_t) * (64 + 2 * (size_t)total));
     const size_t o_state = o_part + up(sizeof(double) * NP * (size_t)n_blocks);
     const size_t o_tab = o_state + up(sizeof(IcpState) * Q);
-    const size_t tab_words = 4 * (size_t)Q + 2;
+    const size_t tab_words = 4 * (size_t)Q + 2 + (a.inits ? 12 * (size_t)Q : 0);  // (+ the guesses of the pairs)
     const size_t o_nrm = o_tab + up(sizeof(uint32_t) * tab_words);
     const size_t bytes = o_nrm + (plane ? sizeof(float4) * a.n : 0);
     StreamAlloc<char> mem_alloc(st);
@@ -1122,6 +1158,8 @@ int icp_batch_dev(Ctx *ctx, const IcpBatchArgs &a, pcr_icp_result *results) {
     memcpy(h_tab + Q + 1, blk_off.data(), sizeof(uint32_t) * (Q + 1));
     memcpy(h_tab + 2 * Q + 2, tgt_frame.data(), sizeof(uint32_t) * Q);
     memcpy(h_tab + 3 * Q + 2, src_begin.data(), sizeof(uint32_t) * Q);
+    if (a.inits)
+        for (int q = 0; q < Q; q++) memcpy(h_tab + 4 * Q + 2 + 12 * q, a.inits + 12 * (size_t)act[q], sizeof(float) * 12);
     PCR_CUDA(ctx, cudaMemcpyAsync(d_tab, h_tab, sizeof(uint32_t) * tab_words, cudaMemcpyHostToDevice, st));
     IcpBatchPairs bp;
     bp.cur_off = d_tab;
@@ -1129,6 +1167,7 @@ int icp_batch_dev(Ctx *ctx, const IcpBatchArgs &a, pcr_icp_result *results) {
     bp.tgt_frame = d_tab + 2 * Q + 2;
     bp.src_begin = d_tab + 3 * Q + 2;
     bp.n_pairs = Q;
+    const float *d_inits = a.inits ? (const float *)(d_tab + 4 * Q + 2) : nullptr;
 
     if (plane) {
         pack_normals_kernel<<<(unsigned)((a.n + 255) / 256), 256, 0, st>>>(a.d_nx, a.d_ny, a.d_nz, a.n, nrm4);
@@ -1148,13 +1187,15 @@ int icp_batch_dev(Ctx *ctx, const IcpBatchArgs &a, pcr_icp_result *results) {
         uint32_t *vA = (uint32_t *)(sm + up(2 * sizeof(unsigned long long) * total)), *vB = vA + total;
         uint32_t *hist = (uint32_t *)((char *)vA + up(2 * sizeof(uint32_t) * total));
         const unsigned nb = (total + 255) / 256;
-        icp_batch_bin_key_kernel<<<nb, 256, 0, st>>>(a.d_x, a.d_y, a.d_z, bp, total, tgt->grids, cell_bits, kA, vA);
+        (a.inits ? icp_batch_bin_key_kernel<true> : icp_batch_bin_key_kernel<false>)<<<nb, 256, 0, st>>>(
+            a.d_x, a.d_y, a.d_z, bp, total, tgt->grids, cell_bits, kA, vA, d_inits);
         PCR_LAUNCH_CHECK(ctx);
         PCR_TRY(radix_sort_pairs_dev(ctx, &kA, &vA, &kB, &vB, total, key_bits, hist));
-        icp_batch_bin_gather_kernel<<<nb, 256, 0, st>>>(a.d_x, a.d_y, a.d_z, bp, total, cell_bits, kA, vA, cur);
+        (a.inits ? icp_batch_bin_gather_kernel<true> : icp_batch_bin_gather_kernel<false>)<<<nb, 256, 0, st>>>(
+            a.d_x, a.d_y, a.d_z, bp, total, cell_bits, kA, vA, cur, d_inits);
         PCR_LAUNCH_CHECK(ctx);
     }
-    icp_batch_init_kernel<<<(Q + 127) / 128, 128, 0, st>>>(d_states, Q, active);
+    (a.inits ? icp_batch_init_kernel<true> : icp_batch_init_kernel<false>)<<<(Q + 127) / 128, 128, 0, st>>>(d_states, Q, active, d_inits);
     PCR_LAUNCH_CHECK(ctx);
 
     auto one_pass = [&](int metrics_only) -> int {

@@ -346,9 +346,10 @@ struct IcpArgs {
     size_t nt;
     const float *d_nx, *d_ny, *d_nz;  // nullptr for point-to-point
     pcr_icp_params params;
+    const float *init = nullptr;  // host, 12 floats (row-major R, then t): the loop's start; nullptr = identity
 };
 int icp_dev(Ctx *ctx, const IcpArgs &a, pcr_icp_result *result);
-// Pairs of frames of one buffer (pcr_icp_point_to_*_batch, arguments checked by the caller, results preset to the identity).
+// Pairs of frames of one buffer (pcr_icp_point_to_*_batch, arguments checked by the caller, results preset to each pair's start).
 struct IcpBatchArgs {
     const float *d_x, *d_y, *d_z;  // every frame, back to back
     size_t n;
@@ -358,6 +359,7 @@ struct IcpBatchArgs {
     const uint32_t *pairs;            // host: pair p = (source frame, target frame)
     size_t n_pairs;
     pcr_icp_params params;
+    const float *inits = nullptr;  // host, 12 floats per pair (row-major R, then t): each pair's start; nullptr = identity
 };
 int icp_batch_dev(Ctx *ctx, const IcpBatchArgs &a, pcr_icp_result *results);
 int find_correspondences_dev(Index *target, const float *dsx, const float *dsy, const float *dsz,
