@@ -163,6 +163,15 @@ int pcr_ctx_set_query_sharding(pcr_ctx *ctx, int enable);
  * GPU can then play every rank in turn and the test checks that the parts are disjoint and add up to the unsharded
  * result (tests/test_gpu_parity.py).  Not for production use. */
 int pcr_ctx_debug_set_shard(pcr_ctx *ctx, int rank, int world_size);
+/* Test hook: the self-query K-nearest-neighbour lists of every point of a batch of frames (frame f = input points
+ * [frame_offsets[f], frame_offsets[f+1])), as the fused SOR -> normals pass searches them: the exact search of the product,
+ * lists kept.  Row i of idx_out (n x K) is input point i's list in ascending (d^2, index) order, as batch input indices;
+ * count_out[i] = valid entries, 0xff = no list (a non-finite point, or a query the search left to a coarser level, where no
+ * list is kept).  routes_out: [0] normal (+ heavy) queries, [1] dense, [2] sparse, [3] follow-up, [4] handed back by the cell
+ * tiles, [5] deferred by level 0, [6..7] 0; words 0-4 come from the class split of level 0, which only runs for K <= 21.
+ * K must be in 2..32.  Not for production use. */
+int pcr_debug_self_knn_lists(pcr_ctx *ctx, const float *x, const float *y, const float *z, const uint64_t *frame_offsets,
+                             size_t n_frames, size_t K, uint32_t *idx_out, uint8_t *count_out, uint64_t routes_out[8]);
 
 /* ---- spatial index (KdTree) ------------------------------------------------------------------ */
 /* k_hint: the k the index will mostly be queried with (0 = unknown); only steers the cell size. */

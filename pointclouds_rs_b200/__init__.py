@@ -1153,6 +1153,30 @@ def radius_outlier_removal_batch(points: np.ndarray, frame_offsets: Sequence[int
     return keep[:n], kept[:nf]
 
 
+DEBUG_ROUTES = ("normal", "dense", "sparse", "follow_up", "handed_back", "deferred")
+
+
+def debug_self_knn_lists(points: np.ndarray, frame_offsets: Sequence[int], K: int, ctx: Optional[Context] = None):
+    """Test hook (pcr_debug_self_knn_lists): the K-nearest-neighbour list of every point among the points of its own frame,
+    as the fused SOR -> normals pass searches it.  -> (idx (N,K) u32 frame-local, count (N,) u8 (0xff = no list), routes
+    dict of the level-0 query counts named by DEBUG_ROUTES)."""
+    pts, off = _batch_frames(points, frame_offsets)
+    ctx = ctx or default_context()
+    x, y, z = _soa(pts)
+    n, nf = len(pts), len(off) - 1
+    idx = np.full((max(n, 1), K), 0xFFFFFFFF, np.uint32)
+    cnt = np.full(max(n, 1), 0xFF, np.uint8)
+    routes = np.zeros(8, np.uint64)
+    st = _ffi.load().pcr_debug_self_knn_lists(ctx._h, _p(x, _ffi.f32p), _p(y, _ffi.f32p), _p(z, _ffi.f32p), _p(off, _ffi.u64p), nf,
+                                              int(K), _p(idx, _ffi.u32p), _p(cnt, _ffi.u8p), _p(routes, _ffi.u64p))
+    _ffi.check(st, ctx._h)
+    idx, cnt = idx[:n], cnt[:n]
+    frame = np.repeat(np.arange(nf), np.diff(off).astype(np.int64))
+    valid = idx != 0xFFFFFFFF
+    idx[valid] -= off[frame].astype(np.uint32)[:, None].repeat(K, 1)[valid]
+    return idx, cnt, {name: int(routes[i]) for i, name in enumerate(DEBUG_ROUTES)}
+
+
 def _frame_lists(lists, off):
     """Checks and stacks one frame-local index list per frame -> (indices u32, list offsets (F+1,) u64); IndexError names
     the frame of an index outside it."""

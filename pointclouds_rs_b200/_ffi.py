@@ -72,6 +72,7 @@ SIGNATURES = {
     "pcr_ctx_get_knn_counters": (C.c_int, [vp, u64p]),
     "pcr_ctx_set_query_sharding": (C.c_int, [vp, C.c_int]),
     "pcr_ctx_debug_set_shard": (C.c_int, [vp, C.c_int, C.c_int]),
+    "pcr_debug_self_knn_lists": (C.c_int, [vp, f32p, f32p, f32p, u64p, C.c_size_t, C.c_size_t, u32p, u8p, u64p]),
     "pcr_ctx_set_timing": (C.c_int, [vp, C.c_int]),
     "pcr_ctx_get_timing": (C.c_int, [vp, C.POINTER(C.c_double), u64p]),
     "pcr_comm_unique_id": (C.c_int, [vp]),

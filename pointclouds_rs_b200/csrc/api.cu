@@ -1911,6 +1911,85 @@ int pcr_sor_normals_batch(pcr_ctx *ctx, const float *x, const float *y, const fl
     PCR_API_END(c)
 }
 
+// Test hook: the self-query search of the fused SOR -> normals pass (batch_core), lists kept, read back in input order.
+int pcr_debug_self_knn_lists(pcr_ctx *ctx, const float *x, const float *y, const float *z, const uint64_t *frame_offsets, size_t n_frames,
+                             size_t K, uint32_t *idx_out, uint8_t *count_out, uint64_t routes_out[8]) {
+    if (!ctx) return fail(nullptr, PCR_ERR_INVALID_ARG, "ctx is NULL");
+    Ctx *c = &ctx->c;
+    if (!routes_out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    memset(routes_out, 0, sizeof(uint64_t) * 8);
+    if (K < 2 || K > 32) return fail(c, PCR_ERR_UNSUPPORTED, "debug_self_knn_lists: K = %zu outside 2..32", K);
+    if (n_frames == 0) return PCR_OK;
+    PCR_TRY(offsets_check(c, "frame_offsets", frame_offsets, n_frames));
+    const size_t n = (size_t)frame_offsets[n_frames];
+    if (n == 0) return PCR_OK;
+    if (!x || !y || !z || !idx_out || !count_out) return fail(c, PCR_ERR_INVALID_ARG, "null pointer");
+    PCR_TRY(batch_size_check(c, n, n_frames));
+    PCR_API_BEGIN
+    DevSetter ds(c);
+    float *dx, *dy, *dz;
+    PCR_TRY(stage_xyz(c, c->b_in, x, y, z, n, &dx, &dy, &dz));
+    StreamAlloc<float> mean_mem(c->stream);
+    StreamAlloc<uint32_t> list_mem(c->stream);
+    PCR_CUDA(c, mean_mem.alloc(sizeof(float) * n));
+    SorLists sl;  // (the layout batch_core allocates)
+    sl.K = K;
+    sl.stride = (n + 63) & ~(size_t)63;
+    PCR_CUDA(c, list_mem.alloc(sizeof(uint32_t) * (K * sl.stride + sl.stride + 64) + sl.stride));
+    sl.lists = list_mem.p;
+    sl.fallback = sl.lists + K * sl.stride;
+    sl.cnt = (uint8_t *)(sl.fallback + sl.stride + 64);
+    PCR_CUDA(c, cudaMemsetAsync(sl.fallback + sl.stride, 0, 64 * sizeof(uint32_t), c->stream));
+    PCR_CUDA(c, cudaMemsetAsync(sl.cnt, 0xff, sl.stride, c->stream));
+    sl.initialised = true;
+    BuildOpts bo;
+    bo.k_hint = K;
+    bo.self_knn = true;
+    bo.n_frames = (int)n_frames;
+    bo.transient = true;
+    bo.frame_offsets = frame_offsets;
+    Index *ix = nullptr;
+    PCR_TRY(index_build_dev(c, dx, dy, dz, n, bo, &ix));
+    const IndexPtr guard(ix);
+    PCR_TRY(sor_mean_dist_dev(ix, K - 1, mean_mem.p, &sl));
+    const size_t m = ix->n_indexed;
+    std::vector<uint32_t> lists(K * m);
+    std::vector<uint8_t> cnt(m);
+    std::vector<float4> sorted(m);
+    uint32_t counters[16] = {};
+    for (size_t j = 0; j < K && m > 0; j++)
+        PCR_CUDA(c, cudaMemcpyAsync(lists.data() + j * m, sl.lists + j * sl.stride, sizeof(uint32_t) * m, cudaMemcpyDeviceToHost, c->stream));
+    if (m > 0) {
+        PCR_CUDA(c, cudaMemcpyAsync(cnt.data(), sl.cnt, m, cudaMemcpyDeviceToHost, c->stream));
+        PCR_CUDA(c, cudaMemcpyAsync(sorted.data(), ix->sorted, sizeof(float4) * m, cudaMemcpyDeviceToHost, c->stream));
+        PCR_CUDA(c, cudaMemcpyAsync(counters, c->b_list.p, sizeof(counters), cudaMemcpyDeviceToHost, c->stream));
+    }
+    PCR_CUDA(c, cudaStreamSynchronize(c->stream));
+    memset(count_out, 0xff, n);
+    for (size_t i = 0; i < n * K; i++) idx_out[i] = 0xffffffffu;
+    size_t no_list = 0;
+    for (size_t q = 0; q < m; q++) {
+        uint32_t row;
+        memcpy(&row, &sorted[q].w, sizeof(row));
+        count_out[row] = cnt[q];
+        if (cnt[q] == 0xff) {
+            no_list++;
+            continue;
+        }
+        for (size_t j = 0; j < K; j++) idx_out[(size_t)row * K + j] = lists[j * m + q];
+    }
+    // run_levels' level-0 counter words (knn.cu): only the class-split search (K <= kSelMaxK) writes words 0-4.  A finite
+    // point without a list is either a sparse query or one that level 0 deferred to the coarser levels.
+    routes_out[0] = counters[3] + counters[7];  // normal (+ heavy)
+    routes_out[1] = counters[4];                // dense, on the finer level
+    routes_out[2] = counters[5];                // sparse, on the coarser level (no list)
+    routes_out[3] = counters[2];                // follow-up pass
+    routes_out[4] = counters[6];                // handed back by the cell tiles to the warp kernels
+    routes_out[5] = no_list - counters[5];      // deferred by level 0 to the coarser levels (no list)
+    return PCR_OK;
+    PCR_API_END(c)
+}
+
 }  // extern "C"
 
 /* ---- device-resident clouds (SURVEY 8f-3) -------------------------------------------------------------

@@ -2062,9 +2062,11 @@ int normals_from_lists_dev(Index *ix, size_t k, const float vp[3], const SorList
     }
     // The queries that fall back are few, and their count is still on the device: launch their level-0 pass now for a
     // fixed capacity (the kernel reads the count itself) and let the count, the kept count the caller's compaction
-    // wants and the pass's own deferred count come back in ONE round trip.
-    uint32_t *mail = (uint32_t *)ctx->pinned + 40;
-    unsigned long long *mail_kept = (unsigned long long *)((uint32_t *)ctx->pinned + 42);
+    // wants and the pass's own deferred count come back in ONE round trip.  (Words 64..67 of the mailbox: run_levels
+    // copies its counters to words 32..47 on EVERY round trip, so a fallback pass that defers to level 1 would overwrite
+    // a piggy slot inside that block with zeros -- a kept count of 0 and a lost second pass.)
+    uint32_t *mail = (uint32_t *)ctx->pinned + 64;
+    unsigned long long *mail_kept = (unsigned long long *)((uint32_t *)ctx->pinned + 66);
     ctx->piggy.clear();
     ctx->piggy.push_back({mail, d_fb_count, sizeof(uint32_t)});
     if (d_kept0 && h_kept0) ctx->piggy.push_back({mail_kept, d_kept0, sizeof(unsigned long long)});

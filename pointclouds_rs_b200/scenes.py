@@ -194,3 +194,131 @@ def voxel_downsample_np(pts: np.ndarray, voxel_size: float) -> np.ndarray:
     np.add.at(sums, seg, p[order])  # unbuffered: sequential f32 adds in input order
     cnt = np.bincount(seg).astype(np.float32)
     return (sums / cnt[:, None]).astype(np.float32)
+
+
+# ---------------------------------------------------------------------------------------------------
+# Adversarial scenes for the exact KNN engine (tests/test_knn_routes.py).  Each one is built to reach a route or a branch
+# of the level-0 self-query search that the gentle scenes above seldom reach: exact distance ties at the k-th place,
+# duplicate points, candidate counts beyond what one cell tile can stage, k-th neighbours far outside the uniform-sheet
+# model, queries on cell faces and degenerate (flat) grids.
+# ---------------------------------------------------------------------------------------------------
+
+def tie_grid(seed: int = 1, dims=(160, 160, 4), occupancy: float = 0.3) -> np.ndarray:
+    """A random `occupancy` share of the integer box `dims`, rows shuffled, scaled by 2^-4 and offset by 4096.  Every
+    coordinate, difference and d^2 is exact in f32, so equal distances are equal bits: most queries have a tie across the
+    k-th place (the index breaks it).  The cell tile's ranking puts such ties in (d^2, index) order with its bubble pass
+    (tile_fix), and the thread-per-query selection of external queries with its slow exact path (sel_exact_slow).  The
+    tie groups stay within the tile's 32 slots for k <= 21, so the tile's exact-tie hand-back is left to dup_cloud."""
+    rng = np.random.default_rng(seed)
+    nx, ny, nz = dims
+    sites = np.flatnonzero(rng.random(nx * ny * nz) < occupancy)
+    rng.shuffle(sites)
+    ijk = np.stack(np.unravel_index(sites, dims), 1).astype(np.float32)
+    return np.ascontiguousarray(ijk * np.float32(1.0 / 16.0) + np.float32(4096.0), np.float32)
+
+
+def dup_cloud(seed: int = 2, counts=(8_000, 400, 70, 500), max_copies: int = 6, n_big: int = 4, big_copies: int = 40,
+              n_nonfinite: int = 7) -> np.ndarray:
+    """A KITTI-shaped frame in which every point is repeated 1..max_copies times at scattered indices: groups of points at
+    d^2 = 0 larger than a small k, whose members only the index tells apart.  `n_big` of the scattered noise points are
+    repeated `big_copies` times: more candidates at d^2 = 0 than the cell tile's 32 slots, which it hands back to the warp
+    kernels.  A few non-finite rows keep no list."""
+    rng = np.random.default_rng(seed)
+    base = kitti_scene(seed, counts)
+    rep = rng.integers(1, max_copies + 1, len(base))
+    rep[0] = max_copies  # (at least one group of the largest size)
+    rep[len(base) - n_big:] = big_copies  # (the last rows of kitti_scene are its noise points)
+    pts = np.repeat(base, rep, axis=0)
+    pts = pts[rng.permutation(len(pts))]
+    bad = rng.choice(len(pts), n_nonfinite, replace=False)
+    pts[bad[0::3], 0] = np.nan
+    pts[bad[1::3], 1] = np.inf
+    pts[bad[2::3], 2] = -np.inf
+    return np.ascontiguousarray(pts, np.float32)
+
+
+def density_ramp(seed: int = 3, n_sheet: int = 30_000, ratio: float = 100.0, n_box: int = 1_500) -> np.ndarray:
+    """A 40 x 10 m sheet whose density rises `ratio`-fold along x, plus three compact 0.3 m boxes.  One cell size serves
+    the whole frame, so the candidates in a query's 27 cells run from a handful to thousands: past the tile kernel's
+    dense-class bound (128), the selection histogram's (384) and what one sub-tile can stage (512 points), which forces
+    the smaller sub-tile attempts and the dense class on the finer level."""
+    rng = np.random.default_rng(seed)
+    u = rng.random(n_sheet)
+    x = 40.0 * np.log1p(u * (ratio - 1.0)) / np.log(ratio)  # density proportional to ratio^(x / 40)
+    sheet = np.column_stack([x, rng.uniform(0.0, 10.0, n_sheet), rng.normal(0.0, 0.01, n_sheet)])
+    parts = [sheet]
+    for cx, cy in ((5.0, 5.0), (20.0, 2.0), (38.0, 8.0)):
+        parts.append(np.column_stack([rng.uniform(cx, cx + 0.3, n_box), rng.uniform(cy, cy + 0.3, n_box), rng.uniform(0.1, 0.4, n_box)]))
+    pts = np.vstack(parts)
+    return np.ascontiguousarray(pts[rng.permutation(len(pts))], np.float32)
+
+
+def wires(seed: int = 4, n_sheet: int = 20_000, n_wires: int = 6, spacing: float = 0.3, n_isolated: int = 40) -> np.ndarray:
+    """Sparse polylines 3-6 m above a 20 x 20 m sheet, and isolated points tens of metres away.  A wire point's k-th
+    neighbour lies k/2 spacings along the wire, far beyond what the sheet's density predicts (the selection's histogram
+    has to widen); the isolated points have almost no candidates in their cells (the sparse class, searched on the
+    coarser level) or need the coarser levels altogether."""
+    rng = np.random.default_rng(seed)
+    parts = [np.column_stack([rng.uniform(0.0, 20.0, n_sheet), rng.uniform(0.0, 20.0, n_sheet), rng.normal(0.0, 0.02, n_sheet)])]
+    for _ in range(n_wires):
+        a = np.append(rng.uniform(0.0, 20.0, 2), rng.uniform(3.0, 6.0))
+        b = np.append(rng.uniform(0.0, 20.0, 2), rng.uniform(3.0, 6.0))
+        m = max(2, int(np.linalg.norm(b - a) / spacing))
+        t = np.linspace(0.0, 1.0, m)[:, None]
+        parts.append(a + t * (b - a) + rng.normal(0.0, 0.005, (m, 3)))
+    iso = rng.uniform(-60.0, 80.0, (n_isolated, 3))
+    iso[:, 2] = rng.uniform(10.0, 40.0, n_isolated)
+    parts.append(iso)
+    pts = np.vstack(parts)
+    return np.ascontiguousarray(pts[rng.permutation(len(pts))], np.float32)
+
+
+def faces(seed: int = 5, n: int = 25_000, dims=(128, 128, 16)) -> np.ndarray:
+    """Distinct random sites of the 2^-4 lattice in an 8 x 8 x 1 m box.  With a cell size of 0.25 (four lattice steps),
+    a quarter of the coordinates lie exactly on a cell face on each axis, and candidates lie exactly at the ring bound of
+    the search's stopping rule; d^2 is exact, so ties are exact too."""
+    rng = np.random.default_rng(seed)
+    sites = rng.choice(dims[0] * dims[1] * dims[2], n, replace=False)
+    ijk = np.stack(np.unravel_index(sites, dims), 1).astype(np.float32)
+    return np.ascontiguousarray(ijk * np.float32(1.0 / 16.0), np.float32)
+
+
+def flat(seed: int = 6, n_sheet: int = 20_000, n_line: int = 2_000) -> np.ndarray:
+    """An exactly planar sheet (z = 0) and an exactly straight line in the same plane: the grid has one cell along z, so
+    every cube of cells is cut by the grid boundary."""
+    rng = np.random.default_rng(seed)
+    sheet = np.column_stack([rng.uniform(0.0, 20.0, n_sheet), rng.uniform(0.0, 20.0, n_sheet), np.zeros(n_sheet)])
+    line = np.column_stack([rng.uniform(0.0, 30.0, n_line), np.full(n_line, -5.0), np.zeros(n_line)])
+    pts = np.vstack([sheet, line])
+    return np.ascontiguousarray(pts[rng.permutation(len(pts))], np.float32)
+
+
+def straight_line(seed: int = 7, n: int = 3_000) -> np.ndarray:
+    """Points of one exactly straight line along x: a grid of one cell on two axes."""
+    rng = np.random.default_rng(seed)
+    return np.ascontiguousarray(np.column_stack([rng.uniform(-10.0, 10.0, n), np.full(n, 2.5), np.full(n, -1.0)]), np.float32)
+
+
+ADVERSARIAL = {
+    "tie_grid": tie_grid,
+    "dup_cloud": dup_cloud,
+    "density_ramp": density_ramp,
+    "wires": wires,
+    "faces": faces,
+    "flat": flat,
+}
+
+
+def adversarial_batch(seed: int = 8):
+    """The adversarial scenes as frames of one batch, with the small frames a batch meets: 95, 96 and 97 points (either
+    side of the size below which a frame is scanned whole), seven points (fewer than most k), one point, an empty frame and
+    a straight line.  -> (points (N,3) f32, frame offsets (F+1,) u64)."""
+    rng = np.random.default_rng(seed)
+    frames = [f() for f in ADVERSARIAL.values()]
+    frames += [uniform_cube(95, seed + 1, 0, 2), uniform_cube(96, seed + 2, 0, 2), uniform_cube(97, seed + 3, 0, 2),
+               uniform_cube(7, seed + 4, 0, 1), uniform_cube(1, seed + 5), np.zeros((0, 3), np.float32), straight_line()]
+    order = rng.permutation(len(frames))
+    frames = [frames[i] for i in order]
+    off = np.zeros(len(frames) + 1, np.uint64)
+    off[1:] = np.cumsum([len(f) for f in frames])
+    return np.ascontiguousarray(np.vstack(frames), np.float32), off

@@ -34,12 +34,14 @@ SCENES = {
     "line": lambda: np.stack([np.arange(300, dtype=np.float32), np.zeros(300, np.float32), np.zeros(300, np.float32)], 1),
     "tiny5": lambda: scenes.uniform_cube(5, 1, 0, 1),
     "plane_far_outlier": lambda: np.vstack([scenes.kitti_scene(4, (5_000, 10, 10, 10)), [[4000.0, -3000.0, 900.0]]]).astype(np.float32),
+    **scenes.ADVERSARIAL,  # exact ties, duplicates, density ramps, far k-th neighbours, cell faces, flat grids
 }
 
 
 def _queries(pts, rng):
     own = pts[rng.integers(0, len(pts), min(len(pts), 1500))]
-    lo, hi = pts.min(0), pts.max(0)
+    fin = pts[np.isfinite(pts).all(1)]
+    lo, hi = fin.min(0), fin.max(0)
     ext = rng.uniform(lo - 0.3 * (hi - lo) - 1, hi + 0.3 * (hi - lo) + 1, (400, 3)).astype(np.float32)
     far = np.array([[1e6, 1e6, 1e6], [-5e4, 0, 0], [0, 0, 1e-30]], np.float32)
     bad = np.array([[np.nan, 0, 0], [0, np.inf, 0], [0, 0, -np.inf]], np.float32)
@@ -47,7 +49,7 @@ def _queries(pts, rng):
 
 
 @pytest.mark.parametrize("scene", list(SCENES))
-@pytest.mark.parametrize("k", [1, 2, 11, 20, 32, 33, 70])
+@pytest.mark.parametrize("k", [1, 2, 11, 12, 13, 20, 21, 22, 32, 33, 70])
 def test_knn_bit_exact(pcr, oracle, scene, k):
     pts = SCENES[scene]()
     rng = np.random.default_rng(11)
@@ -94,7 +96,8 @@ def test_knn_edge_cases(pcr):
 
 @pytest.mark.parametrize("scene,k,std", [("kitti20k", 10, 1.0), ("kitti20k", 20, 2.0), ("cube20k", 10, 1.0),
                                          ("lattice1000", 5, 3.0), ("dupes", 4, 1.0), ("plane_far_outlier", 10, 1.0),
-                                         ("kitti20k", 40, 1.0)])
+                                         ("kitti20k", 40, 1.0)]
+                         + [(name, k, 1.0) for name in scenes.ADVERSARIAL for k in (10, 20, 21, 31)])
 def test_sor_bit_exact(pcr, oracle, scene, k, std):
     pts = SCENES[scene]()
     keep, kept, mean_d, stats = pcr.sor_mask(_cloud(pcr, pts), k, std, want_mean=True)
@@ -406,6 +409,19 @@ def test_fused_lists_equal_the_two_step_path(pcr, oracle, k_sor, std, k_nrm):
     most lists lose more neighbours than their margin and the fallback search carries the result; the normals must be
     BIT-identical to estimate_normals on the filtered cloud (same kernels' arithmetic, same neighbour order)."""
     pts = np.vstack([scenes.kitti_scene(31, (6_000, 300, 60, 140)), [[np.nan, 0, 0], [1, np.inf, 2]]]).astype(np.float32)
+    _fused_equals_two_step(pcr, oracle, pts, k_sor, std, k_nrm, check_angles=True)
+
+
+@pytest.mark.parametrize("k_sor,std,k_nrm", [(10, 1.0, 20), (5, 0.0, 8), (31, 1.0, 10), (10, 0.3, 31), (3, 1.0, 1)])
+@pytest.mark.parametrize("scene", ["tie_grid", "dup_cloud"])
+def test_fused_lists_equal_the_two_step_path_on_ties(pcr, oracle, scene, k_sor, std, k_nrm):
+    """The same on clouds where most lists depend on the index tie-break (exact d^2 ties, duplicate points): a shared
+    wrong member would not cancel out, because the filtered cloud renumbers the points.  (The oracle's normals are not
+    compared here: symmetric neighbourhoods leave the smallest eigenvector undetermined.)"""
+    _fused_equals_two_step(pcr, oracle, scenes.ADVERSARIAL[scene](), k_sor, std, k_nrm, check_angles=False)
+
+
+def _fused_equals_two_step(pcr, oracle, pts, k_sor, std, k_nrm, check_angles):
     off = np.array([0, len(pts)], np.uint64)
     keep, nrm, kept = pcr.sor_normals_batch(pts, off, k_sor, std, k_nrm)
     o_keep, _, _ = oracle.sor(pts, k_sor, std, threads=T)
@@ -413,10 +429,32 @@ def test_fused_lists_equal_the_two_step_path(pcr, oracle, k_sor, std, k_nrm):
     sel = np.nonzero(o_keep)[0]
     two_step = pcr.normals_array(_cloud(pcr, pts[sel]), k_nrm)      # a fresh search on the filtered cloud
     assert np.array_equal(nrm[sel].view(np.uint32), two_step.view(np.uint32))
-    assert np.nanmax(_angles(nrm[sel], oracle.normals(pts[sel], k_nrm, threads=T))) < 1e-4
+    if check_angles:
+        assert np.nanmax(_angles(nrm[sel], oracle.normals(pts[sel], k_nrm, threads=T))) < 1e-4
     assert (nrm[o_keep == 0] == 0).all()
     dev = pcr.DeviceCloud.from_numpy(pts).sor_normals(k_sor, std, k_nrm)
     assert np.array_equal(dev.to_numpy(), pts[sel], equal_nan=True) and np.array_equal(dev.normals_to_numpy().view(np.uint32), two_step.view(np.uint32))
+
+
+@pytest.mark.parametrize("cap", [None, "5"])
+@pytest.mark.parametrize("scene", ["dup_cloud", "wires"])
+def test_fused_fallback_that_defers_keeps_its_counts(pcr, oracle, monkeypatch, scene, cap):
+    """The fallback search of the fused path can defer queries to level 1.  Its own round trips must not clobber the
+    fallback count and the kept count that ride along with its first one: a lost kept count made the device-resident
+    form return an empty cloud, a lost fallback count skipped the queries beyond the blind pass's capacity."""
+    if cap:
+        monkeypatch.setenv("PCR_FALLBACK_CAP", cap)
+    pts = scenes.ADVERSARIAL[scene]()
+    for k_sor, std, k_nrm in ((10, 1.0, 20), (5, 0.0, 8)):
+        o_keep, _, _ = oracle.sor(pts, k_sor, std, threads=T)
+        sel = np.nonzero(o_keep)[0]
+        two_step = pcr.normals_array(_cloud(pcr, pts[sel]), k_nrm)
+        dev = pcr.DeviceCloud.from_numpy(pts).sor_normals(k_sor, std, k_nrm)
+        assert np.array_equal(dev.to_numpy(), pts[sel], equal_nan=True), (k_sor, std, k_nrm)
+        assert np.array_equal(dev.normals_to_numpy().view(np.uint32), two_step.view(np.uint32)), (k_sor, std, k_nrm)
+        keep, nrm, kept = pcr.sor_normals_batch(pts, [0, len(pts)], k_sor, std, k_nrm)
+        assert np.array_equal(keep, o_keep) and kept[0] == len(sel)
+        assert np.array_equal(nrm[sel].view(np.uint32), two_step.view(np.uint32)), (k_sor, std, k_nrm)
 
 
 def test_fused_fallback_beyond_the_blind_pass(pcr, monkeypatch):
